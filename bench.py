@@ -4,6 +4,7 @@
 Contract (see README / DESIGN.md §measurement):
   python bench.py --gpus N --steps K --warmup W            our arm (B200 kernels)
   python bench.py --impl reference --gpus N ...           CPU arm (oracle port; ducc0 unavailable)
+  python bench.py ... --dump-outputs DIR                    also write what the last timed step computed (DIR/*.npy)
 One JSON line on stdout from rank 0.  N>1 is launched with torch.distributed.run, one rank per GPU.
 Multi-band workloads (c2) are ONE job whose bands are partitioned over the N GPUs (strong scaling:
 longest-processing-time-first assignment, then the plane transforms of the heaviest bands are offloaded
@@ -113,6 +114,29 @@ def make_inputs(cfg, band, with_vis=False):
     return d, cell, x
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays, nout):
+    """--dump-outputs: write each array (torch tensor or numpy, float32 / float64) as out_dir/<name>.npy.  `nout` arrays
+    share DUMP_BYTES; an array larger than its share is written as a fixed seeded sample of its flattened elements (the
+    same positions in every run), so that two builds can be compared output for output."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    positions = {}  # (numel, k) -> sorted sample positions, drawn once for all arrays of that size
+    for name, a in arrays.items():
+        t = torch.as_tensor(a)
+        assert t.dtype in (torch.float32, torch.float64), (name, t.dtype)
+        k = (DUMP_BYTES // nout - 4096) // t.element_size()  # (4096: room for the .npy header)
+        if t.numel() > k:
+            if (t.numel(), k) not in positions:  # (at most k distinct positions, without a permutation of all numel)
+                idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), k))
+                positions[t.numel(), k] = torch.from_numpy(idx)
+            t = t.reshape(-1)[positions[t.numel(), k].to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def cpu_hessian_sample(cfg, band, row_step, nthreads_note=True):
     """Time the CPU restatement (oracle/cwgridder) on a bounded sample: the plane work (FFTs, screens)
     in full, the per-visibility loops on every `row_step`-th row; extrapolate the latter."""
@@ -139,26 +163,29 @@ def cpu_hessian_sample(cfg, band, row_step, nthreads_note=True):
     t_bin = time.perf_counter() - t0
     td, tg = {}, {}
     mv = cw.dirty2vis_c(plan, sub, freq, x.astype(np.float64), mask, b=b, timings=td)
-    cw.vis2dirty_c(plan, sub, freq, mv, wgt, mask, b=b, timings=tg)
+    img = cw.vis2dirty_c(plan, sub, freq, mv, wgt, mask, b=b, timings=tg)
     scale = nvis_full / nvis_s
     t_planes = td["planes"] + tg["planes"]
     t_vis = (td["vis"] + tg["vis"] + td["prep"] + tg["prep"]) * scale
     t_full = t_planes + t_vis
     return dict(value=nvis_full / t_full / 1e6, t_full=t_full, t_planes=t_planes, t_vis_sample=t_vis / scale,
                 t_bin_sample=t_bin, nvis_sample=nvis_s, nvis_full=nvis_full, cores=cw.nthreads(),
-                plan=dict(W=plan.W, sigma=plan.sigma, nu=plan.nu, nplanes=plan.nplanes))
+                plan=dict(W=plan.W, sigma=plan.sigma, nu=plan.nu, nplanes=plan.nplanes), image=img)
 
 
 def run_reference(args, cfg):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 3))  # each step = one Hessian apply of band 0 on the host (seconds of CPU work)
+    steps = args.steps  # each step = one Hessian apply of band 0 on the host (seconds of CPU work)
     vals, last = [], None
     for it in range(min(args.warmup, 1) + steps):
         last = cpu_hessian_sample(cfg, 0, args.cpu_row_step)
         if it >= min(args.warmup, 1):
             vals.append(last["value"])
+    if args.dump_outputs:  # (fp64; with --cpu-row-step n > 1 the image of every n-th row only)
+        name = "hessian_band0" if args.cpu_row_step == 1 else f"hessian_band0_rows_every{args.cpu_row_step}"
+        dump_outputs(args.dump_outputs, {name: last["image"]}, 1)
     v = float(np.mean(vals))
     how = ("all rows" if args.cpu_row_step == 1 else
            f"every {args.cpu_row_step}th row for the per-visibility loops ({last['nvis_sample']} vis, extrapolated)")
@@ -245,6 +272,8 @@ def run_c3(args, cfg):
     launches = _lib.load().pfbg_launch_count() - launches0
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f"model_band{b}": x[i] for i, b in enumerate(bands)}, cfg["nbands"])
     ms_it = (times[nshort + args.steps] - times[nshort]) / args.steps * 1e3
     t = torch.tensor([ms_it, times[nshort + args.steps] * 1e3], dtype=torch.float64, device=dev)
     if world > 1:
@@ -379,6 +408,9 @@ def run_c5(args, cfg):
     launches = _lib.load().pfbg_launch_count() - launches0
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f"hessian_rank{rank}_batch{i}": b["out_d"] for i, b in enumerate(batches)},
+                     world * len(batches))
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     nv = torch.tensor([float(nvis_local)], dtype=torch.float64, device=dev)
     la = torch.tensor([float(launches)], dtype=torch.float64, device=dev)
@@ -663,6 +695,9 @@ def run_ours(args, cfg):
     sampler.join()
     if split:
         split.check()
+    if args.dump_outputs and (strong or rank == 0):  # (one job per GPU: rank 0's job)
+        dump_outputs(args.dump_outputs, {f"hessian_band{bd['b']}": bd["out_d"] for bd in bands},
+                     nbands if strong else len(bands))
     ms_ranks = [float(v) / args.steps for v in gather_obj(ms_total)]
     launches_all = int(sum(gather_obj(int(launches))))
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
@@ -977,7 +1012,12 @@ def main():
     ap.add_argument("--strong", action="store_true", help="(default for multi-band workloads) kept for compatibility")
     ap.add_argument("--no-offload", action="store_true", help="band partition only, no plane offload")
     ap.add_argument("--bands", default="", help="restrict the job to these bands, e.g. 7,0 (development)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (at most 64 MB, "
+                         "a fixed seeded sample of larger outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, cfg)
