@@ -757,7 +757,9 @@ static void par_memcpy(void* dst, const void* src, size_t n) {
   const int nt = host_threads();
   if (nt == 1 || n < (size_t)(1 << 20)) { memcpy(dst, src, n); return; }
   std::vector<std::thread> th;
-  size_t per = ((n / nt) + 63) & ~(size_t)63;
+  // ceil(n / nt) rounded up to 64 bytes: the nt chunks cover all n bytes (floor(n / nt) would drop the last n % nt
+  // when it is a multiple of 64)
+  const size_t per = ((n + nt - 1) / nt + 63) & ~(size_t)63;
   for (int t = 0; t < nt; ++t) {
     size_t off = (size_t)t * per;
     if (off >= n) break;
@@ -797,7 +799,7 @@ extern "C" int pfbg_host_hash64(const void* ptr, uint64_t bytes, uint64_t* out) 
   if (nt == 1) { *out = hash_range(p, n, 0); return PFBG_OK; }
   std::vector<uint64_t> part(nt, 0);
   std::vector<std::thread> th;
-  const size_t per = ((n / nt) + 63) & ~(size_t)63;
+  const size_t per = ((n + nt - 1) / nt + 63) & ~(size_t)63;  // covers all n bytes (see par_memcpy)
   for (int t = 0; t < nt; ++t) {
     const size_t off = (size_t)t * per;
     if (off >= n) break;
