@@ -1,8 +1,10 @@
 /*
- * pfbsara.h — C ABI of the device SARA backward step (SURVEY.md §8 row f2): the wavelet dictionary
- * Psi (analysis `dot`, synthesis `hdot`), the fused l21 dual update, and the element-wise pieces of the
- * primal-dual iteration.  Same conventions as pfbgrid.h: every entry point returns 0 or a PFBG_ERR_* code,
- * pfbg_last_error() holds the message, plain pointers and sizes only.
+ * pfbsara.h — C ABI of the device backward steps of the deconvolution major cycle:
+ *   - SARA (SURVEY.md §8 row f2): the wavelet dictionary Psi (analysis `dot`, synthesis `hdot`), the fused l21 dual
+ *     update, and the element-wise pieces of the primal-dual iteration;
+ *   - the Clark CLEAN minor cycle of `pfb kclean` (core/kclean.py:203-218 -> deconv/clark.py).
+ * Same conventions as pfbgrid.h: every entry point returns 0 or a PFBG_ERR_* code, pfbg_last_error() holds the
+ * message, plain pointers and sizes only.
  *
  * Reference interfaces replaced (paths relative to /root/reference/src/pfb_imaging):
  *   - Psi / PsiNocopyt .dot / .hdot  (operators/psi.py:549-664; PsiBand :231-372, PsiBandNocopyt :466-530;
@@ -12,6 +14,7 @@
  *   - _nb_extrapolate_dual, _nb_primal_step, _nb_norm_diff (opt/primal_dual.py:16-61),
  *     positivity / positivity_band (prox/positivity.py:13-38)                               -> pfbs_extrapolate /
  *                                                                                              pfbs_primal_step / pfbs_norm_diff
+ *   - clark (deconv/clark.py), semantics as restated in oracle/clark_np.py                  -> pfbs_clark_run
  */
 #ifndef PFBSARA_H
 #define PFBSARA_H
@@ -75,6 +78,38 @@ int pfbs_norm_diff(int32_t precision, int32_t device, const void* x, const void*
  * the device-resident conjugate gradients (opt/pcg.py:35-41, 77-85) */
 int pfbs_dot2(int32_t precision, int32_t device, const void* a, const void* b, const void* c, const void* d, int64_t n,
               double* out2, void* stream);
+
+/*
+ * Clark CLEAN minor cycle (fp64 only).  Images are (nband, nx, ny), raster index p = i*ny + j; the PSF is
+ * (nband, nx_psf, ny_psf) with its centre at (nx_psf/2, ny_psf/2), nx <= nx_psf, ny <= ny_psf.  `psfhat` is its
+ * r2c half spectrum rfft2(ifftshift(PSF)), (nband, nx_psf, ny_psf/2+1) complex128.  create uploads both once (one PSF
+ * convolver per band) so that a handle serves every major cycle of a deconvolution; psf / psfhat are device pointers
+ * when `flags` has PFBG_DEVICE_PTRS.
+ *
+ * run: R = dirty, model = 0; per major iteration k (at most maxit):
+ *   s(p) = |sum_b R_b(p)| over pixels with mask[p] != 0 (mask NULL: all), Rmax = max s, on the first pass
+ *   tol = max(pf Rmax, threshold); stop when Rmax <= tol;  A = {masked p : s(p) >= subpf Rmax} (raster order);
+ *   subminor components while the peak of s over A > max(subpf Rmax, threshold), at most submaxit: a* = first
+ *   maximum, d_b = gamma R_b(a*) / peak_b (0 where peak_b <= 0), model_b(a*) += d_b, R_b(a) -= d_b PSF_b(c + a - a*)
+ *   on A;  then R = dirty - PSF (*) model through psfhat.
+ * dirty, model, residual (nband, nx, ny) and mask (nx, ny) uint8 are device pointers with PFBG_DEVICE_PTRS (the call is
+ * then asynchronous after its last host decision), else host pointers.  Info, host arrays: niter; per major iteration
+ * rmax[k], nactive[k] = |A|, nsub[k] components; peaks (capacity peaks_cap >= maxit * submaxit) the raster index of
+ * every component in order; times_ms (optional, 3 per major iteration): search + compaction, subminor (with the
+ * model update), residual step, from CUDA events.
+ */
+#define PFBS_CLARK_MAX_BANDS 1024
+
+typedef struct pfbs_clark pfbs_clark;
+
+int pfbs_clark_create(int32_t precision, int32_t device, int32_t nband, int32_t nx, int32_t ny, int32_t nx_psf,
+                      int32_t ny_psf, const void* psf, const void* psfhat, uint32_t flags, void* stream,
+                      pfbs_clark** out);
+int pfbs_clark_run(pfbs_clark* h, const void* dirty, const uint8_t* mask, void* model, void* residual,
+                   double threshold, double gamma, double pf, int32_t maxit, double subpf, int32_t submaxit,
+                   int32_t* niter, double* rmax, int64_t* nactive, int32_t* nsub, int64_t* peaks, int64_t peaks_cap,
+                   float* times_ms, uint32_t flags, void* stream);
+int pfbs_clark_destroy(pfbs_clark* h);
 
 #ifdef __cplusplus
 }

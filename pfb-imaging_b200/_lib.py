@@ -117,6 +117,10 @@ SIGNATURES = {
     "pfbs_primal_step": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _dbl, _i32, _i32, _i64, _vp]),
     "pfbs_dot2": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _i64, C.POINTER(_dbl), _vp]),
     "pfbs_norm_diff": (C.c_int, [_i32, _i32, _vp, _vp, _i64, C.POINTER(_dbl), _vp]),
+    "pfbs_clark_create": (C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _u32, _vp, C.POINTER(_vp)]),
+    "pfbs_clark_destroy": (C.c_int, [_vp]),
+    "pfbs_clark_run": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _dbl, _dbl, _dbl, _i32, _dbl, _i32, C.POINTER(_i32), _vp, _vp,
+                                 _vp, _vp, _i64, _vp, _u32, _vp]),
 }
 
 _lib = None
@@ -128,7 +132,7 @@ _UNITS = {
     "pfbgrid.cu": ["common.cuh", "fft.cuh", "fused_fft.cuh", "kernels.cuh", "psfconv.cuh", "runs.cuh", "runs_mma.cuh", "weighting.cuh",
                    "cols2_api.h", "fused_common.cuh", "../../include/pfbgrid.h"],
     "colsfft.cu": ["common.cuh", "fft.cuh", "fft2.cuh", "cols2.cuh", "rows2.cuh", "cols2_api.h", "fused_common.cuh"],
-    "pfbsara.cu": ["sara.cuh", "../../include/pfbsara.h", "../../include/pfbgrid.h"],
+    "pfbsara.cu": ["sara.cuh", "clean.cuh", "../../include/pfbsara.h", "../../include/pfbgrid.h"],
 }
 
 

@@ -1,11 +1,18 @@
-// C-ABI of the device SARA backward step (include/pfbsara.h); kernels in sara.cuh.
+// C-ABI of the device backward steps (include/pfbsara.h): SARA (kernels in sara.cuh) and the Clark minor cycle
+// (clean.cuh).
 #include <cuda_runtime.h>
 
+#include <thrust/iterator/counting_iterator.h>
+
+#include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <cub/device/device_select.cuh>
 #include <vector>
 
 #include "../../include/pfbsara.h"
+#include "clean.cuh"
 #include "sara.cuh"
 
 // error plumbing shared with pfbgrid.cu (same shared library)
@@ -394,4 +401,207 @@ extern "C" int pfbs_dot2(int32_t precision, int32_t device, const void* a, const
     if (precision == PFBG_F32) k_dot2<float><<<grd, 256, 0, s>>>((const float*)a, (const float*)b, (const float*)c, (const float*)d, n, acc);
     else k_dot2<double><<<grd, 256, 0, s>>>((const double*)a, (const double*)b, (const double*)c, (const double*)d, n, acc);
   });
+}
+
+// ---------------------------------------------------------------------------
+// Clark CLEAN minor cycle (clean.cuh)
+// ---------------------------------------------------------------------------
+struct pfbs_clark {
+  int device = 0, nband = 0, nx = 0, ny = 0, nxp = 0, nyp = 0;
+  int npix = 0, search_grid = 0, sub_grid = 0, log_cap = 0;
+  std::vector<double> peak;
+  std::vector<pfbg_conv*> conv;
+  double *psf = nullptr, *peak_d = nullptr, *ID = nullptr, *R = nullptr, *model = nullptr, *s = nullptr;
+  double *RA = nullptr, *SA = nullptr, *cand_s = nullptr, *slot_s = nullptr, *slot_r = nullptr, *log_d = nullptr;
+  int *idx = nullptr, *cand_i = nullptr, *slot_a = nullptr, *log_p = nullptr, *ints = nullptr;  // ints: best_i, nsel, count
+  int2* ij = nullptr;
+  uint8_t* mask = nullptr;
+  void* cub_tmp = nullptr;
+  size_t cub_bytes = 0;
+  cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+};
+
+extern "C" int pfbs_clark_destroy(pfbs_clark* h) {
+  if (!h) return PFBG_OK;
+  cudaSetDevice(h->device);
+  for (pfbg_conv* cv : h->conv) pfbg_conv_destroy(cv);
+  void* all[] = {h->psf, h->peak_d, h->ID, h->R, h->model, h->s, h->RA, h->SA, h->cand_s, h->slot_s, h->slot_r,
+                 h->log_d, h->idx, h->cand_i, h->slot_a, h->log_p, h->ints, h->ij, h->mask, h->cub_tmp};
+  for (void* q : all)
+    if (q) cudaFree(q);
+  for (cudaEvent_t e : h->ev)
+    if (e) cudaEventDestroy(e);
+  delete h;
+  return PFBG_OK;
+}
+
+extern "C" int pfbs_clark_create(int32_t precision, int32_t device, int32_t nband, int32_t nx, int32_t ny,
+                                 int32_t nx_psf, int32_t ny_psf, const void* psf, const void* psfhat, uint32_t flags,
+                                 void* stream, pfbs_clark** out) {
+  if (!out || !psf || !psfhat) return pfbg_fail(PFBG_ERR_ARG, "null argument");
+  *out = nullptr;
+  if (precision != PFBG_F64) return pfbg_fail(PFBG_ERR_ARG, "the Clark minor cycle is fp64 only");
+  if (nband < 1 || nband > PFBS_CLARK_MAX_BANDS) return pfbg_fail(PFBG_ERR_ARG, "nband %d not in 1..%d", nband, PFBS_CLARK_MAX_BANDS);
+  if (nx < 1 || ny < 1 || nx_psf < nx || ny_psf < ny)
+    return pfbg_fail(PFBG_ERR_ARG, "need 0 < nx <= nx_psf and 0 < ny <= ny_psf (got %d x %d, PSF %d x %d)", nx, ny, nx_psf, ny_psf);
+  if ((int64_t)nx * ny > INT32_MAX) return pfbg_fail(PFBG_ERR_ARG, "nx * ny must be below 2^31");
+  int ndev = 0;
+  SCK(cudaGetDeviceCount(&ndev));
+  if (device < 0 || device >= ndev) return pfbg_fail(PFBG_ERR_ARG, "device %d out of range", device);
+  SCK(cudaSetDevice(device));
+  int coop = 0, nsm = 0, occ = 0;
+  SCK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device));
+  if (!coop) return pfbg_fail(PFBG_ERR_CUDA, "device %d does not support cooperative launches", device);
+  SCK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
+  SCK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_clark_subminor, CLK_THREADS, (size_t)nband * sizeof(double)));
+  if (occ < 1) return pfbg_fail(PFBG_ERR_CUDA, "the subminor kernel cannot be resident");
+  cudaStream_t s = (cudaStream_t)stream;
+  const cudaMemcpyKind kind = (flags & PFBG_DEVICE_PTRS) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+  pfbs_clark* h = new pfbs_clark();
+  h->device = device; h->nband = nband; h->nx = nx; h->ny = ny; h->nxp = nx_psf; h->nyp = ny_psf;
+  h->npix = nx * ny;
+  // at most 2 CTAs per SM: every CTA reads every candidate slot once per component, so the slot traffic grows with
+  // the square of the grid, while 2 x 148 x 256 threads already give each thread < 2 entries at |A| ~ 10^5
+  h->sub_grid = nsm * (occ < 2 ? occ : 2);
+  h->search_grid = nsm * 4;
+  const size_t npix = h->npix, nb = nband;
+  const size_t plane = (size_t)nx_psf * ny_psf;
+  auto fail_free = [&](int rc) { pfbs_clark_destroy(h); return rc; };
+  auto alloc = [&](void** p, size_t bytes) -> int {
+    cudaError_t e = cudaMalloc(p, bytes);
+    if (e != cudaSuccess) { *p = nullptr; cudaGetLastError(); return pfbg_fail(PFBG_ERR_NOMEM, "cudaMalloc of %zu bytes failed: %s", bytes, cudaGetErrorString(e)); }
+    return PFBG_OK;
+  };
+  int rc = PFBG_OK;
+  void** bufs[] = {(void**)&h->psf, (void**)&h->ID, (void**)&h->R, (void**)&h->model, (void**)&h->s, (void**)&h->RA,
+                   (void**)&h->SA, (void**)&h->idx, (void**)&h->ij, (void**)&h->mask, (void**)&h->peak_d,
+                   (void**)&h->cand_s, (void**)&h->cand_i, (void**)&h->slot_s, (void**)&h->slot_a, (void**)&h->slot_r,
+                   (void**)&h->ints};
+  const size_t sizes[] = {nb * plane * 8, nb * npix * 8, nb * npix * 8, nb * npix * 8, npix * 8, nb * npix * 8,
+                          npix * 8, npix * 4, npix * 8, npix, nb * 8,
+                          (size_t)(h->search_grid + 1) * 8, (size_t)h->search_grid * 4, 2 * (size_t)h->sub_grid * 8,
+                          2 * (size_t)h->sub_grid * 4, 2 * (size_t)h->sub_grid * nb * 8, 4 * 4};
+  for (size_t k = 0; k < sizeof(sizes) / sizeof(sizes[0]) && rc == PFBG_OK; ++k) rc = alloc(bufs[k], sizes[k]);
+  if (rc) return fail_free(rc);
+  ClarkActive pred{h->s, 0.0};
+  cudaError_t e = cub::DeviceSelect::If(nullptr, h->cub_bytes, thrust::counting_iterator<int>(0), h->idx, h->ints + 1,
+                                        h->npix, pred, s);
+  if (e != cudaSuccess) { cudaGetLastError(); return fail_free(pfbg_fail(PFBG_ERR_CUDA, "cub select sizing failed: %s", cudaGetErrorString(e))); }
+  if ((rc = alloc(&h->cub_tmp, h->cub_bytes))) return fail_free(rc);
+  e = cudaMemcpyAsync(h->psf, psf, nb * plane * 8, kind, s);
+  h->peak.resize(nband);
+  const size_t centre = (size_t)(nx_psf / 2) * ny_psf + ny_psf / 2;
+  for (int b = 0; b < nband && e == cudaSuccess; ++b)
+    e = cudaMemcpyAsync(&h->peak[b], h->psf + b * plane + centre, 8, cudaMemcpyDeviceToHost, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  if (e == cudaSuccess) e = cudaMemcpy(h->peak_d, h->peak.data(), nb * 8, cudaMemcpyHostToDevice);
+  for (int k = 0; k < 4 && e == cudaSuccess; ++k) e = cudaEventCreate(&h->ev[k]);
+  if (e != cudaSuccess) { cudaGetLastError(); return fail_free(pfbg_fail(PFBG_ERR_CUDA, "PSF upload failed: %s", cudaGetErrorString(e))); }
+  h->conv.assign(nband, nullptr);
+  const size_t half = (size_t)nx_psf * (ny_psf / 2 + 1) * 16;
+  for (int b = 0; b < nband; ++b) {
+    if ((rc = pfbg_conv_create(PFBG_F64, device, nx, ny, nx_psf, ny_psf, &h->conv[b]))) return fail_free(rc);
+    if ((rc = pfbg_conv_set_kernel(h->conv[b], (const char*)psfhat + b * half, 1, flags & PFBG_DEVICE_PTRS, stream)))
+      return fail_free(rc);
+  }
+  *out = h;
+  return PFBG_OK;
+}
+
+static int clark_log_reserve(pfbs_clark* h, int n) {
+  if (n <= h->log_cap) return PFBG_OK;
+  if (h->log_p) cudaFree(h->log_p);
+  if (h->log_d) cudaFree(h->log_d);
+  h->log_p = nullptr; h->log_d = nullptr; h->log_cap = 0;
+  SRC(stage_alloc((void**)&h->log_p, (size_t)n * 4));
+  SRC(stage_alloc((void**)&h->log_d, (size_t)n * h->nband * 8));
+  h->log_cap = n;
+  return PFBG_OK;
+}
+
+extern "C" int pfbs_clark_run(pfbs_clark* h, const void* dirty, const uint8_t* mask, void* model, void* residual,
+                              double threshold, double gamma, double pf, int32_t maxit, double subpf, int32_t submaxit,
+                              int32_t* niter, double* rmax, int64_t* nactive, int32_t* nsub, int64_t* peaks,
+                              int64_t peaks_cap, float* times_ms, uint32_t flags, void* stream) {
+  if (!h || !dirty || !model || !residual || !niter) return pfbg_fail(PFBG_ERR_ARG, "null argument");
+  if (!(threshold >= 0.0) || threshold == HUGE_VAL) return pfbg_fail(PFBG_ERR_ARG, "threshold must be finite and >= 0");
+  if (!(gamma > 0.0 && gamma <= 1.0)) return pfbg_fail(PFBG_ERR_ARG, "gamma must be in (0, 1]");
+  if (!(pf >= 0.0) || pf == HUGE_VAL) return pfbg_fail(PFBG_ERR_ARG, "pf must be finite and >= 0");
+  if (!(subpf > 0.0 && subpf < 1.0)) return pfbg_fail(PFBG_ERR_ARG, "subpf must be in (0, 1)");
+  if (maxit < 0 || submaxit < 1) return pfbg_fail(PFBG_ERR_ARG, "need maxit >= 0 and submaxit >= 1");
+  if (maxit > 0 && (!rmax || !nactive || !nsub || !peaks)) return pfbg_fail(PFBG_ERR_ARG, "null info buffer");
+  if (peaks_cap < (int64_t)maxit * submaxit) return pfbg_fail(PFBG_ERR_ARG, "peaks holds %lld entries, maxit * submaxit = %lld",
+                                                              (long long)peaks_cap, (long long)maxit * submaxit);
+  SCK(cudaSetDevice(h->device));
+  SRC(clark_log_reserve(h, submaxit));
+  cudaStream_t s = (cudaStream_t)stream;
+  const bool dev = flags & PFBG_DEVICE_PTRS;
+  const int npix = h->npix, nband = h->nband;
+  const size_t ib = (size_t)nband * npix * 8;
+  SCK(cudaMemcpyAsync(h->ID, dirty, ib, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
+  if (mask) SCK(cudaMemcpyAsync(h->mask, mask, npix, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
+  SCK(cudaMemcpyAsync(h->R, h->ID, ib, cudaMemcpyDeviceToDevice, s));
+  SCK(cudaMemsetAsync(h->model, 0, ib, s));
+  double tol = -1.0;
+  int k = 0;
+  int64_t npeaks = 0;
+  for (;; ++k) {
+    if (times_ms) SCK(cudaEventRecord(h->ev[0], s));
+    k_clark_search<<<h->search_grid, CLK_THREADS, 0, s>>>(h->R, nband, npix, mask ? h->mask : nullptr, h->s, h->cand_s, h->cand_i);
+    k_clark_best<<<1, CLK_THREADS, 0, s>>>(h->cand_s, h->cand_i, h->search_grid, h->cand_s + h->search_grid, h->ints);
+    pfbg_count_launch(); pfbg_count_launch();
+    SCK(cudaGetLastError());
+    double Rmax = 0.0;
+    SCK(cudaMemcpyAsync(&Rmax, h->cand_s + h->search_grid, 8, cudaMemcpyDeviceToHost, s));
+    SCK(cudaStreamSynchronize(s));
+    if (Rmax < 0.0) Rmax = 0.0;  // no pixel is searched
+    if (k == 0) tol = std::max(pf * Rmax, threshold);
+    if (!(Rmax > tol) || k >= maxit) break;
+    const ClarkActive pred{h->s, subpf * Rmax};
+    SCK(cub::DeviceSelect::If(h->cub_tmp, h->cub_bytes, thrust::counting_iterator<int>(0), h->idx, h->ints + 1, npix, pred, s));
+    int nA = 0;
+    SCK(cudaMemcpyAsync(&nA, h->ints + 1, 4, cudaMemcpyDeviceToHost, s));
+    SCK(cudaStreamSynchronize(s));
+    const int ga = std::min((nA + CLK_THREADS - 1) / CLK_THREADS, h->search_grid);
+    k_clark_gather<<<std::max(ga, 1), CLK_THREADS, 0, s>>>(h->R, h->s, nband, npix, h->ny, h->idx, nA, h->RA, h->SA, h->ij);
+    pfbg_count_launch();
+    SCK(cudaGetLastError());
+    if (times_ms) SCK(cudaEventRecord(h->ev[1], s));
+    ClarkSub c{h->RA, h->SA, h->ij, nA, nband, h->ny, h->psf, h->peak_d, h->nxp, h->nyp, h->nxp / 2, h->nyp / 2,
+               gamma, std::max(subpf * Rmax, threshold), submaxit, h->slot_s, h->slot_a, h->slot_r, h->log_p, h->log_d,
+               h->ints + 2};
+    const int grid = std::max(1, std::min((nA + CLK_THREADS - 1) / CLK_THREADS, h->sub_grid));
+    void* args[] = {&c};
+    SCK(cudaLaunchCooperativeKernel((const void*)k_clark_subminor, dim3(grid), dim3(CLK_THREADS), args,
+                                    (size_t)nband * sizeof(double), s));
+    pfbg_count_launch();
+    k_clark_replay<<<(nband + 31) / 32, 32, 0, s>>>(h->model, nband, npix, h->log_p, h->log_d, h->ints + 2);
+    pfbg_count_launch();
+    SCK(cudaGetLastError());
+    if (times_ms) SCK(cudaEventRecord(h->ev[2], s));
+    for (int b = 0; b < nband; ++b)
+      SRC(pfbg_conv_apply(h->conv[b], h->model + (int64_t)b * npix, nullptr, 0.0, h->R + (int64_t)b * npix, PFBG_DEVICE_PTRS, stream));
+    k_clark_resid<<<h->search_grid, CLK_THREADS, 0, s>>>(h->ID, h->R, (int64_t)nband * npix);
+    pfbg_count_launch();
+    SCK(cudaGetLastError());
+    if (times_ms) SCK(cudaEventRecord(h->ev[3], s));
+    int cnt = 0;
+    SCK(cudaMemcpyAsync(&cnt, h->ints + 2, 4, cudaMemcpyDeviceToHost, s));
+    SCK(cudaStreamSynchronize(s));
+    std::vector<int> lp(cnt);
+    if (cnt) SCK(cudaMemcpy(lp.data(), h->log_p, (size_t)cnt * 4, cudaMemcpyDeviceToHost));
+    for (int t = 0; t < cnt; ++t) peaks[npeaks + t] = lp[t];
+    npeaks += cnt;
+    rmax[k] = Rmax;
+    nactive[k] = nA;
+    nsub[k] = cnt;
+    if (times_ms)
+      for (int t = 0; t < 3; ++t) SCK(cudaEventElapsedTime(&times_ms[3 * k + t], h->ev[t], h->ev[t + 1]));
+  }
+  *niter = k;
+  const cudaMemcpyKind back = dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+  SCK(cudaMemcpyAsync(model, h->model, ib, back, s));
+  SCK(cudaMemcpyAsync(residual, h->R, ib, back, s));
+  if (!dev) SCK(cudaStreamSynchronize(s));
+  return PFBG_OK;
 }
