@@ -250,6 +250,9 @@ int pfbg_conv_destroy(pfbg_conv* conv);
 int pfbg_conv_set_kernel(pfbg_conv* conv, const void* khat, int32_t half, uint32_t flags, void* stream);
 int pfbg_conv_apply(pfbg_conv* conv, const void* x, const void* beam, double eta, void* out, uint32_t flags,
                     void* stream);
+/* Read-only: the column-block width C (1, 2 or 4 columns per CTA of the column pass) and the CTA size of the
+ * row passes that this convolver runs with.  Either output pointer may be NULL. */
+int pfbg_conv_info(const pfbg_conv* conv, int32_t* col_block, int32_t* row_threads);
 
 /*
  * Band split across two GPUs, one process per GPU (SURVEY §8e; the reference runs one actor per band,
@@ -300,7 +303,7 @@ int pfbg_weight_data_corr(int32_t precision, int32_t device, const void* data, c
 
 /*
  * Unit-test hook for the in-shared-memory FFT engine behind the fused plane transforms:
- * `batch` transforms of length n (2^a 3^b 5^c 7^d), complex of `precision`, host pointers.
+ * `batch` transforms of length n (2^a 3^b 5^c 7^d 11^e), complex of `precision`, host pointers.
  * mode 0 = decimation in frequency, 1 = decimation in time; inverse != 0 -> e^{+2 pi i nk/n}.
  */
 int pfbg_debug_fft1d(int32_t precision, int32_t device, int32_t n, int32_t batch, const void* in,

@@ -85,6 +85,7 @@ SIGNATURES = {
     "pfbg_conv_destroy": (C.c_int, [_vp]),
     "pfbg_conv_set_kernel": (C.c_int, [_vp, _vp, _i32, _u32, _vp]),
     "pfbg_conv_apply": (C.c_int, [_vp, _vp, _vp, _dbl, _vp, _u32, _vp]),
+    "pfbg_conv_info": (C.c_int, [_vp, C.POINTER(_i32), C.POINTER(_i32)]),
     "pfbg_debug_fft1d": (C.c_int, [_i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32]),
     "pfbg_debug_es_fast64": (C.c_int, [_i32, _i64, _vp, C.c_double, _vp]),
     "pfbg_weight_data_corr": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i64, _i64, _i64, _i64,

@@ -22,7 +22,7 @@ import math
 import numpy as np
 
 from . import _lib
-from .wgridder import current_device
+from .wgridder import content_hash, current_device
 
 MAX_BANDS = 1024  # PFBS_CLARK_MAX_BANDS
 
@@ -145,12 +145,12 @@ _CLARK_CACHE: dict = {}
 
 
 def _clark_for(psf, psfhat, nx, ny):
-    """A cached :class:`Clark`, keyed like ``psf._convolver_for``: the PSF buffer, its shape, the image size and a
-    strided checksum of its content (a PSF rewritten in place rebuilds the handle)."""
+    """A cached :class:`Clark`, keyed like ``psf._convolver_for``: the PSF and spectrum buffers, their shapes, the image
+    size and a hash of the full content of both (a PSF or spectrum rewritten in place rebuilds the handle)."""
     psf = np.asarray(psf)
     key = (psf.ctypes.data, psf.shape, psf.dtype.str, int(nx), int(ny),
            None if psfhat is None else (np.asarray(psfhat).ctypes.data, np.asarray(psfhat).shape))
-    chk = float(np.abs(psf.ravel()[:: max(1, psf.size // 1024)]).sum())
+    chk = (content_hash(psf), None if psfhat is None else content_hash(psfhat))
     hit = _CLARK_CACHE.get(key)
     if hit is not None and hit[1] == chk:
         return hit[0]

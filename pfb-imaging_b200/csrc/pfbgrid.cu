@@ -2239,7 +2239,7 @@ extern "C" int pfbg_weight_data_corr(int32_t precision, int32_t device, const vo
 template <typename T>
 static int debug_fft_t(int n, int batch, const void* in, void* out, int mode, int inverse) {
   FftDesc d;
-  if (!factorize(n, d, sizeof(T) == 4 ? 16 : 8)) return fail(PFBG_ERR_ARG, "n=%d is not 2^a 3^b 5^c 7^d", n);
+  if (!factorize(n, d, sizeof(T) == 4 ? 16 : 8)) return fail(PFBG_ERR_ARG, "n=%d is not 2^a 3^b 5^c 7^d 11^e", n);
   size_t bytes = (size_t)n * sizeof(cx2<T>);
   if (fft_smem_bytes<T>(n) > kMaxSmem) return fail(PFBG_ERR_ARG, "n=%d does not fit shared memory", n);
   std::vector<cx2<T>> tw(n);
@@ -2417,6 +2417,14 @@ extern "C" int pfbg_conv_create(int32_t precision, int32_t device, int32_t nx, i
   int rc = precision == PFBG_F32 ? conv_setup_t<float>(cv) : conv_setup_t<double>(cv);
   if (rc) { pfbg_conv_destroy(cv); return rc; }
   *out = cv;
+  return PFBG_OK;
+}
+
+// the column-block width and the row-pass CTA size conv_setup_t / conv_apply_t chose (read-only, for tests)
+extern "C" int pfbg_conv_info(const pfbg_conv* cv, int32_t* col_block, int32_t* row_threads_out) {
+  if (!cv) return fail(PFBG_ERR_ARG, "null argument");
+  if (col_block) *col_block = cv->col_c;
+  if (row_threads_out) *row_threads_out = row_threads(cv->ct.nyp, 256);
   return PFBG_OK;
 }
 

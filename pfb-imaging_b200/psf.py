@@ -20,7 +20,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .wgridder import current_device
+from .wgridder import content_hash, current_device
 
 _RDT = {np.dtype(np.float32): (_lib.PFBG_F32, np.complex64), np.dtype(np.float64): (_lib.PFBG_F64, np.complex128)}
 
@@ -97,7 +97,7 @@ def _convolver_for(khat, nx, ny, lastsize, rdt):
     nx_psf = khat.shape[0]
     ny_psf = int(lastsize) if lastsize is not None else 2 * (khat.shape[1] - 1)
     key = (khat.ctypes.data, khat.shape, khat.dtype.str, nx, ny, ny_psf, np.dtype(rdt).str)
-    chk = float(np.abs(khat.ravel()[:: max(1, khat.size // 1024)]).sum())
+    chk = content_hash(khat)  # the whole spectrum: an in-place edit of any element rebuilds the convolver
     hit = _CONV_CACHE.get(key)
     if hit is not None and hit[1] == chk:
         return hit[0]
@@ -174,7 +174,7 @@ def hess_direct_slice(x, xpad=None, xhat=None, xout=None, abspsf=None, taperxy=N
     x = np.asarray(x)
     abspsf = np.asarray(abspsf)
     key = (abspsf.ctypes.data, abspsf.shape, float(eta), mode, x.shape, np.dtype(x.dtype).str, int(lastsize))
-    chk = float(np.abs(abspsf.ravel()[:: max(1, abspsf.size // 1024)]).sum())
+    chk = content_hash(abspsf)
     hit = _DIRECT_CACHE.get(key)
     if hit is None or hit[1] != chk:
         if hit is not None:
@@ -216,8 +216,6 @@ class HessianTree:
     def __init__(self, partitions, nx, ny, nx_psf, ny_psf, eta=0.0, nthreads=1, wsum=None, device=None):
         if not partitions:
             raise ValueError("HessianTree requires at least one partition")
-        from .wgridder import content_hash
-
         self.parts = partitions
         self.nx, self.ny, self.nx_psf, self.ny_psf = nx, ny, nx_psf, ny_psf
         self.eta, self.nthreads = eta, nthreads
