@@ -23,6 +23,9 @@
  *   - _compute_counts / counts_to_weights
  *       (utils/weighting.py:81-140, 143-208)                -> pfbg_counts /
  *                                                              pfbg_counts_to_weights
+ *   - the same per snapshot of `pfb hci`
+ *       (utils/stokes2im.py:563-604)                        -> pfbg_counts_to_weights_batch /
+ *                                                              pfbg_bind_weights_robust
  *   - the l2 re-weighting block of image_data_products
  *       (operators/gridder.py:509-532)                      -> pfbg_l2_reweight
  */
@@ -220,6 +223,35 @@ int pfbg_counts_to_weights(int32_t precision, int32_t device, void* counts, cons
                            int32_t nchan, int32_t ncorr, int32_t nx, int32_t ny, double cell_x,
                            double cell_y, double robust, double usign, double vsign, uint32_t flags,
                            void* stream);
+
+/*
+ * Briggs / uniform weights of a batch of snapshots (`pfb hci`, utils/stokes2im.py:563-604).  Snapshot b owns the rows
+ * [row_offsets[b], row_offsets[b+1]) of uvw (nrow,3), mask (nrow,nchan) u8 or NULL and wgt (nrow,nchan) of
+ * `precision` (one correlation); freq (nchan) is shared.  Each snapshot gets its own (nx_pad, ny_pad) counts grid,
+ * its own sums and ssq, so wgt ends as it would after, for every snapshot on its own,
+ *     pfbg_counts(rows of b) -> counts_b;  pfbg_counts_to_weights(counts_b, rows of b, robust)
+ * A snapshot without any counts (no rows, all flagged, all off the grid) keeps its weights.  wgt is updated in place;
+ * counts (nbatch, nx_pad, ny_pad) of `precision` receives the re-weighted grids when not NULL.  row_offsets is a host
+ * array whatever `flags` says; it must rise monotonically from 0 to nrow.  Everything is checked before any launch.
+ * Scratch held for the call: nbatch * nx_pad * ny_pad * sizeof(real) bytes of counts (2.1 GB for 256 snapshots on a
+ * 1024^2 pad in fp64, 1.07 GB in fp32; none when `counts` is a device pointer), 24 B per snapshot and 4 B per row.
+ */
+int pfbg_counts_to_weights_batch(int32_t precision, int32_t device, int32_t nbatch, const int64_t* row_offsets,
+                                 const double* uvw, const double* freq, const uint8_t* mask, void* wgt, int64_t nrow,
+                                 int32_t nchan, int32_t nx_pad, int32_t ny_pad, double cell_x, double cell_y,
+                                 double robust, double usign, double vsign, void* counts, uint32_t flags,
+                                 void* stream);
+
+/*
+ * The same for the batch a plan holds (pfbg_plan_set_batch + pfbg_bind_vis_batch), on the device: wgt (nrow,nchan)
+ * of the plan's precision is copied into the plan's bound weights and re-weighted there, per snapshot, from the
+ * bound uvw, mask and rows; pfbg_grid / pfbg_degrid / pfbg_hessian with wgt == NULL then use them.  The cell of a
+ * sample is the one pfbg_counts gives for freq when the bound fscale is the rounded quotient freq / c.  The plan keeps
+ * nbatch * nx_pad * ny_pad * sizeof(real) + 24 nbatch bytes of counts scratch for the next call (2.1 GB for 256
+ * snapshots on a 1024^2 pad in fp64, 1.07 GB in fp32).  PFBG_ERR_STATE for a plan without a bound batch.
+ */
+int pfbg_bind_weights_robust(pfbg_plan* plan, const void* wgt, int32_t nx_pad, int32_t ny_pad, double cell_x,
+                             double cell_y, double robust, double usign, double vsign, uint32_t flags, void* stream);
 
 /*
  * l2 (Student-t) re-weighting of the natural weights from residual visibilities — the block

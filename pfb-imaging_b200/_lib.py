@@ -93,6 +93,9 @@ SIGNATURES = {
     "pfbg_debug_fft2": (C.c_int, [_i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32]),
     "pfbg_counts_to_weights": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _i32,
                                          _dbl, _dbl, _dbl, _dbl, _dbl, _u32, _vp]),
+    "pfbg_counts_to_weights_batch": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32,
+                                               _dbl, _dbl, _dbl, _dbl, _dbl, _vp, _u32, _vp]),
+    "pfbg_bind_weights_robust": (C.c_int, [_vp, _vp, _i32, _i32, _dbl, _dbl, _dbl, _dbl, _dbl, _u32, _vp]),
     "pfbg_l2_reweight": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _i64, _i32, _dbl, _vp, _vp, _u32, _vp]),
     "pfbg_host_hash64": (C.c_int, [_vp, C.c_uint64, C.POINTER(C.c_uint64)]),
     "pfbg_ipc_export": (C.c_int, [_vp, _vp]),

@@ -4,7 +4,9 @@
 #include <cufft.h>
 #include <cub/device/device_radix_sort.cuh>
 
+#include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <mutex>
 #include <climits>
 #include <cstdarg>
@@ -126,6 +128,7 @@ struct pfbg_plan {
   bool grid_lazy = false;      // PFBG_PLAN_EXTERNAL_STACK: no stack until one is lent
   DevBuf uvw, fscale, mask;    // bound geometry
   DevBuf wgt;                  // bound weights (nrow,nchan) T
+  DevBuf wcounts;              // pfbg_bind_weights_robust: (nbatch,nx_pad,ny_pad) T counts + 3 sums per snapshot
   DevBuf sorted_idx;           // (nactive) u32
   DevBuf recs;                 // (nactive) VisRec<T>, bucket order (run kernels, W <= 8)
   bool use_runs = false;
@@ -225,7 +228,7 @@ extern "C" int pfbg_plan_destroy(pfbg_plan* pl) {
   cudaSetDevice(pl->device);
   if (pl->fft_ok) cufftDestroy(pl->fft);
   if (pl->grid_external) { pl->grid.p = nullptr; pl->grid.bytes = 0; }
-  DevBuf* all[] = {&pl->corr, &pl->grid, &pl->uvw, &pl->fscale, &pl->mask, &pl->wgt, &pl->sorted_idx, &pl->srt_ka, &pl->srt_kb, &pl->srt_va, &pl->srt_vb, &pl->srt_tmp,
+  DevBuf* all[] = {&pl->corr, &pl->grid, &pl->uvw, &pl->fscale, &pl->mask, &pl->wgt, &pl->wcounts, &pl->sorted_idx, &pl->srt_ka, &pl->srt_kb, &pl->srt_va, &pl->srt_vb, &pl->srt_tmp,
                    &pl->xshare, &pl->partial, &pl->mailbox, &pl->x_local,
                    &pl->row_snap, &pl->snap_w0, &pl->snap_pbase, &pl->snap_np, &pl->plane_w, &pl->plane_img,
                    &pl->recs, &pl->mvis, &pl->tw_u, &pl->tw_v, &pl->rev_u, &pl->rev_v, &pl->pos_v, &pl->pos_u, &pl->cellflags, &pl->accimg, &pl->nutab, &pl->img_in, &pl->img_out, &pl->img_beam, &pl->vis_stage, &pl->wgt_stage,
@@ -2017,6 +2020,49 @@ struct TmpBufs {
   }
 };
 
+// reduction launch of the counts kernels: blockIdx.y over up to kCountsGridsPerLaunch grids, ~1184 CTAs in all
+static dim3 counts_rgrid(int64_t ngrid) {
+  const int gy = (int)std::min<int64_t>(ngrid, kCountsGridsPerLaunch);
+  return dim3((unsigned)std::max(8, 1184 / gy), (unsigned)gy);
+}
+
+template <typename T>
+static int launch_counts(cudaStream_t s, const WParams& w, const double* uvw, const double* scale, const uint8_t* mask,
+                         const int* row_snap, const T* wgt, T* counts, size_t cbytes) {
+  CK(cudaMemsetAsync(counts, 0, cbytes, s));
+  const int64_t nvis = w.nrow * w.nchan;
+  if (nvis > 0) {
+    k_counts<T><<<(unsigned)((nvis + 255) / 256), 256, 0, s>>>(w, uvw, scale, mask, row_snap, wgt, counts, nullptr);
+    LAUNCHED();
+    CK(cudaGetLastError());
+  }
+  return PFBG_OK;
+}
+
+// counts (nsnap * ncorr grids) -> Briggs / uniform weights, in place on counts and wgt (weighting.py:143-208);
+// sums: 3 * nsnap * ncorr doubles of scratch.  No host synchronisation.
+template <typename T>
+static int launch_reweight(cudaStream_t s, const WParams& w, const double* uvw, const double* scale,
+                           const uint8_t* mask, const int* row_snap, int64_t nsnap, T* counts, double* sums,
+                           double robust, T* wgt) {
+  const int64_t ncell = (int64_t)w.nx * w.ny, ngrid = nsnap * w.ncorr, nvis = w.nrow * w.nchan;
+  const dim3 rg = counts_rgrid(ngrid);
+  CK(cudaMemsetAsync(sums, 0, (size_t)ngrid * 3 * sizeof(double), s));
+  k_counts_sums<T><<<rg, 256, 0, s>>>(counts, ncell, (int)ngrid, sums);
+  LAUNCHED();
+  if (robust > -2.0) {
+    const double numsqrt = 5.0 * pow(10.0, -robust);
+    k_counts_scale<T><<<rg, 256, 0, s>>>(counts, ncell, w.ncorr, (int)ngrid, sums, numsqrt * numsqrt);
+    LAUNCHED();
+  }
+  if (nvis > 0) {
+    k_apply_counts<T><<<(unsigned)((nvis + 255) / 256), 256, 0, s>>>(w, uvw, scale, mask, row_snap, counts, wgt);
+    LAUNCHED();
+  }
+  CK(cudaGetLastError());
+  return PFBG_OK;
+}
+
 extern "C" int pfbg_counts(int32_t precision, int32_t device, const double* uvw, const double* freq,
                            const uint8_t* mask, const void* wgt, int64_t nrow, int32_t nchan, int32_t ncorr,
                            int32_t nx, int32_t ny, double cell_x, double cell_y, double usign, double vsign,
@@ -2037,17 +2083,11 @@ extern "C" int pfbg_counts(int32_t precision, int32_t device, const double* uvw,
   if (mask) CKRC(t.get(&dmask, mask, (size_t)nvis, dev, true, s));
   CKRC(t.get(&dwgt, wgt, (size_t)ncorr * nvis * rb, dev, true, s));
   CKRC(t.get(&dcounts, counts, cbytes, dev, false, s));
-  CK(cudaMemsetAsync(dcounts, 0, cbytes, s));
   WParams w = make_wparams(nrow, nchan, ncorr, nx, ny, cell_x, cell_y, usign, vsign);
-  if (nvis > 0) {
-    unsigned grd = (unsigned)((nvis + 255) / 256);
-    if (precision == PFBG_F32)
-      k_counts<float><<<grd, 256, 0, s>>>(w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, (const float*)dwgt, (float*)dcounts, nullptr);
-    else
-      k_counts<double><<<grd, 256, 0, s>>>(w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, (const double*)dwgt, (double*)dcounts, nullptr);
-    LAUNCHED();
-    CK(cudaGetLastError());
-  }
+  if (precision == PFBG_F32)
+    CKRC(launch_counts<float>(s, w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, (const float*)dwgt, (float*)dcounts, cbytes));
+  else
+    CKRC(launch_counts<double>(s, w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, (const double*)dwgt, (double*)dcounts, cbytes));
   if (!dev) {
     CK(cudaMemcpyAsync(counts, dcounts, cbytes, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
@@ -2070,7 +2110,7 @@ extern "C" int pfbg_counts_cells(int32_t device, const double* uvw, const double
   CKRC(t.get(&dcells, cells, (size_t)nvis * 8, false, false, 0));
   WParams w = make_wparams(nrow, nchan, 1, nx, ny, cell_x, cell_y, usign, vsign);
   if (nvis > 0) {
-    k_counts<float><<<(unsigned)((nvis + 255) / 256), 256>>>(w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, nullptr, (int32_t*)dcells);
+    k_counts<float><<<(unsigned)((nvis + 255) / 256), 256>>>(w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, nullptr, nullptr, (int32_t*)dcells);
     LAUNCHED();
     CK(cudaGetLastError());
     CK(cudaMemcpy(cells, dcells, (size_t)nvis * 8, cudaMemcpyDeviceToHost));
@@ -2099,38 +2139,118 @@ extern "C" int pfbg_counts_to_weights(int32_t precision, int32_t device, void* c
   if (mask) CKRC(t.get(&dmask, mask, (size_t)nvis, dev, true, s));
   CKRC(t.get(&dwgt, wgt, wbytes, dev, true, s));
   CKRC(t.get(&dcounts, counts, cbytes, dev, true, s));
-  CKRC(t.get(&dsums, nullptr, (2 * 16 + 1) * 8, false, false, s));
-  CK(cudaMemsetAsync(dsums, 0, (2 * 16 + 1) * 8, s));
-  dim3 rgrid(592, ncorr);
-  if (precision == PFBG_F32) k_counts_sums<float><<<rgrid, 256, 0, s>>>((const float*)dcounts, ncell, ncorr, (double*)dsums);
-  else k_counts_sums<double><<<rgrid, 256, 0, s>>>((const double*)dcounts, ncell, ncorr, (double*)dsums);
-  LAUNCHED();
-  double sums[33];
-  CK(cudaMemcpyAsync(sums, dsums, sizeof sums, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  if (sums[2 * ncorr] == 0.0) return PFBG_OK;  // `if not counts.any(): return weight`
-  if (robust > -2.0) {
-    double numsqrt = 5.0 * pow(10.0, -robust);
-    double ssq[16];
-    for (int c = 0; c < ncorr; ++c) ssq[c] = numsqrt * numsqrt * sums[2 * c + 1] / sums[2 * c];
-    CK(cudaMemcpyAsync(dsums, ssq, ncorr * 8, cudaMemcpyHostToDevice, s));
-    if (precision == PFBG_F32) k_counts_scale<float><<<rgrid, 256, 0, s>>>((float*)dcounts, ncell, (const double*)dsums);
-    else k_counts_scale<double><<<rgrid, 256, 0, s>>>((double*)dcounts, ncell, (const double*)dsums);
-    LAUNCHED();
-  }
+  CKRC(t.get(&dsums, nullptr, (size_t)ncorr * 3 * 8, false, false, s));
   WParams w = make_wparams(nrow, nchan, ncorr, nx, ny, cell_x, cell_y, usign, vsign);
-  if (nvis > 0) {
-    unsigned grd = (unsigned)((nvis + 255) / 256);
-    if (precision == PFBG_F32) k_apply_counts<float><<<grd, 256, 0, s>>>(w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, (const float*)dcounts, (float*)dwgt);
-    else k_apply_counts<double><<<grd, 256, 0, s>>>(w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, (const double*)dcounts, (double*)dwgt);
-    LAUNCHED();
-    CK(cudaGetLastError());
-  }
+  if (precision == PFBG_F32)
+    CKRC(launch_reweight<float>(s, w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, 1, (float*)dcounts, (double*)dsums, robust, (float*)dwgt));
+  else
+    CKRC(launch_reweight<double>(s, w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, 1, (double*)dcounts, (double*)dsums, robust, (double*)dwgt));
   if (!dev) {
     CK(cudaMemcpyAsync(wgt, dwgt, wbytes, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(counts, dcounts, cbytes, cudaMemcpyDeviceToHost, s));
   }
   CK(cudaStreamSynchronize(s));
+  return PFBG_OK;
+}
+
+// Arguments of the batched re-weighting, checked before anything is launched.
+static int check_batch_weights(int64_t nbatch, const int64_t* row_offsets, int64_t nrow, int32_t nx_pad,
+                               int32_t ny_pad, double cell_x, double cell_y) {
+  if (nbatch < 1) return fail(PFBG_ERR_ARG, "nbatch must be positive");
+  if (!row_offsets) return fail(PFBG_ERR_ARG, "null row_offsets");
+  if (row_offsets[0] != 0 || row_offsets[nbatch] != nrow) return fail(PFBG_ERR_ARG, "row_offsets must run from 0 to nrow = %lld", (long long)nrow);
+  for (int64_t b = 0; b < nbatch; ++b)
+    if (row_offsets[b + 1] < row_offsets[b]) return fail(PFBG_ERR_ARG, "row_offsets must not decrease (snapshot %lld)", (long long)b);
+  if (nx_pad <= 0 || ny_pad <= 0) return fail(PFBG_ERR_ARG, "pad sizes must be positive, got %d x %d", nx_pad, ny_pad);
+  if (!std::isfinite(cell_x) || !std::isfinite(cell_y) || !(cell_x > 0) || !(cell_y > 0))
+    return fail(PFBG_ERR_ARG, "cell sizes must be finite and positive");
+  return PFBG_OK;
+}
+
+extern "C" int pfbg_counts_to_weights_batch(int32_t precision, int32_t device, int32_t nbatch, const int64_t* row_offsets,
+                                            const double* uvw, const double* freq, const uint8_t* mask, void* wgt,
+                                            int64_t nrow, int32_t nchan, int32_t nx_pad, int32_t ny_pad, double cell_x,
+                                            double cell_y, double robust, double usign, double vsign, void* counts,
+                                            uint32_t flags, void* stream) {
+  if (precision != PFBG_F32 && precision != PFBG_F64) return fail(PFBG_ERR_ARG, "bad precision");
+  if (nrow < 0 || nchan <= 0) return fail(PFBG_ERR_ARG, "bad nrow / nchan");
+  if (!freq || (nrow > 0 && (!uvw || !wgt))) return fail(PFBG_ERR_ARG, "null argument");
+  CKRC(check_batch_weights(nbatch, row_offsets, nrow, nx_pad, ny_pad, cell_x, cell_y));
+  std::vector<int> rs((size_t)(nrow > 0 ? nrow : 1));
+  for (int b = 0; b < nbatch; ++b)
+    for (int64_t r = row_offsets[b]; r < row_offsets[b + 1]; ++r) rs[(size_t)r] = b;
+  CK(cudaSetDevice(device));
+  cudaStream_t s = (cudaStream_t)stream;
+  const bool dev = flags & PFBG_DEVICE_PTRS;
+  const size_t rb = precision == PFBG_F32 ? 4 : 8;
+  const int64_t nvis = nrow * nchan;
+  const size_t cbytes = (size_t)nbatch * nx_pad * ny_pad * rb, wbytes = (size_t)nvis * rb;
+  TmpBufs t;
+  void *duvw, *dfreq, *dmask = nullptr, *dwgt, *dcounts, *dsums, *drs;
+  CKRC(t.get(&duvw, uvw, (size_t)nrow * 24, dev, true, s));
+  CKRC(t.get(&dfreq, freq, (size_t)nchan * 8, dev, true, s));
+  if (mask) CKRC(t.get(&dmask, mask, (size_t)nvis, dev, true, s));
+  CKRC(t.get(&dwgt, wgt, wbytes, dev, true, s));
+  CKRC(t.get(&dcounts, counts, cbytes, dev && counts, false, s));
+  CKRC(t.get(&dsums, nullptr, (size_t)nbatch * 3 * 8, false, false, s));
+  CKRC(t.get(&drs, rs.data(), rs.size() * 4, false, true, s));
+  WParams w = make_wparams(nrow, nchan, 1, nx_pad, ny_pad, cell_x, cell_y, usign, vsign);
+  const double* u = (const double*)duvw;
+  const double* f = (const double*)dfreq;
+  const uint8_t* m = (const uint8_t*)dmask;
+  const int* r = (const int*)drs;
+  if (precision == PFBG_F32) {
+    CKRC(launch_counts<float>(s, w, u, f, m, r, (const float*)dwgt, (float*)dcounts, cbytes));
+    CKRC(launch_reweight<float>(s, w, u, f, m, r, nbatch, (float*)dcounts, (double*)dsums, robust, (float*)dwgt));
+  } else {
+    CKRC(launch_counts<double>(s, w, u, f, m, r, (const double*)dwgt, (double*)dcounts, cbytes));
+    CKRC(launch_reweight<double>(s, w, u, f, m, r, nbatch, (double*)dcounts, (double*)dsums, robust, (double*)dwgt));
+  }
+  if (!dev) {
+    if (nvis > 0) CK(cudaMemcpyAsync(wgt, dwgt, wbytes, cudaMemcpyDeviceToHost, s));
+    if (counts) CK(cudaMemcpyAsync(counts, dcounts, cbytes, cudaMemcpyDeviceToHost, s));
+  }
+  CK(cudaStreamSynchronize(s));
+  return PFBG_OK;
+}
+
+extern "C" int pfbg_bind_weights_robust(pfbg_plan* pl, const void* wgt, int32_t nx_pad, int32_t ny_pad, double cell_x,
+                                        double cell_y, double robust, double usign, double vsign, uint32_t flags,
+                                        void* stream) {
+  if (!pl) return fail(PFBG_ERR_ARG, "null plan");
+  if (!pl->gp.row_snap || !pl->bound) return fail(PFBG_ERR_STATE, "the plan holds no batch of snapshots: pfbg_plan_set_batch and pfbg_bind_vis_batch first");
+  if (!wgt && pl->nvis > 0) return fail(PFBG_ERR_ARG, "null wgt");
+  if (nx_pad <= 0 || ny_pad <= 0) return fail(PFBG_ERR_ARG, "pad sizes must be positive, got %d x %d", nx_pad, ny_pad);
+  if (!std::isfinite(cell_x) || !std::isfinite(cell_y) || !(cell_x > 0) || !(cell_y > 0))
+    return fail(PFBG_ERR_ARG, "cell sizes must be finite and positive");
+  CK(cudaSetDevice(pl->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  pl->has_wgt = false;
+  if (pl->nvis == 0) return PFBG_OK;
+  const size_t rb = real_bytes(pl);
+  const size_t cbytes = (size_t)pl->nbatch * nx_pad * ny_pad * rb, coff = (cbytes + 255) & ~(size_t)255;
+  CKRC(dev_alloc(pl, pl->wgt, (size_t)pl->nvis * rb));
+  CKRC(dev_alloc(pl, pl->wcounts, coff + (size_t)pl->nbatch * 3 * sizeof(double)));
+  CK(cudaMemcpyAsync(pl->wgt.p, wgt, (size_t)pl->nvis * rb, (flags & PFBG_DEVICE_PTRS) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
+  // the bound fscale is fl(freq / c): a division by lightspeed = 1 reproduces pfbg_counts' cell exactly
+  WParams w = make_wparams(pl->nrow, pl->gp.nchan, 1, nx_pad, ny_pad, cell_x, cell_y, usign, vsign);
+  w.lightspeed = 1.0;
+  const double* u = (const double*)pl->uvw.p;
+  const double* f = (const double*)pl->fscale.p;
+  const uint8_t* m = pl->has_mask ? (const uint8_t*)pl->mask.p : nullptr;
+  const int* r = pl->gp.row_snap;
+  double* sums = (double*)((char*)pl->wcounts.p + coff);
+  if (pl->precision == PFBG_F32) {
+    float* c = (float*)pl->wcounts.p;
+    CKRC(launch_counts<float>(s, w, u, f, m, r, (const float*)pl->wgt.p, c, cbytes));
+    CKRC(launch_reweight<float>(s, w, u, f, m, r, pl->nbatch, c, sums, robust, (float*)pl->wgt.p));
+  } else {
+    double* c = (double*)pl->wcounts.p;
+    CKRC(launch_counts<double>(s, w, u, f, m, r, (const double*)pl->wgt.p, c, cbytes));
+    CKRC(launch_reweight<double>(s, w, u, f, m, r, pl->nbatch, c, sums, robust, (double*)pl->wgt.p));
+  }
+  if (!(flags & PFBG_DEVICE_PTRS)) CK(cudaStreamSynchronize(s));  // the caller may free its host array on return
+  pl->has_wgt = true;
   return PFBG_OK;
 }
 

@@ -2,6 +2,11 @@
 // the Briggs / uniform re-weighting that divides by it.  The integer cell index
 // follows /root/reference/src/pfb_imaging/utils/weighting.py:115-135 operation
 // for operation in fp64 without FMA contraction (bit-exact contract).
+//
+// Every kernel takes a batch of snapshots (pfb hci, utils/stokes2im.py:563-604): row r belongs to snapshot
+// row_snap[r] (row_snap == NULL: one snapshot), whose ncorr grids start at grid snapshot * ncorr of the counts cube
+// (nsnap * ncorr, nx, ny).  No sample reaches another snapshot's grids, and each grid has its own sums and ssq, so a
+// batch computes what one call per snapshot computes.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -9,13 +14,18 @@
 struct WParams {
   int64_t nrow;
   int nchan, ncorr, nx, ny;
+  // scale[f] / lightspeed is f/c: freq with lightspeed = c, or a bound fscale = fl(freq / c) with lightspeed = 1
+  // (an exact division, so both give the same cell)
   double u_cell, v_cell, umax, vmax, usign, vsign, lightspeed;
 };
 
+// grids of one launch of the reduction kernels along blockIdx.y; the kernels stride over further grids
+constexpr int kCountsGridsPerLaunch = 64;
+
 // returns false when the sample falls off the grid
 __device__ __forceinline__ bool uv_cell(const WParams& w, const double* __restrict__ uvw,
-                                        const double* __restrict__ freq, int64_t r, int f, int& ui, int& vi) {
-  double cn = __ddiv_rn(freq[f], w.lightspeed);
+                                        const double* __restrict__ scale, int64_t r, int f, int& ui, int& vi) {
+  double cn = __ddiv_rn(scale[f], w.lightspeed);
   double u = __dmul_rn(__dmul_rn(uvw[3 * r + 0], cn), w.usign);
   double v = __dmul_rn(__dmul_rn(uvw[3 * r + 1], cn), w.vsign);
   if (v < 0) { u = -u; v = -v; }
@@ -28,10 +38,16 @@ __device__ __forceinline__ bool uv_cell(const WParams& w, const double* __restri
   return true;
 }
 
+// first cell of correlation c of the snapshot of row r
+__device__ __forceinline__ int64_t grid_base(const WParams& w, const int* __restrict__ row_snap, int64_t r, int c) {
+  const int64_t snap = row_snap ? row_snap[r] : 0;
+  return (snap * w.ncorr + c) * w.nx * (int64_t)w.ny;
+}
+
 template <typename T>
-__global__ void k_counts(WParams w, const double* __restrict__ uvw, const double* __restrict__ freq,
-                         const uint8_t* __restrict__ mask, const T* __restrict__ wgt, T* __restrict__ counts,
-                         int32_t* __restrict__ cell_dump) {
+__global__ void k_counts(WParams w, const double* __restrict__ uvw, const double* __restrict__ scale,
+                         const uint8_t* __restrict__ mask, const int* __restrict__ row_snap, const T* __restrict__ wgt,
+                         T* __restrict__ counts, int32_t* __restrict__ cell_dump) {
   int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   int64_t nvis = w.nrow * w.nchan;
   if (k >= nvis) return;
@@ -40,52 +56,62 @@ __global__ void k_counts(WParams w, const double* __restrict__ uvw, const double
   if (cell_dump) { cell_dump[2 * k] = -1; cell_dump[2 * k + 1] = -1; }
   if (mask && !mask[k]) return;
   int ui, vi;
-  if (!uv_cell(w, uvw, freq, r, f, ui, vi)) return;
+  if (!uv_cell(w, uvw, scale, r, f, ui, vi)) return;
   if (cell_dump) { cell_dump[2 * k] = ui; cell_dump[2 * k + 1] = vi; }
   if (!counts) return;
   for (int c = 0; c < w.ncorr; ++c) {
     T v = wgt[(int64_t)c * nvis + k];
-    atomicAdd(&counts[((int64_t)c * w.nx + ui) * w.ny + vi], v);
+    atomicAdd(&counts[grid_base(w, row_snap, r, c) + (int64_t)ui * w.ny + vi], v);
   }
 }
 
-// per-correlation sum(c^2) and sum(c) -> sums[2*corr], sums[2*corr+1]; any-nonzero flag in sums[2*ncorr]
+// per grid g of ngrid: sum(c^2) -> sums[3g], sum(c) -> sums[3g+1], 1 -> sums[3g+2] when any cell is non-zero
 template <typename T>
-__global__ void k_counts_sums(const T* __restrict__ counts, int64_t ncell, int ncorr, double* __restrict__ sums) {
-  int c = blockIdx.y;
-  const T* p = counts + (int64_t)c * ncell;
-  double s2 = 0, s1 = 0;
-  bool nz = false;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ncell; i += (int64_t)gridDim.x * blockDim.x) {
-    double v = (double)p[i];
-    s2 += v * v;
-    s1 += v;
-    nz |= (v != 0.0);
+__global__ void k_counts_sums(const T* __restrict__ counts, int64_t ncell, int ngrid, double* __restrict__ sums) {
+  for (int g = blockIdx.y; g < ngrid; g += gridDim.y) {
+    const T* p = counts + (int64_t)g * ncell;
+    double s2 = 0, s1 = 0;
+    bool nz = false;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ncell; i += (int64_t)gridDim.x * blockDim.x) {
+      double v = (double)p[i];
+      s2 += v * v;
+      s1 += v;
+      nz |= (v != 0.0);
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+      s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+      s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+    }
+    nz = __any_sync(0xffffffffu, nz);
+    if ((threadIdx.x & 31) == 0) {
+      atomicAdd(&sums[3 * g], s2);
+      atomicAdd(&sums[3 * g + 1], s1);
+      if (nz) sums[3 * g + 2] = 1.0;
+    }
   }
-  for (int o = 16; o > 0; o >>= 1) {
-    s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-    s1 += __shfl_xor_sync(0xffffffffu, s1, o);
-  }
-  nz = __any_sync(0xffffffffu, nz);
-  if ((threadIdx.x & 31) == 0) {
-    atomicAdd(&sums[2 * c], s2);
-    atomicAdd(&sums[2 * c + 1], s1);
-    if (nz) sums[2 * ncorr] = 1.0;
+}
+
+// Briggs: counts = counts * ssq + 1 with ssq = numsq * sum(c) / sum(c^2) of the grid (weighting.py:162-174).  A
+// snapshot whose grids are all zero is left as it is (`if not counts.any(): return weight`), so its weights are too.
+template <typename T>
+__global__ void k_counts_scale(T* __restrict__ counts, int64_t ncell, int ncorr, int ngrid,
+                               const double* __restrict__ sums, double numsq) {
+  for (int g = blockIdx.y; g < ngrid; g += gridDim.y) {
+    const int g0 = g - g % ncorr;
+    bool any = false;
+    for (int c = 0; c < ncorr; ++c) any |= sums[3 * (g0 + c) + 2] != 0.0;
+    if (!any) continue;
+    const T s = (T)(numsq * sums[3 * g + 1] / sums[3 * g]);
+    T* p = counts + (int64_t)g * ncell;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ncell; i += (int64_t)gridDim.x * blockDim.x)
+      p[i] = p[i] * s + (T)1;
   }
 }
 
 template <typename T>
-__global__ void k_counts_scale(T* __restrict__ counts, int64_t ncell, const double* __restrict__ ssq) {
-  int c = blockIdx.y;
-  T s = (T)ssq[c];
-  T* p = counts + (int64_t)c * ncell;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ncell; i += (int64_t)gridDim.x * blockDim.x)
-    p[i] = p[i] * s + (T)1;
-}
-
-template <typename T>
-__global__ void k_apply_counts(WParams w, const double* __restrict__ uvw, const double* __restrict__ freq,
-                               const uint8_t* __restrict__ mask, const T* __restrict__ counts, T* __restrict__ wgt) {
+__global__ void k_apply_counts(WParams w, const double* __restrict__ uvw, const double* __restrict__ scale,
+                               const uint8_t* __restrict__ mask, const int* __restrict__ row_snap,
+                               const T* __restrict__ counts, T* __restrict__ wgt) {
   int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   int64_t nvis = w.nrow * w.nchan;
   if (k >= nvis) return;
@@ -93,9 +119,9 @@ __global__ void k_apply_counts(WParams w, const double* __restrict__ uvw, const 
   int f = (int)(k - r * w.nchan);
   if (mask && !mask[k]) return;
   int ui, vi;
-  if (!uv_cell(w, uvw, freq, r, f, ui, vi)) return;
+  if (!uv_cell(w, uvw, scale, r, f, ui, vi)) return;
   for (int c = 0; c < w.ncorr; ++c) {
-    T cv = counts[((int64_t)c * w.nx + ui) * w.ny + vi];
+    T cv = counts[grid_base(w, row_snap, r, c) + (int64_t)ui * w.ny + vi];
     if (cv > (T)0) wgt[(int64_t)c * nvis + k] /= cv;
   }
 }

@@ -4,7 +4,8 @@
 ``filter_extreme_counts`` (:212-226), ``box_sum_counts`` (:229-254), and the l2 re-weighting block of
 ``image_data_products`` (``operators/gridder.py:509-532`` -> ``l2_reweight``) — with the
 same positional signatures and in-place behaviour (``counts_to_weights`` mutates
-both ``weight`` and ``counts``).  The histogram / gather run in
+both ``weight`` and ``counts``), plus ``counts_to_weights_batch``, the same pair for each snapshot of a
+``pfb hci`` batch in one call.  The histogram / gather run in
 ``libpfbgrid.so`` (``csrc/weighting.cuh``); the median filter and the box sum are
 small image-sized host operations and stay in numpy/scipy.
 """
@@ -94,6 +95,46 @@ def counts_to_weights(counts, uvw, freq, weight, mask, nx, ny, cell_size_x, cell
     if w is not weight:
         weight[...] = w
     if c is not counts:
+        counts[...] = c
+    return weight
+
+
+def counts_to_weights_batch(uvw, freq, weight, mask, row_offsets, nx_pad, ny_pad, cellx, celly, robust, usign=1.0,
+                            vsign=-1.0, counts=None):
+    """Briggs/uniform weights of a batch of snapshots sharing `freq`, in place on `weight` (nrow, nchan) and returned.
+
+    Rows ``[row_offsets[s], row_offsets[s+1])`` of `uvw`, `weight` and `mask` are snapshot s.  Each snapshot ends
+    with the weights this pair of calls gives it on its own (the per-snapshot weighting of utils/stokes2im.py:563-604):
+
+        c = _compute_counts(uvw_s, freq, mask_s, weight_s[None], nx_pad, ny_pad, cellx, celly, weight.dtype, 1, usign, vsign)
+        counts_to_weights(c, uvw_s, freq, weight_s[None], mask_s, nx_pad, ny_pad, cellx, celly, robust, usign, vsign)
+
+    One counts grid per snapshot, all on the device in one launch sequence.  `counts`, when given, is an
+    (nsnap, nx_pad, ny_pad) array of the weights' dtype that receives the grids as ``counts_to_weights`` leaves them.
+    ``filter_extreme_counts`` / ``box_sum_counts`` are not applied; callers that need them keep the per-snapshot calls."""
+    if not isinstance(weight, np.ndarray) or weight.ndim != 2:
+        raise ValueError("weight must be an ndarray of shape (nrow, nchan)")
+    nrow, nchan = weight.shape
+    dt = weight.dtype
+    prec = _prec(dt)
+    uvw, freq, mask = _geom(uvw, freq, mask, nrow, nchan)
+    ro = np.ascontiguousarray(row_offsets, dtype=np.int64)
+    if ro.ndim != 1 or ro.size < 2 or ro[-1] != nrow:
+        raise ValueError(f"row_offsets must be 1-D, one entry more than the snapshots, and end at nrow = {nrow}")
+    nsnap = ro.size - 1
+    if counts is not None and (not isinstance(counts, np.ndarray) or counts.dtype != dt
+                               or counts.shape != (nsnap, int(nx_pad), int(ny_pad))):
+        raise ValueError(f"counts must be an ({nsnap}, {int(nx_pad)}, {int(ny_pad)}) array of the weights' dtype")
+    w = weight if weight.flags.c_contiguous else np.ascontiguousarray(weight)
+    c = None if counts is None else (counts if counts.flags.c_contiguous else np.empty(counts.shape, dt))
+    lib = _lib.load()
+    _lib.check(lib.pfbg_counts_to_weights_batch(prec, current_device(), nsnap, _p(ro), _p(uvw), _p(freq), _p(mask),
+                                                _p(w), nrow, nchan, int(nx_pad), int(ny_pad), float(cellx),
+                                                float(celly), float(robust), float(usign), float(vsign), _p(c),
+                                                _lib.HOST_PTRS, None))
+    if w is not weight:
+        weight[...] = w
+    if c is not None and c is not counts:
         counts[...] = c
     return weight
 

@@ -15,7 +15,7 @@ import weakref
 import numpy as np
 
 from . import _lib
-from .plan import LIGHTSPEED, Plan, make_batch_plan, make_plan, w_range
+from .plan import LIGHTSPEED, Plan, good_size, make_batch_plan, make_plan, w_range
 
 _PREC = {"single": _lib.PFBG_F32, "double": _lib.PFBG_F64}
 _RDT = {"single": np.float32, "double": np.float64}
@@ -172,6 +172,16 @@ class GridderPlan:
         if wgt is not None:
             wgt = self._check_wgt(wgt)
         _lib.check(self._lib.pfbg_bind_weights(self._h, _ptr(wgt), _lib.HOST_PTRS, stream))
+        return self
+
+    def bind_robust_weights(self, wgt, nx_pad, ny_pad, cellx, celly, robust, usign=1.0, vsign=-1.0, stream=None):
+        """Bind the Briggs/uniform weights of every snapshot of the bound batch, computed on the device from the
+        natural weights `wgt` (nrow, nchan) as ``weighting.counts_to_weights_batch`` computes them, without the
+        weights coming back to the host (``pfbg_bind_weights_robust``).  Later calls without `wgt` use them."""
+        wgt = self._check_wgt(wgt)
+        _lib.check(self._lib.pfbg_bind_weights_robust(self._h, _ptr(wgt), int(nx_pad), int(ny_pad), float(cellx),
+                                                      float(celly), float(robust), float(usign), float(vsign),
+                                                      _lib.HOST_PTRS, stream))
         return self
 
     def info(self) -> dict:
@@ -647,10 +657,16 @@ def batch_plan_for(uvw_list, freq, *, npix_x, npix_y, pixsize_x, pixsize_y, cent
 def vis2dirty_batch(*, uvw, freq, vis, wgt=None, mask=None, npix_x, npix_y, pixsize_x, pixsize_y, center_x=0.0,
                     center_y=0.0, epsilon, flip_u=False, flip_v=False, flip_w=False, do_wgridding=True, divide_by_n=True,
                     nthreads=1, sigma_min=1.1, sigma_max=2.6, double_precision_accumulation=False, verbosity=0,
-                    dirty=None, extra_vis=()):
+                    dirty=None, extra_vis=(), robustness=None, nx_pad=None, ny_pad=None):
     """``vis2dirty`` for a list of snapshots of one geometry: `uvw`, `vis`, `wgt`, `mask` are lists (one entry per
     snapshot, `freq` is shared); returns ``(nsnap, npix_x, npix_y)``.  `extra_vis`: further lists of visibilities
-    gridded with the same binding (the PSF visibilities of stokes2im.py:660-683); then a tuple of cubes comes back."""
+    gridded with the same binding (the PSF visibilities of stokes2im.py:660-683); then a tuple of cubes comes back.
+
+    `robustness`: grid with each snapshot's Briggs weights (utils/stokes2im.py:563-604), computed on the device from
+    `wgt` (ones when None) on an (nx_pad, ny_pad) counts grid with cells (pixsize_x, pixsize_y), as
+    ``weighting.counts_to_weights_batch`` computes them.  The pad defaults to ``plan.good_size(2 * npix)``, which
+    admits the factors 2, 3, 5, 7; the reference's ducc0 ``good_size`` also admits 11, so pass the pad where the two
+    differ.  ``filter_extreme_counts`` / ``box_sum_counts`` are not applied."""
     nsnap = len(uvw)
     prec = _precision_of(np.asarray(vis[0]).dtype, "vis")
     gp = batch_plan_for(uvw, freq, npix_x=npix_x, npix_y=npix_y, pixsize_x=pixsize_x, pixsize_y=pixsize_y,
@@ -659,6 +675,12 @@ def vis2dirty_batch(*, uvw, freq, vis, wgt=None, mask=None, npix_x, npix_y, pixs
                         precision=prec, mask_list=mask, pooled=True)
     with gp as g:
         w = None if wgt is None else np.concatenate([np.asarray(a) for a in wgt], axis=0)
+        if robustness is not None:
+            g.bind_robust_weights(np.ones((g.nrow, g.nchan), g.rdt) if w is None else w,
+                                  good_size(2 * npix_x) if nx_pad is None else nx_pad,
+                                  good_size(2 * npix_y) if ny_pad is None else ny_pad, pixsize_x, pixsize_y, robustness,
+                                  usign=1.0 if flip_u else -1.0, vsign=1.0 if flip_v else -1.0)
+            w = None  # grid with the bound robust weights
         outs = []
         for k, vl in enumerate((vis,) + tuple(extra_vis)):
             if len(vl) != nsnap:
