@@ -285,6 +285,22 @@ int pfbg_conv_apply(pfbg_conv* conv, const void* x, const void* beam, double eta
 /* Read-only: the column-block width C (1, 2 or 4 columns per CTA of the column pass) and the CTA size of the
  * row passes that this convolver runs with.  Either output pointer may be NULL. */
 int pfbg_conv_info(const pfbg_conv* conv, int32_t* col_block, int32_t* row_threads);
+/*
+ * Analytic kernel (`pfb restore`): the multiplier becomes the DFT on the padded grid of the periodised, pixel-sampled
+ * Gaussian g(x, y) = exp(-4 ln 2 (x'^2 / emaj^2 + y'^2 / emin^2)), (x', y') the pixel offsets rotated by pa, evaluated
+ * inside the column pass (no spectrum is stored).  Beams are (emaj, emin, pa): FWHMs in pixels, emaj >= emin >= 1,
+ * the major axis along (cos pa, sin pa) in the (axis 0, axis 1) plane.  from == NULL: convolution with `to`; else the
+ * ratio K_to / K_from that takes an image at resolution `from` to resolution `to`, which needs S_to - S_from positive
+ * semi-definite (S the beam covariances).  The alias sums keep every term above 1e-18 of the peak (plain) or of the
+ * largest term of each sum (ratio).  norm_kernel != 0: unit-sum kernels, else peak 1.  PFBG_ERR_ARG for a beam below
+ * 1 px, emaj < emin, a `to` that does not contain `from`, or (ratio only) an axis ratio above about 30.
+ * pfbg_conv_set_kernel switches back; the stored spectrum is allocated by set_kernel (so an out-of-memory failure
+ * shows there, and leaves the previous kernel in place) and released here, after a device synchronisation.
+ */
+int pfbg_conv_set_gauss(pfbg_conv* conv, const double to[3], const double from[3], int32_t norm_kernel);
+/* out = crop(IFFT(FFT(pad(x)) * K)) + add, the sum taken in the row epilogue; pointers as in pfbg_conv_apply.  With
+ * PFBG_DEVICE_PTRS, `add` must not alias `out` (host pointers are staged, so there they may). */
+int pfbg_conv_apply_add(pfbg_conv* conv, const void* x, const void* add, void* out, uint32_t flags, void* stream);
 
 /*
  * Band split across two GPUs, one process per GPU (SURVEY §8e; the reference runs one actor per band,

@@ -17,6 +17,7 @@ LIB_PATH = os.environ.get("PFBG_LIB") or os.path.join(HERE, "libpfbgrid.so")  # 
 CSRC = os.path.join(HERE, "csrc")
 
 PFBG_F32, PFBG_F64 = 0, 1
+PFBG_ERR_ARG = 1
 HOST_PTRS, DEVICE_PTRS, APPLY_WGT, NO_MASK_ZERO = 0, 1, 2, 4
 PINNED_IN, PINNED_OUT, BEAM_CACHED = 16, 32, 64
 PLAN_EXTERNAL_STACK = 1
@@ -86,6 +87,8 @@ SIGNATURES = {
     "pfbg_conv_set_kernel": (C.c_int, [_vp, _vp, _i32, _u32, _vp]),
     "pfbg_conv_apply": (C.c_int, [_vp, _vp, _vp, _dbl, _vp, _u32, _vp]),
     "pfbg_conv_info": (C.c_int, [_vp, C.POINTER(_i32), C.POINTER(_i32)]),
+    "pfbg_conv_set_gauss": (C.c_int, [_vp, C.POINTER(_dbl), C.POINTER(_dbl), _i32]),
+    "pfbg_conv_apply_add": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _vp]),
     "pfbg_debug_fft1d": (C.c_int, [_i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32]),
     "pfbg_debug_es_fast64": (C.c_int, [_i32, _i64, _vp, C.c_double, _vp]),
     "pfbg_weight_data_corr": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i64, _i64, _i64, _i64,

@@ -66,10 +66,69 @@ k_conv_rows_fwd(ConvTabs ct, const T* __restrict__ x, const T* __restrict__ beam
   }
 }
 
-// column block: forward along u, multiply by khat[k][b], inverse along u, keep rows < nx
-template <typename T, int C>
+// The multiplier of the column pass at spectral cell (k, b0 + c): k is the row of the full spectrum (the digit-reversed
+// position already resolved), b0 + c the column.  KhatMul reads the stored spectrum; GaussMul evaluates the transfer
+// function of a pixel-sampled Gaussian where it is used, so nothing is stored.
+struct KhatMul {
+  template <typename T>
+  __device__ __forceinline__ cx2<T> operator()(const ConvTabs& ct, const cx2<T>* __restrict__ khat, int k, int b0,
+                                               int c) const {
+    return khat[(int64_t)k * ct.nyp + b0 + c];
+  }
+};
+
+// DFT on the padded grid of the periodised, pixel-sampled Gaussian g(x) = exp(-x^T S^-1 x / 2), by Poisson summation:
+//     K(f) = amp * sum_{m in Z^2, |m_i| <= M} exp(q(f + m)),   q(f) = -2 pi^2 f^T S f,
+// f = (k~ / nxp, l~ / nyp) the signed frequencies.  q[] holds (-2 pi^2 S00, -4 pi^2 S01, -2 pi^2 S11), so
+// q(f) = q[0] fx^2 + q[1] fx fy + q[2] fy^2.  Every alias term is the exp of its own exponent (a product of separately
+// exponentiated factors overflows for wide beams).  ratio != 0: K_to / K_from, each sum scaled by the exp of its
+// largest exponent (the m = 0 term whenever f is S-nearest to the origin), so that neither sum underflows and the
+// quotient of the two scales, exp(qmax_to - qmax_from) <= 1 for S_to - S_from positive semi-definite, cannot overflow.
+struct GaussMul {
+  double q_to[3], q_from[3];
+  double amp;  // plain: 2 pi sqrt(det S) (peak 1) or 1 / sum (unit sum); ratio: amp_to / amp_from
+  int M, ratio;
+
+  __device__ __forceinline__ double qform(const double* q, double fx, double fy) const {
+    return q[0] * fx * fx + q[1] * fx * fy + q[2] * fy * fy;
+  }
+  // sum_m exp(q(f + m) - shift), shift = max_m q(f + m) when scaled
+  __device__ __forceinline__ double alias_sum(const double* q, double fx, double fy, bool scaled, double& shift) const {
+    shift = 0.0;
+    if (scaled) {
+      shift = -INFINITY;
+      for (int mx = -M; mx <= M; ++mx)
+        for (int my = -M; my <= M; ++my) shift = fmax(shift, qform(q, fx + mx, fy + my));
+    }
+    double acc = 0.0;
+    for (int mx = -M; mx <= M; ++mx)
+      for (int my = -M; my <= M; ++my) acc += exp(qform(q, fx + mx, fy + my) - shift);
+    return acc;
+  }
+  template <typename T>
+  __device__ __forceinline__ cx2<T> operator()(const ConvTabs& ct, const cx2<T>* __restrict__, int k, int b0,
+                                               int c) const {
+    const int l = b0 + c;
+    const double fx = (double)(2 * k > ct.nxp ? k - ct.nxp : k) / (double)ct.nxp;
+    const double fy = (double)(2 * l > ct.nyp ? l - ct.nyp : l) / (double)ct.nyp;
+    double v;
+    if (!ratio) {
+      double s0;
+      v = amp * alias_sum(q_to, fx, fy, false, s0);
+    } else {
+      double st, sf;
+      const double nt = alias_sum(q_to, fx, fy, true, st);
+      const double nf = alias_sum(q_from, fx, fy, true, sf);
+      v = amp * exp(st - sf) * (nt / nf);
+    }
+    return {(T)v, (T)0};
+  }
+};
+
+// column block: forward along u, multiply by mul(k, b), inverse along u, keep rows < nx
+template <typename T, int C, class Mul>
 __global__ void __launch_bounds__(512)
-k_conv_cols(ConvTabs ct, const cx2<T>* __restrict__ khat, cx2<T>* __restrict__ tmp) {
+k_conv_cols(ConvTabs ct, const cx2<T>* __restrict__ khat, cx2<T>* __restrict__ tmp, Mul mul) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   cx2<T>* s = reinterpret_cast<cx2<T>*>(smem_raw);
   const int tid = threadIdx.x, nthr = blockDim.x;
@@ -97,7 +156,7 @@ k_conv_cols(ConvTabs ct, const cx2<T>* __restrict__ khat, cx2<T>* __restrict__ t
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int w = w0 + u * nthr;
-      if (w < ct.nxp * C) kv[u] = khat[(int64_t)ct.rev_u[w / C] * ct.nyp + b0 + (w % C)];
+      if (w < ct.nxp * C) kv[u] = mul(ct, khat, ct.rev_u[w / C], b0, w % C);
     }
 #pragma unroll
     for (int u = 0; u < U; ++u) {

@@ -334,8 +334,8 @@ def image_data_products(dsl, dsp, nx, ny, nx_psf, ny_psf, cellx, celly, output_n
     `dsl` = list of ``.xds`` groups (paths or dataset-likes with VIS, WEIGHT (corr,row,chan), MASK, UVW, FREQ, BEAM,
     l_beam, m_beam), concatenated along rows; `dsp` = optional dataset with the prior WEIGHT for the l2
     re-weighting; products are written to the zarr group `output_name` and ``{residual, psf, wsum, timeid}`` is
-    returned.  ``PSFPARSN`` needs the reference's jax / scikit-image ``fitcleanbeam``: pass it as `fit_psf`,
-    otherwise that variable is not written."""
+    returned.  ``PSFPARSN`` is written when a fitter is passed as `fit_psf` (``restore.fitcleanbeam``), otherwise
+    that variable is not written."""
     from .store import Dataset
 
     flip_u, flip_v, flip_w, x0, y0 = wgridder_conventions(l0, m0)
@@ -575,8 +575,8 @@ def grid_partition(part, counts, nx, ny, nx_psf, ny_psf, cell_rad, robustness=No
     reduced counts grid, then DIRTY, PSF, PSFHAT, BEAM, WSUM and the imaging WEIGHT.
 
     `part` is duck-typed: attributes ``UVW, VIS, WEIGHT, MASK, FREQ, BEAM, l_beam, m_beam`` exposing
-    ``.values`` (xarray) or plain arrays.  ``PSFPARSN`` needs the reference's jax/scikit-image
-    ``fitcleanbeam`` (out of scope); pass ``fit_psf`` to supply it, otherwise the key is omitted."""
+    ``.values`` (xarray) or plain arrays.  ``PSFPARSN`` is returned when a fitter is passed as ``fit_psf``
+    (``restore.fitcleanbeam``), otherwise the key is omitted."""
     from .weighting import counts_to_weights
 
     flip_u, flip_v, flip_w, x0, y0 = wgridder_conventions(l0, m0)

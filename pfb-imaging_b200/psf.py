@@ -26,7 +26,8 @@ _RDT = {np.dtype(np.float32): (_lib.PFBG_F32, np.complex64), np.dtype(np.float64
 
 
 class PsfConvolver:
-    """out = beam * crop(IFFT(FFT(pad(beam * x)) * khat)) + eta * x for one band."""
+    """out = beam * crop(IFFT(FFT(pad(beam * x)) * khat)) + eta * x for one band.  After :meth:`set_gauss` the
+    multiplier is the transfer function of a pixel-sampled Gaussian (or a ratio of two), evaluated on the device."""
 
     def __init__(self, nx, ny, nx_psf, ny_psf, dtype=np.float64, device=None):
         self.rdt = np.dtype(dtype)
@@ -54,7 +55,27 @@ class PsfConvolver:
         _lib.check(self._lib.pfbg_conv_set_kernel(self._h, C.c_void_p(k.ctypes.data), half, _lib.HOST_PTRS, None))
         return self
 
-    def apply(self, x, beam=None, eta=None, out=None):
+    def set_gauss(self, beam_to, beam_from=None, norm_kernel=False):
+        """Switch to the analytic kernel of ``restore.py``: convolution with the pixel-sampled Gaussian `beam_to`, or,
+        with `beam_from`, the conversion of an image at resolution `beam_from` to `beam_to`.  Beams are
+        ``(emaj, emin, pa)`` in pixels (FWHMs, ``emaj >= emin >= 1``); `norm_kernel`: unit-sum instead of peak-1
+        kernels.  ValueError for a sub-pixel beam or a `beam_to` that does not contain `beam_from`.  The stored
+        spectrum of :meth:`set_kernel`, if any, is released."""
+        def arr(b):
+            b = np.asarray(b, dtype=np.float64).reshape(-1)
+            if b.size != 3:
+                raise ValueError("a beam is (emaj, emin, pa)")
+            return (C.c_double * 3)(*b)
+
+        rc = self._lib.pfbg_conv_set_gauss(self._h, arr(beam_to), None if beam_from is None else arr(beam_from),
+                                           int(bool(norm_kernel)))
+        if rc == _lib.PFBG_ERR_ARG:
+            raise ValueError(self._lib.pfbg_last_error().decode())
+        _lib.check(rc)
+        return self
+
+    def apply(self, x, beam=None, eta=None, out=None, add=None):
+        """`add`: ``crop(IFFT(FFT(pad(x)) * K)) + add``, the sum taken on the device (no `beam`, no `eta`)."""
         x = np.ascontiguousarray(x, dtype=self.rdt)
         if x.shape != (self.nx, self.ny):
             raise ValueError(f"x shape {x.shape} != ({self.nx}, {self.ny})")
@@ -62,18 +83,35 @@ class PsfConvolver:
             beam = np.ascontiguousarray(beam, dtype=self.rdt)
             if beam.shape != x.shape:
                 raise ValueError("beam shape does not match the image")
+        if add is not None:
+            if beam is not None or eta:
+                raise ValueError("add= takes neither beam nor eta")
+            add = np.ascontiguousarray(add, dtype=self.rdt)
+            if add.shape != x.shape:
+                raise ValueError("add shape does not match the image")
         res = np.empty_like(x) if out is None else out
         tmp = res if (res.flags.c_contiguous and res.dtype == self.rdt) else np.empty_like(x)
-        _lib.check(self._lib.pfbg_conv_apply(self._h, C.c_void_p(x.ctypes.data),
-                                             None if beam is None else C.c_void_p(beam.ctypes.data),
-                                             float(eta) if eta else 0.0, C.c_void_p(tmp.ctypes.data),
-                                             _lib.HOST_PTRS, None))
+        if add is not None:
+            _lib.check(self._lib.pfbg_conv_apply_add(self._h, C.c_void_p(x.ctypes.data), C.c_void_p(add.ctypes.data),
+                                                     C.c_void_p(tmp.ctypes.data), _lib.HOST_PTRS, None))
+        else:
+            _lib.check(self._lib.pfbg_conv_apply(self._h, C.c_void_p(x.ctypes.data),
+                                                 None if beam is None else C.c_void_p(beam.ctypes.data),
+                                                 float(eta) if eta else 0.0, C.c_void_p(tmp.ctypes.data),
+                                                 _lib.HOST_PTRS, None))
         if tmp is not res:
             res[...] = tmp
         return res
 
-    def apply_dev(self, x_ptr, out_ptr, beam_ptr=None, eta=None, stream=None):
-        """Same operator on device pointers (asynchronous on `stream`): what the device-resident deconvolution loops call."""
+    def apply_dev(self, x_ptr, out_ptr, beam_ptr=None, eta=None, stream=None, add_ptr=None):
+        """Same operator on device pointers (asynchronous on `stream`): what the device-resident deconvolution loops call.
+        `add_ptr`: ``out = crop(IFFT(FFT(pad(x)) * K)) + add`` (no beam, no eta)."""
+        if add_ptr is not None:
+            if beam_ptr is not None or eta:
+                raise ValueError("add_ptr takes neither beam_ptr nor eta")
+            _lib.check(self._lib.pfbg_conv_apply_add(self._h, C.c_void_p(int(x_ptr)), C.c_void_p(int(add_ptr)),
+                                                     C.c_void_p(int(out_ptr)), _lib.DEVICE_PTRS, stream))
+            return
         _lib.check(self._lib.pfbg_conv_apply(self._h, C.c_void_p(int(x_ptr)), None if beam_ptr is None else C.c_void_p(int(beam_ptr)),
                                              float(eta) if eta else 0.0, C.c_void_p(int(out_ptr)), _lib.DEVICE_PTRS, stream))
 
