@@ -301,6 +301,15 @@ int pfbg_conv_set_gauss(pfbg_conv* conv, const double to[3], const double from[3
 /* out = crop(IFFT(FFT(pad(x)) * K)) + add, the sum taken in the row epilogue; pointers as in pfbg_conv_apply.  With
  * PFBG_DEVICE_PTRS, `add` must not alias `out` (host pointers are staged, so there they may). */
 int pfbg_conv_apply_add(pfbg_conv* conv, const void* x, const void* add, void* out, uint32_t flags, void* stream);
+/*
+ * Direct inverse of the Hessian (operators/hessian.py:213-248 hess_direct_slice) from the stored spectrum, fp64 only:
+ *     out = taper * crop( IFFT( FFT( pad(taper * x) ) * (Re khat + c)^s ) ),   s = -1 if inverse else +1
+ * taper may be NULL; no ridge term.  Re khat + c and its reciprocal are formed in fp64 with IEEE division, so the
+ * output equals that of a convolver whose kernel was set to those doubles.  Pointers as in pfbg_conv_apply.
+ * PFBG_ERR_STATE for a convolver without a stored spectrum (no kernel, or pfbg_conv_set_gauss).
+ */
+int pfbg_conv_apply_shifted(pfbg_conv* conv, const void* x, const void* taper, double c, int32_t inverse, void* out,
+                            uint32_t flags, void* stream);
 
 /*
  * Band split across two GPUs, one process per GPU (SURVEY §8e; the reference runs one actor per band,

@@ -111,6 +111,28 @@ int pfbs_clark_run(pfbs_clark* h, const void* dirty, const uint8_t* mask, void* 
                    float* times_ms, uint32_t flags, void* stream);
 int pfbs_clark_destroy(pfbs_clark* h);
 
+/*
+ * Conjugate gradients on the PSF-convolution Hessian of every band at once (HessPSF.idot(mode="psf"),
+ * operators/hessian.py:357-436), fp64 only.  Per band b, solvers.pcg with no preconditioner on
+ *     A_b v = beam_b conv_b(beam_b v) + eta_b v      (pfbg_conv_apply(conv[b], v, beam[b], eta[b]))
+ * rhs and x are (nband, nx, ny) device arrays, npix = nx * ny; x holds the starting point on entry and the solution on
+ * return.  beam[b] may be NULL.  The convolvers are borrowed (any kernel mode) and must share (nx, ny) and `device`.
+ * work: device memory of at least pfbs_psf_cg_work_bytes(nband, npix) bytes (r, p, Ap and the reductions).
+ * Stopping rules as pcg: iterate while (eps > tol or k < minit) and k < maxit and stalls < 5, each band on its own;
+ * a band that stops is frozen and its convolutions are skipped.  Host outputs per band: iters, eps and stop, one of
+ * the PFBS_CG_* codes below.  All reductions are deterministic.  Synchronises `stream` once per iteration.
+ */
+#define PFBS_CG_CONVERGED 1
+#define PFBS_CG_MAXIT 2
+#define PFBS_CG_STALLED 3
+#define PFBS_CG_ZERO_RESIDUAL 4 /* r = A x - b had r.r not > 0: x is left as it was */
+#define PFBS_CG_EXACT 5         /* rho == 0 and p.Ap == 0: the iterate is the solution */
+
+int64_t pfbs_psf_cg_work_bytes(int32_t nband, int64_t npix); /* -1 for nband < 1 or npix < 1 */
+int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv, const void* const* beam, const double* eta,
+                const void* rhs, void* x, int64_t npix, double tol, int32_t maxit, int32_t minit, void* work,
+                int64_t work_bytes, int32_t* iters, double* eps, int32_t* stop, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -89,6 +89,7 @@ SIGNATURES = {
     "pfbg_conv_info": (C.c_int, [_vp, C.POINTER(_i32), C.POINTER(_i32)]),
     "pfbg_conv_set_gauss": (C.c_int, [_vp, C.POINTER(_dbl), C.POINTER(_dbl), _i32]),
     "pfbg_conv_apply_add": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _vp]),
+    "pfbg_conv_apply_shifted": (C.c_int, [_vp, _vp, _vp, _dbl, _i32, _vp, _u32, _vp]),
     "pfbg_debug_fft1d": (C.c_int, [_i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32]),
     "pfbg_debug_es_fast64": (C.c_int, [_i32, _i64, _vp, C.c_double, _vp]),
     "pfbg_weight_data_corr": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i64, _i64, _i64, _i64,
@@ -128,6 +129,9 @@ SIGNATURES = {
     "pfbs_clark_destroy": (C.c_int, [_vp]),
     "pfbs_clark_run": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _dbl, _dbl, _dbl, _i32, _dbl, _i32, C.POINTER(_i32), _vp, _vp,
                                  _vp, _vp, _i64, _vp, _u32, _vp]),
+    "pfbs_psf_cg_work_bytes": (_i64, [_i32, _i64]),
+    "pfbs_psf_cg": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _dbl, _i32, _i32, _vp, _i64, _vp, _vp, _vp,
+                              _vp]),
 }
 
 _lib = None
@@ -139,7 +143,7 @@ _UNITS = {
     "pfbgrid.cu": ["common.cuh", "fft.cuh", "fused_fft.cuh", "kernels.cuh", "psfconv.cuh", "runs.cuh", "runs_mma.cuh", "weighting.cuh",
                    "cols2_api.h", "fused_common.cuh", "../../include/pfbgrid.h"],
     "colsfft.cu": ["common.cuh", "fft.cuh", "fft2.cuh", "cols2.cuh", "rows2.cuh", "cols2_api.h", "fused_common.cuh"],
-    "pfbsara.cu": ["sara.cuh", "clean.cuh", "../../include/pfbsara.h", "../../include/pfbgrid.h"],
+    "pfbsara.cu": ["sara.cuh", "clean.cuh", "cg.cuh", "../../include/pfbsara.h", "../../include/pfbgrid.h"],
 }
 
 

@@ -2515,6 +2515,11 @@ static int conv_setup_t(pfbg_conv* cv) {
   CK(cudaFuncSetAttribute(k_conv_cols<T, 4, GaussMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
   CK(cudaFuncSetAttribute(k_conv_cols<T, 2, GaussMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
   CK(cudaFuncSetAttribute(k_conv_cols<T, 1, GaussMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+  if constexpr (sizeof(T) == 8) {  // pfbg_conv_apply_shifted is fp64 only
+    CK(cudaFuncSetAttribute(k_conv_cols<T, 4, ShiftMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+    CK(cudaFuncSetAttribute(k_conv_cols<T, 2, ShiftMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+    CK(cudaFuncSetAttribute(k_conv_cols<T, 1, ShiftMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+  }
   return PFBG_OK;
 }
 
@@ -2720,16 +2725,23 @@ static void conv_cols_launch(const pfbg_conv* cv, const Mul& mul, cudaStream_t s
   else k_conv_cols<T, 1, Mul><<<ncol, 512, csm, s>>>(ct, kh, tmp, mul);
 }
 
-// xin != NULL: out += eta * xin in the row epilogue (the ridge term of the Hessian, or eta = 1 for apply_add)
+// xin != NULL: out += eta * xin in the row epilogue (the ridge term of the Hessian, or eta = 1 for apply_add).
+// shift != NULL (fp64, stored spectrum): the column pass multiplies by ShiftMul instead of the convolver's own kernel.
 template <typename T>
 static int conv_apply_t(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta, void* out,
-                        cudaStream_t s) {
+                        cudaStream_t s, const ShiftMul* shift) {
   const ConvTabs& ct = cv->ct;
   const int rt = row_threads(ct.nyp, 256);
   k_conv_rows_fwd<T><<<(ct.nx + 1) / 2, rt, fft_smem_bytes<T>(ct.nyp), s>>>(ct, (const T*)x, (const T*)beam, (cx2<T>*)cv->tmp);
   LAUNCHED();
-  if (cv->gauss) conv_cols_launch<T>(cv, cv->gm, s);
-  else conv_cols_launch<T>(cv, KhatMul{}, s);
+  if constexpr (sizeof(T) == 8) {
+    if (shift) conv_cols_launch<T>(cv, *shift, s);
+    else if (cv->gauss) conv_cols_launch<T>(cv, cv->gm, s);
+    else conv_cols_launch<T>(cv, KhatMul{}, s);
+  } else {
+    if (cv->gauss) conv_cols_launch<T>(cv, cv->gm, s);
+    else conv_cols_launch<T>(cv, KhatMul{}, s);
+  }
   LAUNCHED();
   const double scale = 1.0 / ((double)ct.nxp * (double)ct.nyp);
   k_conv_rows_inv<T><<<(ct.nx + 1) / 2, rt, fft_smem_bytes<T>(ct.nyp), s>>>(ct, (const cx2<T>*)cv->tmp, (const T*)beam,
@@ -2742,7 +2754,7 @@ static int conv_apply_t(pfbg_conv* cv, const void* x, const void* beam, const vo
 // out = beam * crop(IFFT(FFT(pad(beam * x)) * K)) + eta * xin; host pointers are staged through d_x / d_beam / d_out
 // (apply_add passes no beam, so its `add` image rides in d_beam)
 static int conv_apply_any(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta, void* out,
-                          uint32_t flags, void* stream) {
+                          uint32_t flags, void* stream, const ShiftMul* shift = nullptr) {
   if (!cv || !x || !out) return fail(PFBG_ERR_ARG, "null argument");
   if (!cv->has_kernel) return fail(PFBG_ERR_STATE, "no kernel set");
   CK(cudaSetDevice(cv->device));
@@ -2759,8 +2771,8 @@ static int conv_apply_any(pfbg_conv* cv, const void* x, const void* beam, const 
     else if (xin) { CK(cudaMemcpyAsync(cv->d_beam, xin, ib, cudaMemcpyHostToDevice, s)); dxin = cv->d_beam; }
     dout = cv->d_out;
   }
-  CKRC(cv->precision == PFBG_F32 ? conv_apply_t<float>(cv, dx, db, dxin, eta, dout, s)
-                                 : conv_apply_t<double>(cv, dx, db, dxin, eta, dout, s));
+  CKRC(cv->precision == PFBG_F32 ? conv_apply_t<float>(cv, dx, db, dxin, eta, dout, s, nullptr)
+                                 : conv_apply_t<double>(cv, dx, db, dxin, eta, dout, s, shift));
   if (!dev) {
     CK(cudaMemcpyAsync(out, dout, ib, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
@@ -2779,4 +2791,22 @@ extern "C" int pfbg_conv_apply_add(pfbg_conv* cv, const void* x, const void* add
                                    void* stream) {
   if (!add) return fail(PFBG_ERR_ARG, "null argument");
   return conv_apply_any(cv, x, nullptr, add, 1.0, out, flags, stream);
+}
+
+// out = taper * crop(IFFT(FFT(pad(taper * x)) * (Re khat + c)^(+-1)))   (taper may be NULL; no ridge term)
+extern "C" int pfbg_conv_apply_shifted(pfbg_conv* cv, const void* x, const void* taper, double c, int32_t inverse,
+                                       void* out, uint32_t flags, void* stream) {
+  if (!cv || !x || !out) return fail(PFBG_ERR_ARG, "null argument");
+  if (cv->precision != PFBG_F64) return fail(PFBG_ERR_ARG, "the shifted spectrum is fp64 only");
+  if (!cv->has_kernel || cv->gauss || !cv->khat)
+    return fail(PFBG_ERR_STATE, "the shifted spectrum needs a stored spectrum (pfbg_conv_set_kernel)");
+  const ShiftMul sh{c, inverse ? 1 : 0};
+  return conv_apply_any(cv, x, taper, nullptr, 0.0, out, flags, stream, &sh);
+}
+
+// what the batched solvers of pfbsara.cu check before borrowing a convolver (not part of the C ABI)
+int pfbg_conv_props(const pfbg_conv* cv, int* precision, int* device, int* nx, int* ny, int* has_kernel) {
+  if (!cv) return fail(PFBG_ERR_ARG, "null convolver");
+  *precision = cv->precision; *device = cv->device; *nx = cv->ct.nx; *ny = cv->ct.ny; *has_kernel = cv->has_kernel;
+  return PFBG_OK;
 }

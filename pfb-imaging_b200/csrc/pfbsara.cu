@@ -1,5 +1,5 @@
-// C-ABI of the device backward steps (include/pfbsara.h): SARA (kernels in sara.cuh) and the Clark minor cycle
-// (clean.cuh).
+// C-ABI of the device backward steps (include/pfbsara.h): SARA (kernels in sara.cuh), the Clark minor cycle
+// (clean.cuh) and the batched conjugate gradients of HessPSF.idot (cg.cuh).
 #include <cuda_runtime.h>
 
 #include <thrust/iterator/counting_iterator.h>
@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "../../include/pfbsara.h"
+#include "cg.cuh"
 #include "clean.cuh"
 #include "sara.cuh"
 
@@ -603,5 +604,107 @@ extern "C" int pfbs_clark_run(pfbs_clark* h, const void* dirty, const uint8_t* m
   SCK(cudaMemcpyAsync(model, h->model, ib, back, s));
   SCK(cudaMemcpyAsync(residual, h->R, ib, back, s));
   if (!dev) SCK(cudaStreamSynchronize(s));
+  return PFBG_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Batched conjugate gradients on the PSF-convolution Hessian (cg.cuh)
+// ---------------------------------------------------------------------------
+int pfbg_conv_props(const pfbg_conv* cv, int* precision, int* device, int* nx, int* ny, int* has_kernel);
+
+static const int64_t kCgAlign = 256;
+static int64_t cg_round(int64_t b) { return (b + kCgAlign - 1) / kCgAlign * kCgAlign; }
+static int cg_grid(int64_t npix) { return (int)std::min<int64_t>((npix + CG_THREADS - 1) / CG_THREADS, CG_GMAX); }
+
+extern "C" int64_t pfbs_psf_cg_work_bytes(int32_t nband, int64_t npix) {
+  if (nband < 1 || npix < 1) return -1;
+  return 3 * cg_round((int64_t)nband * npix * 8) + cg_round((int64_t)nband * CG_GMAX * 2 * 8) +
+         cg_round((int64_t)nband * (int64_t)sizeof(CgCtl));
+}
+
+// a device array on `device` (or managed memory)
+static bool cg_on_device(const void* p, int device) {
+  cudaPointerAttributes a{};
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+  return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == device;
+}
+
+extern "C" int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv, const void* const* beam,
+                           const double* eta, const void* rhs, void* x, int64_t npix, double tol, int32_t maxit,
+                           int32_t minit, void* work, int64_t work_bytes, int32_t* iters, double* eps, int32_t* stop,
+                           void* stream) {
+  if (!conv || !beam || !eta || !rhs || !x || !work || !iters || !eps || !stop)
+    return pfbg_fail(PFBG_ERR_ARG, "null argument");
+  if (nband < 1 || nband > 65535) return pfbg_fail(PFBG_ERR_ARG, "nband %d not in 1..65535", nband);
+  if (!(tol >= 0.0) || maxit < 0 || minit < 0) return pfbg_fail(PFBG_ERR_ARG, "need tol >= 0, maxit >= 0, minit >= 0");
+  int ndev = 0;
+  SCK(cudaGetDeviceCount(&ndev));
+  if (device < 0 || device >= ndev) return pfbg_fail(PFBG_ERR_ARG, "device %d out of range", device);
+  int nx0 = 0, ny0 = 0;
+  for (int b = 0; b < nband; ++b) {
+    int prec = 0, dev = 0, nx = 0, ny = 0, hk = 0;
+    if (!conv[b]) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is NULL", b);
+    SRC(pfbg_conv_props(conv[b], &prec, &dev, &nx, &ny, &hk));
+    if (prec != PFBG_F64) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is not fp64", b);
+    if (dev != device) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is on device %d, not %d", b, dev, device);
+    if (!hk) return pfbg_fail(PFBG_ERR_STATE, "convolver %d has no kernel", b);
+    if (b == 0) { nx0 = nx; ny0 = ny; }
+    else if (nx != nx0 || ny != ny0)
+      return pfbg_fail(PFBG_ERR_ARG, "convolver %d images are %d x %d, convolver 0's %d x %d", b, nx, ny, nx0, ny0);
+  }
+  if (npix != (int64_t)nx0 * ny0) return pfbg_fail(PFBG_ERR_ARG, "npix %lld != nx * ny = %lld", (long long)npix, (long long)nx0 * ny0);
+  const int64_t need = pfbs_psf_cg_work_bytes(nband, npix);
+  if (work_bytes < need) return pfbg_fail(PFBG_ERR_ARG, "work holds %lld bytes, %lld needed", (long long)work_bytes, (long long)need);
+  SCK(cudaSetDevice(device));
+  if (!cg_on_device(rhs, device) || !cg_on_device(x, device) || !cg_on_device(work, device))
+    return pfbg_fail(PFBG_ERR_ARG, "rhs, x and work must be device arrays on device %d", device);
+  for (int b = 0; b < nband; ++b)
+    if (beam[b] && !cg_on_device(beam[b], device)) return pfbg_fail(PFBG_ERR_ARG, "beam %d is not a device array on device %d", b, device);
+
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t vb = cg_round((int64_t)nband * npix * 8);
+  double* r = (double*)work;
+  double* p = (double*)((char*)work + vb);
+  double* ap = (double*)((char*)work + 2 * vb);
+  double* part = (double*)((char*)work + 3 * vb);
+  CgCtl* ctl = (CgCtl*)((char*)part + cg_round((int64_t)nband * CG_GMAX * 2 * 8));
+  const int G = cg_grid(npix);
+  const dim3 grd(G, nband);
+  const double* xd = (const double*)x;
+  std::vector<CgCtl> h(nband);
+  auto apply = [&](const double* in, double* out, int b) {
+    return pfbg_conv_apply(conv[b], in + b * npix, beam[b], eta[b], out + b * npix, PFBG_DEVICE_PTRS, stream);
+  };
+  auto read_ctl = [&]() -> int {
+    SCK(cudaMemcpyAsync(h.data(), ctl, (size_t)nband * sizeof(CgCtl), cudaMemcpyDeviceToHost, s));
+    SCK(cudaStreamSynchronize(s));
+    return PFBG_OK;
+  };
+
+  for (int b = 0; b < nband; ++b) SRC(apply(xd, r, b));  // r = A x
+  k_cg_init<<<grd, CG_THREADS, 0, s>>>((const double*)rhs, r, p, npix, part);
+  k_cg_init_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G, tol, maxit, minit);
+  pfbg_count_launch(); pfbg_count_launch();
+  SCK(cudaGetLastError());
+  SRC(read_ctl());
+  for (;;) {
+    bool any = false;
+    for (int b = 0; b < nband; ++b)
+      if (h[b].stop == CG_RUNNING) { any = true; SRC(apply(p, ap, b)); }  // stopped bands skip their convolution
+    if (!any) break;
+    k_cg_dots<<<grd, CG_THREADS, 0, s>>>(ctl, p, ap, npix, part);
+    k_cg_dots_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G);
+    k_cg_update<<<grd, CG_THREADS, 0, s>>>(ctl, (double*)x, r, p, ap, npix, part);
+    k_cg_update_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G, tol, maxit, minit);
+    k_cg_direction<<<grd, CG_THREADS, 0, s>>>(ctl, p, r, npix);
+    for (int t = 0; t < 5; ++t) pfbg_count_launch();
+    SCK(cudaGetLastError());
+    SRC(read_ctl());
+  }
+  for (int b = 0; b < nband; ++b) {
+    iters[b] = h[b].k;
+    eps[b] = h[b].eps;
+    stop[b] = h[b].stop;
+  }
   return PFBG_OK;
 }

@@ -125,6 +125,19 @@ struct GaussMul {
   }
 };
 
+// (Re khat + c) or its reciprocal as a real multiplier: the direct inverse of the Hessian (hess_direct_slice) from the
+// convolver's own spectrum, without a second stored one.  fp64 sum and IEEE quotient, the doubles numpy forms.
+struct ShiftMul {
+  double c;
+  int inverse;
+  template <typename T>
+  __device__ __forceinline__ cx2<T> operator()(const ConvTabs& ct, const cx2<T>* __restrict__ khat, int k, int b0,
+                                               int col) const {
+    const double v = (double)khat[(int64_t)k * ct.nyp + b0 + col].x + c;
+    return {(T)(inverse ? 1.0 / v : v), (T)0};
+  }
+};
+
 // column block: forward along u, multiply by mul(k, b), inverse along u, keep rows < nx
 template <typename T, int C, class Mul>
 __global__ void __launch_bounds__(512)

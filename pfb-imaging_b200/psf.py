@@ -115,6 +115,28 @@ class PsfConvolver:
         _lib.check(self._lib.pfbg_conv_apply(self._h, C.c_void_p(int(x_ptr)), None if beam_ptr is None else C.c_void_p(int(beam_ptr)),
                                              float(eta) if eta else 0.0, C.c_void_p(int(out_ptr)), _lib.DEVICE_PTRS, stream))
 
+    def apply_shifted(self, x, taper=None, c=0.0, inverse=True):
+        """``taper * crop(IFFT(FFT(pad(taper * x)) * (Re khat + c)^(+-1)))`` (fp64, stored spectrum): the direct
+        inverse of :func:`hess_direct_slice` from this convolver's own spectrum (`inverse`: the reciprocal)."""
+        x = np.ascontiguousarray(x, dtype=self.rdt)
+        if x.shape != (self.nx, self.ny):
+            raise ValueError(f"x shape {x.shape} != ({self.nx}, {self.ny})")
+        if taper is not None:
+            taper = np.ascontiguousarray(taper, dtype=self.rdt)
+            if taper.shape != x.shape:
+                raise ValueError("taper shape does not match the image")
+        res = np.empty_like(x)
+        _lib.check(self._lib.pfbg_conv_apply_shifted(self._h, C.c_void_p(x.ctypes.data),
+                                                     None if taper is None else C.c_void_p(taper.ctypes.data), float(c),
+                                                     int(bool(inverse)), C.c_void_p(res.ctypes.data), _lib.HOST_PTRS, None))
+        return res
+
+    def apply_shifted_dev(self, x_ptr, out_ptr, taper_ptr=None, c=0.0, inverse=True, stream=None):
+        """:meth:`apply_shifted` on device pointers (asynchronous on `stream`)."""
+        _lib.check(self._lib.pfbg_conv_apply_shifted(self._h, C.c_void_p(int(x_ptr)),
+                                                     None if taper_ptr is None else C.c_void_p(int(taper_ptr)), float(c),
+                                                     int(bool(inverse)), C.c_void_p(int(out_ptr)), _lib.DEVICE_PTRS, stream))
+
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
             self._lib.pfbg_conv_destroy(self._h)
@@ -343,9 +365,17 @@ class HessTreeRay:
         return self._pool.get_mem()
 
 
+CG_STOP = {1: "converged", 2: "maxit", 3: "stalled", 4: "initial residual zero", 5: "exact"}  # pfbsara.h PFBS_CG_*
+
+
 class HessPSF:
     """Cube-level PSF-convolution Hessian with the reference's constructor and ``dot`` / ``idot(mode="psf")``
-    (operators/hessian.py:251-436); one device convolver per band."""
+    (operators/hessian.py:251-436); one device convolver per band.
+
+    numpy in, numpy out as in the reference.  A float64 CUDA tensor on the convolvers' device, ``(nband, nx, ny)`` or
+    ``(nx, ny)`` when ``nband == 1``, stays on the device: ``dot`` and ``idot`` then return a new ``(nband, nx, ny)``
+    tensor computed on torch's current stream, ``idot(mode="psf")`` solves every band in one batched CG
+    (``pfbs_psf_cg``) and leaves the per-band ``iters`` / ``eps`` / ``stop`` in :attr:`last_idot_info`."""
 
     def __init__(self, nx, ny, abspsf, beam=None, eta=1.0, nthreads=1, cgtol=1e-3, cgmaxit=300, cgverbose=2, cgrf=25,
                  taper_width=32, min_beam=5e-3):
@@ -367,10 +397,13 @@ class HessPSF:
         self.min_beam = min_beam
         self.conv = [PsfConvolver(nx, ny, self.nx_psf, self.ny_psf, dtype=np.float64).set_kernel(abspsf[b])
                      for b in range(self.nband)]
+        self._dev_consts = None  # device copies of the beams and the taper, uploaded on the first device call
+        self.last_idot_info = None
 
     def set_beam(self, beam):
         assert beam.shape == (self.nband, self.nx, self.ny)
         self.beam = beam
+        self._dev_consts = None
 
     def _cube(self, x):
         if x.ndim == 3:
@@ -379,7 +412,86 @@ class HessPSF:
             return x[None]
         raise ValueError("Unsupported number of input dimensions")
 
+    def _dev_input(self, x):
+        """The (nband, nx, ny) contiguous view of a device input; raises before anything is launched."""
+        import torch
+
+        if x.dtype != torch.float64:
+            raise TypeError(f"device input must be float64, got {x.dtype}")
+        if x.dim() == 2 and self.nband == 1:
+            x = x[None]
+        if tuple(x.shape) != (self.nband, self.nx, self.ny):
+            raise ValueError(f"input shape {tuple(x.shape)} does not match ({self.nband}, {self.nx}, {self.ny})")
+        if x.device.index != self.conv[0].device:
+            raise ValueError(f"input is on {x.device}, the operator on cuda:{self.conv[0].device}")
+        return x.contiguous()
+
+    def _consts(self, device):
+        import torch
+
+        if self._dev_consts is None:
+            up = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).to(device)  # noqa: E731
+            self._dev_consts = dict(beam=[None if b is None else up(b) for b in self.beam], taper=up(self.taperxy))
+        return self._dev_consts
+
+    def _direct_dev(self, xt, out, consts, stream):
+        """Device :meth:`_direct` of every band: the same shifted spectrum from each band's own convolver."""
+        c0 = np.sqrt(self.nx * self.ny)
+        for b in range(self.nband):
+            self.conv[b].apply_shifted_dev(xt[b].data_ptr(), out[b].data_ptr(), consts["taper"].data_ptr(),
+                                           c=float(self.eta[b]) * c0, inverse=True, stream=stream)
+
+    def _dot_dev(self, x):
+        import torch
+
+        xt = self._dev_input(x)
+        consts = self._consts(xt.device)
+        s = torch.cuda.current_stream(xt.device).cuda_stream
+        out = torch.empty_like(xt)
+        for b in range(self.nband):
+            bm = consts["beam"][b]
+            self.conv[b].apply_dev(xt[b].data_ptr(), out[b].data_ptr(), None if bm is None else bm.data_ptr(),
+                                   float(self.eta[b]), s)
+        return out
+
+    def _idot_dev(self, x, mode, x0, init_x0):
+        import torch
+
+        xt = self._dev_input(x)
+        if mode not in ("direct", "psf"):
+            raise ValueError(f"Unknown mode {mode}")
+        consts = self._consts(xt.device)
+        s = torch.cuda.current_stream(xt.device).cuda_stream
+        if mode == "direct":
+            out = torch.empty_like(xt)
+            self._direct_dev(xt, out, consts, s)
+            for b, bm in enumerate(consts["beam"]):
+                if bm is not None:
+                    mask = (out[b] > 0) & (bm > self.min_beam)
+                    out[b] = torch.where(mask, out[b] / (bm * bm), out[b])
+            return out
+        # the starting point of the host path: the direct estimate, or zero (a passed x0 is not used, as there)
+        if x0 is None and init_x0:
+            sol = torch.empty_like(xt)
+            self._direct_dev(xt, sol, consts, s)
+        else:
+            sol = torch.zeros_like(xt)
+        lib, nb, npix = self.conv[0]._lib, self.nband, self.nx * self.ny
+        nbytes = int(lib.pfbs_psf_cg_work_bytes(nb, npix))
+        work = torch.empty(nbytes, dtype=torch.uint8, device=xt.device)
+        iters, eps, stop = (C.c_int32 * nb)(), (C.c_double * nb)(), (C.c_int32 * nb)()
+        _lib.check(lib.pfbs_psf_cg(self.conv[0].device, nb, (C.c_void_p * nb)(*[c._h.value for c in self.conv]),
+                                   (C.c_void_p * nb)(*[None if bm is None else bm.data_ptr() for bm in consts["beam"]]),
+                                   (C.c_double * nb)(*[float(e) for e in self.eta]), C.c_void_p(xt.data_ptr()),
+                                   C.c_void_p(sol.data_ptr()), npix, float(self.cgtol), int(self.cgmaxit), 3,
+                                   C.c_void_p(work.data_ptr()), nbytes, iters, eps, stop, s))
+        self.last_idot_info = dict(iters=np.array(iters[:], dtype=np.int64), eps=np.array(eps[:]),
+                                   stop=[CG_STOP.get(v, str(v)) for v in stop])
+        return sol
+
     def dot(self, x):
+        if getattr(x, "is_cuda", False):
+            return self._dot_dev(x)
         xt = self._cube(x)
         if xt.shape != (self.nband, self.nx, self.ny):
             raise AssertionError("input shape does not match the operator")
@@ -403,6 +515,8 @@ class HessPSF:
         not used there either, hessian.py:372-390)."""
         from .solvers import pcg
 
+        if getattr(x, "is_cuda", False):
+            return self._idot_dev(x, mode, x0, init_x0)
         xt = self._cube(x)
         if xt.shape != (self.nband, self.nx, self.ny):
             raise AssertionError("input shape does not match the operator")
@@ -433,6 +547,7 @@ class HessPSF:
     def close(self):
         for c in self.conv:
             c.close()
+        self._dev_consts = None
 
 
 class PsfGradient:
