@@ -52,13 +52,20 @@ def kernel_ft(xi, W, beta):
 # --------------------------------------------------------------------------
 # kernel 1 oracle: bit-exact coordinates, first-cell indices, sort keys
 # --------------------------------------------------------------------------
-def bin_indices(plan, uvw, freq, mask=None):
+def bin_indices(plan, uvw, freq, mask=None, row_offsets=None, snap_w0=None, snap_np=None):
     """Per-visibility grid coordinates and the sorted bucket order.
 
     Returns a dict with, for the *active* samples (mask != 0) in row-major
     (row, chan) order: flat index `idx`, `iu0, iv0, ip0` (int32; first touched
     cell per axis, iu0/iv0 may be negative = periodic wrap), `key` (uint64) and
     `order` (stable argsort of key), plus `gu, gv, gw` (fp64 grid coordinates).
+
+    Batched snapshots (`row_offsets`, `snap_w0`, `snap_np`, as given to
+    ``pfbg_plan_set_batch`` / ``pfbg_bind_vis_batch``; ``plan.nplanes`` is the
+    total): rows [row_offsets[s], row_offsets[s+1]) take their plane from
+    snapshot s's own w0, are clamped to its own snap_np[s] planes and are
+    shifted by its plane base (the sum of the plane counts before it);
+    `snap` holds each sample's snapshot.
     """
     uvw = np.asarray(uvw, dtype=np.float64)
     freq = np.asarray(freq, dtype=np.float64)
@@ -85,13 +92,27 @@ def bin_indices(plan, uvw, freq, mask=None):
 
     gu, iu0 = coord(ut, plan.pixsize_x, plan.nu)
     gv, iv0 = coord(vt, plan.pixsize_y, plan.nv)
+    if row_offsets is None:
+        w0 = plan.w0
+        hi = plan.nplanes - W
+        pbase = 0
+        snap = np.zeros((nrow, 1), dtype=np.int64)
+    else:
+        ro = np.asarray(row_offsets, dtype=np.int64)
+        npl = np.asarray(snap_np, dtype=np.int64)
+        snap = np.repeat(np.arange(ro.size - 1), np.diff(ro))[:, None]
+        w0 = np.asarray(snap_w0, dtype=np.float64)[snap]
+        hi = npl[snap] - W
+        pbase = np.concatenate([[0], np.cumsum(npl)[:-1]])[snap]
     if plan.do_wgridding:
-        gw = (wt - plan.w0) / plan.dw
+        gw = (wt - w0) / plan.dw
         ip0 = np.floor(gw - 0.5 * W).astype(np.int64) + 1
-        ip0 = np.clip(ip0, -int(getattr(plan, "pmirror", 0)), plan.nplanes - W)
+        ip0 = np.clip(ip0, -int(getattr(plan, "pmirror", 0)), hi)
     else:
         gw = np.zeros_like(wt)
         ip0 = np.zeros(wt.shape, dtype=np.int64)
+    gw = gw + pbase  # absolute plane units (exact: small integers), as the device adds them
+    ip0 = ip0 + pbase
 
     if mask is None:
         active = np.ones((nrow, nchan), dtype=bool)
@@ -113,6 +134,7 @@ def bin_indices(plan, uvw, freq, mask=None):
         idx=idx.astype(np.int64), iu0=iu0.astype(np.int32), iv0=iv0.astype(np.int32),
         ip0=ip0.astype(np.int32), key=key, order=order.astype(np.int64), gu=gu, gv=gv, gw=gw,
         ut=ut.ravel()[idx], vt=vt.ravel()[idx], wt=wt.ravel()[idx], conj=fold.ravel()[idx],
+        snap=np.broadcast_to(snap, (nrow, nchan)).ravel()[idx],
     )
 
 

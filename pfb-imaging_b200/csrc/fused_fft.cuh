@@ -37,7 +37,11 @@ k_rows_fwd(GParams p, FusedTabs ft, const T* __restrict__ x, const T* __restrict
   __syncthreads();
   const double wq = ft.plane_w ? ft.plane_w[q] : p.w0 + q * p.dw;
   const int64_t row = (int64_t)i * p.ny;
-  if (ft.plane_img) x += (int64_t)ft.plane_img[q] * p.nx * p.ny;  // this plane's snapshot image
+  if (ft.plane_img) {  // this plane's snapshot image and beam
+    const int64_t off = (int64_t)ft.plane_img[q] * p.nx * p.ny;
+    x += off;
+    if (beam) beam += off;
+  }
   const bool vec_ok = (p.ny & 7) == 0 &&
                       (((uintptr_t)x | (uintptr_t)corr | (uintptr_t)beam) & 15) == 0;  // caller-owned device pointers
   if (vec_ok) {
@@ -338,14 +342,15 @@ template <typename T>
 __global__ void k_finish_image(int64_t npix, int64_t npix_img, const double* __restrict__ acc,
                                const double* __restrict__ acc2, const T* __restrict__ corr, const T* __restrict__ beam,
                                const T* __restrict__ xin, double inv_wsum, double eta, T* __restrict__ out) {
-  // npix = nbatch * npix_img: the images of a batch share the correction (and beam) of their common geometry
+  // npix = nbatch * npix_img: the images of a batch share the correction of their common geometry; every snapshot
+  // has its own beam
   int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= npix) return;
   const int64_t kc = npix == npix_img ? k : k % npix_img;
   double a = acc[k];
   if (acc2) a += acc2[k];
   double r = a * (double)corr[kc];
-  if (beam) r *= (double)beam[kc];
+  if (beam) r *= (double)beam[k];
   r *= inv_wsum;
   if (xin) r += eta * (double)xin[k];
   out[k] = (T)r;

@@ -44,18 +44,22 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
   const int64_t row = (int64_t)i * p.ny;
   const float* xa = x;
   const float* xb = x;
-  if (ft.plane_img) {  // batched snapshots: every plane has its own image
-    xa += (int64_t)ft.plane_img[qa] * p.nx * p.ny;
-    xb += (int64_t)ft.plane_img[qb] * p.nx * p.ny;
+  const float* ba = beam;
+  const float* bb = beam;
+  if (ft.plane_img) {  // batched snapshots: every plane has its own image and beam
+    const int64_t oa = (int64_t)ft.plane_img[qa] * p.nx * p.ny, ob = (int64_t)ft.plane_img[qb] * p.nx * p.ny;
+    xa += oa;
+    xb += ob;
+    if (beam) { ba += oa; bb += ob; }
   }
-  const bool same_x = xa == xb;
+  const bool same_x = xa == xb;  // (then ba == bb too)
   const float mb = two ? 1.f : 0.f;
   const bool vec_ok = (p.ny & 7) == 0 && (((uintptr_t)x | (uintptr_t)corr | (uintptr_t)beam) & 15) == 0;
   if (vec_ok) {
     // 4 consecutive pixels per step (hy % 4 == 0, so a group never straddles the wrap), two steps in flight
     const int ng = p.ny >> 2;
     for (int g0 = tid; g0 < ng; g0 += 2 * nthr) {
-      float xv[2][4], yv[2][4], cv[2][4], bv[2][4];
+      float xv[2][4], yv[2][4], cv[2][4], bv[2][4], bw[2][4];
       double nuv[2][4];
       int pv[2][4];
 #pragma unroll
@@ -66,7 +70,10 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
           load4(xa + row + j, xv[u]);
           if (!same_x) load4(xb + row + j, yv[u]);
           load4(corr + row + j, cv[u]);
-          if (beam) load4(beam + row + j, bv[u]);
+          if (beam) {
+            load4(ba + row + j, bv[u]);
+            if (!same_x) load4(bb + row + j, bw[u]);
+          }
           if (p.do_wgridding) load4(ft.nutab + row + j, nuv[u]);
           const int jp = j - hy;
           load4(pos_v + (jp < 0 ? jp + nv : jp), pv[u]);
@@ -77,10 +84,13 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
         if (g0 + u * nthr < ng) {
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
-            float cb = cv[u][e];
-            if (beam) cb *= bv[u][e];
+            float cb = cv[u][e], cbb = cb;
+            if (beam) {
+              cb *= bv[u][e];
+              cbb = same_x ? cb : cbb * bw[u][e];
+            }
             const float va = xv[u][e] * cb;
-            const float vb = (same_x ? xv[u][e] : yv[u][e]) * cb * mb;
+            const float vb = (same_x ? xv[u][e] : yv[u][e]) * cbb * mb;
             if (va == 0.f && vb == 0.f) continue;  // the buffer is zero already
             float4 v = make_float4(va, vb, 0.f, 0.f);
             if (p.do_wgridding) {
@@ -97,9 +107,8 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
   } else {
     for (int j = tid; j < p.ny; j += nthr) {
       const int64_t pix = row + j;
-      float cb = corr[pix];
-      if (beam) cb *= beam[pix];
-      const float va = xa[pix] * cb, vb = xb[pix] * cb * mb;
+      const float c = corr[pix];
+      const float va = xa[pix] * (beam ? c * ba[pix] : c), vb = xb[pix] * (beam ? c * bb[pix] : c) * mb;
       float4 v = make_float4(va, vb, 0.f, 0.f);
       if (p.do_wgridding) {
         float ca, sa, c2, s2;

@@ -1,7 +1,8 @@
 """GPU: batched snapshots (BASELINE config 5, `pfb hci`): many small images of one geometry through ONE bin / sort
 and one launch of every kernel (pfbg_plan_set_batch / pfbg_bind_vis_batch).  Every snapshot is checked against the
 explicit DFT with the settings of the reference's snapshot imager (utils/stokes2im.py:635-683: divide_by_n=True,
-sigma_min = min_padding = 2) and against the one-shot call on that snapshot alone."""
+sigma_min = min_padding = 2) and against the one-shot call on that snapshot alone.  These are toy sizes (5 snapshots
+of 64 x 48); tests/test_gpu_batch_production.py runs the benchmark's production shape (256 snapshots of 512^2)."""
 import numpy as np
 import pytest
 

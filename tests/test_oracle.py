@@ -1,4 +1,5 @@
 """CPU: the oracle against the reference's own known-answer vectors and identities."""
+import dataclasses
 import os
 
 import numpy as np
@@ -88,6 +89,37 @@ def test_bin_indices_invariants():
     std = wg.bin_indices(_plan(p, 1e-5, mirror=False), p["uvw"], p["freq"], p["mask"])
     assert std["ip0"].min() >= 0
     assert (np.diff(b["key"][b["order"]].astype(np.int64)) >= 0).all()
+
+
+def test_bin_indices_of_a_batch():
+    """Batched snapshots: each sample's plane comes from its own snapshot's w0 and plane block.  A batch of one
+    snapshot whose block is the plan's own stack bins like the plan; in a batch of three, snapshot s's samples bin
+    like the one-snapshot plan of its block, shifted by the planes before it."""
+    from pfb_imaging_b200.plan import make_batch_plan
+
+    ps = [small_problem(nrow=120 + 30 * s, seed=s, wscale=1.0 + 8.0 * s * s) for s in range(3)]
+    freq, cell = ps[0]["freq"], ps[0]["cell"]
+    wr = [w_range(p["uvw"], freq) for p in ps]
+    plan, w0, npl = make_batch_plan(wr, nx=64, ny=48, pixsize_x=cell, pixsize_y=cell, epsilon=1e-5, flip_v=True)
+    assert len(set(npl.tolist())) > 1
+    plan.nplanes = int(npl.sum())
+    uvw = np.concatenate([p["uvw"] for p in ps])
+    mask = np.concatenate([p["mask"] for p in ps])
+    ro = np.concatenate([[0], np.cumsum([p["uvw"].shape[0] for p in ps])])
+    b = wg.bin_indices(plan, uvw, freq, mask, row_offsets=ro, snap_w0=w0, snap_np=npl)
+    pbase = np.concatenate([[0], np.cumsum(npl)[:-1]])
+    for s, p in enumerate(ps):
+        one = dataclasses.replace(plan, w0=float(w0[s]), nplanes=int(npl[s]))
+        ref = wg.bin_indices(one, p["uvw"], freq, p["mask"])
+        sel = b["snap"] == s
+        assert np.array_equal(b["ip0"][sel], ref["ip0"] + pbase[s])
+        assert np.array_equal(b["iu0"][sel], ref["iu0"]) and np.array_equal(b["iv0"][sel], ref["iv0"])
+        assert b["ip0"][sel].min() >= pbase[s] and b["ip0"][sel].max() + plan.W <= pbase[s] + npl[s]
+    solo = wg.bin_indices(plan, uvw, freq, mask, row_offsets=[0, uvw.shape[0]], snap_w0=[plan.w0],
+                          snap_np=[plan.nplanes])
+    whole = wg.bin_indices(plan, uvw, freq, mask)
+    for k in ("iu0", "iv0", "ip0", "key", "order"):
+        assert np.array_equal(solo[k], whole[k]), k
 
 
 # --- weighting -------------------------------------------------------------
