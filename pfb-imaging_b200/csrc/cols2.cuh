@@ -26,7 +26,6 @@
 #include "cols2_api.h"
 
 #define COLS2_THREADS 384      // radix-16 stages, 128 registers per thread
-#define COLS2_THREADS_R8 768   // radix-8 stages (Cols2Args.du = the radix-8 factorisation): <= 85 registers, 24 warps
 #define COLS2_BOX_BIG 256
 #define COLS2_BOX_SMALL 32
 
@@ -37,9 +36,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
 }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   asm volatile(
@@ -61,36 +57,15 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
       : "memory");
 }
 
-__device__ __forceinline__ void tma_load_2d_hint(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar,
-                                                 uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3}], "
-      "[%4], %5;" ::"r"(smem_u32(dst)),
-      "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar)), "l"(policy)
-      : "memory");
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-
 // rows [r0, r1) of the four columns starting at column `col` of stack row block `rowbase` -> buffer rows [r0, r1)
 __device__ __forceinline__ void cols2_load_rows(float4* buf, const CUtensorMap* mbig, const CUtensorMap* msmall, int col,
-                                                int rowbase, int r0, int r1, uint64_t* bar, bool keep) {
+                                                int rowbase, int r0, int r1, uint64_t* bar) {
   int r = r0;
-  if (keep) {  // the neighbouring column pair (next item of this CTA) lives in the same 32-byte sectors
-    const uint64_t pol = l2_policy_evict_last();
-    for (; r + COLS2_BOX_BIG <= r1; r += COLS2_BOX_BIG) tma_load_2d_hint(buf + 2 * r, mbig, 2 * col, rowbase + r, bar, pol);
-    for (; r < r1; r += COLS2_BOX_SMALL) tma_load_2d_hint(buf + 2 * r, msmall, 2 * col, rowbase + r, bar, pol);
-    return;
-  }
   for (; r + COLS2_BOX_BIG <= r1; r += COLS2_BOX_BIG) tma_load_2d(buf + 2 * r, mbig, 2 * col, rowbase + r, bar);
   for (; r < r1; r += COLS2_BOX_SMALL) tma_load_2d(buf + 2 * r, msmall, 2 * col, rowbase + r, bar);
 }
 
-template <bool R8>
-__global__ void __launch_bounds__(R8 ? COLS2_THREADS_R8 : COLS2_THREADS, 1)
+__global__ void __launch_bounds__(COLS2_THREADS, 1)
 k_cols2(const __grid_constant__ CUtensorMap mbig, const __grid_constant__ CUtensorMap msmall,
         const __grid_constant__ Cols2Args a, float2* __restrict__ out) {
   extern __shared__ __align__(1024) unsigned char smem_raw1k[];
@@ -100,7 +75,7 @@ k_cols2(const __grid_constant__ CUtensorMap mbig, const __grid_constant__ CUtens
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + (size_t)nu * 32);
   float2* twtab = reinterpret_cast<float2*>(bar + 8);                                    // two-level twiddle table
   unsigned short* pos16 = reinterpret_cast<unsigned short*>(twtab + p2_tw_entries(nu));  // k -> position, nu entries
-  constexpr int NTHR = R8 ? COLS2_THREADS_R8 : COLS2_THREADS;
+  constexpr int NTHR = COLS2_THREADS;
   const int tid = threadIdx.x;
   const P2Tw tw = p2_tw_fill(twtab, a.tw_u, nu, tid, NTHR);
   for (int k = tid; k < nu; k += NTHR) pos16[k] = (unsigned short)a.pos_u[k];
@@ -109,16 +84,12 @@ k_cols2(const __grid_constant__ CUtensorMap mbig, const __grid_constant__ CUtens
     fence_proxy_async();
   }
   __syncthreads();
-  // contiguous range of (plane, column block) items of this CTA
+  // work items: (plane, column block)
   const int nblk = a.b_len >> 2;
   const int64_t nitems = (int64_t)a.nq * nblk;
   // items are dealt round-robin: neighbouring column blocks (which share 64-byte DRAM atoms) are loaded by
-  // neighbouring CTAs at about the same time, so one DRAM access serves both (PFBG_COLS2_DEBUG=16: contiguous
-  // ranges per CTA instead — measured 2.7x the DRAM reads, the L2 does not keep the neighbour for the next item)
-  const bool contiguous = (a.debug & 16) != 0;
-  const int64_t it0 = contiguous ? nitems * blockIdx.x / gridDim.x : blockIdx.x;
-  const int64_t it1 = contiguous ? nitems * (blockIdx.x + 1) / gridDim.x : nitems;
-  const int64_t istep = contiguous ? 1 : gridDim.x;
+  // neighbouring CTAs at about the same time, so one DRAM access serves both (contiguous ranges per CTA were
+  // measured at 2.7x the DRAM reads: the L2 does not keep the neighbour for the next item)
   uint32_t phase = 0;
   // loaded row segments [s0a, s1a) and [s0b, s1b); everything else is zero
   int s0a, s1a, s0b, s1b;
@@ -130,28 +101,19 @@ k_cols2(const __grid_constant__ CUtensorMap mbig, const __grid_constant__ CUtens
     else { s0a = a.a_lo; s1a = nu; s0b = 0; s1b = end - nu; }
   }
   const uint32_t tx_bytes = (uint32_t)((s1a - s0a) + (s1b - s0b)) * 32u;
-  const bool keep = (a.debug & 8) != 0;
   const int inmode = a.inverse ? P2_IN_AOS_SWAP : P2_IN_AOS;
   const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
 
-  for (int64_t it = it0; it < it1; it += istep) {
+  for (int64_t it = blockIdx.x; it < nitems; it += gridDim.x) {
     const int q = (int)(it / nblk), j = (int)(it - (int64_t)q * nblk);
     int col = a.b_lo + 4 * j;
     if (col >= a.nv) col -= a.nv;
     // ---- fill: the copy engine brings the data rows, the threads zero the rest (disjoint rows)
-    if (a.debug & 1) {
-      // debugging aid (PFBG_COLS2_DEBUG=1): plain copies instead of the TMA unit
-      const float2* g = a.dbg_stack + ((int64_t)(a.q0 + q - a.slot0) * nu) * a.nv + col;
-      for (int e = s0a * 2 + tid; e < s1a * 2; e += NTHR)
-        s[e] = *reinterpret_cast<const float4*>(g + (int64_t)(e >> 1) * a.nv + 2 * (e & 1));
-      for (int e = s0b * 2 + tid; e < s1b * 2; e += NTHR)
-        s[e] = *reinterpret_cast<const float4*>(g + (int64_t)(e >> 1) * a.nv + 2 * (e & 1));
-      if (tid == 0) mbar_arrive(bar);
-    } else if (tid == 0) {
+    if (tid == 0) {
       const int rowbase = (a.q0 + q - a.slot0) * nu;
       mbar_expect_tx(bar, tx_bytes);
-      cols2_load_rows(s, &mbig, &msmall, col, rowbase, s0a, s1a, bar, keep);
-      cols2_load_rows(s, &mbig, &msmall, col, rowbase, s0b, s1b, bar, keep);
+      cols2_load_rows(s, &mbig, &msmall, col, rowbase, s0a, s1a, bar);
+      cols2_load_rows(s, &mbig, &msmall, col, rowbase, s0b, s1b, bar);
     }
     if (s1b > s0b) {  // two segments: the gap between them ([s1a, s0b) forward, [s1b, s0a) inverse)
       const int z0 = !a.inverse ? s1a : s1b, z1 = !a.inverse ? s0b : s0a;
@@ -163,12 +125,10 @@ k_cols2(const __grid_constant__ CUtensorMap mbig, const __grid_constant__ CUtens
     mbar_wait(bar, phase);
     phase ^= 1;
     __syncthreads();  // everybody's zero rows are in place
-    p2_fft_dif<2, R8 ? 8 : 16>(s, tw, a.du, inmode, tid, NTHR);
+    p2_fft_dif<2>(s, tw, a.du, inmode, tid, NTHR);
     // ---- write-back: one 32-byte sector per row
     float2* go = out + (int64_t)(a.q0 + q) * nu * a.nv + col;  // `out` is biased: logical plane q at out + q nu nv
-    if (a.debug & 2) {
-      // debugging aid: no write-back
-    } else if (!a.inverse) {
+    if (!a.inverse) {
 #pragma unroll 4
       for (int t = tid; t < a.a_len; t += NTHR) {  // rows of the active window
         int k = a.a_lo + t;

@@ -12,8 +12,6 @@ struct Cols2Args {
   int q0, nq;                // logical planes [q0, q0 + nq)
   int slot0;                 // logical plane stored in slot 0 of the local stack (tensor-map row = (q - slot0) nu + a)
   int inverse;
-  int debug;                 // PFBG_COLS2_DEBUG bits: 1 = manual copy instead of TMA, 2 = no write-back, 4 = 128-byte hardware swizzle in the map (faults)
-  const float2* dbg_stack;
 };
 
 // true when the pair-engine column kernels can serve this geometry (fp32 only): two nu x 16-byte buffers fit shared
@@ -23,16 +21,17 @@ bool cols2_supported(int nu, int nv, int nx, const FftDesc& du);
 // `stack_planes` planes: what the tensor maps describe and the loads read), `out` = where the result rows go,
 // biased so that logical plane q sits at out + q nu nv (the local stack, or a peer-mapped one).
 // Returns cudaSuccess or the failing error; *what names the failing step.
-cudaError_t cols2_launch(const Cols2Args& a, bool r8, const float2* stack, int stack_planes, float2* out,
-                         cudaStream_t s, const char** what);
+cudaError_t cols2_launch(const Cols2Args& a, const float2* stack, int stack_planes, float2* out, cudaStream_t s,
+                         const char** what);
 // engine unit test: `batch` CTAs, each transforming 2 NP interleaved length-n arrays (see k_fft2_debug)
 cudaError_t fft2_debug_launch(const FftDesc& d, int np, const float2* tw, const int* rev, const float2* in, float2* out,
                               int batch, int inverse, int aos);
 
 // Row passes on the pair engine (rows2.cuh, fp32): the same image row of two neighbouring planes per CTA.
-// `stack_biased`: logical plane q at stack_biased + q nu nv.  Planes [ft.q0, ft.q0 + nq).
+// `stack_biased`: logical plane q at stack_biased + q nu nv.  Planes [ft.q0, ft.q0 + nq); nq must be even
+// (cudaErrorInvalidValue otherwise).
 bool rows2_supported(int nv);
-cudaError_t rows2_fwd_launch(const GParams& g, const FusedTabs& ft, int nq, bool fast, bool r8, const float* x,
-                             const float* beam, const float* corr, float2* stack_biased, cudaStream_t s);
-cudaError_t rows2_inv_launch(const GParams& g, const FusedTabs& ft, int nq, bool fast, bool r8,
-                             const float2* stack_biased, double* accimg, cudaStream_t s);
+cudaError_t rows2_fwd_launch(const GParams& g, const FusedTabs& ft, int nq, bool fast, const float* x, const float* beam,
+                             const float* corr, float2* stack_biased, cudaStream_t s);
+cudaError_t rows2_inv_launch(const GParams& g, const FusedTabs& ft, int nq, bool fast, const float2* stack_biased,
+                             double* accimg, cudaStream_t s);

@@ -2,7 +2,6 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <atomic>
-#include <cstdlib>
 #include <mutex>
 #include "cols2.cuh"
 #include "rows2.cuh"
@@ -38,30 +37,25 @@ bool cols2_supported(int nu, int nv, int nx, const FftDesc& du) {
 }
 
 // (2 nv floats, rows) view of the plane stack, boxes of 8 floats (four columns = one 32-byte sector per row) x `box_rows` rows, dense in shared
-// memory (a 128-byte hardware swizzle of 16-byte-wide boxes faults on B200; the first FFT stage swizzles instead)
-static bool encode_map(CUtensorMap* m, const float2* stack, int nv, int64_t rows, int box_rows, bool swz = false) {
+// memory (a 128-byte hardware swizzle of 16-byte-wide boxes faults on B200, so the first FFT stage swizzles instead)
+static bool encode_map(CUtensorMap* m, const float2* stack, int nv, int64_t rows, int box_rows) {
   const cuuint64_t gdim[2] = {(cuuint64_t)2 * nv, (cuuint64_t)rows};
   const cuuint64_t gstride[1] = {(cuuint64_t)nv * 8};
   const cuuint32_t box[2] = {8, (cuuint32_t)box_rows};
   const cuuint32_t estr[2] = {1, 1};
   return encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)stack, gdim, gstride, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, swz ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-cudaError_t cols2_launch(const Cols2Args& a_in, bool r8, const float2* stack, int stack_planes, float2* out,
-                         cudaStream_t s, const char** what) {
+cudaError_t cols2_launch(const Cols2Args& a, const float2* stack, int stack_planes, float2* out, cudaStream_t s,
+                         const char** what) {
   static std::atomic<int> attr_done{0};
-  Cols2Args a = a_in;
-  const char* dbg = getenv("PFBG_COLS2_DEBUG");
-  a.debug = dbg ? atoi(dbg) : 0;
-  a.dbg_stack = stack;
   *what = "";
   if (a.nq <= 0 || a.b_len <= 0) return cudaSuccess;
   alignas(64) CUtensorMap mbig, msmall;
   const int64_t rows = (int64_t)stack_planes * a.nu;
-  if (!encode_map(&mbig, stack, a.nv, rows, COLS2_BOX_BIG, (a.debug & 4) != 0) ||
-      !encode_map(&msmall, stack, a.nv, rows, COLS2_BOX_SMALL, (a.debug & 4) != 0)) {
+  if (!encode_map(&mbig, stack, a.nv, rows, COLS2_BOX_BIG) || !encode_map(&msmall, stack, a.nv, rows, COLS2_BOX_SMALL)) {
     *what = "cuTensorMapEncodeTiled";
     return cudaErrorInvalidValue;
   }
@@ -70,15 +64,13 @@ cudaError_t cols2_launch(const Cols2Args& a_in, bool r8, const float2* stack, in
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
   if (e != cudaSuccess) { *what = "device query"; return e; }
   if (!(attr_done.load() & (1 << (dev & 31)))) {
-    e = cudaFuncSetAttribute(k_cols2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCols2MaxSmem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_cols2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCols2MaxSmem);
+    e = cudaFuncSetAttribute(k_cols2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCols2MaxSmem);
     if (e != cudaSuccess) { *what = "cudaFuncSetAttribute(k_cols2)"; return e; }
     attr_done.fetch_or(1 << (dev & 31));
   }
   const int64_t nitems = (int64_t)a.nq * (a.b_len / 4);
   const int grid = (int)(nitems < nsm ? nitems : nsm);
-  if (r8) k_cols2<true><<<grid, COLS2_THREADS_R8, cols2_smem(a.nu), s>>>(mbig, msmall, a, out);
-  else k_cols2<false><<<grid, COLS2_THREADS, cols2_smem(a.nu), s>>>(mbig, msmall, a, out);
+  k_cols2<<<grid, COLS2_THREADS, cols2_smem(a.nu), s>>>(mbig, msmall, a, out);
   *what = "k_cols2 launch";
   return cudaGetLastError();
 }
@@ -140,10 +132,9 @@ cudaError_t fft2_debug_launch(const FftDesc& d, int np, const float2* tw, const 
 
 // ---- row passes on the pair engine (rows2.cuh) --------------------------------------------------------------------
 static size_t rows2_smem(int nv) { return (size_t)nv * 16 + (size_t)((nv + 63) / 64 + 64) * 8; }
-static int rows2_threads(int nv, bool r8) {
-  int t = ((nv / (r8 ? 8 : 16) + 1) / 2 + 31) & ~31;  // two butterflies of the widest stage per thread
-  const int cap = r8 ? ROWS2_THREADS_R8 : ROWS2_THREADS;
-  return t < 32 ? 32 : (t > cap ? cap : t);
+static int rows2_threads(int nv) {
+  const int t = ((nv / 16 + 1) / 2 + 31) & ~31;  // two butterflies of the widest stage per thread
+  return t < 32 ? 32 : (t > ROWS2_THREADS ? ROWS2_THREADS : t);
 }
 
 bool rows2_supported(int nv) { return nv % 32 == 0 && rows2_smem(nv) <= kCols2MaxSmem; }
@@ -155,52 +146,40 @@ static cudaError_t rows2_attr(K kern) {
   return e;
 }
 
-cudaError_t rows2_fwd_launch(const GParams& g, const FusedTabs& ft, int nq, bool fast, bool r8, const float* x,
-                             const float* beam, const float* corr, float2* stack_biased, cudaStream_t s) {
+cudaError_t rows2_fwd_launch(const GParams& g, const FusedTabs& ft, int nq, bool fast, const float* x, const float* beam,
+                             const float* corr, float2* stack_biased, cudaStream_t s) {
   static std::atomic<int> attr_done{0};
+  if (nq & 1) return cudaErrorInvalidValue;  // every CTA transforms a full pair of planes
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return e;
   if (!(attr_done.load() & (1 << (dev & 31)))) {
-    if ((e = rows2_attr(k_rows2_fwd<false, false>)) != cudaSuccess || (e = rows2_attr(k_rows2_fwd<true, false>)) != cudaSuccess ||
-        (e = rows2_attr(k_rows2_fwd<false, true>)) != cudaSuccess || (e = rows2_attr(k_rows2_fwd<true, true>)) != cudaSuccess)
-      return e;
+    if ((e = rows2_attr(k_rows2_fwd<false>)) != cudaSuccess || (e = rows2_attr(k_rows2_fwd<true>)) != cudaSuccess) return e;
     attr_done.fetch_or(1 << (dev & 31));
   }
-  const dim3 grid((nq + 1) / 2, g.nx);
-  const int nt = rows2_threads(g.nv, r8);
+  const dim3 grid(nq / 2, g.nx);
+  const int nt = rows2_threads(g.nv);
   const size_t sm = rows2_smem(g.nv);
-  if (r8) {
-    if (fast) k_rows2_fwd<true, true><<<grid, nt, sm, s>>>(g, ft, nq, x, beam, corr, stack_biased);
-    else k_rows2_fwd<false, true><<<grid, nt, sm, s>>>(g, ft, nq, x, beam, corr, stack_biased);
-  } else {
-    if (fast) k_rows2_fwd<true, false><<<grid, nt, sm, s>>>(g, ft, nq, x, beam, corr, stack_biased);
-    else k_rows2_fwd<false, false><<<grid, nt, sm, s>>>(g, ft, nq, x, beam, corr, stack_biased);
-  }
+  if (fast) k_rows2_fwd<true><<<grid, nt, sm, s>>>(g, ft, x, beam, corr, stack_biased);
+  else k_rows2_fwd<false><<<grid, nt, sm, s>>>(g, ft, x, beam, corr, stack_biased);
   return cudaGetLastError();
 }
 
-cudaError_t rows2_inv_launch(const GParams& g, const FusedTabs& ft, int nq, bool fast, bool r8,
-                             const float2* stack_biased, double* accimg, cudaStream_t s) {
+cudaError_t rows2_inv_launch(const GParams& g, const FusedTabs& ft, int nq, bool fast, const float2* stack_biased,
+                             double* accimg, cudaStream_t s) {
   static std::atomic<int> attr_done{0};
+  if (nq & 1) return cudaErrorInvalidValue;  // every CTA transforms a full pair of planes
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return e;
   if (!(attr_done.load() & (1 << (dev & 31)))) {
-    if ((e = rows2_attr(k_rows2_inv<false, false>)) != cudaSuccess || (e = rows2_attr(k_rows2_inv<true, false>)) != cudaSuccess ||
-        (e = rows2_attr(k_rows2_inv<false, true>)) != cudaSuccess || (e = rows2_attr(k_rows2_inv<true, true>)) != cudaSuccess)
-      return e;
+    if ((e = rows2_attr(k_rows2_inv<false>)) != cudaSuccess || (e = rows2_attr(k_rows2_inv<true>)) != cudaSuccess) return e;
     attr_done.fetch_or(1 << (dev & 31));
   }
-  const dim3 grid((nq + 1) / 2, g.nx);
-  const int nt = rows2_threads(g.nv, r8);
+  const dim3 grid(nq / 2, g.nx);
+  const int nt = rows2_threads(g.nv);
   const size_t sm = rows2_smem(g.nv);
-  if (r8) {
-    if (fast) k_rows2_inv<true, true><<<grid, nt, sm, s>>>(g, ft, nq, stack_biased, accimg);
-    else k_rows2_inv<false, true><<<grid, nt, sm, s>>>(g, ft, nq, stack_biased, accimg);
-  } else {
-    if (fast) k_rows2_inv<true, false><<<grid, nt, sm, s>>>(g, ft, nq, stack_biased, accimg);
-    else k_rows2_inv<false, false><<<grid, nt, sm, s>>>(g, ft, nq, stack_biased, accimg);
-  }
+  if (fast) k_rows2_inv<true><<<grid, nt, sm, s>>>(g, ft, stack_biased, accimg);
+  else k_rows2_inv<false><<<grid, nt, sm, s>>>(g, ft, stack_biased, accimg);
   return cudaGetLastError();
 }

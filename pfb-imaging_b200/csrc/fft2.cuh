@@ -302,13 +302,10 @@ __device__ __forceinline__ void p2_stage_pick(float4* s, const P2Tw& tw, int N, 
   p2_stage<R, NP, 0, VAR>(s, tw, N, L, swap, tid, nthr);
 }
 
-// MAXR = 8: the factorisation holds no radix-16 stage (kernels compiled for 85 registers leave that code out)
-template <int NP, int VAR, int MAXR>
+template <int NP, int VAR>
 __device__ __forceinline__ void p2_stage_dispatch(int r, float4* s, const P2Tw& tw, int N, int L, int swap, int tid,
                                                   int nthr) {
-  if constexpr (MAXR >= 16) {
-    if (r == 16) { p2_stage_pick<16, NP, VAR>(s, tw, N, L, swap, tid, nthr); return; }
-  }
+  if (r == 16) { p2_stage_pick<16, NP, VAR>(s, tw, N, L, swap, tid, nthr); return; }
   switch (r) {
     case 8: p2_stage_pick<8, NP, VAR>(s, tw, N, L, swap, tid, nthr); break;
     case 4: p2_stage_pick<4, NP, VAR>(s, tw, N, L, swap, tid, nthr); break;
@@ -328,14 +325,14 @@ __device__ __forceinline__ void p2_sync(int nthr) { asm volatile("bar.sync 1, %0
 
 // Forward DIF transform of the NP * 2 interleaved length-N arrays.  The caller makes the input visible to the
 // `nthr` transform threads first; on return every stage is complete and synchronised among them.
-template <int NP, int MAXR = 16>
+template <int NP>
 __device__ __forceinline__ void p2_fft_dif(float4* s, const P2Tw& tw, const FftDesc& d, int inmode, int tid, int nthr) {
   int L = d.n;
   for (int st = 0; st < d.nstage; ++st) {
     if (st == 0 && inmode != P2_IN_PAIR)
-      p2_stage_dispatch<NP, P2_DIF_DENSE, MAXR>(d.radix[0], s, tw, d.n, L, inmode == P2_IN_AOS_SWAP, tid, nthr);
+      p2_stage_dispatch<NP, P2_DIF_DENSE>(d.radix[0], s, tw, d.n, L, inmode == P2_IN_AOS_SWAP, tid, nthr);
     else
-      p2_stage_dispatch<NP, P2_DIF, MAXR>(d.radix[st], s, tw, d.n, L, 0, tid, nthr);
+      p2_stage_dispatch<NP, P2_DIF>(d.radix[st], s, tw, d.n, L, 0, tid, nthr);
     L /= d.radix[st];
     p2_sync(nthr);
   }
@@ -343,12 +340,12 @@ __device__ __forceinline__ void p2_fft_dif(float4* s, const P2Tw& tw, const FftD
 
 // Forward DIT transform: the input element n sits at (swizzled) position posmap[n] (digit-reversed), the output is
 // in natural order.
-template <int NP, int MAXR = 16>
+template <int NP>
 __device__ __forceinline__ void p2_fft_dit(float4* s, const P2Tw& tw, const FftDesc& d, int tid, int nthr) {
   int L = 1;
   for (int st = d.nstage - 1; st >= 0; --st) {
     L *= d.radix[st];
-    p2_stage_dispatch<NP, P2_DIT, MAXR>(d.radix[st], s, tw, d.n, L, 0, tid, nthr);
+    p2_stage_dispatch<NP, P2_DIT>(d.radix[st], s, tw, d.n, L, 0, tid, nthr);
     p2_sync(nthr);
   }
 }

@@ -11,11 +11,6 @@ struct FusedTabs {
   const int* rev_v;
   const int* pos_v;          // k -> pos (DIT input scatter)
   const int* pos_u;          // k -> pos along u (drain loops of the column kernels walk k)
-  // fp32 pair engine (fft2.cuh): radix-8 factorisations (72 instead of 128 registers per thread: twice the resident
-  // warps) and their digit tables; null / n = 0 when unused
-  FftDesc du8, dv8;
-  const int* pos_u8;
-  const int* pos_v8;
   const double* nutab;       // (nx,ny) fp64: n - 1 + nshift per pixel (w-screen phase = w_p * nutab, up to 1e3 turns)
   // cells any bound sample can touch: rows [a_lo, a_lo+a_len) and columns [b_lo, b_lo+b_len), circular
   int a_lo, a_len, b_lo, b_len;

@@ -146,13 +146,12 @@ struct pfbg_plan {
   cudaEvent_t stage_ev[16]{};
   bool stage_ev_ok = false;
   // fused FFT path (fused_fft.cuh)
-  DevBuf tw_u, tw_v, rev_u, rev_v, pos_v, pos_u, pos_u8, pos_v8, cellflags, accimg, nutab;
+  DevBuf tw_u, tw_v, rev_u, rev_v, pos_v, pos_u, cellflags, accimg, nutab;
   FusedTabs ftabs{};
   bool fused = false;          // tables built and sizes fit shared memory
   int col_c = 4;               // columns per CTA in the column passes
   bool cols2 = false;          // fp32: TMA-fed pair-engine column kernels (cols2.cuh) serve this geometry
   bool rows2 = false;          // fp32: pair-engine row kernels (rows2.cuh), two planes per CTA
-  bool rows_r8 = false, cols_r8 = false;  // ... on radix-8 stages with twice the threads
   cufftHandle fft = 0;
   int fft_batch = 1;           // planes per cuFFT execution (a divisor of nplanes; bounds the work area)
   bool fft_ok = false;
@@ -515,28 +514,6 @@ static int fused_setup_t(pfbg_plan* pl) {
     pl->cols2 = !(ce && strcmp(ce, "old") == 0) && pl->col_c == full_c && cols2_supported(g.nu, g.nv, g.nx, du);
     const char* re = getenv("PFBG_ROWS");  // PFBG_ROWS=old: one plane per CTA (k_rows_fwd / k_rows_inv)
     pl->rows2 = !(re && strcmp(re, "old") == 0) && rows2_supported(g.nv);
-    // radix-8 factorisations for the pair engine (PFBG_R8: bit 0 rows, bit 1 columns)
-    ft.du8.n = ft.dv8.n = 0;
-    ft.pos_u8 = ft.pos_v8 = nullptr;
-    const char* r8e = getenv("PFBG_R8");
-    const int r8 = r8e ? atoi(r8e) : 0;
-    FftDesc d8;
-    if ((r8 & 1) && pl->rows2 && factorize(g.nv, d8, 8)) {
-      digit_tables(d8, rev, pos);
-      CKRC(dev_alloc(pl, pl->pos_v8, (size_t)g.nv * 4));
-      CK(cudaMemcpy(pl->pos_v8.p, pos.data(), (size_t)g.nv * 4, cudaMemcpyHostToDevice));
-      ft.dv8 = d8;
-      ft.pos_v8 = (const int*)pl->pos_v8.p;
-      pl->rows_r8 = true;
-    }
-    if ((r8 & 2) && pl->cols2 && factorize(g.nu, d8, 8) && cols2_supported(g.nu, g.nv, g.nx, d8)) {
-      digit_tables(d8, rev, pos);
-      CKRC(dev_alloc(pl, pl->pos_u8, (size_t)g.nu * 4));
-      CK(cudaMemcpy(pl->pos_u8.p, pos.data(), (size_t)g.nu * 4, cudaMemcpyHostToDevice));
-      ft.du8 = d8;
-      ft.pos_u8 = (const int*)pl->pos_u8.p;
-      pl->cols_r8 = true;
-    }
   }
   pl->fused = true;
   return PFBG_OK;
@@ -924,14 +901,6 @@ static int run_slice(const pfbg_plan* pl, int64_t nact, int warps_per_cta, int c
   return (int)(sl < RUN_SLICE_TAIL ? RUN_SLICE_TAIL : (sl > RUN_SLICE ? RUN_SLICE : sl));
 }
 
-// resident CTAs per SM of the run kernels (PFBG_GRID_CTAS / PFBG_DEG_CTAS override the defaults: fewer CTAs leave
-// room for the kernels of another band running on a second stream)
-static int run_ctas(const char* env, int dflt) {
-  const char* e = getenv(env);
-  const int v = e ? atoi(e) : 0;
-  return v >= 1 && v <= dflt ? v : dflt;
-}
-
 static int run_blocks(const pfbg_plan* pl, int64_t nact, int warps_per_cta, int ctas_per_sm) {
   int sm = 148;
   cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, pl->device);
@@ -1181,7 +1150,7 @@ static int run_spread(pfbg_plan* pl, cudaStream_t s, const void* vis, int64_t rs
   } else if (pl->nactive > 0 && pl->use_runs) {
     unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + 16);  // slice counter of this launch
     CK(cudaMemsetAsync(queue, 0, 8, s));
-    const int ctas = run_ctas("PFBG_GRID_CTAS", 3);
+    const int ctas = 3;  // resident CTAs per SM
     const int slice = run_slice(pl, pl->nactive, RUN_WARPS, ctas);
     k_grid_runs<T><<<run_blocks(pl, pl->nactive, RUN_WARPS, ctas), RUN_WARPS * 32, 0, s>>>(
         pl->gp, (const VisRec<T>*)pl->recs.p, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p,
@@ -1240,7 +1209,7 @@ static int run_gather(pfbg_plan* pl, cudaStream_t s, const void* wgt, void* vis_
   } else if (pl->nactive > 0 && pl->use_runs) {
     unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + 24);
     CK(cudaMemsetAsync(queue, 0, 8, s));
-    const int ctas = run_ctas("PFBG_DEG_CTAS", 5);
+    const int ctas = 5;  // resident CTAs per SM
     const int slice = run_slice(pl, pl->nactive, DEG_WARPS, ctas);
     k_degrid_runs<T><<<run_blocks(pl, pl->nactive, DEG_WARPS, ctas), DEG_WARPS * 32, 0, s>>>(
         pl->gp, (const VisRec<T>*)pl->recs.p, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out,
@@ -1281,22 +1250,9 @@ static int run_grid2img(pfbg_plan* pl, cudaStream_t s, const void* beam, const v
   return PFBG_OK;
 }
 
-// planes of a row pass that go through the pair engine: all of an even count, all but the last of an odd one
-// (PFBG_ROWS_ODD=pair keeps the last plane there too: A/B)
-static int rows_odd_split(int nq) {
-  if (!(nq & 1)) return nq;
-  const char* e = getenv("PFBG_ROWS_ODD");
-  if (e && strcmp(e, "pair") == 0) return nq;
-  return nq - 1;
-}
-
 // threads per CTA for a row transform: the multiple of 32 (<= cap, >= cap/2) that balances the
 // radix-16 stage best (n/16 butterflies)
 static int row_threads(int n, int cap, int radix = 16) {
-  if (const char* e = getenv("PFBG_ROW_THREADS")) {  // tuning hook
-    const int t = atoi(e);
-    if (t >= 32 && t <= cap && t % 32 == 0) return t;
-  }
   int nb = n / radix, best = cap;
   double best_eff = 0.0;
   for (int t = cap; t >= cap / 2; t -= 32) {
@@ -1313,16 +1269,15 @@ static int run_cols2(pfbg_plan* pl, cudaStream_t s, const FusedTabs& ft, int slo
                      float2* out_biased) {
   const GParams& g = pl->gp;
   Cols2Args a;
-  a.du = pl->cols_r8 ? ft.du8 : ft.du;
+  a.du = ft.du;
   a.tw_u = (const float2*)ft.tw_u;
-  a.pos_u = pl->cols_r8 ? ft.pos_u8 : ft.pos_u;
+  a.pos_u = ft.pos_u;
   a.nu = g.nu; a.nv = g.nv; a.nx = g.nx;
   a.a_lo = ft.a_lo; a.a_len = ft.a_len; a.b_lo = ft.b_lo; a.b_len = ft.b_len;
   a.q0 = ft.q0; a.nq = nq; a.slot0 = slot0;
   a.inverse = inverse ? 1 : 0;
-  a.debug = 0; a.dbg_stack = nullptr;
   const char* what = "";
-  cudaError_t e = cols2_launch(a, pl->cols_r8, (const float2*)pl->grid.p, pl->stack_planes, out_biased, s, &what);
+  cudaError_t e = cols2_launch(a, (const float2*)pl->grid.p, pl->stack_planes, out_biased, s, &what);
   if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "%s: %s", what, cudaGetErrorString(e));
   LAUNCHED();
   return PFBG_OK;
@@ -1359,9 +1314,9 @@ static int run_fused_fwd(pfbg_plan* pl, cudaStream_t s, const void* x, const voi
   int nq2 = 0;  // planes that go through the pair engine
   if constexpr (sizeof(T) == 4) {
     if (pl->rows2) {
-      nq2 = rows_odd_split(nq);
+      nq2 = nq & ~1;
       if (nq2 > 0) {
-        cudaError_t e = rows2_fwd_launch(g, ft, nq2, g.fast_screen != 0, pl->rows_r8, (const float*)x, (const float*)beam,
+        cudaError_t e = rows2_fwd_launch(g, ft, nq2, g.fast_screen != 0, (const float*)x, (const float*)beam,
                                          (const float*)pl->corr.p, (float2*)stack, s);
         if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "k_rows2_fwd launch: %s", cudaGetErrorString(e));
         LAUNCHED();
@@ -1433,9 +1388,9 @@ static int run_fused_inv_acc(pfbg_plan* pl, cudaStream_t s, int q0, int nq, cons
   int nq2 = 0;  // planes that go through the pair engine (see run_fused_fwd)
   if constexpr (sizeof(T) == 4) {
     if (pl->rows2) {
-      nq2 = rows_odd_split(nq);
+      nq2 = nq & ~1;
       if (nq2 > 0) {
-        cudaError_t e = rows2_inv_launch(g, ft, nq2, g.fast_screen != 0, pl->rows_r8, (const float2*)stack, (double*)pl->accimg.p, s);
+        cudaError_t e = rows2_inv_launch(g, ft, nq2, g.fast_screen != 0, (const float2*)stack, (double*)pl->accimg.p, s);
         if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "k_rows2_inv launch: %s", cudaGetErrorString(e));
         LAUNCHED();
       }

@@ -5,7 +5,8 @@
 //   * the butterflies run two-wide (FADD2 / FMUL2 / FFMA2): half the math instructions per plane,
 //   * the grid direction adds the two planes' contributions to the fp64 image with ONE RED.F64 per pixel instead of two.
 // Shared memory: nv pair elements of 16 bytes {re_q, re_q+1, im_q, im_q+1} (XOR-swizzled) + the two-level twiddle table;
-// two CTAs per SM at nv = 6144.  A launch over an odd number of planes leaves the second half of the last pair empty.
+// two CTAs per SM at nv = 6144.  A launch covers an even number of planes (the last plane of an odd count goes to the
+// one-plane kernel).
 //
 //   k_rows2_fwd (degrid direction): pad + beam + correction + w-screen of both planes built in shared memory at the
 //                                   digit-reversed positions, DIT transform (natural-order output), the active columns
@@ -18,21 +19,18 @@
 #include "fft2.cuh"
 
 #define ROWS2_THREADS 192    // radix-16 stages: 128 registers per thread, two CTAs of 6 warps per SM
-#define ROWS2_THREADS_R8 384 // radix-8 stages (ft.dv8 / ft.pos_v8): <= 85 registers, two CTAs of 12 warps per SM
 
-template <bool FAST, bool R8>
-__global__ void __launch_bounds__(R8 ? ROWS2_THREADS_R8 : ROWS2_THREADS, 2)
-k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const float* __restrict__ beam,
+template <bool FAST>
+__global__ void __launch_bounds__(ROWS2_THREADS, 2)
+k_rows2_fwd(GParams p, FusedTabs ft, const float* __restrict__ x, const float* __restrict__ beam,
             const float* __restrict__ corr, float2* __restrict__ grid) {
   extern __shared__ __align__(1024) unsigned char smem_raw1k[];
   float4* s = reinterpret_cast<float4*>(smem_raw1k);
   const int tid = threadIdx.x, nthr = blockDim.x, i = blockIdx.y;
   const int nv = p.nv, hy = p.ny / 2;
-  const FftDesc& dv = R8 ? ft.dv8 : ft.dv;
-  const int* __restrict__ pos_v = R8 ? ft.pos_v8 : ft.pos_v;
-  const int qa = 2 * blockIdx.x + ft.q0;
-  const bool two = 2 * (int)blockIdx.x + 1 < nq;
-  const int qb = two ? qa + 1 : qa;
+  const FftDesc& dv = ft.dv;
+  const int* __restrict__ pos_v = ft.pos_v;
+  const int qa = 2 * blockIdx.x + ft.q0, qb = qa + 1;
   const P2Tw tw = p2_tw_fill(reinterpret_cast<float2*>(s + nv), (const float2*)ft.tw_v, nv, tid, nthr);
   const int ip = i - p.nx / 2;
   const int a = ip < 0 ? ip + p.nu : ip;
@@ -53,7 +51,6 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
     if (beam) { ba += oa; bb += ob; }
   }
   const bool same_x = xa == xb;  // (then ba == bb too)
-  const float mb = two ? 1.f : 0.f;
   const bool vec_ok = (p.ny & 7) == 0 && (((uintptr_t)x | (uintptr_t)corr | (uintptr_t)beam) & 15) == 0;
   if (vec_ok) {
     // 4 consecutive pixels per step (hy % 4 == 0, so a group never straddles the wrap), two steps in flight
@@ -90,7 +87,7 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
               cbb = same_x ? cb : cbb * bw[u][e];
             }
             const float va = xv[u][e] * cb;
-            const float vb = (same_x ? xv[u][e] : yv[u][e]) * cbb * mb;
+            const float vb = (same_x ? xv[u][e] : yv[u][e]) * cbb;
             if (va == 0.f && vb == 0.f) continue;  // the buffer is zero already
             float4 v = make_float4(va, vb, 0.f, 0.f);
             if (p.do_wgridding) {
@@ -108,7 +105,7 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
     for (int j = tid; j < p.ny; j += nthr) {
       const int64_t pix = row + j;
       const float c = corr[pix];
-      const float va = xa[pix] * (beam ? c * ba[pix] : c), vb = xb[pix] * (beam ? c * bb[pix] : c) * mb;
+      const float va = xa[pix] * (beam ? c * ba[pix] : c), vb = xb[pix] * (beam ? c * bb[pix] : c);
       float4 v = make_float4(va, vb, 0.f, 0.f);
       if (p.do_wgridding) {
         float ca, sa, c2, s2;
@@ -121,7 +118,7 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
     }
   }
   __syncthreads();
-  p2_fft_dit<1, R8 ? 8 : 16>(s, tw, dv, tid, nthr);
+  p2_fft_dit<1>(s, tw, dv, tid, nthr);
   // only the active columns are written (window bounds are multiples of 32): two columns per step and plane
   float2* da = grid + ((int64_t)qa * p.nu + a) * nv;
   float2* db = grid + ((int64_t)qb * p.nu + a) * nv;
@@ -132,22 +129,20 @@ k_rows2_fwd(GParams p, FusedTabs ft, int nq, const float* __restrict__ x, const 
     if (n >= nv) n -= nv;
     const float4 v0 = s[sw2(n)], v1 = s[sw2(n + 1)];  // {re_a, re_b, im_a, im_b}
     *reinterpret_cast<float4*>(da + n) = make_float4(v0.x, v0.z, v1.x, v1.z);
-    if (two) *reinterpret_cast<float4*>(db + n) = make_float4(v0.y, v0.w, v1.y, v1.w);
+    *reinterpret_cast<float4*>(db + n) = make_float4(v0.y, v0.w, v1.y, v1.w);
   }
 }
 
-template <bool FAST, bool R8>
-__global__ void __launch_bounds__(R8 ? ROWS2_THREADS_R8 : ROWS2_THREADS, 2)
-k_rows2_inv(GParams p, FusedTabs ft, int nq, const float2* __restrict__ grid, double* __restrict__ accimg) {
+template <bool FAST>
+__global__ void __launch_bounds__(ROWS2_THREADS, 2)
+k_rows2_inv(GParams p, FusedTabs ft, const float2* __restrict__ grid, double* __restrict__ accimg) {
   extern __shared__ __align__(1024) unsigned char smem_raw1k[];
   float4* s = reinterpret_cast<float4*>(smem_raw1k);
   const int tid = threadIdx.x, nthr = blockDim.x, i = blockIdx.y;
   const int nv = p.nv, hy = p.ny / 2;
-  const FftDesc& dv = R8 ? ft.dv8 : ft.dv;
-  const int* __restrict__ pos_v = R8 ? ft.pos_v8 : ft.pos_v;
-  const int qa = 2 * blockIdx.x + ft.q0;
-  const bool two = 2 * (int)blockIdx.x + 1 < nq;
-  const int qb = two ? qa + 1 : qa;
+  const FftDesc& dv = ft.dv;
+  const int* __restrict__ pos_v = ft.pos_v;
+  const int qa = 2 * blockIdx.x + ft.q0, qb = qa + 1;
   const P2Tw tw = p2_tw_fill(reinterpret_cast<float2*>(s + nv), (const float2*)ft.tw_v, nv, tid, nthr);
   const int ip = i - p.nx / 2;
   const int a = ip < 0 ? ip + p.nu : ip;
@@ -160,21 +155,19 @@ k_rows2_inv(GParams p, FusedTabs ft, int nq, const float2* __restrict__ grid, do
     if (n >= nv) n -= nv;
     s[sw2(n)] = z;
   }
-  const float mb = two ? 1.f : 0.f;
   const int npair = ft.b_len >> 1;
 #pragma unroll 4
   for (int r = tid; r < npair; r += nthr) {
     int n = ft.b_lo + 2 * r;
     if (n >= nv) n -= nv;
     const float4 va = *reinterpret_cast<const float4*>(sa_ + n);  // {re(n), im(n), re(n+1), im(n+1)} of plane a
-    float4 vb = *reinterpret_cast<const float4*>(sb_ + n);
-    vb.x *= mb; vb.y *= mb; vb.z *= mb; vb.w *= mb;
+    const float4 vb = *reinterpret_cast<const float4*>(sb_ + n);
     // swap-in: the engine transforms (im, re), which makes the forward transform the inverse one
     s[sw2(n)] = make_float4(va.y, vb.y, va.x, vb.x);
     s[sw2(n + 1)] = make_float4(va.w, vb.w, va.z, vb.z);
   }
   __syncthreads();
-  p2_fft_dif<1, R8 ? 8 : 16>(s, tw, dv, P2_IN_PAIR, tid, nthr);
+  p2_fft_dif<1>(s, tw, dv, P2_IN_PAIR, tid, nthr);
   const double wa = ft.plane_w ? ft.plane_w[qa] : p.w0 + qa * p.dw;
   const double wb = ft.plane_w ? ft.plane_w[qb] : p.w0 + qb * p.dw;
   const int64_t row = (int64_t)i * p.ny;
@@ -219,7 +212,7 @@ k_rows2_inv(GParams p, FusedTabs ft, int nq, const float2* __restrict__ grid, do
               atomicAdd(dsta + 4 * g + e, (double)ra + (double)rb);
             } else {
               atomicAdd(dsta + 4 * g + e, (double)ra);
-              if (two) atomicAdd(dstb + 4 * g + e, (double)rb);
+              atomicAdd(dstb + 4 * g + e, (double)rb);
             }
           }
         }
@@ -244,7 +237,7 @@ k_rows2_inv(GParams p, FusedTabs ft, int nq, const float2* __restrict__ grid, do
         atomicAdd(dsta + j, (double)ra + (double)rb);
       } else {
         atomicAdd(dsta + j, (double)ra);
-        if (two) atomicAdd(dstb + j, (double)rb);
+        atomicAdd(dstb + j, (double)rb);
       }
     }
   }

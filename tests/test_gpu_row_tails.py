@@ -7,8 +7,8 @@ input, and a caller may pass views into a larger device buffer.
 
 Which row kernel runs: fp32 plans whose nv fits the pair engine (rows2_supported: nv % 32 == 0, which padded_size
 always gives, and ~14 k cells of shared memory) run all planes of an even count and all but the last of an odd one
-on k_rows2_*, the last one on k_rows_*; PFBG_ROWS=old runs every plane on k_rows_*, PFBG_ROWS_ODD=pair the last one in
-a half-empty pair.  fp64 plans always run k_rows_*; beyond ROWS_BIG_SMEM (fused_common.cuh) of shared memory per row
+on k_rows2_*, the last one on k_rows_*; PFBG_ROWS=old runs every plane on k_rows_*.  fp64 plans always run
+k_rows_*; beyond ROWS_BIG_SMEM (fused_common.cuh) of shared memory per row
 the BIG variants (PFBG_ROWS_SMALL=1: the ordinary ones).  A plan with nv % 32 != 0 cannot be made (plan.padded_size
 rounds nv up to a multiple of 32), so the one-plane kernels are reached through fp64, the odd last plane and
 PFBG_ROWS=old instead.
@@ -106,8 +106,7 @@ def _check_arms(a, b, prec, what):
 @pytest.mark.parametrize("ny", [250, 252, 254])
 def test_scalar_row_branches(gpu, monkeypatch, ny, prec, fast, planes):
     """ny % 8 in {2, 4, 6}: fp32 on the pair engine (nv = 512) with the fast w-screen on and off, fp64 on the one-plane
-    kernels; odd and even plane counts.  fp32: against the last plane in a pair slot and every plane on the one-plane
-    kernels at round-off."""
+    kernels; odd and even plane counts.  fp32: against every plane on the one-plane kernels at round-off."""
     if not fast and prec == "single":
         monkeypatch.setenv("PFBG_FAST_SCREEN", "0")
     nx = 64
@@ -123,11 +122,8 @@ def test_scalar_row_branches(gpu, monkeypatch, ny, prec, fast, planes):
             assert pl.fast_screen == fast, f"fixture no longer exercises fast_screen = {fast}"
         out = _apply(gp, r)
         _check_dft(p, r, out, EPS[prec], f"rows ny={ny} {prec} fast={fast} {planes} P={pl.nplanes}")
-        if prec == "double":
-            return
-        monkeypatch.setenv("PFBG_ROWS_ODD", "pair")  # read per call
-        _check_arms(out, _apply(gp, r), prec, "PFBG_ROWS_ODD=pair")
-    monkeypatch.delenv("PFBG_ROWS_ODD")
+    if prec == "double":
+        return
     monkeypatch.setenv("PFBG_ROWS", "old")  # read when the plan sets up its transforms
     with _plan(p, prec) as gp:
         _check_arms(out, _apply(gp, r), prec, "PFBG_ROWS=old")

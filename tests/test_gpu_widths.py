@@ -216,8 +216,8 @@ def _parity_plan(p, w, sigma, wgrid):
 @pytest.mark.parametrize("fast", [1, 0])
 def test_row_passes_with_odd_and_even_plane_counts(gpu, monkeypatch, planes, fast):
     """nplanes = 1 (no w-gridding), odd >= 3 and even >= 4 through the fp32 row passes, fast w-screen on and off:
-    against the DFT at the bound, and against the last plane in a pair slot (PFBG_ROWS_ODD=pair) and the one-plane
-    row kernels for every plane (PFBG_ROWS=old) at fp32 round-off.  (Two planes occur only as split subsets, below.)"""
+    against the DFT at the bound, and against the one-plane row kernels for every plane (PFBG_ROWS=old) at fp32
+    round-off.  (Two planes occur only as split subsets, below.)"""
     w, sigma = 6, 2.0
     p = _parity_problem(0 if planes == "even" else 1, w, sigma)
     if not fast:
@@ -235,15 +235,11 @@ def test_row_passes_with_odd_and_even_plane_counts(gpu, monkeypatch, planes, fas
         assert gp.plan.fast_screen == (fast if wgrid else 0)
         res["split"] = _apply(gp, r)
         _check_bound(gp, _dft_errors(prob, "single", res["split"]), f"rows/{planes}")
-        monkeypatch.setenv("PFBG_ROWS_ODD", "pair")
-        res["pair"] = _apply(gp, r)
-    monkeypatch.delenv("PFBG_ROWS_ODD")
     monkeypatch.setenv("PFBG_ROWS", "old")
     with _parity_plan(p, w, sigma, wgrid) as gp:
         res["old"] = _apply(gp, r)
-    for arm in ("pair", "old"):
-        for a, b, what in zip(res["split"], res[arm], ("degrid", "grid", "hessian")):
-            assert rel_l2(a, b) <= 3e-6, (arm, what, rel_l2(a, b))
+    for a, b, what in zip(res["split"], res["old"], ("degrid", "grid", "hessian")):
+        assert rel_l2(a, b) <= 3e-6, ("old", what, rel_l2(a, b))
 
 
 @pytest.mark.parametrize("parity", [1, 0])
