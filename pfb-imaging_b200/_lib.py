@@ -10,6 +10,7 @@ import ctypes as C
 import os
 import subprocess
 import sys
+from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
@@ -137,23 +138,28 @@ SIGNATURES = {
 _lib = None
 
 
-# translation units of libpfbgrid.so and the files each one includes (incremental rebuilds: the gridder
-# unit takes ~2 minutes to compile, the others seconds)
+# translation units of libpfbgrid.so and every file each one includes, directly or not (incremental rebuilds: the
+# gridder unit takes minutes to compile, the others seconds; tests/test_build_units.py keeps the lists exact)
 _UNITS = {
-    "pfbgrid.cu": ["common.cuh", "fft.cuh", "fused_fft.cuh", "kernels.cuh", "psfconv.cuh", "runs.cuh", "runs_mma.cuh", "weighting.cuh",
-                   "cols2_api.h", "fused_common.cuh", "../../include/pfbgrid.h"],
-    "colsfft.cu": ["common.cuh", "fft.cuh", "fft2.cuh", "cols2.cuh", "rows2.cuh", "cols2_api.h", "fused_common.cuh"],
-    "pfbsara.cu": ["sara.cuh", "clean.cuh", "cg.cuh", "../../include/pfbsara.h", "../../include/pfbgrid.h"],
+    "pfbgrid.cu": ["common.cuh", "fft.cuh", "fused_fft.cuh", "kernels.cuh", "runs.cuh", "runs_mma.cuh", "cols2_api.h",
+                   "fused_common.cuh", "fft_host.h", "host.h", "../../include/pfbgrid.h"],
+    "colsfft.cu": ["common.cuh", "fft.cuh", "fft2.cuh", "cols2.cuh", "rows2.cuh", "cols2_api.h", "fused_common.cuh",
+                   "fft_host.h", "host.h", "../../include/pfbgrid.h"],
+    "psfconv.cu": ["psfconv.cuh", "fft.cuh", "fft_host.h", "host.h", "../../include/pfbgrid.h"],
+    "weighting.cu": ["weighting.cuh", "common.cuh", "host.h", "../../include/pfbgrid.h"],
+    "pfbsara.cu": ["sara.cuh", "clean.cuh", "cg.cuh", "host.h", "../../include/pfbsara.h", "../../include/pfbgrid.h"],
 }
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
-    """Compile ``csrc/*.cu`` for sm_100a into ``libpfbgrid.so`` (in-tree), one object per translation unit."""
+    """Compile ``csrc/*.cu`` for sm_100a into ``libpfbgrid.so`` (in-tree), one object per translation unit.
+
+    Stale units compile concurrently, so a clean build takes about as long as the slowest unit."""
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
     objdir = os.path.join(HERE, "build")
     os.makedirs(objdir, exist_ok=True)
     flags = [f for f in NVCC_FLAGS if f != "-shared"]
-    objs, relink = [], force or not os.path.exists(LIB_PATH)
+    objs, stale = [], []
     for unit, deps in _UNITS.items():
         src = os.path.join(CSRC, unit)
         obj = os.path.join(objdir, unit.replace(".cu", ".o"))
@@ -164,13 +170,15 @@ def build(force: bool = False, verbose: bool = False) -> str:
             if verbose:
                 cmd.insert(1, "-Xptxas=-v")
                 print(" ".join(cmd), file=sys.stderr)
-            res = subprocess.run(cmd, capture_output=True, text=True)
-            if res.returncode != 0:
-                raise RuntimeError(f"nvcc failed:\n{res.stdout}\n{res.stderr}")
-            if verbose:
-                print(res.stderr, file=sys.stderr)
-            relink = True
-    if relink or any(os.path.getmtime(o) > os.path.getmtime(LIB_PATH) for o in objs):
+            stale.append(cmd)
+    with ThreadPoolExecutor(max_workers=max(1, len(stale))) as pool:
+        results = list(pool.map(lambda cmd: subprocess.run(cmd, capture_output=True, text=True), stale))
+    for res in results:
+        if res.returncode != 0:
+            raise RuntimeError(f"nvcc failed:\n{res.stdout}\n{res.stderr}")
+        if verbose:
+            print(res.stderr, file=sys.stderr)
+    if stale or not os.path.exists(LIB_PATH) or any(os.path.getmtime(o) > os.path.getmtime(LIB_PATH) for o in objs):
         cmd = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", *objs, "-o", LIB_PATH, "-lcufft",
                "-Xlinker", "-rpath=/usr/local/cuda/lib64"]
         res = subprocess.run(cmd, capture_output=True, text=True)

@@ -23,9 +23,6 @@ bool cols2_supported(int nu, int nv, int nx, const FftDesc& du);
 // Returns cudaSuccess or the failing error; *what names the failing step.
 cudaError_t cols2_launch(const Cols2Args& a, const float2* stack, int stack_planes, float2* out, cudaStream_t s,
                          const char** what);
-// engine unit test: `batch` CTAs, each transforming 2 NP interleaved length-n arrays (see k_fft2_debug)
-cudaError_t fft2_debug_launch(const FftDesc& d, int np, const float2* tw, const int* rev, const float2* in, float2* out,
-                              int batch, int inverse, int aos);
 
 // Row passes on the pair engine (rows2.cuh, fp32): the same image row of two neighbouring planes per CTA.
 // `stack_biased`: logical plane q at stack_biased + q nu nv.  Planes [ft.q0, ft.q0 + nq); nq must be even

@@ -1,12 +1,13 @@
-// Translation unit of the pair-engine column transforms (cols2.cuh): tensor-map encoding, launch, engine unit test.
+// Translation unit of the pair-engine column transforms (cols2.cuh): tensor-map encoding, launch, and the unit-test
+// hooks of both shared-memory FFT engines (fft.cuh, fft2.cuh).
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <atomic>
 #include <mutex>
 #include "cols2.cuh"
+#include "fft_host.h"
+#include "host.h"
 #include "rows2.cuh"
-
-static const size_t kCols2MaxSmem = 232448;  // 227 KB opt-in dynamic shared memory per CTA on sm_100
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -31,7 +32,7 @@ static size_t cols2_smem(int nu) { return (size_t)nu * 32 + 64 + (size_t)((nu + 
 bool cols2_supported(int nu, int nv, int nx, const FftDesc& du) {
   if (nu > 65535) return false;
   if (!p2_dense_ok(du, 2)) return false;
-  if (cols2_smem(nu) > kCols2MaxSmem) return false;
+  if (cols2_smem(nu) > kMaxSmem) return false;
   if ((nx / 2) % COLS2_BOX_SMALL || nu % COLS2_BOX_SMALL || nv % 32 || nx % 2) return false;
   return encode_fn() != nullptr;
 }
@@ -64,7 +65,7 @@ cudaError_t cols2_launch(const Cols2Args& a, const float2* stack, int stack_plan
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
   if (e != cudaSuccess) { *what = "device query"; return e; }
   if (!(attr_done.load() & (1 << (dev & 31)))) {
-    e = cudaFuncSetAttribute(k_cols2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCols2MaxSmem);
+    e = cudaFuncSetAttribute(k_cols2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem);
     if (e != cudaSuccess) { *what = "cudaFuncSetAttribute(k_cols2)"; return e; }
     attr_done.fetch_or(1 << (dev & 31));
   }
@@ -113,14 +114,14 @@ __global__ void __launch_bounds__(256) k_fft2_debug(FftDesc d, const float2* __r
   }
 }
 
-cudaError_t fft2_debug_launch(const FftDesc& d, int np, const float2* tw, const int* rev, const float2* in, float2* out,
-                              int batch, int inverse, int aos) {
+static cudaError_t fft2_debug_launch(const FftDesc& d, int np, const float2* tw, const int* rev, const float2* in,
+                                     float2* out, int batch, int inverse, int aos) {
   const size_t sm = (size_t)d.n * np * 16 + (size_t)((d.n + 63) / 64 + 64) * 8;
-  if (sm > kCols2MaxSmem || (np != 1 && np != 2 && np != 4)) return cudaErrorInvalidValue;
+  if (sm > kMaxSmem || (np != 1 && np != 2 && np != 4)) return cudaErrorInvalidValue;
   if (aos == 1 && !p2_dense_ok(d, np)) return cudaErrorInvalidValue;
   cudaError_t e;
 #define FFT2_DEBUG_CASE(NPV)                                                                                          \
-  e = cudaFuncSetAttribute(k_fft2_debug<NPV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCols2MaxSmem);       \
+  e = cudaFuncSetAttribute(k_fft2_debug<NPV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem);       \
   if (e != cudaSuccess) return e;                                                                                      \
   k_fft2_debug<NPV><<<batch, 256, sm>>>(d, tw, rev, in, out, inverse, aos);
   if (np == 1) { FFT2_DEBUG_CASE(1) }
@@ -130,6 +131,64 @@ cudaError_t fft2_debug_launch(const FftDesc& d, int np, const float2* tw, const 
   return cudaGetLastError();
 }
 
+extern "C" int pfbg_debug_fft2(int32_t device, int32_t n, int32_t np, int32_t batch, const void* in, void* out,
+                               int32_t inverse, int32_t aos) {
+  if (!in || !out || n < 2 || batch < 1) return fail(PFBG_ERR_ARG, "bad argument");
+  CK(cudaSetDevice(device));
+  FftDesc d;
+  if (!factorize(n, d, 16)) return fail(PFBG_ERR_ARG, "n=%d is not 2^a 3^b 5^c 7^d 11^e", n);
+  const std::vector<cx2<float>> tw = twiddles<float>(n);
+  std::vector<int> rev, pos;
+  digit_tables(d, rev, pos);
+  const size_t bytes = (size_t)n * 8 * 2 * np * batch;
+  TmpBufs t;
+  void *dtw, *drev, *din, *dout;
+  CKRC(t.get(&dtw, tw.data(), (size_t)n * 8, false, true, 0));
+  CKRC(t.get(&drev, rev.data(), (size_t)n * 4, false, true, 0));
+  CKRC(t.get(&din, in, bytes, false, true, 0));
+  CKRC(t.get(&dout, out, bytes, false, false, 0));
+  cudaError_t e = fft2_debug_launch(d, np, (const float2*)dtw, (const int*)drev, (const float2*)din, (float2*)dout, batch,
+                                    inverse, aos);
+  if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "fft2 debug launch: %s", cudaGetErrorString(e));
+  LAUNCHED();
+  CK(cudaMemcpy(out, dout, bytes, cudaMemcpyDeviceToHost));
+  return PFBG_OK;
+}
+
+// ---- engine unit test of the one-plane FFT (fft.cuh) ---------------------------------------------------------------
+template <typename T>
+static int debug_fft_t(int n, int batch, const void* in, void* out, int mode, int inverse) {
+  FftDesc d;
+  if (!factorize(n, d, sizeof(T) == 4 ? 16 : 8)) return fail(PFBG_ERR_ARG, "n=%d is not 2^a 3^b 5^c 7^d 11^e", n);
+  size_t bytes = (size_t)n * sizeof(cx2<T>);
+  if (fft_smem_bytes<T>(n) > kMaxSmem) return fail(PFBG_ERR_ARG, "n=%d does not fit shared memory", n);
+  const std::vector<cx2<T>> tw = twiddles<T>(n);
+  std::vector<int> rev, pos;
+  digit_tables(d, rev, pos);
+  TmpBufs t;
+  void *dtw, *drev, *dpos, *din, *dout;
+  CKRC(t.get(&dtw, tw.data(), bytes, false, true, 0));
+  CKRC(t.get(&drev, rev.data(), (size_t)n * 4, false, true, 0));
+  CKRC(t.get(&dpos, pos.data(), (size_t)n * 4, false, true, 0));
+  CKRC(t.get(&din, in, bytes * batch, false, true, 0));
+  CKRC(t.get(&dout, out, bytes * batch, false, false, 0));
+  CK(cudaFuncSetAttribute(k_fft_debug<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+  k_fft_debug<T><<<batch, 256, fft_smem_bytes<T>(n)>>>(d, (const cx2<T>*)dtw, (const int*)drev, (const int*)dpos, (const cx2<T>*)din,
+                                        (cx2<T>*)dout, mode, inverse);
+  LAUNCHED();
+  CK(cudaGetLastError());
+  CK(cudaMemcpy(out, dout, bytes * batch, cudaMemcpyDeviceToHost));
+  return PFBG_OK;
+}
+
+extern "C" int pfbg_debug_fft1d(int32_t precision, int32_t device, int32_t n, int32_t batch, const void* in,
+                                void* out, int32_t mode, int32_t inverse) {
+  if (!in || !out || n < 2 || batch < 1) return fail(PFBG_ERR_ARG, "bad argument");
+  CK(cudaSetDevice(device));
+  return precision == PFBG_F32 ? debug_fft_t<float>(n, batch, in, out, mode, inverse)
+                               : debug_fft_t<double>(n, batch, in, out, mode, inverse);
+}
+
 // ---- row passes on the pair engine (rows2.cuh) --------------------------------------------------------------------
 static size_t rows2_smem(int nv) { return (size_t)nv * 16 + (size_t)((nv + 63) / 64 + 64) * 8; }
 static int rows2_threads(int nv) {
@@ -137,11 +196,11 @@ static int rows2_threads(int nv) {
   return t < 32 ? 32 : (t > ROWS2_THREADS ? ROWS2_THREADS : t);
 }
 
-bool rows2_supported(int nv) { return nv % 32 == 0 && rows2_smem(nv) <= kCols2MaxSmem; }
+bool rows2_supported(int nv) { return nv % 32 == 0 && rows2_smem(nv) <= kMaxSmem; }
 
 template <typename K>
 static cudaError_t rows2_attr(K kern) {
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCols2MaxSmem);
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
   return e;
 }

@@ -22,7 +22,8 @@
 #include "runs_mma.cuh"
 #include "fused_fft.cuh"
 #include "cols2_api.h"
-#include "weighting.cuh"
+#include "fft_host.h"
+#include "host.h"
 
 // ---------------------------------------------------------------------------
 // error plumbing
@@ -30,17 +31,6 @@
 static thread_local std::string g_err;
 static std::atomic<int64_t> g_launches{0};
 
-static int fail(int code, const char* fmt, ...) {
-  char buf[1024];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof buf, fmt, ap);
-  va_end(ap);
-  g_err = buf;
-  return code;
-}
-
-// used by the other translation units of this library (pfbsara.cu)
 int pfbg_fail(int code, const char* fmt, ...) {
   char buf[1024];
   va_list ap;
@@ -52,7 +42,7 @@ int pfbg_fail(int code, const char* fmt, ...) {
 }
 void pfbg_count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
-// Small device scratch blocks (256 B) for the scalar reductions of both translation units: a caller holds a block
+// Small device scratch blocks (256 B) for the scalar reductions of every translation unit: a caller holds a block
 // for the duration of its call, so two host threads (or two streams driven from different threads) on one device
 // never share an accumulator; blocks are recycled, never freed while the process lives (no cudaMalloc / cudaFree
 // inside solver loops).
@@ -78,13 +68,6 @@ void pfbg_scratch_put(int device, void* p) {
   g_scratch_free[device].push_back(p);
 }
 
-#define CK(call)                                                                           \
-  do {                                                                                     \
-    cudaError_t e_ = (call);                                                               \
-    if (e_ != cudaSuccess)                                                                 \
-      return fail(PFBG_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_),   \
-                  __FILE__, __LINE__);                                                     \
-  } while (0)
 #define CKFFT(call)                                                                        \
   do {                                                                                     \
     cufftResult r_ = (call);                                                               \
@@ -92,12 +75,6 @@ void pfbg_scratch_put(int device, void* p) {
       return fail(PFBG_ERR_CUFFT, "%s failed: cufft status %d (%s:%d)", #call, (int)r_,    \
                   __FILE__, __LINE__);                                                     \
   } while (0)
-#define CKRC(call)              \
-  do {                          \
-    int rc_ = (call);           \
-    if (rc_ != PFBG_OK) return rc_; \
-  } while (0)
-#define LAUNCHED() (g_launches.fetch_add(1, std::memory_order_relaxed))
 
 extern "C" const char* pfbg_last_error(void) { return g_err.c_str(); }
 extern "C" int pfbg_version(void) { return 100; }
@@ -374,64 +351,13 @@ static int plan_create_impl(const pfbg_plan_desc* d, int stack_planes, pfbg_plan
 // ---------------------------------------------------------------------------
 // fused FFT tables
 // ---------------------------------------------------------------------------
-// maxr: largest power-of-two radix (16 in fp32; 8 in fp64, whose radix-16 butterfly needs ~250 registers and
-// leaves one 8-warp CTA per SM)
-static bool factorize(int n, FftDesc& d, int maxr = 16) {
-  d.n = n;
-  d.nstage = 0;
-  int m = n;
-  const int odd[4] = {11, 7, 5, 3};
-  for (int r : odd)
-    while (m % r == 0) {
-      if (d.nstage >= FFT_MAX_STAGES) return false;
-      d.radix[d.nstage++] = r;
-      m /= r;
-    }
-  int a = 0;
-  while (m % 2 == 0) { m /= 2; ++a; }
-  if (m != 1) return false;
-  const int lg = maxr >= 16 ? 4 : 3;
-  while (a >= lg) {
-    if (d.nstage >= FFT_MAX_STAGES) return false;
-    d.radix[d.nstage++] = 1 << lg;
-    a -= lg;
-  }
-  if (a > 0) {
-    if (d.nstage >= FFT_MAX_STAGES) return false;
-    d.radix[d.nstage++] = 1 << a;
-  }
-  return true;
-}
-
-static void digit_tables(const FftDesc& d, std::vector<int>& rev, std::vector<int>& pos) {
-  rev.assign(d.n, 0);
-  pos.assign(d.n, 0);
-  for (int k = 0; k < d.n; ++k) {
-    int kk = k, M = d.n, p = 0;
-    for (int s = 0; s < d.nstage; ++s) {
-      M /= d.radix[s];
-      p += (kk % d.radix[s]) * M;
-      kk /= d.radix[s];
-    }
-    pos[k] = p;
-    rev[p] = k;
-  }
-}
-
 template <typename T>
 static int upload_twiddles(pfbg_plan* pl, DevBuf& buf, int n) {
-  std::vector<cx2<T>> tw(n);
-  for (int t = 0; t < n; ++t) {
-    double ang = -2.0 * M_PI * (double)t / (double)n;
-    tw[t].x = (T)cos(ang);
-    tw[t].y = (T)sin(ang);
-  }
+  const std::vector<cx2<T>> tw = twiddles<T>(n);
   CKRC(dev_alloc(pl, buf, (size_t)n * sizeof(cx2<T>)));
   CK(cudaMemcpy(buf.p, tw.data(), (size_t)n * sizeof(cx2<T>), cudaMemcpyHostToDevice));
   return PFBG_OK;
 }
-
-static const size_t kMaxSmem = 232448;  // 227 KB opt-in dynamic shared memory per CTA on sm_100
 
 template <typename T>
 static int fused_setup_t(pfbg_plan* pl) {
@@ -448,15 +374,11 @@ static int fused_setup_t(pfbg_plan* pl) {
     const int v = atoi(cc);
     if (v == 1 || v == 2 || v == 4) pl->col_c = v < full_c ? v : full_c;
   }
-  const int want_c = pl->col_c;
   while (pl->col_c > 1 && fft_smem_bytes<T>(g.nu * pl->col_c) > kMaxSmem) pl->col_c /= 2;
-  // measured on B200 (15360^2 x 63 planes): with narrower-than-sector column blocks and one row CTA
-  // per SM the fused kernels lose to cuFFT (710 ms vs 520 ms per apply), so large grids stay on cuFFT
-  // unless PFBG_FFT=fused asks for them
-  // ... but half-sector blocks still win: measured at 8640^2 (the PSF grid of a 4096^2 field, 12 planes) the fused path
-  // takes 20.6 ms per Hessian apply against cuFFT's 25.9 ms in fp32 (34.6 vs 48.1 ms in fp64) and needs no work area
-  // and quarter-sector blocks (fp32 grids up to ~27k) are on par: 15360^2 x 33 planes, 312 ms fused vs 339 ms cuFFT
-  if (pl->col_c * 4 < want_c && !(env && strcmp(env, "fused") == 0)) return PFBG_OK;
+  // Narrower column blocks stay fused, measured on B200: half-sector blocks win at 8640^2 (the PSF grid of a 4096^2
+  // field, 12 planes: 20.6 ms per Hessian apply against cuFFT's 25.9 ms in fp32, 34.6 vs 48.1 ms in fp64, and no work
+  // area) and quarter-sector blocks (fp32 grids up to ~27k) are on par (15360^2 x 33 planes: 312 ms vs 339 ms).
+  // cuFFT takes what the shared-memory engine cannot: rows or one-column blocks beyond shared memory, other primes.
   if (fft_smem_bytes<T>(g.nv) > kMaxSmem) return PFBG_OK;
   if (fft_smem_bytes<T>(g.nu * pl->col_c) > kMaxSmem) return PFBG_OK;
   FftDesc du, dv;
@@ -919,11 +841,18 @@ static int wide_blocks(const pfbg_plan* pl, int64_t nact, int team) {
   return (int)(want < cap ? (want > 0 ? want : 1) : cap);
 }
 
-// fp64, 9 <= W <= 12: the DMMA run kernels (runs_mma.cuh) unless PFBG_WIDE_MMA=0 asks for the scalar team kernels
-static bool use_mma(const pfbg_plan* pl) {
-  if (pl->precision == PFBG_F32 || pl->gp.W < 9 || pl->gp.W > 12) return false;
-  const char* e = getenv("PFBG_WIDE_MMA");
-  return !(e && e[0] == '0');
+// kernel family of the spreading / gathering passes of a binding: direct (no per-sample records), the one-warp run
+// kernels (W <= 8), the scalar team kernels wide<3, 6, 4> (W <= 12) and wide<2, 8, 8>, or in fp64 at 9 <= W <= 12 the
+// DMMA run kernels (runs_mma.cuh) unless PFBG_WIDE_MMA=0 asks for the scalar team kernels
+enum RunArm { ARM_DIRECT, ARM_RUNS, ARM_WIDE6, ARM_WIDE8, ARM_MMA };
+static RunArm run_arm(const pfbg_plan* pl) {
+  if (!pl->use_runs) return ARM_DIRECT;
+  if (pl->gp.W <= 8) return ARM_RUNS;
+  if (pl->precision == PFBG_F64 && pl->gp.W <= 12) {
+    const char* e = getenv("PFBG_WIDE_MMA");
+    if (!(e && e[0] == '0')) return ARM_MMA;
+  }
+  return pl->gp.W <= 12 ? ARM_WIDE6 : ARM_WIDE8;
 }
 
 static int mma_blocks(const pfbg_plan* pl, int64_t nact) {
@@ -1088,6 +1017,34 @@ extern "C" int pfbg_bind_weights(pfbg_plan* pl, const void* wgt, uint32_t flags,
   return PFBG_OK;
 }
 
+extern "C" int pfbg_bind_weights_robust(pfbg_plan* pl, const void* wgt, int32_t nx_pad, int32_t ny_pad, double cell_x,
+                                        double cell_y, double robust, double usign, double vsign, uint32_t flags,
+                                        void* stream) {
+  if (!pl) return fail(PFBG_ERR_ARG, "null plan");
+  if (!pl->gp.row_snap || !pl->bound) return fail(PFBG_ERR_STATE, "the plan holds no batch of snapshots: pfbg_plan_set_batch and pfbg_bind_vis_batch first");
+  if (!wgt && pl->nvis > 0) return fail(PFBG_ERR_ARG, "null wgt");
+  if (nx_pad <= 0 || ny_pad <= 0) return fail(PFBG_ERR_ARG, "pad sizes must be positive, got %d x %d", nx_pad, ny_pad);
+  if (!std::isfinite(cell_x) || !std::isfinite(cell_y) || !(cell_x > 0) || !(cell_y > 0))
+    return fail(PFBG_ERR_ARG, "cell sizes must be finite and positive");
+  CK(cudaSetDevice(pl->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  pl->has_wgt = false;
+  if (pl->nvis == 0) return PFBG_OK;
+  const size_t rb = real_bytes(pl);
+  const size_t cbytes = (size_t)pl->nbatch * nx_pad * ny_pad * rb, coff = (cbytes + 255) & ~(size_t)255;
+  CKRC(dev_alloc(pl, pl->wgt, (size_t)pl->nvis * rb));
+  CKRC(dev_alloc(pl, pl->wcounts, coff + (size_t)pl->nbatch * 3 * sizeof(double)));
+  CK(cudaMemcpyAsync(pl->wgt.p, wgt, (size_t)pl->nvis * rb, (flags & PFBG_DEVICE_PTRS) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
+  // the bound fscale is fl(freq / c): a division by lightspeed = 1 reproduces pfbg_counts' cell exactly
+  CKRC(pfbg_counts_reweight(pl->precision, s, pl->nrow, pl->gp.nchan, nx_pad, ny_pad, cell_x, cell_y, usign, vsign, 1.0,
+                            (const double*)pl->uvw.p, (const double*)pl->fscale.p,
+                            pl->has_mask ? (const uint8_t*)pl->mask.p : nullptr, pl->gp.row_snap, pl->nbatch, robust,
+                            pl->wcounts.p, (double*)((char*)pl->wcounts.p + coff), pl->wgt.p));
+  if (!(flags & PFBG_DEVICE_PTRS)) CK(cudaStreamSynchronize(s));  // the caller may free its host array on return
+  pl->has_wgt = true;
+  return PFBG_OK;
+}
+
 extern "C" int pfbg_bin_dump(pfbg_plan* pl, int32_t* iu0, int32_t* iv0, int32_t* ip0, uint64_t* key,
                              uint32_t* sorted_idx) {
   if (!pl) return fail(PFBG_ERR_ARG, "null plan");
@@ -1124,46 +1081,44 @@ template <typename T>
 static int run_spread(pfbg_plan* pl, cudaStream_t s, const void* vis, int64_t rs, int64_t cs, const void* wgt,
                       int vis_sorted, int apply_phase) {
   using C = typename cplx_of<T>::type;
-  if (pl->nactive > 0 && pl->use_runs && pl->gp.W > 8) {
-    unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + 16);  // slice counter of this launch
-    CK(cudaMemsetAsync(queue, 0, 8, s));
-    bool mma = false;
-    if constexpr (sizeof(T) == 8) {
-      if (use_mma(pl)) {
-        mma = true;
+  if (pl->nactive == 0) return PFBG_OK;
+  const RunArm arm = run_arm(pl);
+  const VisRec<T>* recs = (const VisRec<T>*)pl->recs.p;
+  unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + 16);  // slice counter of this launch
+  if (arm != ARM_DIRECT) CK(cudaMemsetAsync(queue, 0, 8, s));
+  switch (arm) {
+    case ARM_MMA:
+      if constexpr (sizeof(T) == 8)
         k_grid_runs_mma<<<mma_blocks(pl, pl->nactive), MMA_R * MMA_TEAMS * 32, 0, s>>>(
-            pl->gp, (const VisRec<double>*)pl->recs.p, pl->nactive, (const double2*)vis, rs, cs, (const double*)wgt,
-            (double2*)pl->grid.p, vis_sorted, apply_phase, queue);
-      }
-    }
-    if (mma) {
-    } else if (pl->gp.W <= 12)
+            pl->gp, recs, pl->nactive, (const double2*)vis, rs, cs, (const double*)wgt, (double2*)pl->grid.p,
+            vis_sorted, apply_phase, queue);
+      break;
+    case ARM_WIDE6:
       k_grid_runs_wide<T, 3, 6, 4><<<wide_blocks(pl, pl->nactive, 4), WIDE_WARPS * 32, 0, s>>>(
-          pl->gp, (const VisRec<T>*)pl->recs.p, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p,
-          vis_sorted, apply_phase, queue);
-    else
+          pl->gp, recs, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p, vis_sorted, apply_phase,
+          queue);
+      break;
+    case ARM_WIDE8:
       k_grid_runs_wide<T, 2, 8, 8><<<wide_blocks(pl, pl->nactive, 8), WIDE_WARPS * 32, 0, s>>>(
-          pl->gp, (const VisRec<T>*)pl->recs.p, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p,
-          vis_sorted, apply_phase, queue);
-    LAUNCHED();
-    CK(cudaGetLastError());
-  } else if (pl->nactive > 0 && pl->use_runs) {
-    unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + 16);  // slice counter of this launch
-    CK(cudaMemsetAsync(queue, 0, 8, s));
-    const int ctas = 3;  // resident CTAs per SM
-    const int slice = run_slice(pl, pl->nactive, RUN_WARPS, ctas);
-    k_grid_runs<T><<<run_blocks(pl, pl->nactive, RUN_WARPS, ctas), RUN_WARPS * 32, 0, s>>>(
-        pl->gp, (const VisRec<T>*)pl->recs.p, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p,
-        vis_sorted, apply_phase, queue, slice);
-    LAUNCHED();
-    CK(cudaGetLastError());
-  } else if (pl->nactive > 0) {
-    k_grid_direct<T><<<grid_blocks(pl, pl->nactive), 256, 0, s>>>(
-        pl->gp, (const double*)pl->uvw.p, (const double*)pl->fscale.p, (const uint32_t*)pl->sorted_idx.p, pl->nactive,
-        (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p, vis_sorted, apply_phase);
-    LAUNCHED();
-    CK(cudaGetLastError());
+          pl->gp, recs, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p, vis_sorted, apply_phase,
+          queue);
+      break;
+    case ARM_RUNS: {
+      const int ctas = 3;  // resident CTAs per SM
+      const int slice = run_slice(pl, pl->nactive, RUN_WARPS, ctas);
+      k_grid_runs<T><<<run_blocks(pl, pl->nactive, RUN_WARPS, ctas), RUN_WARPS * 32, 0, s>>>(
+          pl->gp, recs, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p, vis_sorted, apply_phase,
+          queue, slice);
+      break;
+    }
+    case ARM_DIRECT:
+      k_grid_direct<T><<<grid_blocks(pl, pl->nactive), 256, 0, s>>>(
+          pl->gp, (const double*)pl->uvw.p, (const double*)pl->fscale.p, (const uint32_t*)pl->sorted_idx.p, pl->nactive,
+          (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p, vis_sorted, apply_phase);
+      break;
   }
+  LAUNCHED();
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
@@ -1171,7 +1126,11 @@ template <typename T>
 static int run_gather(pfbg_plan* pl, cudaStream_t s, const void* wgt, void* vis_out, void* out_sorted, int apply_phase,
                       int vis_zeroed = 0) {
   using C = typename cplx_of<T>::type;
-  if (pl->nactive > 0 && pl->use_runs && pl->gp.W > 8) {
+  if (pl->nactive == 0) return PFBG_OK;
+  const RunArm arm = run_arm(pl);
+  const VisRec<T>* recs = (const VisRec<T>*)pl->recs.p;
+  const bool team = arm == ARM_WIDE6 || arm == ARM_WIDE8 || arm == ARM_MMA;
+  if (team) {
     // the R warps of a team add their row-partials atomically: start from zero
     if (out_sorted) CK(cudaMemsetAsync(out_sorted, 0, (size_t)pl->nactive * sizeof(C), s));
     else if (!pl->has_mask) CK(cudaMemsetAsync(vis_out, 0, (size_t)pl->nvis * sizeof(C), s));
@@ -1179,50 +1138,48 @@ static int run_gather(pfbg_plan* pl, cudaStream_t s, const void* wgt, void* vis_
       k_zero_active<C><<<(unsigned)((pl->nactive + 255) / 256), 256, 0, s>>>((C*)vis_out, (const uint32_t*)pl->sorted_idx.p, pl->nactive);
       LAUNCHED();
     }
-    unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + 32);  // one slice counter per row group (<= 8)
-    CK(cudaMemsetAsync(queue, 0, 64, s));
-    bool mma = false;
-    if constexpr (sizeof(T) == 8) {
-      if (use_mma(pl)) {
-        mma = true;
-        k_degrid_runs_mma<<<mma_blocks(pl, pl->nactive), MMA_R * MMA_TEAMS * 32, 0, s>>>(
-            pl->gp, (const VisRec<double>*)pl->recs.p, pl->nactive, (const double2*)pl->grid.p, (const double*)wgt,
-            (double2*)vis_out, (double2*)out_sorted, apply_phase, queue);
-      }
-    }
-    const size_t psm = (size_t)WIDE_WARPS * 16 * 32 * sizeof(C);  // per-sample lane partials (see k_degrid_runs_wide)
-    // (per device and cheap: set on every launch rather than caching it per process)
-    if (mma) {
-    } else if (pl->gp.W <= 12) CK(cudaFuncSetAttribute(k_degrid_runs_wide<T, 3, 6, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
-    else CK(cudaFuncSetAttribute(k_degrid_runs_wide<T, 2, 8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
-    if (mma) {
-    } else if (pl->gp.W <= 12)
-      k_degrid_runs_wide<T, 3, 6, 4><<<wide_blocks(pl, pl->nactive, 4), WIDE_WARPS * 32, psm, s>>>(
-          pl->gp, (const VisRec<T>*)pl->recs.p, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out,
-          (C*)out_sorted, apply_phase, queue);
-    else
-      k_degrid_runs_wide<T, 2, 8, 8><<<wide_blocks(pl, pl->nactive, 8), WIDE_WARPS * 32, psm, s>>>(
-          pl->gp, (const VisRec<T>*)pl->recs.p, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out,
-          (C*)out_sorted, apply_phase, queue);
-    LAUNCHED();
-    CK(cudaGetLastError());
-  } else if (pl->nactive > 0 && pl->use_runs) {
-    unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + 24);
-    CK(cudaMemsetAsync(queue, 0, 8, s));
-    const int ctas = 5;  // resident CTAs per SM
-    const int slice = run_slice(pl, pl->nactive, DEG_WARPS, ctas);
-    k_degrid_runs<T><<<run_blocks(pl, pl->nactive, DEG_WARPS, ctas), DEG_WARPS * 32, 0, s>>>(
-        pl->gp, (const VisRec<T>*)pl->recs.p, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out,
-        (C*)out_sorted, apply_phase, queue, slice);
-    LAUNCHED();
-    CK(cudaGetLastError());
-  } else if (pl->nactive > 0) {
-    k_degrid_direct<T><<<grid_blocks(pl, pl->nactive), 256, 0, s>>>(
-        pl->gp, (const double*)pl->uvw.p, (const double*)pl->fscale.p, (const uint32_t*)pl->sorted_idx.p, pl->nactive,
-        (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out, (C*)out_sorted, apply_phase);
-    LAUNCHED();
-    CK(cudaGetLastError());
   }
+  // slice counters of this launch: one per row group (<= 8) for the team kernels
+  unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + (team ? 32 : 24));
+  if (arm != ARM_DIRECT) CK(cudaMemsetAsync(queue, 0, team ? 64 : 8, s));
+  // per-sample lane partials of the team kernels (see k_degrid_runs_wide); the attribute is per device and cheap: set
+  // on every launch rather than cached per process
+  const size_t psm = (size_t)WIDE_WARPS * 16 * 32 * sizeof(C);
+  switch (arm) {
+    case ARM_MMA:
+      if constexpr (sizeof(T) == 8)
+        k_degrid_runs_mma<<<mma_blocks(pl, pl->nactive), MMA_R * MMA_TEAMS * 32, 0, s>>>(
+            pl->gp, recs, pl->nactive, (const double2*)pl->grid.p, (const double*)wgt, (double2*)vis_out,
+            (double2*)out_sorted, apply_phase, queue);
+      break;
+    case ARM_WIDE6:
+      CK(cudaFuncSetAttribute(k_degrid_runs_wide<T, 3, 6, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
+      k_degrid_runs_wide<T, 3, 6, 4><<<wide_blocks(pl, pl->nactive, 4), WIDE_WARPS * 32, psm, s>>>(
+          pl->gp, recs, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out, (C*)out_sorted, apply_phase,
+          queue);
+      break;
+    case ARM_WIDE8:
+      CK(cudaFuncSetAttribute(k_degrid_runs_wide<T, 2, 8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
+      k_degrid_runs_wide<T, 2, 8, 8><<<wide_blocks(pl, pl->nactive, 8), WIDE_WARPS * 32, psm, s>>>(
+          pl->gp, recs, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out, (C*)out_sorted, apply_phase,
+          queue);
+      break;
+    case ARM_RUNS: {
+      const int ctas = 5;  // resident CTAs per SM
+      const int slice = run_slice(pl, pl->nactive, DEG_WARPS, ctas);
+      k_degrid_runs<T><<<run_blocks(pl, pl->nactive, DEG_WARPS, ctas), DEG_WARPS * 32, 0, s>>>(
+          pl->gp, recs, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out, (C*)out_sorted, apply_phase,
+          queue, slice);
+      break;
+    }
+    case ARM_DIRECT:
+      k_degrid_direct<T><<<grid_blocks(pl, pl->nactive), 256, 0, s>>>(
+          pl->gp, (const double*)pl->uvw.p, (const double*)pl->fscale.p, (const uint32_t*)pl->sorted_idx.p, pl->nactive,
+          (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out, (C*)out_sorted, apply_phase);
+      break;
+  }
+  LAUNCHED();
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
@@ -1250,19 +1207,6 @@ static int run_grid2img(pfbg_plan* pl, cudaStream_t s, const void* beam, const v
   return PFBG_OK;
 }
 
-// threads per CTA for a row transform: the multiple of 32 (<= cap, >= cap/2) that balances the
-// radix-16 stage best (n/16 butterflies)
-static int row_threads(int n, int cap, int radix = 16) {
-  int nb = n / radix, best = cap;
-  double best_eff = 0.0;
-  for (int t = cap; t >= cap / 2; t -= 32) {
-    int per = (nb + t - 1) / t;
-    double eff = (double)nb / ((double)per * t);
-    if (eff > best_eff + 1e-9) { best_eff = eff; best = t; }
-  }
-  return best;
-}
-
 // TMA-fed pair-engine column pass (cols2.cuh) over logical planes [ft.q0, ft.q0 + nq): loads come from the local
 // stack (slot 0 = logical plane slot0), results go to `out_biased` (logical plane q at out_biased + q nu nv)
 static int run_cols2(pfbg_plan* pl, cudaStream_t s, const FusedTabs& ft, int slot0, int nq, bool inverse,
@@ -1283,6 +1227,89 @@ static int run_cols2(pfbg_plan* pl, cudaStream_t s, const FusedTabs& ft, int slo
   return PFBG_OK;
 }
 
+// Row pass of planes [ft.q0, ft.q0 + nq): the first nq2 on the pair engine (fp32, two planes per CTA; a last odd plane
+// would cost a whole pair slot there, the one-plane kernel does it for ~0.55 of one: C2 has 4 bands with an odd plane
+// count), the rest on the one-plane kernel, whose BIG variant (480-768 threads) takes rows whose FFT leaves one CTA per
+// SM unless PFBG_ROWS_SMALL asks for the small one
+struct RowSplit { int nq2, threads; bool big; };
+template <typename T>
+static RowSplit row_split(const pfbg_plan* pl, int nq) {
+  const bool big = fft_smem_bytes<T>(pl->gp.nv) > (size_t)ROWS_BIG_SMEM && !getenv("PFBG_ROWS_SMALL");
+  const int cap = !big ? ROWS_MAX_THREADS : sizeof(T) == 4 ? ROWS_BIG_THREADS_F32 : ROWS_BIG_THREADS_F64;
+  return {sizeof(T) == 4 && pl->rows2 ? nq & ~1 : 0, row_threads(pl->gp.nv, cap, sizeof(T) == 8 ? 8 : 16), big};
+}
+
+// forward row pass (pad + screen the image, FFT along v) of planes [ft.q0, ft.q0 + nq) into the biased stack
+template <typename T>
+static int run_rows_fwd(pfbg_plan* pl, cudaStream_t s, const FusedTabs& ft, int nq, const void* x, const void* beam,
+                        typename cplx_of<T>::type* stack) {
+  const GParams& g = pl->gp;
+  const RowSplit r = row_split<T>(pl, nq);
+  const int nq2 = r.nq2;
+  if constexpr (sizeof(T) == 4) {
+    if (nq2 > 0) {
+      cudaError_t e = rows2_fwd_launch(g, ft, nq2, g.fast_screen != 0, (const float*)x, (const float*)beam,
+                                       (const float*)pl->corr.p, (float2*)stack, s);
+      if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "k_rows2_fwd launch: %s", cudaGetErrorString(e));
+      LAUNCHED();
+    }
+  }
+  if (nq2 < nq) {
+    auto k_rows = r.big ? &k_rows_fwd<T, false, true> : &k_rows_fwd<T, false>;
+    if constexpr (sizeof(T) == 4) {
+      if (g.fast_screen) k_rows = r.big ? &k_rows_fwd<T, true, true> : &k_rows_fwd<T, true>;
+    }
+    FusedTabs ft1 = ft;
+    ft1.q0 = ft.q0 + nq2;
+    k_rows<<<dim3(nq - nq2, g.nx), r.threads, fft_smem_bytes<T>(g.nv), s>>>(g, ft1, (const T*)x, (const T*)beam,
+                                                                        (const T*)pl->corr.p, stack);
+    LAUNCHED();
+  }
+  CK(cudaGetLastError());
+  return PFBG_OK;
+}
+
+// inverse row pass (FFT along v, screen + crop) of planes [ft.q0, ft.q0 + nq), accumulated into accimg
+template <typename T>
+static int run_rows_inv(pfbg_plan* pl, cudaStream_t s, const FusedTabs& ft, int nq,
+                        const typename cplx_of<T>::type* stack) {
+  const GParams& g = pl->gp;
+  const RowSplit r = row_split<T>(pl, nq);
+  const int nq2 = r.nq2;
+  if constexpr (sizeof(T) == 4) {
+    if (nq2 > 0) {
+      cudaError_t e = rows2_inv_launch(g, ft, nq2, g.fast_screen != 0, (const float2*)stack, (double*)pl->accimg.p, s);
+      if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "k_rows2_inv launch: %s", cudaGetErrorString(e));
+      LAUNCHED();
+    }
+  }
+  if (nq2 < nq) {
+    auto k_rows = r.big ? &k_rows_inv<T, false, true> : &k_rows_inv<T, false>;
+    if constexpr (sizeof(T) == 4) {
+      if (g.fast_screen) k_rows = r.big ? &k_rows_inv<T, true, true> : &k_rows_inv<T, true>;
+    }
+    FusedTabs ft1 = ft;
+    ft1.q0 = ft.q0 + nq2;
+    k_rows<<<dim3(nq - nq2, g.nx), r.threads, fft_smem_bytes<T>(g.nv), s>>>(g, ft1, stack, (double*)pl->accimg.p);
+    LAUNCHED();
+  }
+  CK(cudaGetLastError());
+  return PFBG_OK;
+}
+
+// one-plane column pass (fused_fft.cuh) of planes [ft.q0, ft.q0 + nq) in blocks of pl->col_c columns, src -> dst
+template <typename T>
+static int run_cols(pfbg_plan* pl, cudaStream_t s, const FusedTabs& ft, int nq, bool inverse,
+                    const typename cplx_of<T>::type* src, typename cplx_of<T>::type* dst) {
+  const int cc = pl->col_c;
+  const auto k_cols = inverse ? (cc == 4 ? &k_cols_inv<T, 4> : cc == 2 ? &k_cols_inv<T, 2> : &k_cols_inv<T, 1>)
+                              : (cc == 4 ? &k_cols_fwd<T, 4> : cc == 2 ? &k_cols_fwd<T, 2> : &k_cols_fwd<T, 1>);
+  k_cols<<<dim3(ft.b_len / cc, nq), 512, fft_smem_bytes<T>(pl->gp.nu * cc), s>>>(pl->gp, ft, src, dst);
+  LAUNCHED();
+  CK(cudaGetLastError());
+  return PFBG_OK;
+}
+
 // Plane subset of the fused transforms: logical planes [q0, q0 + nq).  `stack` is the local plane stack biased so
 // that logical plane q sits at stack + q * nu * nv (a helper of a split band stores plane q0 in slot 0); `remote`
 // (optional) is the peer-mapped stack of the band's owner: the forward column pass then writes there and the
@@ -1291,7 +1318,6 @@ template <typename T>
 static int run_fused_fwd(pfbg_plan* pl, cudaStream_t s, const void* x, const void* beam, int q0 = 0, int nq = -1,
                          void* remote = nullptr) {
   using C = typename cplx_of<T>::type;
-  const int CC = pl->col_c;
   const GParams& g = pl->gp;
   if (nq < 0) nq = g.nplanes - (pl->split_role == 1 ? pl->split_nq : 0);
   if (nq == 0) return PFBG_OK;
@@ -1299,57 +1325,16 @@ static int run_fused_fwd(pfbg_plan* pl, cudaStream_t s, const void* x, const voi
   ft.q0 = q0;
   const int slot0 = pl->split_role == 2 ? g.nplanes - pl->split_nq : 0;  // logical plane held by slot 0
   C* stack = (C*)pl->grid.p - (int64_t)slot0 * g.nu * g.nv;
-  auto k_rows = &k_rows_fwd<T, false>;
-  int rows_cap = ROWS_MAX_THREADS;
-  const bool rows_big = fft_smem_bytes<T>(g.nv) > (size_t)ROWS_BIG_SMEM && !getenv("PFBG_ROWS_SMALL");
-  if (rows_big) {
-    k_rows = &k_rows_fwd<T, false, true>;
-    rows_cap = sizeof(T) == 4 ? ROWS_BIG_THREADS_F32 : ROWS_BIG_THREADS_F64;
-  }
-  if constexpr (sizeof(T) == 4) {
-    if (g.fast_screen) k_rows = rows_big ? &k_rows_fwd<T, true, true> : &k_rows_fwd<T, true>;
-  }
-  // The pair engine transforms two planes per CTA; a last odd plane would cost a whole pair slot there, the one-plane
-  // kernel does it for ~0.55 of one (C2: 4 of the 8 bands have an odd plane count)
-  int nq2 = 0;  // planes that go through the pair engine
-  if constexpr (sizeof(T) == 4) {
-    if (pl->rows2) {
-      nq2 = nq & ~1;
-      if (nq2 > 0) {
-        cudaError_t e = rows2_fwd_launch(g, ft, nq2, g.fast_screen != 0, (const float*)x, (const float*)beam,
-                                         (const float*)pl->corr.p, (float2*)stack, s);
-        if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "k_rows2_fwd launch: %s", cudaGetErrorString(e));
-        LAUNCHED();
-      }
-    }
-  }
-  if (nq2 < nq) {
-    FusedTabs ft1 = ft;
-    ft1.q0 = ft.q0 + nq2;
-    k_rows<<<dim3(nq - nq2, g.nx), row_threads(g.nv, rows_cap, sizeof(T) == 8 ? 8 : 16), fft_smem_bytes<T>(g.nv), s>>>(
-        g, ft1, (const T*)x, (const T*)beam, (const T*)pl->corr.p, stack);
-    LAUNCHED();
-  }
-  CK(cudaGetLastError());
-  const dim3 cgrid(ft.b_len / CC, nq);
-  const size_t csm = fft_smem_bytes<T>(g.nu * CC);
+  CKRC(run_rows_fwd<T>(pl, s, ft, nq, x, beam, stack));
   C* dst = remote ? (C*)remote : stack;
-  if constexpr (sizeof(T) == 4) {
-    if (pl->cols2) return run_cols2(pl, s, ft, slot0, nq, false, (float2*)dst);
-  }
-  if (CC == 4) k_cols_fwd<T, 4><<<cgrid, 512, csm, s>>>(g, ft, stack, dst);
-  else if (CC == 2) k_cols_fwd<T, 2><<<cgrid, 512, csm, s>>>(g, ft, stack, dst);
-  else k_cols_fwd<T, 1><<<cgrid, 512, csm, s>>>(g, ft, stack, dst);
-  LAUNCHED();
-  CK(cudaGetLastError());
-  return PFBG_OK;
+  if (pl->cols2) return run_cols2(pl, s, ft, slot0, nq, false, (float2*)dst);
+  return run_cols<T>(pl, s, ft, nq, false, stack, dst);
 }
 
 // inverse transforms of planes [q0, q0 + nq) accumulated into accimg (zeroed first)
 template <typename T>
 static int run_fused_inv_acc(pfbg_plan* pl, cudaStream_t s, int q0, int nq, const void* remote) {
   using C = typename cplx_of<T>::type;
-  const int CC = pl->col_c;
   const GParams& g = pl->gp;
   FusedTabs ft = pl->ftabs;
   ft.q0 = q0;
@@ -1358,53 +1343,10 @@ static int run_fused_inv_acc(pfbg_plan* pl, cudaStream_t s, int q0, int nq, cons
   const int64_t npix = (int64_t)img_elems(pl);
   CK(cudaMemsetAsync(pl->accimg.p, 0, (size_t)npix * sizeof(double), s));
   if (nq == 0) return PFBG_OK;
-  const dim3 cgrid(ft.b_len / CC, nq);
-  const size_t csm = fft_smem_bytes<T>(g.nu * CC);
-  const C* src = remote ? (const C*)remote : stack;
-  bool done = false;
-  if constexpr (sizeof(T) == 4) {
-    if (pl->cols2 && !remote) {  // (a helper's loads from the owner's peer-mapped stack stay on the old kernel)
-      CKRC(run_cols2(pl, s, ft, slot0, nq, true, (float2*)stack));
-      done = true;
-    }
-  }
-  if (!done) {
-    if (CC == 4) k_cols_inv<T, 4><<<cgrid, 512, csm, s>>>(g, ft, src, stack);
-    else if (CC == 2) k_cols_inv<T, 2><<<cgrid, 512, csm, s>>>(g, ft, src, stack);
-    else k_cols_inv<T, 1><<<cgrid, 512, csm, s>>>(g, ft, src, stack);
-    LAUNCHED();
-    CK(cudaGetLastError());
-  }
-  auto k_rows = &k_rows_inv<T, false>;
-  int rows_cap = ROWS_MAX_THREADS;
-  const bool rows_big = fft_smem_bytes<T>(g.nv) > (size_t)ROWS_BIG_SMEM && !getenv("PFBG_ROWS_SMALL");
-  if (rows_big) {
-    k_rows = &k_rows_inv<T, false, true>;
-    rows_cap = sizeof(T) == 4 ? ROWS_BIG_THREADS_F32 : ROWS_BIG_THREADS_F64;
-  }
-  if constexpr (sizeof(T) == 4) {
-    if (g.fast_screen) k_rows = rows_big ? &k_rows_inv<T, true, true> : &k_rows_inv<T, true>;
-  }
-  int nq2 = 0;  // planes that go through the pair engine (see run_fused_fwd)
-  if constexpr (sizeof(T) == 4) {
-    if (pl->rows2) {
-      nq2 = nq & ~1;
-      if (nq2 > 0) {
-        cudaError_t e = rows2_inv_launch(g, ft, nq2, g.fast_screen != 0, (const float2*)stack, (double*)pl->accimg.p, s);
-        if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "k_rows2_inv launch: %s", cudaGetErrorString(e));
-        LAUNCHED();
-      }
-    }
-  }
-  if (nq2 < nq) {
-    FusedTabs ft1 = ft;
-    ft1.q0 = ft.q0 + nq2;
-    k_rows<<<dim3(nq - nq2, g.nx), row_threads(g.nv, rows_cap, sizeof(T) == 8 ? 8 : 16), fft_smem_bytes<T>(g.nv), s>>>(
-        g, ft1, stack, (double*)pl->accimg.p);
-    LAUNCHED();
-  }
-  CK(cudaGetLastError());
-  return PFBG_OK;
+  // (a helper's loads from the owner's peer-mapped stack stay on the one-plane kernel)
+  if (pl->cols2 && !remote) CKRC(run_cols2(pl, s, ft, slot0, nq, true, (float2*)stack));
+  else CKRC(run_cols<T>(pl, s, ft, nq, true, remote ? (const C*)remote : stack, stack));
+  return run_rows_inv<T>(pl, s, ft, nq, stack);
 }
 
 static int split_wait(pfbg_plan* pl, cudaStream_t s, int slot);
@@ -1464,12 +1406,18 @@ static int zero_planes(pfbg_plan* pl, cudaStream_t s) {
   return PFBG_OK;
 }
 
+// preconditions of pfbg_grid / pfbg_grid_psf / pfbg_degrid / pfbg_hessian; only the Hessian serves a split band
+static int check_apply(const pfbg_plan* pl, bool split_ok) {
+  if (pl->split_role && !split_ok) return fail(PFBG_ERR_STATE, "plan is part of a band split: only pfbg_hessian / pfbg_split_helper_serve");
+  if (!pl->bound) return fail(PFBG_ERR_STATE, "no visibilities bound");
+  if (!pl->grid.p) return fail(PFBG_ERR_STATE, "the plan has no plane stack (created with PFBG_PLAN_EXTERNAL_STACK): lend one with pfbg_plan_set_stack");
+  return PFBG_OK;
+}
+
 extern "C" int pfbg_grid(pfbg_plan* pl, const void* vis, int64_t vis_rs, int64_t vis_cs, const void* wgt,
                          void* dirty, uint32_t flags, void* stream) {
   if (!pl || !dirty) return fail(PFBG_ERR_ARG, "null argument");
-  if (pl->split_role) return fail(PFBG_ERR_STATE, "plan is part of a band split: only pfbg_hessian / pfbg_split_helper_serve");
-  if (!pl->bound) return fail(PFBG_ERR_STATE, "no visibilities bound");
-  if (!pl->grid.p) return fail(PFBG_ERR_STATE, "the plan has no plane stack (created with PFBG_PLAN_EXTERNAL_STACK): lend one with pfbg_plan_set_stack");
+  CKRC(check_apply(pl, false));
   if (!vis && pl->nvis > 0) return fail(PFBG_ERR_ARG, "null vis");
   CK(cudaSetDevice(pl->device));
   cudaStream_t s = (cudaStream_t)stream;
@@ -1504,9 +1452,7 @@ extern "C" int pfbg_grid(pfbg_plan* pl, const void* vis, int64_t vis_rs, int64_t
 extern "C" int pfbg_grid_psf(pfbg_plan* pl, double x0, double y0, double sign, const void* wgt, void* dirty,
                              uint32_t flags, void* stream) {
   if (!pl || !dirty) return fail(PFBG_ERR_ARG, "null argument");
-  if (pl->split_role) return fail(PFBG_ERR_STATE, "plan is part of a band split: only pfbg_hessian / pfbg_split_helper_serve");
-  if (!pl->bound) return fail(PFBG_ERR_STATE, "no visibilities bound");
-  if (!pl->grid.p) return fail(PFBG_ERR_STATE, "the plan has no plane stack (created with PFBG_PLAN_EXTERNAL_STACK): lend one with pfbg_plan_set_stack");
+  CKRC(check_apply(pl, false));
   if (x0 * x0 + y0 * y0 >= 1.0) return fail(PFBG_ERR_ARG, "phase centre outside the unit sphere");
   CK(cudaSetDevice(pl->device));
   cudaStream_t s = (cudaStream_t)stream;
@@ -1544,9 +1490,7 @@ extern "C" int pfbg_grid_psf(pfbg_plan* pl, double x0, double y0, double sign, c
 extern "C" int pfbg_degrid(pfbg_plan* pl, const void* dirty, void* vis, const void* wgt, uint32_t flags,
                            void* stream) {
   if (!pl || !dirty) return fail(PFBG_ERR_ARG, "null argument");
-  if (pl->split_role) return fail(PFBG_ERR_STATE, "plan is part of a band split: only pfbg_hessian / pfbg_split_helper_serve");
-  if (!pl->bound) return fail(PFBG_ERR_STATE, "no visibilities bound");
-  if (!pl->grid.p) return fail(PFBG_ERR_STATE, "the plan has no plane stack (created with PFBG_PLAN_EXTERNAL_STACK): lend one with pfbg_plan_set_stack");
+  CKRC(check_apply(pl, false));
   if (!vis && pl->nvis > 0) return fail(PFBG_ERR_ARG, "null vis");
   CK(cudaSetDevice(pl->device));
   cudaStream_t s = (cudaStream_t)stream;
@@ -1588,8 +1532,7 @@ extern "C" int pfbg_degrid(pfbg_plan* pl, const void* dirty, void* vis, const vo
 extern "C" int pfbg_hessian(pfbg_plan* pl, const void* x, const void* beam, double wsum, double eta, void* out,
                             uint32_t flags, void* stream) {
   if (!pl || !x || !out) return fail(PFBG_ERR_ARG, "null argument");
-  if (!pl->bound) return fail(PFBG_ERR_STATE, "no visibilities bound");
-  if (!pl->grid.p) return fail(PFBG_ERR_STATE, "the plan has no plane stack (created with PFBG_PLAN_EXTERNAL_STACK): lend one with pfbg_plan_set_stack");
+  CKRC(check_apply(pl, true));
   if (pl->split_role == 2) return fail(PFBG_ERR_STATE, "split helper plans only serve (pfbg_split_helper_serve)");
   if (pl->split_role == 1 && !(flags & PFBG_DEVICE_PTRS)) return fail(PFBG_ERR_STATE, "split plans take device pointers");
   CK(cudaSetDevice(pl->device));
@@ -1942,413 +1885,6 @@ extern "C" int pfbg_split_end(pfbg_plan* pl) {
   return PFBG_OK;
 }
 
-// ---------------------------------------------------------------------------
-// imaging weights (utils/weighting.py:81-140, 143-208)
-// ---------------------------------------------------------------------------
-static WParams make_wparams(int64_t nrow, int nchan, int ncorr, int nx, int ny, double cell_x, double cell_y,
-                            double usign, double vsign) {
-  WParams w;
-  w.nrow = nrow; w.nchan = nchan; w.ncorr = ncorr; w.nx = nx; w.ny = ny;
-  w.u_cell = 1.0 / ((double)nx * cell_x);
-  w.umax = fabs(1.0 / cell_x / 2.0);
-  w.v_cell = 1.0 / ((double)ny * cell_y);
-  w.vmax = fabs(1.0 / cell_y / 2.0);
-  w.usign = usign; w.vsign = vsign; w.lightspeed = 299792458.0;
-  return w;
-}
-
-struct TmpBufs {
-  std::vector<void*> ptrs;
-  ~TmpBufs() { for (void* p : ptrs) cudaFree(p); }
-  int get(void** out, const void* src, size_t bytes, bool dev, bool copy, cudaStream_t s) {
-    if (dev) { *out = (void*)src; return PFBG_OK; }
-    void* p = nullptr;
-    cudaError_t e = cudaMalloc(&p, bytes ? bytes : 16);
-    if (e != cudaSuccess) return fail(PFBG_ERR_NOMEM, "cudaMalloc of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
-    ptrs.push_back(p);
-    if (copy && bytes) {
-      e = cudaMemcpyAsync(p, src, bytes, cudaMemcpyHostToDevice, s);
-      if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "H2D copy failed: %s", cudaGetErrorString(e));
-    }
-    *out = p;
-    return PFBG_OK;
-  }
-};
-
-// reduction launch of the counts kernels: blockIdx.y over up to kCountsGridsPerLaunch grids, ~1184 CTAs in all
-static dim3 counts_rgrid(int64_t ngrid) {
-  const int gy = (int)std::min<int64_t>(ngrid, kCountsGridsPerLaunch);
-  return dim3((unsigned)std::max(8, 1184 / gy), (unsigned)gy);
-}
-
-template <typename T>
-static int launch_counts(cudaStream_t s, const WParams& w, const double* uvw, const double* scale, const uint8_t* mask,
-                         const int* row_snap, const T* wgt, T* counts, size_t cbytes) {
-  CK(cudaMemsetAsync(counts, 0, cbytes, s));
-  const int64_t nvis = w.nrow * w.nchan;
-  if (nvis > 0) {
-    k_counts<T><<<(unsigned)((nvis + 255) / 256), 256, 0, s>>>(w, uvw, scale, mask, row_snap, wgt, counts, nullptr);
-    LAUNCHED();
-    CK(cudaGetLastError());
-  }
-  return PFBG_OK;
-}
-
-// counts (nsnap * ncorr grids) -> Briggs / uniform weights, in place on counts and wgt (weighting.py:143-208);
-// sums: 3 * nsnap * ncorr doubles of scratch.  No host synchronisation.
-template <typename T>
-static int launch_reweight(cudaStream_t s, const WParams& w, const double* uvw, const double* scale,
-                           const uint8_t* mask, const int* row_snap, int64_t nsnap, T* counts, double* sums,
-                           double robust, T* wgt) {
-  const int64_t ncell = (int64_t)w.nx * w.ny, ngrid = nsnap * w.ncorr, nvis = w.nrow * w.nchan;
-  const dim3 rg = counts_rgrid(ngrid);
-  CK(cudaMemsetAsync(sums, 0, (size_t)ngrid * 3 * sizeof(double), s));
-  k_counts_sums<T><<<rg, 256, 0, s>>>(counts, ncell, (int)ngrid, sums);
-  LAUNCHED();
-  if (robust > -2.0) {
-    const double numsqrt = 5.0 * pow(10.0, -robust);
-    k_counts_scale<T><<<rg, 256, 0, s>>>(counts, ncell, w.ncorr, (int)ngrid, sums, numsqrt * numsqrt);
-    LAUNCHED();
-  }
-  if (nvis > 0) {
-    k_apply_counts<T><<<(unsigned)((nvis + 255) / 256), 256, 0, s>>>(w, uvw, scale, mask, row_snap, counts, wgt);
-    LAUNCHED();
-  }
-  CK(cudaGetLastError());
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_counts(int32_t precision, int32_t device, const double* uvw, const double* freq,
-                           const uint8_t* mask, const void* wgt, int64_t nrow, int32_t nchan, int32_t ncorr,
-                           int32_t nx, int32_t ny, double cell_x, double cell_y, double usign, double vsign,
-                           void* counts, uint32_t flags, void* stream) {
-  if (!uvw || !freq || !wgt || !counts) return fail(PFBG_ERR_ARG, "null argument");
-  if (nrow < 0 || nchan <= 0 || ncorr <= 0 || nx <= 0 || ny <= 0) return fail(PFBG_ERR_ARG, "bad sizes");
-  if (precision != PFBG_F32 && precision != PFBG_F64) return fail(PFBG_ERR_ARG, "bad precision");
-  CK(cudaSetDevice(device));
-  cudaStream_t s = (cudaStream_t)stream;
-  const bool dev = flags & PFBG_DEVICE_PTRS;
-  const size_t rb = precision == PFBG_F32 ? 4 : 8;
-  const int64_t nvis = nrow * nchan;
-  const size_t cbytes = (size_t)ncorr * nx * ny * rb;
-  TmpBufs t;
-  void *duvw, *dfreq, *dmask = nullptr, *dwgt, *dcounts;
-  CKRC(t.get(&duvw, uvw, (size_t)nrow * 24, dev, true, s));
-  CKRC(t.get(&dfreq, freq, (size_t)nchan * 8, dev, true, s));
-  if (mask) CKRC(t.get(&dmask, mask, (size_t)nvis, dev, true, s));
-  CKRC(t.get(&dwgt, wgt, (size_t)ncorr * nvis * rb, dev, true, s));
-  CKRC(t.get(&dcounts, counts, cbytes, dev, false, s));
-  WParams w = make_wparams(nrow, nchan, ncorr, nx, ny, cell_x, cell_y, usign, vsign);
-  if (precision == PFBG_F32)
-    CKRC(launch_counts<float>(s, w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, (const float*)dwgt, (float*)dcounts, cbytes));
-  else
-    CKRC(launch_counts<double>(s, w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, (const double*)dwgt, (double*)dcounts, cbytes));
-  if (!dev) {
-    CK(cudaMemcpyAsync(counts, dcounts, cbytes, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-  }
-  return PFBG_OK;
-}
-
-// cell index dump for the bit-exact check: cells (nrow,nchan,2) int32, -1 = skipped
-extern "C" int pfbg_counts_cells(int32_t device, const double* uvw, const double* freq, const uint8_t* mask,
-                                 int64_t nrow, int32_t nchan, int32_t nx, int32_t ny, double cell_x, double cell_y,
-                                 double usign, double vsign, int32_t* cells) {
-  if (!uvw || !freq || !cells) return fail(PFBG_ERR_ARG, "null argument");
-  CK(cudaSetDevice(device));
-  const int64_t nvis = nrow * nchan;
-  TmpBufs t;
-  void *duvw, *dfreq, *dmask = nullptr, *dcells;
-  CKRC(t.get(&duvw, uvw, (size_t)nrow * 24, false, true, 0));
-  CKRC(t.get(&dfreq, freq, (size_t)nchan * 8, false, true, 0));
-  if (mask) CKRC(t.get(&dmask, mask, (size_t)nvis, false, true, 0));
-  CKRC(t.get(&dcells, cells, (size_t)nvis * 8, false, false, 0));
-  WParams w = make_wparams(nrow, nchan, 1, nx, ny, cell_x, cell_y, usign, vsign);
-  if (nvis > 0) {
-    k_counts<float><<<(unsigned)((nvis + 255) / 256), 256>>>(w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, nullptr, nullptr, (int32_t*)dcells);
-    LAUNCHED();
-    CK(cudaGetLastError());
-    CK(cudaMemcpy(cells, dcells, (size_t)nvis * 8, cudaMemcpyDeviceToHost));
-  }
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_counts_to_weights(int32_t precision, int32_t device, void* counts, const double* uvw,
-                                      const double* freq, void* wgt, const uint8_t* mask, int64_t nrow,
-                                      int32_t nchan, int32_t ncorr, int32_t nx, int32_t ny, double cell_x,
-                                      double cell_y, double robust, double usign, double vsign, uint32_t flags,
-                                      void* stream) {
-  if (!uvw || !freq || !wgt || !counts) return fail(PFBG_ERR_ARG, "null argument");
-  if (nrow < 0 || nchan <= 0 || ncorr <= 0 || ncorr > 16 || nx <= 0 || ny <= 0) return fail(PFBG_ERR_ARG, "bad sizes");
-  if (precision != PFBG_F32 && precision != PFBG_F64) return fail(PFBG_ERR_ARG, "bad precision");
-  CK(cudaSetDevice(device));
-  cudaStream_t s = (cudaStream_t)stream;
-  const bool dev = flags & PFBG_DEVICE_PTRS;
-  const size_t rb = precision == PFBG_F32 ? 4 : 8;
-  const int64_t nvis = nrow * nchan, ncell = (int64_t)nx * ny;
-  const size_t cbytes = (size_t)ncorr * ncell * rb, wbytes = (size_t)ncorr * nvis * rb;
-  TmpBufs t;
-  void *duvw, *dfreq, *dmask = nullptr, *dwgt, *dcounts, *dsums;
-  CKRC(t.get(&duvw, uvw, (size_t)nrow * 24, dev, true, s));
-  CKRC(t.get(&dfreq, freq, (size_t)nchan * 8, dev, true, s));
-  if (mask) CKRC(t.get(&dmask, mask, (size_t)nvis, dev, true, s));
-  CKRC(t.get(&dwgt, wgt, wbytes, dev, true, s));
-  CKRC(t.get(&dcounts, counts, cbytes, dev, true, s));
-  CKRC(t.get(&dsums, nullptr, (size_t)ncorr * 3 * 8, false, false, s));
-  WParams w = make_wparams(nrow, nchan, ncorr, nx, ny, cell_x, cell_y, usign, vsign);
-  if (precision == PFBG_F32)
-    CKRC(launch_reweight<float>(s, w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, 1, (float*)dcounts, (double*)dsums, robust, (float*)dwgt));
-  else
-    CKRC(launch_reweight<double>(s, w, (const double*)duvw, (const double*)dfreq, (const uint8_t*)dmask, nullptr, 1, (double*)dcounts, (double*)dsums, robust, (double*)dwgt));
-  if (!dev) {
-    CK(cudaMemcpyAsync(wgt, dwgt, wbytes, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(counts, dcounts, cbytes, cudaMemcpyDeviceToHost, s));
-  }
-  CK(cudaStreamSynchronize(s));
-  return PFBG_OK;
-}
-
-// Arguments of the batched re-weighting, checked before anything is launched.
-static int check_batch_weights(int64_t nbatch, const int64_t* row_offsets, int64_t nrow, int32_t nx_pad,
-                               int32_t ny_pad, double cell_x, double cell_y) {
-  if (nbatch < 1) return fail(PFBG_ERR_ARG, "nbatch must be positive");
-  if (!row_offsets) return fail(PFBG_ERR_ARG, "null row_offsets");
-  if (row_offsets[0] != 0 || row_offsets[nbatch] != nrow) return fail(PFBG_ERR_ARG, "row_offsets must run from 0 to nrow = %lld", (long long)nrow);
-  for (int64_t b = 0; b < nbatch; ++b)
-    if (row_offsets[b + 1] < row_offsets[b]) return fail(PFBG_ERR_ARG, "row_offsets must not decrease (snapshot %lld)", (long long)b);
-  if (nx_pad <= 0 || ny_pad <= 0) return fail(PFBG_ERR_ARG, "pad sizes must be positive, got %d x %d", nx_pad, ny_pad);
-  if (!std::isfinite(cell_x) || !std::isfinite(cell_y) || !(cell_x > 0) || !(cell_y > 0))
-    return fail(PFBG_ERR_ARG, "cell sizes must be finite and positive");
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_counts_to_weights_batch(int32_t precision, int32_t device, int32_t nbatch, const int64_t* row_offsets,
-                                            const double* uvw, const double* freq, const uint8_t* mask, void* wgt,
-                                            int64_t nrow, int32_t nchan, int32_t nx_pad, int32_t ny_pad, double cell_x,
-                                            double cell_y, double robust, double usign, double vsign, void* counts,
-                                            uint32_t flags, void* stream) {
-  if (precision != PFBG_F32 && precision != PFBG_F64) return fail(PFBG_ERR_ARG, "bad precision");
-  if (nrow < 0 || nchan <= 0) return fail(PFBG_ERR_ARG, "bad nrow / nchan");
-  if (!freq || (nrow > 0 && (!uvw || !wgt))) return fail(PFBG_ERR_ARG, "null argument");
-  CKRC(check_batch_weights(nbatch, row_offsets, nrow, nx_pad, ny_pad, cell_x, cell_y));
-  std::vector<int> rs((size_t)(nrow > 0 ? nrow : 1));
-  for (int b = 0; b < nbatch; ++b)
-    for (int64_t r = row_offsets[b]; r < row_offsets[b + 1]; ++r) rs[(size_t)r] = b;
-  CK(cudaSetDevice(device));
-  cudaStream_t s = (cudaStream_t)stream;
-  const bool dev = flags & PFBG_DEVICE_PTRS;
-  const size_t rb = precision == PFBG_F32 ? 4 : 8;
-  const int64_t nvis = nrow * nchan;
-  const size_t cbytes = (size_t)nbatch * nx_pad * ny_pad * rb, wbytes = (size_t)nvis * rb;
-  TmpBufs t;
-  void *duvw, *dfreq, *dmask = nullptr, *dwgt, *dcounts, *dsums, *drs;
-  CKRC(t.get(&duvw, uvw, (size_t)nrow * 24, dev, true, s));
-  CKRC(t.get(&dfreq, freq, (size_t)nchan * 8, dev, true, s));
-  if (mask) CKRC(t.get(&dmask, mask, (size_t)nvis, dev, true, s));
-  CKRC(t.get(&dwgt, wgt, wbytes, dev, true, s));
-  CKRC(t.get(&dcounts, counts, cbytes, dev && counts, false, s));
-  CKRC(t.get(&dsums, nullptr, (size_t)nbatch * 3 * 8, false, false, s));
-  CKRC(t.get(&drs, rs.data(), rs.size() * 4, false, true, s));
-  WParams w = make_wparams(nrow, nchan, 1, nx_pad, ny_pad, cell_x, cell_y, usign, vsign);
-  const double* u = (const double*)duvw;
-  const double* f = (const double*)dfreq;
-  const uint8_t* m = (const uint8_t*)dmask;
-  const int* r = (const int*)drs;
-  if (precision == PFBG_F32) {
-    CKRC(launch_counts<float>(s, w, u, f, m, r, (const float*)dwgt, (float*)dcounts, cbytes));
-    CKRC(launch_reweight<float>(s, w, u, f, m, r, nbatch, (float*)dcounts, (double*)dsums, robust, (float*)dwgt));
-  } else {
-    CKRC(launch_counts<double>(s, w, u, f, m, r, (const double*)dwgt, (double*)dcounts, cbytes));
-    CKRC(launch_reweight<double>(s, w, u, f, m, r, nbatch, (double*)dcounts, (double*)dsums, robust, (double*)dwgt));
-  }
-  if (!dev) {
-    if (nvis > 0) CK(cudaMemcpyAsync(wgt, dwgt, wbytes, cudaMemcpyDeviceToHost, s));
-    if (counts) CK(cudaMemcpyAsync(counts, dcounts, cbytes, cudaMemcpyDeviceToHost, s));
-  }
-  CK(cudaStreamSynchronize(s));
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_bind_weights_robust(pfbg_plan* pl, const void* wgt, int32_t nx_pad, int32_t ny_pad, double cell_x,
-                                        double cell_y, double robust, double usign, double vsign, uint32_t flags,
-                                        void* stream) {
-  if (!pl) return fail(PFBG_ERR_ARG, "null plan");
-  if (!pl->gp.row_snap || !pl->bound) return fail(PFBG_ERR_STATE, "the plan holds no batch of snapshots: pfbg_plan_set_batch and pfbg_bind_vis_batch first");
-  if (!wgt && pl->nvis > 0) return fail(PFBG_ERR_ARG, "null wgt");
-  if (nx_pad <= 0 || ny_pad <= 0) return fail(PFBG_ERR_ARG, "pad sizes must be positive, got %d x %d", nx_pad, ny_pad);
-  if (!std::isfinite(cell_x) || !std::isfinite(cell_y) || !(cell_x > 0) || !(cell_y > 0))
-    return fail(PFBG_ERR_ARG, "cell sizes must be finite and positive");
-  CK(cudaSetDevice(pl->device));
-  cudaStream_t s = (cudaStream_t)stream;
-  pl->has_wgt = false;
-  if (pl->nvis == 0) return PFBG_OK;
-  const size_t rb = real_bytes(pl);
-  const size_t cbytes = (size_t)pl->nbatch * nx_pad * ny_pad * rb, coff = (cbytes + 255) & ~(size_t)255;
-  CKRC(dev_alloc(pl, pl->wgt, (size_t)pl->nvis * rb));
-  CKRC(dev_alloc(pl, pl->wcounts, coff + (size_t)pl->nbatch * 3 * sizeof(double)));
-  CK(cudaMemcpyAsync(pl->wgt.p, wgt, (size_t)pl->nvis * rb, (flags & PFBG_DEVICE_PTRS) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
-  // the bound fscale is fl(freq / c): a division by lightspeed = 1 reproduces pfbg_counts' cell exactly
-  WParams w = make_wparams(pl->nrow, pl->gp.nchan, 1, nx_pad, ny_pad, cell_x, cell_y, usign, vsign);
-  w.lightspeed = 1.0;
-  const double* u = (const double*)pl->uvw.p;
-  const double* f = (const double*)pl->fscale.p;
-  const uint8_t* m = pl->has_mask ? (const uint8_t*)pl->mask.p : nullptr;
-  const int* r = pl->gp.row_snap;
-  double* sums = (double*)((char*)pl->wcounts.p + coff);
-  if (pl->precision == PFBG_F32) {
-    float* c = (float*)pl->wcounts.p;
-    CKRC(launch_counts<float>(s, w, u, f, m, r, (const float*)pl->wgt.p, c, cbytes));
-    CKRC(launch_reweight<float>(s, w, u, f, m, r, pl->nbatch, c, sums, robust, (float*)pl->wgt.p));
-  } else {
-    double* c = (double*)pl->wcounts.p;
-    CKRC(launch_counts<double>(s, w, u, f, m, r, (const double*)pl->wgt.p, c, cbytes));
-    CKRC(launch_reweight<double>(s, w, u, f, m, r, pl->nbatch, c, sums, robust, (double*)pl->wgt.p));
-  }
-  if (!(flags & PFBG_DEVICE_PTRS)) CK(cudaStreamSynchronize(s));  // the caller may free its host array on return
-  pl->has_wgt = true;
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_l2_reweight(int32_t precision, int32_t device, const void* resvis, const void* wgtp,
-                                const uint8_t* mask, void* wgt, int64_t nvis, int32_t ncorr, double dof,
-                                double* ovar_out, int32_t* applied, uint32_t flags, void* stream) {
-  if (!resvis || !wgt || !ovar_out || !applied) return fail(PFBG_ERR_ARG, "null argument");
-  if (nvis < 0 || ncorr <= 0 || ncorr > 16) return fail(PFBG_ERR_ARG, "bad sizes");
-  if (precision != PFBG_F32 && precision != PFBG_F64) return fail(PFBG_ERR_ARG, "bad precision");
-  CK(cudaSetDevice(device));
-  cudaStream_t s = (cudaStream_t)stream;
-  const bool dev = flags & PFBG_DEVICE_PTRS;
-  const size_t rb = precision == PFBG_F32 ? 4 : 8;
-  const size_t wbytes = (size_t)ncorr * nvis * rb;
-  *applied = 0;
-  TmpBufs t;
-  void *drv, *dp = nullptr, *dmask = nullptr, *dwgt, *dsums;
-  CKRC(t.get(&drv, resvis, 2 * wbytes, dev, true, s));
-  if (wgtp) CKRC(t.get(&dp, wgtp, wbytes, dev, true, s));
-  if (mask) CKRC(t.get(&dmask, mask, (size_t)nvis, dev, true, s));
-  CKRC(t.get(&dwgt, wgt, wbytes, dev, true, s));
-  // 17 doubles of reduction scratch, held for this call (pfbg_scratch_get: recycled blocks, no cudaMalloc per call)
-  struct Hold {
-    int dev; void* p;
-    ~Hold() { pfbg_scratch_put(dev, p); }
-  } hold{device, pfbg_scratch_get(device)};
-  if (!hold.p) return fail(PFBG_ERR_NOMEM, "no reduction scratch on device %d", device);
-  dsums = hold.p;
-  CK(cudaMemsetAsync(dsums, 0, 17 * 8, s));
-  dim3 rgrid(592, ncorr);
-  if (nvis > 0) {
-    if (precision == PFBG_F32) k_l2_ssq<float><<<rgrid, 256, 0, s>>>((const float*)drv, (const float*)dp, (const uint8_t*)dmask, nvis, (double*)dsums);
-    else k_l2_ssq<double><<<rgrid, 256, 0, s>>>((const double*)drv, (const double*)dp, (const uint8_t*)dmask, nvis, (double*)dsums);
-    LAUNCHED();
-  }
-  double sums[17];
-  CK(cudaMemcpyAsync(sums, dsums, sizeof sums, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  bool all_nonzero = true;
-  for (int c = 0; c < ncorr; ++c) {
-    ovar_out[c] = sums[c] / sums[ncorr];  // 0/0 -> NaN like numpy; NaN is truthy there too
-    if (ovar_out[c] == 0.0) all_nonzero = false;
-  }
-  if (!all_nonzero) return PFBG_OK;
-  CK(cudaMemcpyAsync(dsums, ovar_out, ncorr * 8, cudaMemcpyHostToDevice, s));
-  if (nvis > 0) {
-    if (precision == PFBG_F32) k_l2_apply<float><<<rgrid, 256, 0, s>>>((const float*)drv, (const float*)dp, (float*)dwgt, nvis, (const double*)dsums, dof, dof + 2.0);
-    else k_l2_apply<double><<<rgrid, 256, 0, s>>>((const double*)drv, (const double*)dp, (double*)dwgt, nvis, (const double*)dsums, dof, dof + 2.0);
-    LAUNCHED();
-    CK(cudaGetLastError());
-    if (!dev) CK(cudaMemcpyAsync(wgt, dwgt, wbytes, cudaMemcpyDeviceToHost, s));
-  }
-  CK(cudaStreamSynchronize(s));
-  *applied = 1;
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_weight_data_corr(int32_t precision, int32_t device, const void* data, const void* weight,
-                                     const void* jones, const int32_t* row_t, const int32_t* ant1, const int32_t* ant2,
-                                     int64_t nrow, int32_t nchan, int32_t ncorr, int64_t jones_elems, int64_t js_t,
-                                     int64_t js_a, int64_t js_c, void* vis, void* wgt, uint32_t flags, void* stream) {
-  if (!data || !weight || !jones || !row_t || !ant1 || !ant2 || !vis || !wgt) return fail(PFBG_ERR_ARG, "null argument");
-  if (nrow < 0 || nchan <= 0 || ncorr <= 0 || jones_elems <= 0) return fail(PFBG_ERR_ARG, "bad sizes");
-  if (precision != PFBG_F32 && precision != PFBG_F64) return fail(PFBG_ERR_ARG, "bad precision");
-  CK(cudaSetDevice(device));
-  cudaStream_t s = (cudaStream_t)stream;
-  const bool dev = flags & PFBG_DEVICE_PTRS;
-  const size_t rb = precision == PFBG_F32 ? 4 : 8;
-  const int64_t nvis = nrow * nchan;
-  TmpBufs t;
-  void *dd, *dw, *dj, *dt, *d1, *d2, *dv, *dg;
-  CKRC(t.get(&dd, data, (size_t)nvis * ncorr * 2 * rb, dev, true, s));
-  CKRC(t.get(&dw, weight, (size_t)nvis * ncorr * rb, dev, true, s));
-  CKRC(t.get(&dj, jones, (size_t)jones_elems * 2 * rb, dev, true, s));
-  CKRC(t.get(&dt, row_t, (size_t)nrow * 4, dev, true, s));
-  CKRC(t.get(&d1, ant1, (size_t)nrow * 4, dev, true, s));
-  CKRC(t.get(&d2, ant2, (size_t)nrow * 4, dev, true, s));
-  CKRC(t.get(&dv, vis, (size_t)nvis * 2 * rb, dev, false, s));
-  CKRC(t.get(&dg, wgt, (size_t)nvis * rb, dev, false, s));
-  CK(cudaMemsetAsync(dv, 0, (size_t)nvis * 2 * rb, s));
-  CK(cudaMemsetAsync(dg, 0, (size_t)nvis * rb, s));
-  if (nvis > 0) {
-    const unsigned grd = (unsigned)((nvis + 255) / 256);
-    if (precision == PFBG_F32)
-      k_weight_data_corr<float><<<grd, 256, 0, s>>>((const float2*)dd, (const float*)dw, (const float2*)dj, (const int32_t*)dt,
-                                                      (const int32_t*)d1, (const int32_t*)d2, nrow, nchan, ncorr, js_t, js_a, js_c,
-                                                      (float2*)dv, (float*)dg);
-    else
-      k_weight_data_corr<double><<<grd, 256, 0, s>>>((const double2*)dd, (const double*)dw, (const double2*)dj, (const int32_t*)dt,
-                                                       (const int32_t*)d1, (const int32_t*)d2, nrow, nchan, ncorr, js_t, js_a, js_c,
-                                                       (double2*)dv, (double*)dg);
-    LAUNCHED();
-    CK(cudaGetLastError());
-    if (!dev) {
-      CK(cudaMemcpyAsync(vis, dv, (size_t)nvis * 2 * rb, cudaMemcpyDeviceToHost, s));
-      CK(cudaMemcpyAsync(wgt, dg, (size_t)nvis * rb, cudaMemcpyDeviceToHost, s));
-    }
-  }
-  if (!dev) CK(cudaStreamSynchronize(s));
-  return PFBG_OK;
-}
-
-// ---------------------------------------------------------------------------
-// unit-test hook for the shared-memory FFT engine (fft.cuh)
-// ---------------------------------------------------------------------------
-template <typename T>
-static int debug_fft_t(int n, int batch, const void* in, void* out, int mode, int inverse) {
-  FftDesc d;
-  if (!factorize(n, d, sizeof(T) == 4 ? 16 : 8)) return fail(PFBG_ERR_ARG, "n=%d is not 2^a 3^b 5^c 7^d 11^e", n);
-  size_t bytes = (size_t)n * sizeof(cx2<T>);
-  if (fft_smem_bytes<T>(n) > kMaxSmem) return fail(PFBG_ERR_ARG, "n=%d does not fit shared memory", n);
-  std::vector<cx2<T>> tw(n);
-  for (int t = 0; t < n; ++t) {
-    double ang = -2.0 * M_PI * (double)t / (double)n;
-    tw[t].x = (T)cos(ang);
-    tw[t].y = (T)sin(ang);
-  }
-  std::vector<int> rev, pos;
-  digit_tables(d, rev, pos);
-  TmpBufs t;
-  void *dtw, *drev, *dpos, *din, *dout;
-  CKRC(t.get(&dtw, tw.data(), bytes, false, true, 0));
-  CKRC(t.get(&drev, rev.data(), (size_t)n * 4, false, true, 0));
-  CKRC(t.get(&dpos, pos.data(), (size_t)n * 4, false, true, 0));
-  CKRC(t.get(&din, in, bytes * batch, false, true, 0));
-  CKRC(t.get(&dout, out, bytes * batch, false, false, 0));
-  CK(cudaFuncSetAttribute(k_fft_debug<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  k_fft_debug<T><<<batch, 256, fft_smem_bytes<T>(n)>>>(d, (const cx2<T>*)dtw, (const int*)drev, (const int*)dpos, (const cx2<T>*)din,
-                                        (cx2<T>*)dout, mode, inverse);
-  LAUNCHED();
-  CK(cudaGetLastError());
-  CK(cudaMemcpy(out, dout, bytes * batch, cudaMemcpyDeviceToHost));
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_debug_fft1d(int32_t precision, int32_t device, int32_t n, int32_t batch, const void* in,
-                                void* out, int32_t mode, int32_t inverse) {
-  if (!in || !out || n < 2 || batch < 1) return fail(PFBG_ERR_ARG, "bad argument");
-  CK(cudaSetDevice(device));
-  return precision == PFBG_F32 ? debug_fft_t<float>(n, batch, in, out, mode, inverse)
-                               : debug_fft_t<double>(n, batch, in, out, mode, inverse);
-}
-
 // unit-test hook: the lean fp64 ES tap of the DMMA run kernels (runs_mma.cuh) at n positions x in [-1, 1]
 __global__ void k_debug_es_fast64(const double* __restrict__ x, double beta, int64_t n, double* __restrict__ out) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -2373,395 +1909,3 @@ extern "C" int pfbg_debug_es_fast64(int32_t device, int64_t n, const double* x, 
   return PFBG_OK;
 }
 
-extern "C" int pfbg_debug_fft2(int32_t device, int32_t n, int32_t np, int32_t batch, const void* in, void* out,
-                               int32_t inverse, int32_t aos) {
-  if (!in || !out || n < 2 || batch < 1) return fail(PFBG_ERR_ARG, "bad argument");
-  CK(cudaSetDevice(device));
-  FftDesc d;
-  if (!factorize(n, d, 16)) return fail(PFBG_ERR_ARG, "n=%d is not 2^a 3^b 5^c 7^d 11^e", n);
-  std::vector<cx2<float>> tw(n);
-  for (int t = 0; t < n; ++t) {
-    double ang = -2.0 * M_PI * (double)t / (double)n;
-    tw[t].x = (float)cos(ang);
-    tw[t].y = (float)sin(ang);
-  }
-  std::vector<int> rev, pos;
-  digit_tables(d, rev, pos);
-  const size_t bytes = (size_t)n * 8 * 2 * np * batch;
-  TmpBufs t;
-  void *dtw, *drev, *din, *dout;
-  CKRC(t.get(&dtw, tw.data(), (size_t)n * 8, false, true, 0));
-  CKRC(t.get(&drev, rev.data(), (size_t)n * 4, false, true, 0));
-  CKRC(t.get(&din, in, bytes, false, true, 0));
-  CKRC(t.get(&dout, out, bytes, false, false, 0));
-  cudaError_t e = fft2_debug_launch(d, np, (const float2*)dtw, (const int*)drev, (const float2*)din, (float2*)dout, batch,
-                                    inverse, aos);
-  if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "fft2 debug launch: %s", cudaGetErrorString(e));
-  LAUNCHED();
-  CK(cudaMemcpy(out, dout, bytes, cudaMemcpyDeviceToHost));
-  return PFBG_OK;
-}
-
-// ---------------------------------------------------------------------------
-// PSF-convolution Hessian (psfconv.cuh)
-// ---------------------------------------------------------------------------
-#include "psfconv.cuh"
-
-struct pfbg_conv {
-  int precision = 0, device = 0;
-  ConvTabs ct{};
-  int col_c = 1;
-  void *tw_u = nullptr, *tw_v = nullptr, *rev_u = nullptr, *rev_v = nullptr, *pos_v = nullptr;
-  void *khat = nullptr, *tmp = nullptr, *d_x = nullptr, *d_beam = nullptr, *d_out = nullptr;
-  bool has_kernel = false;
-  bool gauss = false;  // pfbg_conv_set_gauss: the analytic multiplier `gm`, no stored spectrum
-  GaussMul gm{};
-};
-
-template <typename T>
-static int conv_setup_t(pfbg_conv* cv) {
-  const ConvTabs& c0 = cv->ct;
-  FftDesc du, dv;
-  if (!factorize(c0.nxp, du, sizeof(T) == 4 ? 16 : 8) || !factorize(c0.nyp, dv, sizeof(T) == 4 ? 16 : 8))
-    return fail(PFBG_ERR_ARG, "padded sizes %d x %d must be 2^a 3^b 5^c 7^d 11^e", c0.nxp, c0.nyp);
-  if (fft_smem_bytes<T>(c0.nyp) > kMaxSmem) return fail(PFBG_ERR_ARG, "ny_psf=%d too large for the shared-memory FFT", c0.nyp);
-  int cc = (int)(32 / sizeof(cx2<T>));
-  while (cc > 1 && (c0.nyp % cc || fft_smem_bytes<T>(c0.nxp * cc) > kMaxSmem)) cc /= 2;
-  if (fft_smem_bytes<T>(c0.nxp * cc) > kMaxSmem) return fail(PFBG_ERR_ARG, "nx_psf=%d too large for the shared-memory FFT", c0.nxp);
-  cv->col_c = cc;
-  auto up = [&](void** dst, const void* src, size_t bytes) -> int {
-    CK(cudaMalloc(dst, bytes));
-    CK(cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice));
-    return PFBG_OK;
-  };
-  std::vector<cx2<T>> tw;
-  auto mk = [&](int n) {
-    tw.resize(n);
-    for (int t = 0; t < n; ++t) {
-      double ang = -2.0 * M_PI * (double)t / (double)n;
-      tw[t].x = (T)cos(ang);
-      tw[t].y = (T)sin(ang);
-    }
-  };
-  std::vector<int> rev, pos;
-  mk(c0.nxp);
-  CKRC(up(&cv->tw_u, tw.data(), tw.size() * sizeof(cx2<T>)));
-  mk(c0.nyp);
-  CKRC(up(&cv->tw_v, tw.data(), tw.size() * sizeof(cx2<T>)));
-  digit_tables(du, rev, pos);
-  CKRC(up(&cv->rev_u, rev.data(), rev.size() * 4));
-  digit_tables(dv, rev, pos);
-  CKRC(up(&cv->rev_v, rev.data(), rev.size() * 4));
-  CKRC(up(&cv->pos_v, pos.data(), pos.size() * 4));
-  const size_t rb = sizeof(T);
-  CK(cudaMalloc(&cv->tmp, (size_t)c0.nx * c0.nyp * 2 * rb));
-  CK(cudaMalloc(&cv->d_x, (size_t)c0.nx * c0.ny * rb));
-  CK(cudaMalloc(&cv->d_beam, (size_t)c0.nx * c0.ny * rb));
-  CK(cudaMalloc(&cv->d_out, (size_t)c0.nx * c0.ny * rb));
-  ConvTabs& ct = cv->ct;
-  ct.du = du; ct.dv = dv;
-  ct.tw_u = cv->tw_u; ct.tw_v = cv->tw_v;
-  ct.rev_u = (const int*)cv->rev_u; ct.rev_v = (const int*)cv->rev_v; ct.pos_v = (const int*)cv->pos_v;
-  CK(cudaFuncSetAttribute(k_conv_rows_fwd<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  CK(cudaFuncSetAttribute(k_conv_rows_inv<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  CK(cudaFuncSetAttribute(k_conv_cols<T, 4, KhatMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  CK(cudaFuncSetAttribute(k_conv_cols<T, 2, KhatMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  CK(cudaFuncSetAttribute(k_conv_cols<T, 1, KhatMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  CK(cudaFuncSetAttribute(k_conv_cols<T, 4, GaussMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  CK(cudaFuncSetAttribute(k_conv_cols<T, 2, GaussMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  CK(cudaFuncSetAttribute(k_conv_cols<T, 1, GaussMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  if constexpr (sizeof(T) == 8) {  // pfbg_conv_apply_shifted is fp64 only
-    CK(cudaFuncSetAttribute(k_conv_cols<T, 4, ShiftMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-    CK(cudaFuncSetAttribute(k_conv_cols<T, 2, ShiftMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-    CK(cudaFuncSetAttribute(k_conv_cols<T, 1, ShiftMul>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-  }
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_conv_destroy(pfbg_conv* cv) {
-  if (!cv) return PFBG_OK;
-  cudaSetDevice(cv->device);
-  void* all[] = {cv->tw_u, cv->tw_v, cv->rev_u, cv->rev_v, cv->pos_v, cv->khat, cv->tmp, cv->d_x, cv->d_beam, cv->d_out};
-  for (void* p : all)
-    if (p) cudaFree(p);
-  delete cv;
-  return PFBG_OK;
-}
-
-extern "C" int pfbg_conv_create(int32_t precision, int32_t device, int32_t nx, int32_t ny, int32_t nx_psf,
-                                int32_t ny_psf, pfbg_conv** out) {
-  if (!out) return fail(PFBG_ERR_ARG, "null argument");
-  *out = nullptr;
-  if (precision != PFBG_F32 && precision != PFBG_F64) return fail(PFBG_ERR_ARG, "bad precision");
-  if (nx <= 0 || ny <= 0 || nx_psf < nx || ny_psf < ny) return fail(PFBG_ERR_ARG, "need 0 < nx <= nx_psf and 0 < ny <= ny_psf");
-  CK(cudaSetDevice(device));
-  pfbg_conv* cv = new pfbg_conv();
-  cv->precision = precision; cv->device = device;
-  cv->ct.nx = nx; cv->ct.ny = ny; cv->ct.nxp = nx_psf; cv->ct.nyp = ny_psf;
-  int rc = precision == PFBG_F32 ? conv_setup_t<float>(cv) : conv_setup_t<double>(cv);
-  if (rc) { pfbg_conv_destroy(cv); return rc; }
-  *out = cv;
-  return PFBG_OK;
-}
-
-// the column-block width and the row-pass CTA size conv_setup_t / conv_apply_t chose (read-only, for tests)
-extern "C" int pfbg_conv_info(const pfbg_conv* cv, int32_t* col_block, int32_t* row_threads_out) {
-  if (!cv) return fail(PFBG_ERR_ARG, "null argument");
-  if (col_block) *col_block = cv->col_c;
-  if (row_threads_out) *row_threads_out = row_threads(cv->ct.nyp, 256);
-  return PFBG_OK;
-}
-
-// khat: complex multiplier of `precision`; half != 0: (nx_psf, ny_psf/2+1) half spectrum of a real kernel
-// (r2c layout: PSFHAT / abspsf), else the full (nx_psf, ny_psf) spectrum.
-extern "C" int pfbg_conv_set_kernel(pfbg_conv* cv, const void* khat, int32_t half, uint32_t flags, void* stream) {
-  if (!cv || !khat) return fail(PFBG_ERR_ARG, "null argument");
-  CK(cudaSetDevice(cv->device));
-  cudaStream_t s = (cudaStream_t)stream;
-  const ConvTabs& ct = cv->ct;
-  const size_t cb = cv->precision == PFBG_F32 ? 8 : 16;
-  const cudaMemcpyKind kind = (flags & PFBG_DEVICE_PTRS) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-  // the spectrum is allocated here, not at creation: a convolver that only ever runs the analytic kernel never holds it
-  // (an out-of-memory failure therefore shows here, not at pfbg_conv_create; the previous kernel is kept)
-  if (!cv->khat) CK(cudaMalloc(&cv->khat, (size_t)ct.nxp * ct.nyp * cb));
-  if (!half) {
-    // keep the Hermitian part only (all a real image can see; the column stage evaluates half the columns)
-    const size_t fb = (size_t)ct.nxp * ct.nyp * cb;
-    void* df = nullptr;
-    CK(cudaMalloc(&df, fb));
-    cudaError_t e = cudaMemcpyAsync(df, khat, fb, kind, s);
-    if (e == cudaSuccess) {
-      dim3 grd((ct.nyp + 127) / 128, ct.nxp);
-      if (cv->precision == PFBG_F32) k_hermitize<float><<<grd, 128, 0, s>>>(ct.nxp, ct.nyp, (const cx2<float>*)df, (cx2<float>*)cv->khat);
-      else k_hermitize<double><<<grd, 128, 0, s>>>(ct.nxp, ct.nyp, (const cx2<double>*)df, (cx2<double>*)cv->khat);
-      LAUNCHED();
-      e = cudaStreamSynchronize(s);
-    }
-    cudaFree(df);
-    if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "set_kernel failed: %s", cudaGetErrorString(e));
-  } else {
-    const size_t hb = (size_t)ct.nxp * (ct.nyp / 2 + 1) * cb;
-    void* dh = nullptr;
-    CK(cudaMalloc(&dh, hb));
-    cudaError_t e = cudaMemcpyAsync(dh, khat, hb, kind, s);
-    if (e == cudaSuccess) {
-      dim3 grd((ct.nyp + 127) / 128, ct.nxp);
-      if (cv->precision == PFBG_F32) k_expand_half<float><<<grd, 128, 0, s>>>(ct.nxp, ct.nyp, (const cx2<float>*)dh, (cx2<float>*)cv->khat);
-      else k_expand_half<double><<<grd, 128, 0, s>>>(ct.nxp, ct.nyp, (const cx2<double>*)dh, (cx2<double>*)cv->khat);
-      LAUNCHED();
-      e = cudaStreamSynchronize(s);
-    }
-    cudaFree(dh);
-    if (e != cudaSuccess) return fail(PFBG_ERR_CUDA, "set_kernel failed: %s", cudaGetErrorString(e));
-  }
-  CK(cudaStreamSynchronize(s));
-  cv->gauss = false;
-  cv->has_kernel = true;
-  return PFBG_OK;
-}
-
-// Beam (emaj, emin, pa) in pixels -> covariance S of exp(-x^T S^-1 x / 2); emaj, emin are FWHMs, the major axis points
-// along (cos pa, sin pa) in the (axis 0, axis 1) plane.
-static int gauss_cov(const double* b, const char* which, double S[3]) {
-  const double emaj = b[0], emin = b[1], pa = b[2];
-  if (!std::isfinite(emaj) || !std::isfinite(emin) || !std::isfinite(pa))
-    return fail(PFBG_ERR_ARG, "%s beam is not finite", which);
-  if (emin < 1.0) return fail(PFBG_ERR_ARG, "%s beam FWHM %g px is below 1 pixel", which, emin);
-  if (emaj < emin) return fail(PFBG_ERR_ARG, "%s beam has emaj %g < emin %g", which, emaj, emin);
-  const double k = 1.0 / (8.0 * M_LN2);  // sigma^2 = FWHM^2 / (8 ln 2)
-  const double va = emaj * emaj * k, vb = emin * emin * k, c = cos(pa), sn = sin(pa);
-  S[0] = va * c * c + vb * sn * sn;
-  S[1] = (va - vb) * c * sn;
-  S[2] = va * sn * sn + vb * c * c;
-  return PFBG_OK;
-}
-
-static double sym2_min_eig(const double S[3]) {
-  const double m = 0.5 * (S[0] + S[2]), d = hypot(0.5 * (S[0] - S[2]), S[1]);
-  return m - d;
-}
-
-// Alias count of one sum of the ratio mode, where each sum must be accurate relative to its own largest term (the
-// quotient divides the scale out), not to the peak at f = 0.  With m = 0 as the reference kept term, a dropped term m
-// is small enough at every f of the zone [-1/2, 1/2]^2 when
-//     (f + m)^T S (f + m) - f^T S f = m^T S m + 2 m^T S f >= m^T S m - |S m|_1 >= c,   c = -ln(1e-18) / (2 pi^2),
-// so M is the largest |m|_inf of any m that fails this.  Outside |m|_inf <= r0, m^T S m >= lmin r^2 and
-// |S m|_1 <= 2 lmax r make every m pass.  Returns -1 when r0 exceeds kMaxAliasScan (beams with an axis ratio above ~30).
-static constexpr int kMaxAliasScan = 2048;
-static int ratio_alias_M(const double S[3], double c) {
-  const double lmin = sym2_min_eig(S), lmax = S[0] + S[2] - lmin;
-  const double r0 = (lmax + sqrt(lmax * lmax + lmin * c)) / lmin;
-  if (!(r0 <= kMaxAliasScan)) return -1;
-  const int R = (int)ceil(r0);
-  int M = 0;
-  for (int mx = -R; mx <= R; ++mx)
-    for (int my = -R; my <= R; ++my) {
-      const double sx = S[0] * mx + S[1] * my, sy = S[1] * mx + S[2] * my;
-      if (mx * sx + my * sy - fabs(sx) - fabs(sy) < c) M = std::max(M, std::max(std::abs(mx), std::abs(my)));
-    }
-  return M;
-}
-
-// the alias sum of GaussMul at f = 0 (host), for the unit-sum normalisation
-static double gauss_sum0(const double q[3], int M) {
-  double acc = 0.0;
-  for (int mx = -M; mx <= M; ++mx)
-    for (int my = -M; my <= M; ++my) acc += exp(q[0] * mx * mx + q[1] * mx * my + q[2] * my * my);
-  return acc;
-}
-
-// to, from: (emaj, emin, pa) in pixels; from == NULL: plain convolution with the `to` Gaussian, else the ratio
-// K_to / K_from.  norm_kernel != 0: unit sum, else peak 1 (for a ratio, both kernels are normalised the same way).
-extern "C" int pfbg_conv_set_gauss(pfbg_conv* cv, const double* to, const double* from, int32_t norm_kernel) {
-  if (!cv || !to) return fail(PFBG_ERR_ARG, "null argument");
-  double St[3], Sf[3];
-  CKRC(gauss_cov(to, "target", St));
-  if (from) {
-    CKRC(gauss_cov(from, "source", Sf));
-    // converting to a narrower (or differently shaped) beam would divide by a vanishing transfer function
-    const double D[3] = {St[0] - Sf[0], St[1] - Sf[1], St[2] - Sf[2]};
-    const double tol = 1e-9 * fmax(St[0] + St[2], Sf[0] + Sf[2]);
-    if (sym2_min_eig(D) < -tol)
-      return fail(PFBG_ERR_ARG, "target beam (%g, %g, %g) does not contain source beam (%g, %g, %g): S_to - S_from "
-                  "is not positive semi-definite", to[0], to[1], to[2], from[0], from[1], from[2]);
-  }
-  GaussMul g{};
-  const double cdrop = -log(1e-18) / (2.0 * M_PI * M_PI);
-  if (!from) {
-    // plain: an absolute bound suffices.  The dropped alias terms have |f + m| >= M + 1/2, so
-    // q <= -2 pi^2 lmin (M + 1/2)^2, below 1e-18 of the peak when that is <= ln(1e-18) (M = 3 at a 1 px FWHM)
-    const double need = sqrt(cdrop / sym2_min_eig(St)) - 0.5;
-    g.M = need <= 0.0 ? 0 : (int)ceil(need);
-  } else {
-    const int mt = ratio_alias_M(St, cdrop), mf = ratio_alias_M(Sf, cdrop);
-    if (mt < 0 || mf < 0)
-      return fail(PFBG_ERR_ARG, "beam axis ratio too large for a change of resolution (alias scan beyond %d)",
-                  kMaxAliasScan);
-    g.M = std::max(mt, mf);
-  }
-  g.ratio = from != nullptr;
-  const double c2 = -2.0 * M_PI * M_PI;
-  const double qt[3] = {c2 * St[0], 2.0 * c2 * St[1], c2 * St[2]};
-  for (int i = 0; i < 3; ++i) g.q_to[i] = qt[i];
-  auto amp_of = [&](const double* S, const double* q) {
-    return norm_kernel ? 1.0 / gauss_sum0(q, g.M) : 2.0 * M_PI * sqrt(S[0] * S[2] - S[1] * S[1]);
-  };
-  g.amp = amp_of(St, qt);
-  if (from) {
-    const double qf[3] = {c2 * Sf[0], 2.0 * c2 * Sf[1], c2 * Sf[2]};
-    for (int i = 0; i < 3; ++i) g.q_from[i] = qf[i];
-    g.amp /= amp_of(Sf, qf);
-  }
-  if (cv->khat) {  // a Gaussian-mode convolver holds no spectrum
-    CK(cudaSetDevice(cv->device));
-    // an apply still in flight on any stream may read it.  set_gauss takes no stream, and cudaFree synchronises the
-    // device anyway; this happens once per switch from a stored spectrum, never between bands of a Gaussian run.
-    CK(cudaDeviceSynchronize());
-    cudaFree(cv->khat);
-    cv->khat = nullptr;
-  }
-  cv->gm = g;
-  cv->gauss = true;
-  cv->has_kernel = true;
-  return PFBG_OK;
-}
-
-template <typename T, class Mul>
-static void conv_cols_launch(const pfbg_conv* cv, const Mul& mul, cudaStream_t s) {
-  const ConvTabs& ct = cv->ct;
-  const int cc = cv->col_c;
-  const size_t csm = fft_smem_bytes<T>(ct.nxp * cc);
-  // Hermitian symmetry (real image, real kernel): only the columns l <= nyp/2 are transformed (psfconv.cuh)
-  const int ncol = ct.nyp / 2 + 1;
-  const cx2<T>* kh = (const cx2<T>*)cv->khat;
-  cx2<T>* tmp = (cx2<T>*)cv->tmp;
-  if (cc == 4) k_conv_cols<T, 4, Mul><<<(ncol + 3) / 4, 512, csm, s>>>(ct, kh, tmp, mul);
-  else if (cc == 2) k_conv_cols<T, 2, Mul><<<(ncol + 1) / 2, 512, csm, s>>>(ct, kh, tmp, mul);
-  else k_conv_cols<T, 1, Mul><<<ncol, 512, csm, s>>>(ct, kh, tmp, mul);
-}
-
-// xin != NULL: out += eta * xin in the row epilogue (the ridge term of the Hessian, or eta = 1 for apply_add).
-// shift != NULL (fp64, stored spectrum): the column pass multiplies by ShiftMul instead of the convolver's own kernel.
-template <typename T>
-static int conv_apply_t(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta, void* out,
-                        cudaStream_t s, const ShiftMul* shift) {
-  const ConvTabs& ct = cv->ct;
-  const int rt = row_threads(ct.nyp, 256);
-  k_conv_rows_fwd<T><<<(ct.nx + 1) / 2, rt, fft_smem_bytes<T>(ct.nyp), s>>>(ct, (const T*)x, (const T*)beam, (cx2<T>*)cv->tmp);
-  LAUNCHED();
-  if constexpr (sizeof(T) == 8) {
-    if (shift) conv_cols_launch<T>(cv, *shift, s);
-    else if (cv->gauss) conv_cols_launch<T>(cv, cv->gm, s);
-    else conv_cols_launch<T>(cv, KhatMul{}, s);
-  } else {
-    if (cv->gauss) conv_cols_launch<T>(cv, cv->gm, s);
-    else conv_cols_launch<T>(cv, KhatMul{}, s);
-  }
-  LAUNCHED();
-  const double scale = 1.0 / ((double)ct.nxp * (double)ct.nyp);
-  k_conv_rows_inv<T><<<(ct.nx + 1) / 2, rt, fft_smem_bytes<T>(ct.nyp), s>>>(ct, (const cx2<T>*)cv->tmp, (const T*)beam,
-                                                                 (const T*)xin, scale, eta, (T*)out);
-  LAUNCHED();
-  CK(cudaGetLastError());
-  return PFBG_OK;
-}
-
-// out = beam * crop(IFFT(FFT(pad(beam * x)) * K)) + eta * xin; host pointers are staged through d_x / d_beam / d_out
-// (apply_add passes no beam, so its `add` image rides in d_beam)
-static int conv_apply_any(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta, void* out,
-                          uint32_t flags, void* stream, const ShiftMul* shift = nullptr) {
-  if (!cv || !x || !out) return fail(PFBG_ERR_ARG, "null argument");
-  if (!cv->has_kernel) return fail(PFBG_ERR_STATE, "no kernel set");
-  CK(cudaSetDevice(cv->device));
-  cudaStream_t s = (cudaStream_t)stream;
-  const bool dev = flags & PFBG_DEVICE_PTRS;
-  const size_t ib = (size_t)cv->ct.nx * cv->ct.ny * (cv->precision == PFBG_F32 ? 4 : 8);
-  const void *dx = x, *db = beam, *dxin = xin;
-  void* dout = out;
-  if (!dev) {
-    CK(cudaMemcpyAsync(cv->d_x, x, ib, cudaMemcpyHostToDevice, s));
-    dx = cv->d_x;
-    if (beam) { CK(cudaMemcpyAsync(cv->d_beam, beam, ib, cudaMemcpyHostToDevice, s)); db = cv->d_beam; }
-    if (xin == x) dxin = dx;
-    else if (xin) { CK(cudaMemcpyAsync(cv->d_beam, xin, ib, cudaMemcpyHostToDevice, s)); dxin = cv->d_beam; }
-    dout = cv->d_out;
-  }
-  CKRC(cv->precision == PFBG_F32 ? conv_apply_t<float>(cv, dx, db, dxin, eta, dout, s, nullptr)
-                                 : conv_apply_t<double>(cv, dx, db, dxin, eta, dout, s, shift));
-  if (!dev) {
-    CK(cudaMemcpyAsync(out, dout, ib, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-  }
-  return PFBG_OK;
-}
-
-// out = beam * crop(IFFT(FFT(pad(beam * x)) * khat)) + eta * x      (beam may be NULL)
-extern "C" int pfbg_conv_apply(pfbg_conv* cv, const void* x, const void* beam, double eta, void* out, uint32_t flags,
-                               void* stream) {
-  return conv_apply_any(cv, x, beam, eta != 0.0 ? x : nullptr, eta, out, flags, stream);
-}
-
-// out = crop(IFFT(FFT(pad(x)) * K)) + add, the add in the row epilogue (x + 1.0 * add rounds as the separate sum)
-extern "C" int pfbg_conv_apply_add(pfbg_conv* cv, const void* x, const void* add, void* out, uint32_t flags,
-                                   void* stream) {
-  if (!add) return fail(PFBG_ERR_ARG, "null argument");
-  return conv_apply_any(cv, x, nullptr, add, 1.0, out, flags, stream);
-}
-
-// out = taper * crop(IFFT(FFT(pad(taper * x)) * (Re khat + c)^(+-1)))   (taper may be NULL; no ridge term)
-extern "C" int pfbg_conv_apply_shifted(pfbg_conv* cv, const void* x, const void* taper, double c, int32_t inverse,
-                                       void* out, uint32_t flags, void* stream) {
-  if (!cv || !x || !out) return fail(PFBG_ERR_ARG, "null argument");
-  if (cv->precision != PFBG_F64) return fail(PFBG_ERR_ARG, "the shifted spectrum is fp64 only");
-  if (!cv->has_kernel || cv->gauss || !cv->khat)
-    return fail(PFBG_ERR_STATE, "the shifted spectrum needs a stored spectrum (pfbg_conv_set_kernel)");
-  const ShiftMul sh{c, inverse ? 1 : 0};
-  return conv_apply_any(cv, x, taper, nullptr, 0.0, out, flags, stream, &sh);
-}
-
-// what the batched solvers of pfbsara.cu check before borrowing a convolver (not part of the C ABI)
-int pfbg_conv_props(const pfbg_conv* cv, int* precision, int* device, int* nx, int* ny, int* has_kernel) {
-  if (!cv) return fail(PFBG_ERR_ARG, "null convolver");
-  *precision = cv->precision; *device = cv->device; *nx = cv->ct.nx; *ny = cv->ct.ny; *has_kernel = cv->has_kernel;
-  return PFBG_OK;
-}

@@ -14,23 +14,8 @@
 #include "../../include/pfbsara.h"
 #include "cg.cuh"
 #include "clean.cuh"
+#include "host.h"
 #include "sara.cuh"
-
-// error plumbing shared with pfbgrid.cu (same shared library)
-int pfbg_fail(int code, const char* fmt, ...);
-void pfbg_count_launch();
-
-#define SCK(call)                                                                              \
-  do {                                                                                         \
-    cudaError_t e_ = (call);                                                                   \
-    if (e_ != cudaSuccess)                                                                     \
-      return pfbg_fail(PFBG_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-  } while (0)
-#define SRC(call)                   \
-  do {                              \
-    int rc_ = (call);               \
-    if (rc_ != PFBG_OK) return rc_; \
-  } while (0)
 
 struct pfbs_psi {
   int precision = 0, device = 0;
@@ -69,9 +54,9 @@ extern "C" int pfbs_psi_create(int32_t precision, int32_t device, int32_t nband,
   if (nband < 1 || nx < 1 || ny < 1 || nbasis < 1 || nlevel < 1 || nxmax < nx || nymax < ny)
     return pfbg_fail(PFBG_ERR_ARG, "bad sizes");
   int ndev = 0;
-  SCK(cudaGetDeviceCount(&ndev));
+  CK(cudaGetDeviceCount(&ndev));
   if (device < 0 || device >= ndev) return pfbg_fail(PFBG_ERR_ARG, "device %d out of range", device);
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   pfbs_psi* p = new pfbs_psi();
   p->precision = precision; p->device = device; p->nband = nband; p->nx = nx; p->ny = ny;
   p->nbasis = nbasis; p->nlevel = nlevel; p->nxmax = nxmax; p->nymax = nymax;
@@ -127,12 +112,12 @@ template <typename T>
 static int psi_dot_t(pfbs_psi* p, const T* x, T* alpha, cudaStream_t s) {
   const int64_t img = (int64_t)p->nx * p->ny, plane = (int64_t)p->nxmax * p->nymax;
   const int64_t astride = (int64_t)p->nbasis * plane;
-  SCK(cudaMemsetAsync(alpha, 0, (size_t)p->nband * astride * sizeof(T), s));
+  CK(cudaMemsetAsync(alpha, 0, (size_t)p->nband * astride * sizeof(T), s));
   for (int b = 0; b < p->nbasis; ++b) {
     T* ab = alpha + (int64_t)b * plane;
     if (p->K[b] == 0) {
       k_copy2d<T><<<dim3((p->ny + 127) / 128, p->nx, p->nband), 128, 0, s>>>(x, p->ny, img, ab, p->nymax, astride, p->nx, p->ny, 0);
-      pfbg_count_launch();
+      LAUNCHED();
       continue;
     }
     const T* in = x;
@@ -153,11 +138,11 @@ static int psi_dot_t(pfbs_psi* p, const T* x, T* alpha, cudaStream_t s) {
         case 8: k_dwt_level<T, 8><<<grd, 256, 0, s>>>(in, ld_in, nxin, nyin, blk, p->nymax, sx, sy, ap, p->dec[b], bp); break;
         default: k_dwt_level<T, 10><<<grd, 256, 0, s>>>(in, ld_in, nxin, nyin, blk, p->nymax, sx, sy, ap, p->dec[b], bp); break;
       }
-      pfbg_count_launch();
+      LAUNCHED();
       in = ap; ld_in = sy; nxin = sx; nyin = sy; in_stride = (int64_t)p->approx_elems;
     }
   }
-  SCK(cudaGetLastError());
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
@@ -165,12 +150,12 @@ template <typename T>
 static int psi_hdot_t(pfbs_psi* p, const T* alpha, T* x, cudaStream_t s) {
   const int64_t img = (int64_t)p->nx * p->ny, plane = (int64_t)p->nxmax * p->nymax;
   const int64_t astride = (int64_t)p->nbasis * plane;
-  SCK(cudaMemsetAsync(x, 0, (size_t)p->nband * img * sizeof(T), s));
+  CK(cudaMemsetAsync(x, 0, (size_t)p->nband * img * sizeof(T), s));
   for (int b = 0; b < p->nbasis; ++b) {
     const T* ab = alpha + (int64_t)b * plane;
     if (p->K[b] == 0) {
       k_copy2d<T><<<dim3((p->ny + 127) / 128, p->nx, p->nband), 128, 0, s>>>(ab, p->nymax, astride, x, p->ny, img, p->nx, p->ny, 1);
-      pfbg_count_launch();
+      LAUNCHED();
       continue;
     }
     const T* ll = nullptr;  // LL source of the current level: the block's own quadrant at the deepest level
@@ -197,11 +182,11 @@ static int psi_hdot_t(pfbs_psi* p, const T* alpha, T* x, cudaStream_t s) {
         case 8: k_idwt_level<T, 8><<<grd, 256, 0, s>>>(ll, ld_ll, blk, p->nymax, sx, sy, dst, ld_dst, nxo, nyo, p->rec[b], acc, bp); break;
         default: k_idwt_level<T, 10><<<grd, 256, 0, s>>>(ll, ld_ll, blk, p->nymax, sx, sy, dst, ld_dst, nxo, nyo, p->rec[b], acc, bp); break;
       }
-      pfbg_count_launch();
+      LAUNCHED();
       ll = dst; ld_ll = ld_dst; ll_stride = dst_stride;
     }
   }
-  SCK(cudaGetLastError());
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
@@ -210,9 +195,9 @@ static int transpose_planes(const T* src, T* dst, int nplanes, int n0, int n1, c
   for (int z0 = 0; z0 < nplanes; z0 += 65535) {
     const int nz = nplanes - z0 < 65535 ? nplanes - z0 : 65535;
     k_transpose<T><<<dim3((n1 + 31) / 32, (n0 + 31) / 32, nz), dim3(32, 8), 0, s>>>(src + (int64_t)z0 * n0 * n1, dst + (int64_t)z0 * n0 * n1, n0, n1);
-    pfbg_count_launch();
+    LAUNCHED();
   }
-  SCK(cudaGetLastError());
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
@@ -224,43 +209,43 @@ static int psi_apply(pfbs_psi* p, const void* in, void* out, uint32_t flags, cud
   const int nplanes = p->nband * p->nbasis;
   if (fwd) {
     const T* dx = (const T*)in;
-    if (!dev) { SRC(stage_alloc(&p->d_x, xb)); SCK(cudaMemcpyAsync(p->d_x, in, xb, cudaMemcpyHostToDevice, s)); dx = (const T*)p->d_x; }
+    if (!dev) { CKRC(stage_alloc(&p->d_x, xb)); CK(cudaMemcpyAsync(p->d_x, in, xb, cudaMemcpyHostToDevice, s)); dx = (const T*)p->d_x; }
     T* da = (T*)out;
-    if (!dev || tr) { SRC(stage_alloc(&p->d_alpha, ab)); da = (T*)p->d_alpha; }
-    SRC(psi_dot_t<T>(p, dx, da, s));
+    if (!dev || tr) { CKRC(stage_alloc(&p->d_alpha, ab)); da = (T*)p->d_alpha; }
+    CKRC(psi_dot_t<T>(p, dx, da, s));
     if (tr) {
       T* dt = (T*)out;
-      if (!dev) { SRC(stage_alloc(&p->d_alpha_t, ab)); dt = (T*)p->d_alpha_t; }
-      SRC(transpose_planes<T>(da, dt, nplanes, p->nxmax, p->nymax, s));
+      if (!dev) { CKRC(stage_alloc(&p->d_alpha_t, ab)); dt = (T*)p->d_alpha_t; }
+      CKRC(transpose_planes<T>(da, dt, nplanes, p->nxmax, p->nymax, s));
       da = dt;
     }
-    if (!dev) { SCK(cudaMemcpyAsync(out, da, ab, cudaMemcpyDeviceToHost, s)); SCK(cudaStreamSynchronize(s)); }
+    if (!dev) { CK(cudaMemcpyAsync(out, da, ab, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s)); }
   } else {
     const T* da = (const T*)in;
-    if (!dev) { SRC(stage_alloc(tr ? &p->d_alpha_t : &p->d_alpha, ab)); void* st = tr ? p->d_alpha_t : p->d_alpha; SCK(cudaMemcpyAsync(st, in, ab, cudaMemcpyHostToDevice, s)); da = (const T*)st; }
+    if (!dev) { CKRC(stage_alloc(tr ? &p->d_alpha_t : &p->d_alpha, ab)); void* st = tr ? p->d_alpha_t : p->d_alpha; CK(cudaMemcpyAsync(st, in, ab, cudaMemcpyHostToDevice, s)); da = (const T*)st; }
     if (tr) {
-      SRC(stage_alloc(&p->d_alpha, ab));
-      SRC(transpose_planes<T>(da, (T*)p->d_alpha, nplanes, p->nymax, p->nxmax, s));
+      CKRC(stage_alloc(&p->d_alpha, ab));
+      CKRC(transpose_planes<T>(da, (T*)p->d_alpha, nplanes, p->nymax, p->nxmax, s));
       da = (const T*)p->d_alpha;
     }
     T* dx = (T*)out;
-    if (!dev) { SRC(stage_alloc(&p->d_x, xb)); dx = (T*)p->d_x; }
-    SRC(psi_hdot_t<T>(p, da, dx, s));
-    if (!dev) { SCK(cudaMemcpyAsync(out, dx, xb, cudaMemcpyDeviceToHost, s)); SCK(cudaStreamSynchronize(s)); }
+    if (!dev) { CKRC(stage_alloc(&p->d_x, xb)); dx = (T*)p->d_x; }
+    CKRC(psi_hdot_t<T>(p, da, dx, s));
+    if (!dev) { CK(cudaMemcpyAsync(out, dx, xb, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s)); }
   }
   return PFBG_OK;
 }
 
 extern "C" int pfbs_psi_dot(pfbs_psi* p, const void* x, void* alpha, uint32_t flags, void* stream) {
   if (!p || !x || !alpha) return pfbg_fail(PFBG_ERR_ARG, "null argument");
-  SCK(cudaSetDevice(p->device));
+  CK(cudaSetDevice(p->device));
   return p->precision == PFBG_F32 ? psi_apply<float>(p, x, alpha, flags, (cudaStream_t)stream, true)
                                   : psi_apply<double>(p, x, alpha, flags, (cudaStream_t)stream, true);
 }
 
 extern "C" int pfbs_psi_hdot(pfbs_psi* p, const void* alpha, void* x, uint32_t flags, void* stream) {
   if (!p || !x || !alpha) return pfbg_fail(PFBG_ERR_ARG, "null argument");
-  SCK(cudaSetDevice(p->device));
+  CK(cudaSetDevice(p->device));
   return p->precision == PFBG_F32 ? psi_apply<float>(p, alpha, x, flags, (cudaStream_t)stream, false)
                                   : psi_apply<double>(p, alpha, x, flags, (cudaStream_t)stream, false);
 }
@@ -277,7 +262,7 @@ extern "C" int pfbs_dual_update(int32_t precision, int32_t device, const void* v
     return pfbg_fail(PFBG_ERR_ARG, "null argument");
   if (vbar && phase == 1) return pfbg_fail(PFBG_ERR_ARG, "the extrapolated dual is written by phase 0 or 2");
   if (phase < 0 || phase > 2 || nband < 1 || ncoef < 0) return pfbg_fail(PFBG_ERR_ARG, "bad phase / sizes");
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   cudaStream_t s = (cudaStream_t)stream;
   if (ncoef == 0) return PFBG_OK;
   if (precision == PFBG_F32)
@@ -285,8 +270,8 @@ extern "C" int pfbs_dual_update(int32_t precision, int32_t device, const void* v
   else if (precision == PFBG_F64)
     k_dual_update<double><<<nblk(ncoef), 256, 0, s>>>((const double*)vp, (double*)v, (const double*)weight, lam, sigma, nband, ncoef, (double*)bsum, phase, (double*)vbar);
   else return pfbg_fail(PFBG_ERR_ARG, "bad precision");
-  pfbg_count_launch();
-  SCK(cudaGetLastError());
+  LAUNCHED();
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
@@ -294,7 +279,7 @@ extern "C" int pfbs_prox_21m(int32_t precision, int32_t device, const void* v, v
                              double lam, double sigma, int32_t nband, int64_t ncoef, void* stream) {
   if (!v || !result || !weight) return pfbg_fail(PFBG_ERR_ARG, "null argument");
   if (nband < 1 || ncoef < 0 || !(sigma > 0)) return pfbg_fail(PFBG_ERR_ARG, "bad sizes / sigma");
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   cudaStream_t s = (cudaStream_t)stream;
   if (ncoef == 0) return PFBG_OK;
   if (precision == PFBG_F32)
@@ -302,35 +287,35 @@ extern "C" int pfbs_prox_21m(int32_t precision, int32_t device, const void* v, v
   else if (precision == PFBG_F64)
     k_prox_21m<double><<<nblk(ncoef), 256, 0, s>>>((const double*)v, (double*)result, (const double*)weight, lam, sigma, nband, ncoef);
   else return pfbg_fail(PFBG_ERR_ARG, "bad precision");
-  pfbg_count_launch();
-  SCK(cudaGetLastError());
+  LAUNCHED();
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
 extern "C" int pfbs_extrapolate(int32_t precision, int32_t device, const void* v, void* vp, int64_t n, void* stream) {
   if (!v || !vp) return pfbg_fail(PFBG_ERR_ARG, "null argument");
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   cudaStream_t s = (cudaStream_t)stream;
   if (n <= 0) return PFBG_OK;
   if (precision == PFBG_F32) k_extrapolate<float><<<nblk(n), 256, 0, s>>>((const float*)v, (float*)vp, n);
   else if (precision == PFBG_F64) k_extrapolate<double><<<nblk(n), 256, 0, s>>>((const double*)v, (double*)vp, n);
   else return pfbg_fail(PFBG_ERR_ARG, "bad precision");
-  pfbg_count_launch();
-  SCK(cudaGetLastError());
+  LAUNCHED();
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
 extern "C" int pfbs_axpby(int32_t precision, int32_t device, void* out, double a, const void* x, double b, const void* y,
                           int64_t n, void* stream) {
   if (!out || !x || !y) return pfbg_fail(PFBG_ERR_ARG, "null argument");
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   cudaStream_t s = (cudaStream_t)stream;
   if (n <= 0) return PFBG_OK;
   if (precision == PFBG_F32) k_axpby<float><<<nblk(n), 256, 0, s>>>((float*)out, (float)a, (const float*)x, (float)b, (const float*)y, n);
   else if (precision == PFBG_F64) k_axpby<double><<<nblk(n), 256, 0, s>>>((double*)out, a, (const double*)x, b, (const double*)y, n);
   else return pfbg_fail(PFBG_ERR_ARG, "bad precision");
-  pfbg_count_launch();
-  SCK(cudaGetLastError());
+  LAUNCHED();
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
@@ -338,7 +323,7 @@ extern "C" int pfbs_primal_step(int32_t precision, int32_t device, void* x, cons
                                 int32_t positivity, int32_t nband, int64_t npix, void* stream) {
   if (!x || !xp || !xout) return pfbg_fail(PFBG_ERR_ARG, "null argument");
   if (positivity < 0 || positivity > 2 || nband < 1) return pfbg_fail(PFBG_ERR_ARG, "bad positivity mode / nband");
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   cudaStream_t s = (cudaStream_t)stream;
   if (npix <= 0) return PFBG_OK;
   if (precision == PFBG_F32)
@@ -346,16 +331,14 @@ extern "C" int pfbs_primal_step(int32_t precision, int32_t device, void* x, cons
   else if (precision == PFBG_F64)
     k_primal_step<double><<<nblk(npix), 256, 0, s>>>((double*)x, (const double*)xp, (const double*)xout, tau, positivity, nband, npix);
   else return pfbg_fail(PFBG_ERR_ARG, "bad precision");
-  pfbg_count_launch();
-  SCK(cudaGetLastError());
+  LAUNCHED();
+  CK(cudaGetLastError());
   return PFBG_OK;
 }
 
 // two doubles of device scratch for the reductions, held for the duration of the call (pfbgrid.cu: recycled blocks,
 // one per concurrent caller, so host threads / streams on one device never share an accumulator; no cudaMalloc /
 // cudaFree, which synchronises the device, inside the solver loops)
-void* pfbg_scratch_get(int device);
-void pfbg_scratch_put(int device, void* p);
 
 template <typename K>
 static int reduce2(int device, cudaStream_t s, double* out2, K launch) {
@@ -365,12 +348,12 @@ static int reduce2(int device, cudaStream_t s, double* out2, K launch) {
   } hold{device, pfbg_scratch_get(device)};
   double* acc = (double*)hold.p;
   if (!acc) return pfbg_fail(PFBG_ERR_NOMEM, "no reduction scratch on device %d", device);
-  SCK(cudaMemsetAsync(acc, 0, 16, s));
+  CK(cudaMemsetAsync(acc, 0, 16, s));
   launch(acc);
-  pfbg_count_launch();
-  SCK(cudaGetLastError());
-  SCK(cudaMemcpyAsync(out2, acc, 16, cudaMemcpyDeviceToHost, s));
-  SCK(cudaStreamSynchronize(s));
+  LAUNCHED();
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out2, acc, 16, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
   return PFBG_OK;
 }
 
@@ -378,7 +361,7 @@ extern "C" int pfbs_norm_diff(int32_t precision, int32_t device, const void* x, 
                               double* num_den, void* stream) {
   if (!x || !xp || !num_den) return pfbg_fail(PFBG_ERR_ARG, "null argument");
   if (precision != PFBG_F32 && precision != PFBG_F64) return pfbg_fail(PFBG_ERR_ARG, "bad precision");
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   cudaStream_t s = (cudaStream_t)stream;
   num_den[0] = num_den[1] = 0.0;
   if (n <= 0) return PFBG_OK;
@@ -393,7 +376,7 @@ extern "C" int pfbs_dot2(int32_t precision, int32_t device, const void* a, const
                          int64_t n, double* out2, void* stream) {
   if (!a || !b || !c || !d || !out2) return pfbg_fail(PFBG_ERR_ARG, "null argument");
   if (precision != PFBG_F32 && precision != PFBG_F64) return pfbg_fail(PFBG_ERR_ARG, "bad precision");
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   cudaStream_t s = (cudaStream_t)stream;
   out2[0] = out2[1] = 0.0;
   if (n <= 0) return PFBG_OK;
@@ -447,14 +430,14 @@ extern "C" int pfbs_clark_create(int32_t precision, int32_t device, int32_t nban
     return pfbg_fail(PFBG_ERR_ARG, "need 0 < nx <= nx_psf and 0 < ny <= ny_psf (got %d x %d, PSF %d x %d)", nx, ny, nx_psf, ny_psf);
   if ((int64_t)nx * ny > INT32_MAX) return pfbg_fail(PFBG_ERR_ARG, "nx * ny must be below 2^31");
   int ndev = 0;
-  SCK(cudaGetDeviceCount(&ndev));
+  CK(cudaGetDeviceCount(&ndev));
   if (device < 0 || device >= ndev) return pfbg_fail(PFBG_ERR_ARG, "device %d out of range", device);
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   int coop = 0, nsm = 0, occ = 0;
-  SCK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device));
+  CK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device));
   if (!coop) return pfbg_fail(PFBG_ERR_CUDA, "device %d does not support cooperative launches", device);
-  SCK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
-  SCK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_clark_subminor, CLK_THREADS, (size_t)nband * sizeof(double)));
+  CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_clark_subminor, CLK_THREADS, (size_t)nband * sizeof(double)));
   if (occ < 1) return pfbg_fail(PFBG_ERR_CUDA, "the subminor kernel cannot be resident");
   cudaStream_t s = (cudaStream_t)stream;
   const cudaMemcpyKind kind = (flags & PFBG_DEVICE_PTRS) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
@@ -514,8 +497,8 @@ static int clark_log_reserve(pfbs_clark* h, int n) {
   if (h->log_p) cudaFree(h->log_p);
   if (h->log_d) cudaFree(h->log_d);
   h->log_p = nullptr; h->log_d = nullptr; h->log_cap = 0;
-  SRC(stage_alloc((void**)&h->log_p, (size_t)n * 4));
-  SRC(stage_alloc((void**)&h->log_d, (size_t)n * h->nband * 8));
+  CKRC(stage_alloc((void**)&h->log_p, (size_t)n * 4));
+  CKRC(stage_alloc((void**)&h->log_d, (size_t)n * h->nband * 8));
   h->log_cap = n;
   return PFBG_OK;
 }
@@ -533,84 +516,83 @@ extern "C" int pfbs_clark_run(pfbs_clark* h, const void* dirty, const uint8_t* m
   if (maxit > 0 && (!rmax || !nactive || !nsub || !peaks)) return pfbg_fail(PFBG_ERR_ARG, "null info buffer");
   if (peaks_cap < (int64_t)maxit * submaxit) return pfbg_fail(PFBG_ERR_ARG, "peaks holds %lld entries, maxit * submaxit = %lld",
                                                               (long long)peaks_cap, (long long)maxit * submaxit);
-  SCK(cudaSetDevice(h->device));
-  SRC(clark_log_reserve(h, submaxit));
+  CK(cudaSetDevice(h->device));
+  CKRC(clark_log_reserve(h, submaxit));
   cudaStream_t s = (cudaStream_t)stream;
   const bool dev = flags & PFBG_DEVICE_PTRS;
   const int npix = h->npix, nband = h->nband;
   const size_t ib = (size_t)nband * npix * 8;
-  SCK(cudaMemcpyAsync(h->ID, dirty, ib, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
-  if (mask) SCK(cudaMemcpyAsync(h->mask, mask, npix, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
-  SCK(cudaMemcpyAsync(h->R, h->ID, ib, cudaMemcpyDeviceToDevice, s));
-  SCK(cudaMemsetAsync(h->model, 0, ib, s));
+  CK(cudaMemcpyAsync(h->ID, dirty, ib, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
+  if (mask) CK(cudaMemcpyAsync(h->mask, mask, npix, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(h->R, h->ID, ib, cudaMemcpyDeviceToDevice, s));
+  CK(cudaMemsetAsync(h->model, 0, ib, s));
   double tol = -1.0;
   int k = 0;
   int64_t npeaks = 0;
   for (;; ++k) {
-    if (times_ms) SCK(cudaEventRecord(h->ev[0], s));
+    if (times_ms) CK(cudaEventRecord(h->ev[0], s));
     k_clark_search<<<h->search_grid, CLK_THREADS, 0, s>>>(h->R, nband, npix, mask ? h->mask : nullptr, h->s, h->cand_s, h->cand_i);
     k_clark_best<<<1, CLK_THREADS, 0, s>>>(h->cand_s, h->cand_i, h->search_grid, h->cand_s + h->search_grid, h->ints);
-    pfbg_count_launch(); pfbg_count_launch();
-    SCK(cudaGetLastError());
+    LAUNCHED(); LAUNCHED();
+    CK(cudaGetLastError());
     double Rmax = 0.0;
-    SCK(cudaMemcpyAsync(&Rmax, h->cand_s + h->search_grid, 8, cudaMemcpyDeviceToHost, s));
-    SCK(cudaStreamSynchronize(s));
+    CK(cudaMemcpyAsync(&Rmax, h->cand_s + h->search_grid, 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
     if (Rmax < 0.0) Rmax = 0.0;  // no pixel is searched
     if (k == 0) tol = std::max(pf * Rmax, threshold);
     if (!(Rmax > tol) || k >= maxit) break;
     const ClarkActive pred{h->s, subpf * Rmax};
-    SCK(cub::DeviceSelect::If(h->cub_tmp, h->cub_bytes, thrust::counting_iterator<int>(0), h->idx, h->ints + 1, npix, pred, s));
+    CK(cub::DeviceSelect::If(h->cub_tmp, h->cub_bytes, thrust::counting_iterator<int>(0), h->idx, h->ints + 1, npix, pred, s));
     int nA = 0;
-    SCK(cudaMemcpyAsync(&nA, h->ints + 1, 4, cudaMemcpyDeviceToHost, s));
-    SCK(cudaStreamSynchronize(s));
+    CK(cudaMemcpyAsync(&nA, h->ints + 1, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
     const int ga = std::min((nA + CLK_THREADS - 1) / CLK_THREADS, h->search_grid);
     k_clark_gather<<<std::max(ga, 1), CLK_THREADS, 0, s>>>(h->R, h->s, nband, npix, h->ny, h->idx, nA, h->RA, h->SA, h->ij);
-    pfbg_count_launch();
-    SCK(cudaGetLastError());
-    if (times_ms) SCK(cudaEventRecord(h->ev[1], s));
+    LAUNCHED();
+    CK(cudaGetLastError());
+    if (times_ms) CK(cudaEventRecord(h->ev[1], s));
     ClarkSub c{h->RA, h->SA, h->ij, nA, nband, h->ny, h->psf, h->peak_d, h->nxp, h->nyp, h->nxp / 2, h->nyp / 2,
                gamma, std::max(subpf * Rmax, threshold), submaxit, h->slot_s, h->slot_a, h->slot_r, h->log_p, h->log_d,
                h->ints + 2};
     const int grid = std::max(1, std::min((nA + CLK_THREADS - 1) / CLK_THREADS, h->sub_grid));
     void* args[] = {&c};
-    SCK(cudaLaunchCooperativeKernel((const void*)k_clark_subminor, dim3(grid), dim3(CLK_THREADS), args,
+    CK(cudaLaunchCooperativeKernel((const void*)k_clark_subminor, dim3(grid), dim3(CLK_THREADS), args,
                                     (size_t)nband * sizeof(double), s));
-    pfbg_count_launch();
+    LAUNCHED();
     k_clark_replay<<<(nband + 31) / 32, 32, 0, s>>>(h->model, nband, npix, h->log_p, h->log_d, h->ints + 2);
-    pfbg_count_launch();
-    SCK(cudaGetLastError());
-    if (times_ms) SCK(cudaEventRecord(h->ev[2], s));
+    LAUNCHED();
+    CK(cudaGetLastError());
+    if (times_ms) CK(cudaEventRecord(h->ev[2], s));
     for (int b = 0; b < nband; ++b)
-      SRC(pfbg_conv_apply(h->conv[b], h->model + (int64_t)b * npix, nullptr, 0.0, h->R + (int64_t)b * npix, PFBG_DEVICE_PTRS, stream));
+      CKRC(pfbg_conv_apply(h->conv[b], h->model + (int64_t)b * npix, nullptr, 0.0, h->R + (int64_t)b * npix, PFBG_DEVICE_PTRS, stream));
     k_clark_resid<<<h->search_grid, CLK_THREADS, 0, s>>>(h->ID, h->R, (int64_t)nband * npix);
-    pfbg_count_launch();
-    SCK(cudaGetLastError());
-    if (times_ms) SCK(cudaEventRecord(h->ev[3], s));
+    LAUNCHED();
+    CK(cudaGetLastError());
+    if (times_ms) CK(cudaEventRecord(h->ev[3], s));
     int cnt = 0;
-    SCK(cudaMemcpyAsync(&cnt, h->ints + 2, 4, cudaMemcpyDeviceToHost, s));
-    SCK(cudaStreamSynchronize(s));
+    CK(cudaMemcpyAsync(&cnt, h->ints + 2, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
     std::vector<int> lp(cnt);
-    if (cnt) SCK(cudaMemcpy(lp.data(), h->log_p, (size_t)cnt * 4, cudaMemcpyDeviceToHost));
+    if (cnt) CK(cudaMemcpy(lp.data(), h->log_p, (size_t)cnt * 4, cudaMemcpyDeviceToHost));
     for (int t = 0; t < cnt; ++t) peaks[npeaks + t] = lp[t];
     npeaks += cnt;
     rmax[k] = Rmax;
     nactive[k] = nA;
     nsub[k] = cnt;
     if (times_ms)
-      for (int t = 0; t < 3; ++t) SCK(cudaEventElapsedTime(&times_ms[3 * k + t], h->ev[t], h->ev[t + 1]));
+      for (int t = 0; t < 3; ++t) CK(cudaEventElapsedTime(&times_ms[3 * k + t], h->ev[t], h->ev[t + 1]));
   }
   *niter = k;
   const cudaMemcpyKind back = dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-  SCK(cudaMemcpyAsync(model, h->model, ib, back, s));
-  SCK(cudaMemcpyAsync(residual, h->R, ib, back, s));
-  if (!dev) SCK(cudaStreamSynchronize(s));
+  CK(cudaMemcpyAsync(model, h->model, ib, back, s));
+  CK(cudaMemcpyAsync(residual, h->R, ib, back, s));
+  if (!dev) CK(cudaStreamSynchronize(s));
   return PFBG_OK;
 }
 
 // ---------------------------------------------------------------------------
 // Batched conjugate gradients on the PSF-convolution Hessian (cg.cuh)
 // ---------------------------------------------------------------------------
-int pfbg_conv_props(const pfbg_conv* cv, int* precision, int* device, int* nx, int* ny, int* has_kernel);
 
 static const int64_t kCgAlign = 256;
 static int64_t cg_round(int64_t b) { return (b + kCgAlign - 1) / kCgAlign * kCgAlign; }
@@ -638,13 +620,13 @@ extern "C" int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv
   if (nband < 1 || nband > 65535) return pfbg_fail(PFBG_ERR_ARG, "nband %d not in 1..65535", nband);
   if (!(tol >= 0.0) || maxit < 0 || minit < 0) return pfbg_fail(PFBG_ERR_ARG, "need tol >= 0, maxit >= 0, minit >= 0");
   int ndev = 0;
-  SCK(cudaGetDeviceCount(&ndev));
+  CK(cudaGetDeviceCount(&ndev));
   if (device < 0 || device >= ndev) return pfbg_fail(PFBG_ERR_ARG, "device %d out of range", device);
   int nx0 = 0, ny0 = 0;
   for (int b = 0; b < nband; ++b) {
     int prec = 0, dev = 0, nx = 0, ny = 0, hk = 0;
     if (!conv[b]) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is NULL", b);
-    SRC(pfbg_conv_props(conv[b], &prec, &dev, &nx, &ny, &hk));
+    CKRC(pfbg_conv_props(conv[b], &prec, &dev, &nx, &ny, &hk));
     if (prec != PFBG_F64) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is not fp64", b);
     if (dev != device) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is on device %d, not %d", b, dev, device);
     if (!hk) return pfbg_fail(PFBG_ERR_STATE, "convolver %d has no kernel", b);
@@ -655,7 +637,7 @@ extern "C" int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv
   if (npix != (int64_t)nx0 * ny0) return pfbg_fail(PFBG_ERR_ARG, "npix %lld != nx * ny = %lld", (long long)npix, (long long)nx0 * ny0);
   const int64_t need = pfbs_psf_cg_work_bytes(nband, npix);
   if (work_bytes < need) return pfbg_fail(PFBG_ERR_ARG, "work holds %lld bytes, %lld needed", (long long)work_bytes, (long long)need);
-  SCK(cudaSetDevice(device));
+  CK(cudaSetDevice(device));
   if (!cg_on_device(rhs, device) || !cg_on_device(x, device) || !cg_on_device(work, device))
     return pfbg_fail(PFBG_ERR_ARG, "rhs, x and work must be device arrays on device %d", device);
   for (int b = 0; b < nband; ++b)
@@ -676,30 +658,30 @@ extern "C" int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv
     return pfbg_conv_apply(conv[b], in + b * npix, beam[b], eta[b], out + b * npix, PFBG_DEVICE_PTRS, stream);
   };
   auto read_ctl = [&]() -> int {
-    SCK(cudaMemcpyAsync(h.data(), ctl, (size_t)nband * sizeof(CgCtl), cudaMemcpyDeviceToHost, s));
-    SCK(cudaStreamSynchronize(s));
+    CK(cudaMemcpyAsync(h.data(), ctl, (size_t)nband * sizeof(CgCtl), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
     return PFBG_OK;
   };
 
-  for (int b = 0; b < nband; ++b) SRC(apply(xd, r, b));  // r = A x
+  for (int b = 0; b < nband; ++b) CKRC(apply(xd, r, b));  // r = A x
   k_cg_init<<<grd, CG_THREADS, 0, s>>>((const double*)rhs, r, p, npix, part);
   k_cg_init_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G, tol, maxit, minit);
-  pfbg_count_launch(); pfbg_count_launch();
-  SCK(cudaGetLastError());
-  SRC(read_ctl());
+  LAUNCHED(); LAUNCHED();
+  CK(cudaGetLastError());
+  CKRC(read_ctl());
   for (;;) {
     bool any = false;
     for (int b = 0; b < nband; ++b)
-      if (h[b].stop == CG_RUNNING) { any = true; SRC(apply(p, ap, b)); }  // stopped bands skip their convolution
+      if (h[b].stop == CG_RUNNING) { any = true; CKRC(apply(p, ap, b)); }  // stopped bands skip their convolution
     if (!any) break;
     k_cg_dots<<<grd, CG_THREADS, 0, s>>>(ctl, p, ap, npix, part);
     k_cg_dots_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G);
     k_cg_update<<<grd, CG_THREADS, 0, s>>>(ctl, (double*)x, r, p, ap, npix, part);
     k_cg_update_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G, tol, maxit, minit);
     k_cg_direction<<<grd, CG_THREADS, 0, s>>>(ctl, p, r, npix);
-    for (int t = 0; t < 5; ++t) pfbg_count_launch();
-    SCK(cudaGetLastError());
-    SRC(read_ctl());
+    for (int t = 0; t < 5; ++t) LAUNCHED();
+    CK(cudaGetLastError());
+    CKRC(read_ctl());
   }
   for (int b = 0; b < nband; ++b) {
     iters[b] = h[b].k;

@@ -22,7 +22,6 @@ def test_narrow_column_blocks_against_dft(gpu, monkeypatch, colc, prec, eps):
     """k_cols_fwd / k_cols_inv<T, 2> and <T, 1> are what every fp32 grid with nu > ~6.8 k and every fp64 grid with
     nu > ~3.4 k runs (the 8640^2 PSF grid of config 2, all of config 4).  PFBG_COLC forces them at a small size."""
     monkeypatch.setenv("PFBG_COLC", colc)
-    monkeypatch.setenv("PFBG_FFT", "fused")
     W.clear_plan_pool()
     p = small_problem(nrow=700, nchan=3, nx=96, ny=80, seed=31, wscale=2.0)
     rdt, cdt = (np.float32, np.complex64) if prec == "single" else (np.float64, np.complex128)

@@ -31,7 +31,7 @@ ROUNDOFF = {"single": 3e-6, "double": 1e-11}
 DT = {"single": (np.float32, np.complex64), "double": (np.float64, np.complex128)}
 WSUM, ETA = 2.0, 0.25
 ROWS_BIG_SMEM = 113 * 1024  # fused_common.cuh
-COLS2_MAX_SMEM = 232448  # colsfft.cu: kCols2MaxSmem
+COLS2_MAX_SMEM = 232448  # fft_host.h: kMaxSmem
 
 
 def _fft_smem_bytes(n, prec):  # fft.cuh: one pad element per 16 (fp32) / 8 (fp64) elements
