@@ -310,6 +310,16 @@ int pfbg_conv_apply_add(pfbg_conv* conv, const void* x, const void* add, void* o
  */
 int pfbg_conv_apply_shifted(pfbg_conv* conv, const void* x, const void* taper, double c, int32_t inverse, void* out,
                             uint32_t flags, void* stream);
+/*
+ * One term of a sum-over-partitions Hessian (operators/hessian.py:439-522 HessianTree), device arrays only:
+ *     out = scale * beam * crop( IFFT( FFT( pad(beam * x) ) * K ) ) + eta * xin
+ * beam may be NULL; xin is not read when eta == 0 (it may then be NULL).  The epilogue multiplies by
+ * scale / (nx_psf * ny_psf), so scale = 1 and xin = x give the bits of pfbg_conv_apply.  A sum over groups accumulates
+ * through xin with eta = 1, ping-ponging between two buffers: xin must not alias out.  `flags` must hold
+ * PFBG_DEVICE_PTRS; PFBG_ERR_ARG for host pointers, pointers on another device, or a scale that is not finite and > 0.
+ */
+int pfbg_conv_apply_scaled(pfbg_conv* conv, const void* x, const void* beam, const void* xin, double eta, double scale,
+                           void* out, uint32_t flags, void* stream);
 
 /*
  * Band split across two GPUs, one process per GPU (SURVEY §8e; the reference runs one actor per band,

@@ -15,6 +15,7 @@
  *     positivity / positivity_band (prox/positivity.py:13-38)                               -> pfbs_extrapolate /
  *                                                                                              pfbs_primal_step / pfbs_norm_diff
  *   - clark (deconv/clark.py), semantics as restated in oracle/clark_np.py                  -> pfbs_clark_run
+ *   - pcg on HessPSF / HessianTree (operators/hessian.py:357-522, opt/pcg.py:202-314)       -> pfbs_psf_cg / pfbs_tree_cg
  */
 #ifndef PFBSARA_H
 #define PFBSARA_H
@@ -132,6 +133,24 @@ int64_t pfbs_psf_cg_work_bytes(int32_t nband, int64_t npix); /* -1 for nband < 1
 int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv, const void* const* beam, const double* eta,
                 const void* rhs, void* x, int64_t npix, double tol, int32_t maxit, int32_t minit, void* work,
                 int64_t work_bytes, int32_t* iters, double* eps, int32_t* stop, void* stream);
+
+/*
+ * The same conjugate gradients on grouped systems: the corr-0 operator of a band's HessianTree
+ * (operators/hessian.py:439-522), a sum over the beam groups g = group_start[s] .. group_start[s+1]-1 of system s,
+ *     A_s v = scale_s sum_g beam_g conv_g(beam_g v) + eta_s v      (scale_s = 1 / wsum_s)
+ * applied with pfbg_conv_apply_scaled, accumulating through one scratch image.  conv[] and beam[] are the flattened
+ * group lists (beam[g] may be NULL), scale[] and eta[] have one entry per system.  Everything else (layout of rhs and
+ * x, stopping rules, outputs, deterministic reductions, skipped convolutions of stopped systems) is pfbs_psf_cg's,
+ * which is this function with one group per band and scale 1.  PFBG_ERR_ARG also for group_start[0] != 0, a system
+ * without a group, and a scale that is not finite and > 0.
+ * work: at least pfbs_tree_cg_work_bytes(nsys, group_start, npix) bytes, which adds one image to
+ * pfbs_psf_cg_work_bytes when some system has two or more groups (-1 for nsys < 1, npix < 1 or no group_start).
+ */
+int64_t pfbs_tree_cg_work_bytes(int32_t nsys, const int32_t* group_start, int64_t npix);
+int pfbs_tree_cg(int32_t device, int32_t nsys, const int32_t* group_start, pfbg_conv* const* conv,
+                 const void* const* beam, const double* scale, const double* eta, const void* rhs, void* x,
+                 int64_t npix, double tol, int32_t maxit, int32_t minit, void* work, int64_t work_bytes,
+                 int32_t* iters, double* eps, int32_t* stop, void* stream);
 
 #ifdef __cplusplus
 }

@@ -91,6 +91,7 @@ SIGNATURES = {
     "pfbg_conv_set_gauss": (C.c_int, [_vp, C.POINTER(_dbl), C.POINTER(_dbl), _i32]),
     "pfbg_conv_apply_add": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _vp]),
     "pfbg_conv_apply_shifted": (C.c_int, [_vp, _vp, _vp, _dbl, _i32, _vp, _u32, _vp]),
+    "pfbg_conv_apply_scaled": (C.c_int, [_vp, _vp, _vp, _vp, _dbl, _dbl, _vp, _u32, _vp]),
     "pfbg_debug_fft1d": (C.c_int, [_i32, _i32, _i32, _i32, _vp, _vp, _i32, _i32]),
     "pfbg_debug_es_fast64": (C.c_int, [_i32, _i64, _vp, C.c_double, _vp]),
     "pfbg_weight_data_corr": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i64, _i64, _i64, _i64,
@@ -133,6 +134,9 @@ SIGNATURES = {
     "pfbs_psf_cg_work_bytes": (_i64, [_i32, _i64]),
     "pfbs_psf_cg": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _dbl, _i32, _i32, _vp, _i64, _vp, _vp, _vp,
                               _vp]),
+    "pfbs_tree_cg_work_bytes": (_i64, [_i32, _vp, _i64]),
+    "pfbs_tree_cg": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _dbl, _i32, _i32, _vp, _i64, _vp,
+                               _vp, _vp, _vp]),
 }
 
 _lib = None

@@ -11,6 +11,10 @@ completed by one all-reduce, like ``BandPool``).  A worker holds the three roles
   residual  ``load_band`` / ``residual``              exact ``dirty - sum_p R_p^H W_p R_p (beam_p model)``
                                                        (operators/gridder.py:926-1016), data pinned on the device
 
+``hess_dot`` / ``hess_cg`` also take ``(nband, nx, ny)`` float64 CUDA tensors: the cube then stays on the devices
+(bands pinned to another device are copied there and back), and ``hess_cg`` solves the bands of each device in one
+batched ``psf.tree_cg``, the devices concurrently.
+
 ``load_band(store_url, node_name)`` reads the band node of a ``.dt`` zarr store itself (band_worker.py:61-106) through
 ``pfb_imaging_b200.store`` (xarray / zarr are not importable here); `store_url` may also be an already opened tree.
 """
@@ -70,6 +74,12 @@ class _BandWorkerImpl:
 
     def hess_dot(self, x):
         return self._hess.dot(x)
+
+    @property
+    def hess(self):
+        if self._hess is None:
+            raise RuntimeError("no Hessian; call init_hess first")
+        return self._hess
 
     def cg(self, rhs, x0, tol, maxit, minit, verbosity):
         from .solvers import pcg
@@ -152,6 +162,7 @@ class BandWorkerPool:
             self._mine = list(range(nband))
             self._workers = {b: _BandWorkerImpl(self.nthreads_per_band, device=b % ndev) for b in self._mine}
         self.actors = None  # the reference's attribute: no Ray actors here
+        self.last_cg_info = None  # per-band iters / eps / stop of the last device hess_cg
 
     def _map(self, method, per_band_args):
         """Run ``method(*args)`` on the band workers of this process; band -> result."""
@@ -175,17 +186,89 @@ class BandWorkerPool:
                                  etas[b], wsums[b]) for b in range(self.nband)])
 
     def hess_dot(self, x):
+        if getattr(x, "is_cuda", False):
+            return self._complete(self._hess_dot_dev(x))
         out = np.zeros_like(x)
         for b, res in self._map("hess_dot", [(x[b],) for b in range(self.nband)]).items():
             out[b] = res[0]
         return self._complete(out)
 
     def hess_cg(self, rhs, x0, tol, maxit, minit, verbosity):
+        if getattr(rhs, "is_cuda", False):
+            return self._complete(self._hess_cg_dev(rhs, x0, tol, maxit, minit, verbosity))
         out = np.zeros_like(rhs)
         args = [(rhs[b], None if x0 is None else x0[b], tol, maxit, minit, verbosity) for b in range(self.nband)]
         for b, res in self._map("cg", args).items():
             out[b] = res
         return self._complete(out)
+
+    def _dev_cube(self, x, name):
+        """The contiguous (nband, nx, ny) float64 CUDA tensor `x`; raises before anything is launched."""
+        import torch
+
+        if not getattr(x, "is_cuda", False) or x.dtype != torch.float64:
+            raise TypeError(f"{name} must be a float64 CUDA tensor")
+        t = self._workers[self._mine[0]].hess if self._mine else None
+        if t is not None and tuple(x.shape) != (self.nband, t.nx, t.ny):
+            raise ValueError(f"{name} shape {tuple(x.shape)} does not match ({self.nband}, {t.nx}, {t.ny})")
+        return x.contiguous()
+
+    def _hess_dot_dev(self, x):
+        import torch
+
+        x = self._dev_cube(x, "x")
+        out = torch.zeros_like(x) if self._world > 1 else torch.empty_like(x)
+        for b in self._mine:
+            tree = self._workers[b].hess
+            if tree.device == x.device.index:
+                tree._dot_dev(x[b], out=out[b:b + 1])
+            else:
+                out[b].copy_(tree.dot(x[b].to(torch.device("cuda", tree.device)))[0])
+        return out
+
+    def _hess_cg_dev(self, rhs, x0, tol, maxit, minit, verbosity):
+        import torch
+
+        from .psf import tree_cg
+
+        rhs = self._dev_cube(rhs, "rhs")
+        if x0 is not None:
+            x0 = self._dev_cube(x0, "x0")
+            if x0.device != rhs.device:
+                raise ValueError(f"x0 is on {x0.device}, rhs on {rhs.device}")
+        by_dev: dict = {}
+        for b in self._mine:
+            by_dev.setdefault(self._workers[b].hess.device, []).append(b)
+        jobs = []  # the copies run here, on torch's current streams, and each solve on its device's current stream
+        for d, bands in by_dev.items():
+            dev = torch.device("cuda", d)
+            idx = torch.tensor(bands, device=rhs.device)
+            jobs.append((bands, idx, rhs.index_select(0, idx).to(dev),
+                         None if x0 is None else x0.index_select(0, idx).to(dev), torch.cuda.current_stream(dev)))
+
+        def solve(job):
+            bands, _, r, x, st = job
+            return tree_cg([self._workers[b].hess for b in bands], r, x, tol, maxit, minit, stream=st)
+
+        if len(jobs) == 1:
+            results = [solve(jobs[0])]
+        else:  # one host thread per device: the solves synchronise their own stream once per iteration
+            from concurrent.futures import ThreadPoolExecutor
+
+            with ThreadPoolExecutor(len(jobs)) as ex:
+                results = list(ex.map(solve, jobs))
+        out = torch.zeros_like(rhs)
+        info = dict(iters=np.full(self.nband, -1, dtype=np.int64), eps=np.full(self.nband, np.nan),
+                    stop=[None] * self.nband)  # bands of other ranks keep -1 / nan / None
+        for (bands, idx, *_), (sol, inf) in zip(jobs, results):
+            out.index_copy_(0, idx, sol.to(rhs.device))
+            for i, b in enumerate(bands):
+                info["iters"][b], info["eps"][b], info["stop"][b] = inf["iters"][i], inf["eps"][i], inf["stop"][i]
+        self.last_cg_info = info
+        if verbosity:
+            for b in self._mine:
+                print(_pcg_end_message(info["stop"][b], info["iters"][b], info["eps"][b]))
+        return out
 
     # --- Psi role ---
     def init_psi(self, nx, ny, bases, nlevel):
@@ -231,3 +314,14 @@ class BandWorkerPool:
     def close(self):
         for w in self._workers.values():
             w.close()
+
+
+def _pcg_end_message(stop, k, eps):
+    """What ``solvers.pcg`` prints at the end of a solve (verbosity >= 1), from a device stop code."""
+    if stop == "initial residual zero":
+        return "Initial residual is zero"
+    if stop == "maxit":
+        return f"Max iters reached. eps = {eps:.3e}"
+    if stop == "stalled":
+        return f"Stalled after {k} iterations with eps = {eps:.3e}"
+    return f"Success, converged after {k} iterations"

@@ -13,8 +13,12 @@ inline constexpr auto& fail = pfbg_fail;
 void pfbg_count_launch();
 void* pfbg_scratch_get(int device);
 void pfbg_scratch_put(int device, void* p);
-// psfconv.cu: what the batched solvers of pfbsara.cu check before borrowing a convolver
+// psfconv.cu: what the batched solvers of pfbsara.cu check before borrowing a convolver, whether p is a device array
+// on `device`, and pfbg_conv_apply_scaled without its argument checks
 int pfbg_conv_props(const pfbg_conv* cv, int* precision, int* device, int* nx, int* ny, int* has_kernel);
+bool pfbg_on_device(const void* p, int device);
+int pfbg_conv_apply_dev(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta, double scale,
+                        void* out, void* stream);
 // weighting.cu: counts of nsnap snapshots (row_snap: snapshot of each row, NULL for one; scale[f] / lightspeed = f/c),
 // then the Briggs / uniform re-weighting of wgt in place, on stream s.  counts: nsnap * nx * ny reals, sums: 3 * nsnap doubles
 int pfbg_counts_reweight(int precision, cudaStream_t s, int64_t nrow, int nchan, int nx, int ny, double cell_x,

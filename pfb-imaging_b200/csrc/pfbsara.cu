@@ -1,5 +1,5 @@
 // C-ABI of the device backward steps (include/pfbsara.h): SARA (kernels in sara.cuh), the Clark minor cycle
-// (clean.cuh) and the batched conjugate gradients of HessPSF.idot (cg.cuh).
+// (clean.cuh) and the batched conjugate gradients of HessPSF.idot and HessianTree (cg.cuh).
 #include <cuda_runtime.h>
 
 #include <thrust/iterator/counting_iterator.h>
@@ -591,102 +591,142 @@ extern "C" int pfbs_clark_run(pfbs_clark* h, const void* dirty, const uint8_t* m
 }
 
 // ---------------------------------------------------------------------------
-// Batched conjugate gradients on the PSF-convolution Hessian (cg.cuh)
+// Batched conjugate gradients on sums of PSF-convolution terms (cg.cuh): the one CG driver of the library.
+// pfbs_psf_cg is the case of one group per system and scale 1.
 // ---------------------------------------------------------------------------
 
 static const int64_t kCgAlign = 256;
 static int64_t cg_round(int64_t b) { return (b + kCgAlign - 1) / kCgAlign * kCgAlign; }
 static int cg_grid(int64_t npix) { return (int)std::min<int64_t>((npix + CG_THREADS - 1) / CG_THREADS, CG_GMAX); }
 
-extern "C" int64_t pfbs_psf_cg_work_bytes(int32_t nband, int64_t npix) {
-  if (nband < 1 || npix < 1) return -1;
-  return 3 * cg_round((int64_t)nband * npix * 8) + cg_round((int64_t)nband * CG_GMAX * 2 * 8) +
-         cg_round((int64_t)nband * (int64_t)sizeof(CgCtl));
+// r, p, Ap, the partial sums and the CgCtl of every system, then (pingpong) one image for the running sum of a
+// system with two or more groups: the systems are applied one after another on one stream, so they share it
+static int64_t cg_work_bytes(int64_t nsys, int64_t npix, bool pingpong) {
+  return 3 * cg_round(nsys * npix * 8) + cg_round(nsys * CG_GMAX * 2 * 8) + cg_round(nsys * (int64_t)sizeof(CgCtl)) +
+         (pingpong ? cg_round(npix * 8) : 0);
 }
 
-// a device array on `device` (or managed memory)
-static bool cg_on_device(const void* p, int device) {
-  cudaPointerAttributes a{};
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-  return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == device;
+extern "C" int64_t pfbs_psf_cg_work_bytes(int32_t nband, int64_t npix) {
+  if (nband < 1 || npix < 1) return -1;
+  return cg_work_bytes(nband, npix, false);
+}
+
+extern "C" int64_t pfbs_tree_cg_work_bytes(int32_t nsys, const int32_t* group_start, int64_t npix) {
+  if (nsys < 1 || npix < 1 || !group_start) return -1;
+  bool pingpong = false;
+  for (int s = 0; s < nsys; ++s) pingpong |= group_start[s + 1] - group_start[s] >= 2;
+  return cg_work_bytes(nsys, npix, pingpong);
+}
+
+extern "C" int pfbs_tree_cg(int32_t device, int32_t nsys, const int32_t* group_start, pfbg_conv* const* conv,
+                            const void* const* beam, const double* scale, const double* eta, const void* rhs, void* x,
+                            int64_t npix, double tol, int32_t maxit, int32_t minit, void* work, int64_t work_bytes,
+                            int32_t* iters, double* eps, int32_t* stop, void* stream) {
+  if (!group_start || !conv || !beam || !scale || !eta || !rhs || !x || !work || !iters || !eps || !stop)
+    return pfbg_fail(PFBG_ERR_ARG, "null argument");
+  if (nsys < 1 || nsys > 65535) return pfbg_fail(PFBG_ERR_ARG, "nsys %d not in 1..65535", nsys);
+  if (!(tol >= 0.0) || maxit < 0 || minit < 0) return pfbg_fail(PFBG_ERR_ARG, "need tol >= 0, maxit >= 0, minit >= 0");
+  if (group_start[0] != 0) return pfbg_fail(PFBG_ERR_ARG, "group_start[0] = %d, not 0", group_start[0]);
+  for (int s = 0; s < nsys; ++s) {
+    if (group_start[s + 1] <= group_start[s])
+      return pfbg_fail(PFBG_ERR_ARG, "system %d has no group (group_start[%d] = %d, group_start[%d] = %d)", s, s,
+                       group_start[s], s + 1, group_start[s + 1]);
+    if (!(scale[s] > 0.0) || !std::isfinite(scale[s]))
+      return pfbg_fail(PFBG_ERR_ARG, "scale[%d] = %g must be finite and > 0", s, scale[s]);
+  }
+  const int ngroup = group_start[nsys];
+  int ndev = 0;
+  CK(cudaGetDeviceCount(&ndev));
+  if (device < 0 || device >= ndev) return pfbg_fail(PFBG_ERR_ARG, "device %d out of range", device);
+  int nx0 = 0, ny0 = 0;
+  for (int g = 0; g < ngroup; ++g) {
+    int prec = 0, dev = 0, nx = 0, ny = 0, hk = 0;
+    if (!conv[g]) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is NULL", g);
+    CKRC(pfbg_conv_props(conv[g], &prec, &dev, &nx, &ny, &hk));
+    if (prec != PFBG_F64) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is not fp64", g);
+    if (dev != device) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is on device %d, not %d", g, dev, device);
+    if (!hk) return pfbg_fail(PFBG_ERR_STATE, "convolver %d has no kernel", g);
+    if (g == 0) { nx0 = nx; ny0 = ny; }
+    else if (nx != nx0 || ny != ny0)
+      return pfbg_fail(PFBG_ERR_ARG, "convolver %d images are %d x %d, convolver 0's %d x %d", g, nx, ny, nx0, ny0);
+  }
+  if (npix != (int64_t)nx0 * ny0) return pfbg_fail(PFBG_ERR_ARG, "npix %lld != nx * ny = %lld", (long long)npix, (long long)nx0 * ny0);
+  const int64_t need = pfbs_tree_cg_work_bytes(nsys, group_start, npix);
+  if (work_bytes < need) return pfbg_fail(PFBG_ERR_ARG, "work holds %lld bytes, %lld needed", (long long)work_bytes, (long long)need);
+  CK(cudaSetDevice(device));
+  if (!pfbg_on_device(rhs, device) || !pfbg_on_device(x, device) || !pfbg_on_device(work, device))
+    return pfbg_fail(PFBG_ERR_ARG, "rhs, x and work must be device arrays on device %d", device);
+  for (int g = 0; g < ngroup; ++g)
+    if (beam[g] && !pfbg_on_device(beam[g], device)) return pfbg_fail(PFBG_ERR_ARG, "beam %d is not a device array on device %d", g, device);
+
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t vb = cg_round((int64_t)nsys * npix * 8);
+  double* r = (double*)work;
+  double* p = (double*)((char*)work + vb);
+  double* ap = (double*)((char*)work + 2 * vb);
+  double* part = (double*)((char*)work + 3 * vb);
+  CgCtl* ctl = (CgCtl*)((char*)part + cg_round((int64_t)nsys * CG_GMAX * 2 * 8));
+  double* pong = (double*)((char*)ctl + cg_round((int64_t)nsys * (int64_t)sizeof(CgCtl)));
+  const int G = cg_grid(npix);
+  const dim3 grd(G, nsys);
+  const double* xd = (const double*)x;
+  std::vector<CgCtl> h(nsys);
+  // out_s = scale_s sum_g beam_g conv_g(beam_g in_s) + eta_s in_s: the first group adds the ridge term, each later one
+  // adds the running sum (eta = 1) from the other buffer, and the parity puts the last group's output in out_s
+  auto apply = [&](const double* in, double* out, int sys) -> int {
+    const double* xs = in + sys * npix;
+    const double* prev = nullptr;
+    const int g0 = group_start[sys], g1 = group_start[sys + 1];
+    for (int g = g0; g < g1; ++g) {
+      double* dst = ((g1 - 1 - g) & 1) ? pong : out + sys * npix;
+      CKRC(pfbg_conv_apply_dev(conv[g], xs, beam[g], g == g0 ? xs : prev, g == g0 ? eta[sys] : 1.0, scale[sys], dst,
+                               stream));
+      prev = dst;
+    }
+    return PFBG_OK;
+  };
+  auto read_ctl = [&]() -> int {
+    CK(cudaMemcpyAsync(h.data(), ctl, (size_t)nsys * sizeof(CgCtl), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return PFBG_OK;
+  };
+
+  for (int b = 0; b < nsys; ++b) CKRC(apply(xd, r, b));  // r = A x
+  k_cg_init<<<grd, CG_THREADS, 0, s>>>((const double*)rhs, r, p, npix, part);
+  k_cg_init_fin<<<nsys, CG_THREADS, 0, s>>>(ctl, part, G, tol, maxit, minit);
+  LAUNCHED(); LAUNCHED();
+  CK(cudaGetLastError());
+  CKRC(read_ctl());
+  for (;;) {
+    bool any = false;
+    for (int b = 0; b < nsys; ++b)
+      if (h[b].stop == CG_RUNNING) { any = true; CKRC(apply(p, ap, b)); }  // stopped systems skip their convolutions
+    if (!any) break;
+    k_cg_dots<<<grd, CG_THREADS, 0, s>>>(ctl, p, ap, npix, part);
+    k_cg_dots_fin<<<nsys, CG_THREADS, 0, s>>>(ctl, part, G);
+    k_cg_update<<<grd, CG_THREADS, 0, s>>>(ctl, (double*)x, r, p, ap, npix, part);
+    k_cg_update_fin<<<nsys, CG_THREADS, 0, s>>>(ctl, part, G, tol, maxit, minit);
+    k_cg_direction<<<grd, CG_THREADS, 0, s>>>(ctl, p, r, npix);
+    for (int t = 0; t < 5; ++t) LAUNCHED();
+    CK(cudaGetLastError());
+    CKRC(read_ctl());
+  }
+  for (int b = 0; b < nsys; ++b) {
+    iters[b] = h[b].k;
+    eps[b] = h[b].eps;
+    stop[b] = h[b].stop;
+  }
+  return PFBG_OK;
 }
 
 extern "C" int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv, const void* const* beam,
                            const double* eta, const void* rhs, void* x, int64_t npix, double tol, int32_t maxit,
                            int32_t minit, void* work, int64_t work_bytes, int32_t* iters, double* eps, int32_t* stop,
                            void* stream) {
-  if (!conv || !beam || !eta || !rhs || !x || !work || !iters || !eps || !stop)
-    return pfbg_fail(PFBG_ERR_ARG, "null argument");
   if (nband < 1 || nband > 65535) return pfbg_fail(PFBG_ERR_ARG, "nband %d not in 1..65535", nband);
-  if (!(tol >= 0.0) || maxit < 0 || minit < 0) return pfbg_fail(PFBG_ERR_ARG, "need tol >= 0, maxit >= 0, minit >= 0");
-  int ndev = 0;
-  CK(cudaGetDeviceCount(&ndev));
-  if (device < 0 || device >= ndev) return pfbg_fail(PFBG_ERR_ARG, "device %d out of range", device);
-  int nx0 = 0, ny0 = 0;
-  for (int b = 0; b < nband; ++b) {
-    int prec = 0, dev = 0, nx = 0, ny = 0, hk = 0;
-    if (!conv[b]) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is NULL", b);
-    CKRC(pfbg_conv_props(conv[b], &prec, &dev, &nx, &ny, &hk));
-    if (prec != PFBG_F64) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is not fp64", b);
-    if (dev != device) return pfbg_fail(PFBG_ERR_ARG, "convolver %d is on device %d, not %d", b, dev, device);
-    if (!hk) return pfbg_fail(PFBG_ERR_STATE, "convolver %d has no kernel", b);
-    if (b == 0) { nx0 = nx; ny0 = ny; }
-    else if (nx != nx0 || ny != ny0)
-      return pfbg_fail(PFBG_ERR_ARG, "convolver %d images are %d x %d, convolver 0's %d x %d", b, nx, ny, nx0, ny0);
-  }
-  if (npix != (int64_t)nx0 * ny0) return pfbg_fail(PFBG_ERR_ARG, "npix %lld != nx * ny = %lld", (long long)npix, (long long)nx0 * ny0);
-  const int64_t need = pfbs_psf_cg_work_bytes(nband, npix);
-  if (work_bytes < need) return pfbg_fail(PFBG_ERR_ARG, "work holds %lld bytes, %lld needed", (long long)work_bytes, (long long)need);
-  CK(cudaSetDevice(device));
-  if (!cg_on_device(rhs, device) || !cg_on_device(x, device) || !cg_on_device(work, device))
-    return pfbg_fail(PFBG_ERR_ARG, "rhs, x and work must be device arrays on device %d", device);
-  for (int b = 0; b < nband; ++b)
-    if (beam[b] && !cg_on_device(beam[b], device)) return pfbg_fail(PFBG_ERR_ARG, "beam %d is not a device array on device %d", b, device);
-
-  cudaStream_t s = (cudaStream_t)stream;
-  const int64_t vb = cg_round((int64_t)nband * npix * 8);
-  double* r = (double*)work;
-  double* p = (double*)((char*)work + vb);
-  double* ap = (double*)((char*)work + 2 * vb);
-  double* part = (double*)((char*)work + 3 * vb);
-  CgCtl* ctl = (CgCtl*)((char*)part + cg_round((int64_t)nband * CG_GMAX * 2 * 8));
-  const int G = cg_grid(npix);
-  const dim3 grd(G, nband);
-  const double* xd = (const double*)x;
-  std::vector<CgCtl> h(nband);
-  auto apply = [&](const double* in, double* out, int b) {
-    return pfbg_conv_apply(conv[b], in + b * npix, beam[b], eta[b], out + b * npix, PFBG_DEVICE_PTRS, stream);
-  };
-  auto read_ctl = [&]() -> int {
-    CK(cudaMemcpyAsync(h.data(), ctl, (size_t)nband * sizeof(CgCtl), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    return PFBG_OK;
-  };
-
-  for (int b = 0; b < nband; ++b) CKRC(apply(xd, r, b));  // r = A x
-  k_cg_init<<<grd, CG_THREADS, 0, s>>>((const double*)rhs, r, p, npix, part);
-  k_cg_init_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G, tol, maxit, minit);
-  LAUNCHED(); LAUNCHED();
-  CK(cudaGetLastError());
-  CKRC(read_ctl());
-  for (;;) {
-    bool any = false;
-    for (int b = 0; b < nband; ++b)
-      if (h[b].stop == CG_RUNNING) { any = true; CKRC(apply(p, ap, b)); }  // stopped bands skip their convolution
-    if (!any) break;
-    k_cg_dots<<<grd, CG_THREADS, 0, s>>>(ctl, p, ap, npix, part);
-    k_cg_dots_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G);
-    k_cg_update<<<grd, CG_THREADS, 0, s>>>(ctl, (double*)x, r, p, ap, npix, part);
-    k_cg_update_fin<<<nband, CG_THREADS, 0, s>>>(ctl, part, G, tol, maxit, minit);
-    k_cg_direction<<<grd, CG_THREADS, 0, s>>>(ctl, p, r, npix);
-    for (int t = 0; t < 5; ++t) LAUNCHED();
-    CK(cudaGetLastError());
-    CKRC(read_ctl());
-  }
-  for (int b = 0; b < nband; ++b) {
-    iters[b] = h[b].k;
-    eps[b] = h[b].eps;
-    stop[b] = h[b].stop;
-  }
-  return PFBG_OK;
+  std::vector<int32_t> group_start(nband + 1);
+  for (int b = 0; b <= nband; ++b) group_start[b] = b;
+  const std::vector<double> scale(nband, 1.0);
+  return pfbs_tree_cg(device, nband, group_start.data(), conv, beam, scale.data(), eta, rhs, x, npix, tol, maxit, minit,
+                      work, work_bytes, iters, eps, stop, stream);
 }

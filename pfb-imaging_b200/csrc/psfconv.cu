@@ -272,9 +272,11 @@ static void conv_cols_launch(const pfbg_conv* cv, const Mul& mul, cudaStream_t s
 
 // xin != NULL: out += eta * xin in the row epilogue (the ridge term of the Hessian, or eta = 1 for apply_add).
 // shift != NULL (fp64, stored spectrum): the column pass multiplies by ShiftMul instead of the convolver's own kernel.
+// scale multiplies the convolution term: the epilogue factor is scale / (nxp nyp), the same double as 1 / (nxp nyp) at
+// scale = 1.
 template <typename T>
 static int conv_apply_t(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta, void* out,
-                        cudaStream_t s, const ShiftMul* shift) {
+                        cudaStream_t s, const ShiftMul* shift, double scale) {
   const ConvTabs& ct = cv->ct;
   const int rt = row_threads(ct.nyp, 256);
   k_conv_rows_fwd<T><<<(ct.nx + 1) / 2, rt, fft_smem_bytes<T>(ct.nyp), s>>>(ct, (const T*)x, (const T*)beam, (cx2<T>*)cv->tmp);
@@ -288,9 +290,9 @@ static int conv_apply_t(pfbg_conv* cv, const void* x, const void* beam, const vo
     else conv_cols_launch<T>(cv, KhatMul{}, s);
   }
   LAUNCHED();
-  const double scale = 1.0 / ((double)ct.nxp * (double)ct.nyp);
+  const double escale = scale / ((double)ct.nxp * (double)ct.nyp);
   k_conv_rows_inv<T><<<(ct.nx + 1) / 2, rt, fft_smem_bytes<T>(ct.nyp), s>>>(ct, (const cx2<T>*)cv->tmp, (const T*)beam,
-                                                                 (const T*)xin, scale, eta, (T*)out);
+                                                                 (const T*)xin, escale, eta, (T*)out);
   LAUNCHED();
   CK(cudaGetLastError());
   return PFBG_OK;
@@ -299,7 +301,7 @@ static int conv_apply_t(pfbg_conv* cv, const void* x, const void* beam, const vo
 // out = beam * crop(IFFT(FFT(pad(beam * x)) * K)) + eta * xin; host pointers are staged through d_x / d_beam / d_out
 // (apply_add passes no beam, so its `add` image rides in d_beam)
 static int conv_apply_any(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta, void* out,
-                          uint32_t flags, void* stream, const ShiftMul* shift = nullptr) {
+                          uint32_t flags, void* stream, const ShiftMul* shift = nullptr, double scale = 1.0) {
   if (!cv || !x || !out) return fail(PFBG_ERR_ARG, "null argument");
   if (!cv->has_kernel) return fail(PFBG_ERR_STATE, "no kernel set");
   CK(cudaSetDevice(cv->device));
@@ -316,8 +318,8 @@ static int conv_apply_any(pfbg_conv* cv, const void* x, const void* beam, const 
     else if (xin) { CK(cudaMemcpyAsync(cv->d_beam, xin, ib, cudaMemcpyHostToDevice, s)); dxin = cv->d_beam; }
     dout = cv->d_out;
   }
-  CKRC(cv->precision == PFBG_F32 ? conv_apply_t<float>(cv, dx, db, dxin, eta, dout, s, nullptr)
-                                 : conv_apply_t<double>(cv, dx, db, dxin, eta, dout, s, shift));
+  CKRC(cv->precision == PFBG_F32 ? conv_apply_t<float>(cv, dx, db, dxin, eta, dout, s, nullptr, scale)
+                                 : conv_apply_t<double>(cv, dx, db, dxin, eta, dout, s, shift, scale));
   if (!dev) {
     CK(cudaMemcpyAsync(out, dout, ib, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
@@ -336,6 +338,34 @@ extern "C" int pfbg_conv_apply_add(pfbg_conv* cv, const void* x, const void* add
                                    void* stream) {
   if (!add) return fail(PFBG_ERR_ARG, "null argument");
   return conv_apply_any(cv, x, nullptr, add, 1.0, out, flags, stream);
+}
+
+// a device array on `device` (or managed memory)
+bool pfbg_on_device(const void* p, int device) {
+  cudaPointerAttributes a{};
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+  return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == device;
+}
+
+// the unchecked device-pointer body of pfbg_conv_apply_scaled, for the batched solvers (xin is ignored when eta == 0)
+int pfbg_conv_apply_dev(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta, double scale,
+                        void* out, void* stream) {
+  return conv_apply_any(cv, x, beam, eta != 0.0 ? xin : nullptr, eta, out, PFBG_DEVICE_PTRS, stream, nullptr, scale);
+}
+
+// out = scale * beam * crop(IFFT(FFT(pad(beam * x)) * K)) + eta * xin, device arrays only
+extern "C" int pfbg_conv_apply_scaled(pfbg_conv* cv, const void* x, const void* beam, const void* xin, double eta,
+                                      double scale, void* out, uint32_t flags, void* stream) {
+  if (!cv || !x || !out || (eta != 0.0 && !xin)) return fail(PFBG_ERR_ARG, "null argument");
+  if (!(flags & PFBG_DEVICE_PTRS)) return fail(PFBG_ERR_ARG, "pfbg_conv_apply_scaled takes device pointers only");
+  if (!(scale > 0.0) || !std::isfinite(scale)) return fail(PFBG_ERR_ARG, "scale %g must be finite and > 0", scale);
+  if (eta != 0.0 && xin == out) return fail(PFBG_ERR_ARG, "xin must not alias out (accumulate through a second buffer)");
+  CK(cudaSetDevice(cv->device));
+  const void* ptrs[] = {x, beam, eta != 0.0 ? xin : nullptr, out};
+  for (const void* p : ptrs)
+    if (p && !pfbg_on_device(p, cv->device))
+      return fail(PFBG_ERR_ARG, "x, beam, xin and out must be device arrays on device %d", cv->device);
+  return pfbg_conv_apply_dev(cv, x, beam, xin, eta, scale, out, stream);
 }
 
 // out = taper * crop(IFFT(FFT(pad(taper * x)) * (Re khat + c)^(+-1)))   (taper may be NULL; no ridge term)

@@ -271,7 +271,12 @@ class HessianTree:
     `partitions`: dicts with ``psfhat`` (corr, nx_psf, nyo2), ``beam`` (corr, nx, ny), ``wsum`` (corr,).  Partitions
     that share a beam (bit for bit) are merged by linearity — their kernels are summed once at construction — so
     the common case of one beam per band costs one device convolution per correlation whatever the number of
-    partitions; distinct beams keep one convolver each."""
+    partitions; distinct beams keep one convolver each.
+
+    numpy in, numpy out as in the reference.  A float64 CUDA tensor on the tree's :attr:`device`, ``(ncorr, nx, ny)``
+    or ``(nx, ny)`` when ``ncorr == 1``, stays there: ``dot`` returns a new ``(ncorr, nx, ny)`` tensor computed on
+    torch's current stream (``pfbg_conv_apply_scaled`` per group, the groups of a correlation summed through a second
+    buffer).  The beams are uploaded on the first device call."""
 
     def __init__(self, partitions, nx, ny, nx_psf, ny_psf, eta=0.0, nthreads=1, wsum=None, device=None):
         if not partitions:
@@ -302,8 +307,55 @@ class HessianTree:
         for c, beam, khat in groups.values():
             cv = PsfConvolver(nx, ny, nx_psf, ny_psf, dtype=np.float64, device=device).set_kernel(khat)
             self._groups.append((c, beam, cv))
+        self.device = self._groups[0][2].device
+        self._dev_beams = None  # device copies of the group beams, uploaded on the first device call
+
+    def _beams_dev(self):
+        import torch
+
+        if self._dev_beams is None:
+            dev = torch.device("cuda", self.device)
+            self._dev_beams = [None if bm is None else torch.from_numpy(bm).to(dev) for _, bm, _ in self._groups]
+        return self._dev_beams
+
+    def corr_groups(self, c):
+        """(convolver, device beam or None) of every group of correlation c."""
+        return [(cv, bm) for (gc, _, cv), bm in zip(self._groups, self._beams_dev()) if gc == c]
+
+    def _dot_dev(self, x, out=None):
+        import torch
+
+        if x.dtype != torch.float64:
+            raise TypeError(f"device input must be float64, got {x.dtype}")
+        if x.device.index != self.device:
+            raise ValueError(f"input is on {x.device}, the operator on cuda:{self.device}")
+        xt = x if x.dim() == 3 else x[None]
+        ncorr, nx, ny = xt.shape
+        assert ncorr == self.ncorr, f"expected {self.ncorr} correlations on axis 0, got {ncorr}"
+        assert nx == self.nx and ny == self.ny
+        xt = xt.contiguous()
+        out = torch.empty_like(xt) if out is None else out
+        s = torch.cuda.current_stream(xt.device).cuda_stream
+        pong = None
+        for c in range(ncorr):
+            gs = self.corr_groups(c)
+            if len(gs) > 1 and pong is None:
+                pong = torch.empty_like(xt[0])
+            prev = None
+            for i, (cv, bm) in enumerate(gs):
+                # the last group writes out[c]; the ridge term comes in with the first, the running sum with the others
+                dst = out[c] if (len(gs) - 1 - i) % 2 == 0 else pong
+                xin, eta = (xt[c], float(self.eta)) if i == 0 else (prev, 1.0)
+                _lib.check(cv._lib.pfbg_conv_apply_scaled(
+                    cv._h, C.c_void_p(xt[c].data_ptr()), None if bm is None else C.c_void_p(bm.data_ptr()),
+                    C.c_void_p(xin.data_ptr()), eta, 1.0 / float(self.wsum[c]), C.c_void_p(dst.data_ptr()),
+                    _lib.DEVICE_PTRS, s))
+                prev = dst
+        return out
 
     def dot(self, x):
+        if getattr(x, "is_cuda", False):
+            return self._dot_dev(x)
         x = np.asarray(x)
         xtmp = x if x.ndim == 3 else x[None, :, :]
         ncorr, nx, ny = xtmp.shape
@@ -322,11 +374,70 @@ class HessianTree:
         for _, _, cv in self._groups:
             cv.close()
         self._groups = []
+        self._dev_beams = None
+
+
+CG_STOP = {1: "converged", 2: "maxit", 3: "stalled", 4: "initial residual zero", 5: "exact"}  # pfbsara.h PFBS_CG_*
+
+
+def tree_cg(trees, rhs_t, x0_t, tol, maxit, minit, stream=None):
+    """Batched CG over the corr-0 systems of `trees` (HessianTrees on one device, sharing (nx, ny)): solves
+    ``trees[s].dot(v)[0] = rhs_t[s]`` for every s with one ``pfbs_tree_cg``, the stopping rules of ``solvers.pcg``.
+
+    `rhs_t`: ``(len(trees), nx, ny)`` float64 CUDA tensor on the trees' device; `x0_t`: None (start from zero) or a
+    tensor like it, read and not modified.  Runs on `stream` (a ``torch.cuda.Stream``; default: torch's current stream
+    of the device).  Returns the solution and a dict of per-system ``iters``, ``eps`` and ``stop`` (``CG_STOP``
+    strings).  A tree with more than one correlation fails the assertion the host solve fails."""
+    import torch
+
+    n = len(trees)
+    if n == 0:
+        raise ValueError("tree_cg needs at least one tree")
+    t0 = trees[0]
+    for t in trees:
+        assert t.ncorr == 1, f"expected {t.ncorr} correlations on axis 0, got 1"
+        if t.device != t0.device or (t.nx, t.ny) != (t0.nx, t0.ny):
+            raise ValueError("the trees of one batched solve must share the device and (nx, ny)")
+    shape = (n, t0.nx, t0.ny)
+    for name, v in (("rhs", rhs_t), ("x0", x0_t)):
+        if v is None:
+            continue
+        if v.dtype != torch.float64:
+            raise TypeError(f"{name} must be float64, got {v.dtype}")
+        if tuple(v.shape) != shape:
+            raise ValueError(f"{name} shape {tuple(v.shape)} does not match {shape}")
+        if not v.is_cuda or v.device.index != t0.device:
+            raise ValueError(f"{name} is on {v.device}, the trees on cuda:{t0.device}")
+    dev = torch.device("cuda", t0.device)
+    stream = torch.cuda.current_stream(dev) if stream is None else stream
+    with torch.cuda.stream(stream):
+        rhs = rhs_t.contiguous()
+        sol = torch.zeros(shape, dtype=torch.float64, device=dev) if x0_t is None else x0_t.clone(
+            memory_format=torch.contiguous_format)
+        group_start, convs, beams = [0], [], []
+        for t in trees:
+            gs = t.corr_groups(0)
+            convs += [cv._h.value for cv, _ in gs]
+            beams += [None if bm is None else bm.data_ptr() for _, bm in gs]
+            group_start.append(len(convs))
+        lib, ng, npix = _lib.load(), len(convs), t0.nx * t0.ny
+        gs_arr = (C.c_int32 * (n + 1))(*group_start)
+        nbytes = int(lib.pfbs_tree_cg_work_bytes(n, gs_arr, npix))
+        work = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        iters, eps, stop = (C.c_int32 * n)(), (C.c_double * n)(), (C.c_int32 * n)()
+        _lib.check(lib.pfbs_tree_cg(t0.device, n, gs_arr, (C.c_void_p * ng)(*convs), (C.c_void_p * ng)(*beams),
+                                    (C.c_double * n)(*[1.0 / float(t.wsum[0]) for t in trees]),
+                                    (C.c_double * n)(*[float(t.eta) for t in trees]), C.c_void_p(rhs.data_ptr()),
+                                    C.c_void_p(sol.data_ptr()), npix, float(tol), int(maxit), int(minit),
+                                    C.c_void_p(work.data_ptr()), nbytes, iters, eps, stop, stream.cuda_stream))
+    info = dict(iters=np.array(iters[:], dtype=np.int64), eps=np.array(eps[:]), stop=[CG_STOP.get(v, str(v)) for v in stop])
+    return sol, info
 
 
 class HessTreeRay:
     """Cube-level Hessian over per-band :class:`HessianTree` operators held by a band pool
-    (operators/hessian.py:525-615); `workers` is a :class:`pfb_imaging_b200.operators.BandWorkerPool`."""
+    (operators/hessian.py:525-615); `workers` is a :class:`pfb_imaging_b200.operators.BandWorkerPool`.  ``dot`` and
+    ``cg`` take numpy cubes or ``(nband, nx, ny)`` float64 CUDA tensors, which stay on the device."""
 
     def __init__(self, partitions_per_band, nx, ny, nx_psf, ny_psf, etas=0.0, nthreads=1, wsums=None, cg_tol=1e-3,
                  cg_maxit=150, cg_minit=1, cg_verbose=0, workers=None):
@@ -364,8 +475,10 @@ class HessTreeRay:
     def get_mem(self):
         return self._pool.get_mem()
 
-
-CG_STOP = {1: "converged", 2: "maxit", 3: "stalled", 4: "initial residual zero", 5: "exact"}  # pfbsara.h PFBS_CG_*
+    @property
+    def last_cg_info(self):
+        """Per-band ``iters`` / ``eps`` / ``stop`` of the last device :meth:`cg` (``BandWorkerPool.last_cg_info``)."""
+        return self._pool.last_cg_info
 
 
 class HessPSF:
@@ -441,7 +554,7 @@ class HessPSF:
             self.conv[b].apply_shifted_dev(xt[b].data_ptr(), out[b].data_ptr(), consts["taper"].data_ptr(),
                                            c=float(self.eta[b]) * c0, inverse=True, stream=stream)
 
-    def _dot_dev(self, x):
+    def _dot_dev(self, x, out=None):
         import torch
 
         xt = self._dev_input(x)
@@ -554,9 +667,10 @@ class PsfGradient:
     """Gradient of the smooth term of the deconvolution sub-problem, ``grad(x) = hess(x) - dirty`` with the
     PSF-convolution Hessian (the `grad` callables built in ``core/sara.py:300-340`` / ``deconv`` presets), usable both as
     the reference's numpy callable and, through ``device_apply``, inside the device-resident loops of
-    ``pfb_imaging_b200.sara`` (no host round trip per iteration)."""
+    ``pfb_imaging_b200.sara`` (no host round trip per iteration).  `hess` is a :class:`HessPSF` or, for ``pfb deconv``,
+    a :class:`HessTreeRay` (its bands may sit on other devices: the pool copies them there and back)."""
 
-    def __init__(self, hess: HessPSF, dirty):
+    def __init__(self, hess, dirty):
         self.hess = hess
         self.dirty = np.ascontiguousarray(dirty, dtype=np.float64)
         if self.dirty.shape != (hess.nband, hess.nx, hess.ny):
@@ -569,11 +683,16 @@ class PsfGradient:
     def device_apply(self, x_t, out_t):
         import torch
 
+        tree = not isinstance(self.hess, HessPSF)
         if self._dev is None:
             dev = x_t.device
             self._dev = dict(dirty=torch.from_numpy(self.dirty).to(dev),
-                             beam=[None if b is None else torch.from_numpy(np.ascontiguousarray(b, dtype=np.float64)).to(dev)
-                                   for b in self.hess.beam])
+                             beam=[] if tree else [None if b is None else
+                                                   torch.from_numpy(np.ascontiguousarray(b, dtype=np.float64)).to(dev)
+                                                   for b in self.hess.beam])
+        if tree:
+            torch.sub(self.hess.dot(x_t), self._dev["dirty"], out=out_t)
+            return
         s = torch.cuda.current_stream(x_t.device).cuda_stream
         for b in range(self.hess.nband):
             bm = self._dev["beam"][b]
