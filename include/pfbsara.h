@@ -15,7 +15,7 @@
  *     positivity / positivity_band (prox/positivity.py:13-38)                               -> pfbs_extrapolate /
  *                                                                                              pfbs_primal_step / pfbs_norm_diff
  *   - clark (deconv/clark.py), semantics as restated in oracle/clark_np.py                  -> pfbs_clark_run
- *   - pcg on HessPSF / HessianTree (operators/hessian.py:357-522, opt/pcg.py:202-314)       -> pfbs_psf_cg / pfbs_tree_cg
+ *   - pcg on HessPSF / HessianTree (operators/hessian.py:357-522, opt/pcg.py:202-314)       -> pfbs_tree_cg
  */
 #ifndef PFBSARA_H
 #define PFBSARA_H
@@ -113,15 +113,22 @@ int pfbs_clark_run(pfbs_clark* h, const void* dirty, const uint8_t* mask, void* 
 int pfbs_clark_destroy(pfbs_clark* h);
 
 /*
- * Conjugate gradients on the PSF-convolution Hessian of every band at once (HessPSF.idot(mode="psf"),
- * operators/hessian.py:357-436), fp64 only.  Per band b, solvers.pcg with no preconditioner on
- *     A_b v = beam_b conv_b(beam_b v) + eta_b v      (pfbg_conv_apply(conv[b], v, beam[b], eta[b]))
- * rhs and x are (nband, nx, ny) device arrays, npix = nx * ny; x holds the starting point on entry and the solution on
- * return.  beam[b] may be NULL.  The convolvers are borrowed (any kernel mode) and must share (nx, ny) and `device`.
- * work: device memory of at least pfbs_psf_cg_work_bytes(nband, npix) bytes (r, p, Ap and the reductions).
- * Stopping rules as pcg: iterate while (eps > tol or k < minit) and k < maxit and stalls < 5, each band on its own;
- * a band that stops is frozen and its convolutions are skipped.  Host outputs per band: iters, eps and stop, one of
- * the PFBS_CG_* codes below.  All reductions are deterministic.  Synchronises `stream` once per iteration.
+ * Conjugate gradients on grouped PSF-convolution Hessians, every system at once, fp64 only: the corr-0 operator of a
+ * band's HessianTree (operators/hessian.py:439-522), a sum over the beam groups g = group_start[s] ..
+ * group_start[s+1]-1 of system s,
+ *     A_s v = scale_s sum_g beam_g conv_g(beam_g v) + eta_s v      (scale_s = 1 / wsum_s)
+ * applied with pfbg_conv_apply_scaled, accumulating through one scratch image.  HessPSF.idot(mode="psf")
+ * (operators/hessian.py:357-436) is the case of one group per system and scale 1, A_b v = pfbg_conv_apply(conv[b], v,
+ * beam[b], eta[b]).  conv[] and beam[] are the flattened group lists (beam[g] may be NULL), scale[] and eta[] have one
+ * entry per system.  The convolvers are borrowed (any kernel mode) and must share (nx, ny) and `device`.
+ * rhs and x are (nsys, nx, ny) device arrays, npix = nx * ny; x holds the starting point on entry and the solution on
+ * return.  Per system, solvers.pcg with no preconditioner: iterate while (eps > tol or k < minit) and k < maxit and
+ * stalls < 5, each system on its own; a system that stops is frozen and its convolutions are skipped.  Host outputs
+ * per system: iters, eps and stop, one of the PFBS_CG_* codes below.  All reductions are deterministic.  Synchronises
+ * `stream` once per iteration.  PFBG_ERR_ARG also for group_start[0] != 0, a system without a group, and a scale that
+ * is not finite and > 0.
+ * work: device memory of at least pfbs_tree_cg_work_bytes(nsys, group_start, npix) bytes (r, p, Ap, the reductions,
+ * and one more image when some system has two or more groups; -1 for nsys < 1, npix < 1 or no group_start).
  */
 #define PFBS_CG_CONVERGED 1
 #define PFBS_CG_MAXIT 2
@@ -129,23 +136,6 @@ int pfbs_clark_destroy(pfbs_clark* h);
 #define PFBS_CG_ZERO_RESIDUAL 4 /* r = A x - b had r.r not > 0: x is left as it was */
 #define PFBS_CG_EXACT 5         /* rho == 0 and p.Ap == 0: the iterate is the solution */
 
-int64_t pfbs_psf_cg_work_bytes(int32_t nband, int64_t npix); /* -1 for nband < 1 or npix < 1 */
-int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv, const void* const* beam, const double* eta,
-                const void* rhs, void* x, int64_t npix, double tol, int32_t maxit, int32_t minit, void* work,
-                int64_t work_bytes, int32_t* iters, double* eps, int32_t* stop, void* stream);
-
-/*
- * The same conjugate gradients on grouped systems: the corr-0 operator of a band's HessianTree
- * (operators/hessian.py:439-522), a sum over the beam groups g = group_start[s] .. group_start[s+1]-1 of system s,
- *     A_s v = scale_s sum_g beam_g conv_g(beam_g v) + eta_s v      (scale_s = 1 / wsum_s)
- * applied with pfbg_conv_apply_scaled, accumulating through one scratch image.  conv[] and beam[] are the flattened
- * group lists (beam[g] may be NULL), scale[] and eta[] have one entry per system.  Everything else (layout of rhs and
- * x, stopping rules, outputs, deterministic reductions, skipped convolutions of stopped systems) is pfbs_psf_cg's,
- * which is this function with one group per band and scale 1.  PFBG_ERR_ARG also for group_start[0] != 0, a system
- * without a group, and a scale that is not finite and > 0.
- * work: at least pfbs_tree_cg_work_bytes(nsys, group_start, npix) bytes, which adds one image to
- * pfbs_psf_cg_work_bytes when some system has two or more groups (-1 for nsys < 1, npix < 1 or no group_start).
- */
 int64_t pfbs_tree_cg_work_bytes(int32_t nsys, const int32_t* group_start, int64_t npix);
 int pfbs_tree_cg(int32_t device, int32_t nsys, const int32_t* group_start, pfbg_conv* const* conv,
                  const void* const* beam, const double* scale, const double* eta, const void* rhs, void* x,

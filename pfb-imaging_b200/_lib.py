@@ -131,9 +131,6 @@ SIGNATURES = {
     "pfbs_clark_destroy": (C.c_int, [_vp]),
     "pfbs_clark_run": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _dbl, _dbl, _dbl, _i32, _dbl, _i32, C.POINTER(_i32), _vp, _vp,
                                  _vp, _vp, _i64, _vp, _u32, _vp]),
-    "pfbs_psf_cg_work_bytes": (_i64, [_i32, _i64]),
-    "pfbs_psf_cg": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _dbl, _i32, _i32, _vp, _i64, _vp, _vp, _vp,
-                              _vp]),
     "pfbs_tree_cg_work_bytes": (_i64, [_i32, _vp, _i64]),
     "pfbs_tree_cg": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _dbl, _i32, _i32, _vp, _i64, _vp,
                                _vp, _vp, _vp]),

@@ -163,6 +163,7 @@ class BandWorkerPool:
             self._workers = {b: _BandWorkerImpl(self.nthreads_per_band, device=b % ndev) for b in self._mine}
         self.actors = None  # the reference's attribute: no Ray actors here
         self.last_cg_info = None  # per-band iters / eps / stop of the last device hess_cg
+        self._hess_shape = None  # (nband, nx, ny) of init_hess
 
     def _map(self, method, per_band_args):
         """Run ``method(*args)`` on the band workers of this process; band -> result."""
@@ -182,6 +183,7 @@ class BandWorkerPool:
     # --- Hessian role ---
     def init_hess(self, partitions_per_band, nx, ny, nx_psf, ny_psf, etas, wsums):
         """Build per-band HessianTrees; ``partitions_per_band=None`` uses load_bands data."""
+        self._hess_shape = (self.nband, nx, ny)
         self._map("init_hess", [(None if partitions_per_band is None else partitions_per_band[b], nx, ny, nx_psf, ny_psf,
                                  etas[b], wsums[b]) for b in range(self.nband)])
 
@@ -203,15 +205,12 @@ class BandWorkerPool:
         return self._complete(out)
 
     def _dev_cube(self, x, name):
-        """The contiguous (nband, nx, ny) float64 CUDA tensor `x`; raises before anything is launched."""
-        import torch
+        """The contiguous (nband, nx, ny) float64 CUDA tensor `x`, on any device; raises before anything is launched."""
+        from .psf import _dev_cube
 
-        if not getattr(x, "is_cuda", False) or x.dtype != torch.float64:
-            raise TypeError(f"{name} must be a float64 CUDA tensor")
-        t = self._workers[self._mine[0]].hess if self._mine else None
-        if t is not None and tuple(x.shape) != (self.nband, t.nx, t.ny):
-            raise ValueError(f"{name} shape {tuple(x.shape)} does not match ({self.nband}, {t.nx}, {t.ny})")
-        return x.contiguous()
+        if self._hess_shape is None:
+            raise RuntimeError("no Hessian; call init_hess first")
+        return _dev_cube(x, self._hess_shape, None, name)
 
     def _hess_dot_dev(self, x):
         import torch

@@ -22,7 +22,7 @@ import math
 import numpy as np
 
 from . import _lib
-from .wgridder import content_hash, current_device
+from .wgridder import HandleCache, content_hash, current_device
 
 MAX_BANDS = 1024  # PFBS_CLARK_MAX_BANDS
 
@@ -141,7 +141,7 @@ class Clark:
             pass
 
 
-_CLARK_CACHE: dict = {}
+_CLARK_CACHE = HandleCache(2)  # a handle holds the PSF, its spectra and the work arrays: gigabytes at scale
 
 
 def _clark_for(psf, psfhat, nx, ny):
@@ -151,21 +151,11 @@ def _clark_for(psf, psfhat, nx, ny):
     key = (psf.ctypes.data, psf.shape, psf.dtype.str, int(nx), int(ny),
            None if psfhat is None else (np.asarray(psfhat).ctypes.data, np.asarray(psfhat).shape))
     chk = (content_hash(psf), None if psfhat is None else content_hash(psfhat))
-    hit = _CLARK_CACHE.get(key)
-    if hit is not None and hit[1] == chk:
-        return hit[0]
-    if hit is not None:
-        hit[0].close()
-    while len(_CLARK_CACHE) >= 2:  # a handle holds the PSF, its spectra and the work arrays: gigabytes at scale
-        _CLARK_CACHE.pop(next(iter(_CLARK_CACHE)))[0].close()
-    cl = Clark(psf, psfhat, nx=nx, ny=ny)
-    _CLARK_CACHE[key] = (cl, chk, psf, psfhat)
-    return cl
+    return _CLARK_CACHE.get(key, chk, lambda: Clark(psf, psfhat, nx=nx, ny=ny), keep=(psf, psfhat))
 
 
 def clear_clark_cache():
-    while _CLARK_CACHE:
-        _CLARK_CACHE.popitem()[1][0].close()
+    _CLARK_CACHE.clear()
 
 
 def clark(ID, PSF, PSFHAT=None, mask=None, threshold=0.0, gamma=0.05, pf=0.05, maxit=50, subpf=0.5, submaxit=1000):

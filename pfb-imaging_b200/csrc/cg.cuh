@@ -1,4 +1,4 @@
-// Batched conjugate gradients on the PSF-convolution Hessian (pfbs_psf_cg): the vector work of solvers.pcg
+// Batched conjugate gradients on the PSF-convolution Hessian (pfbs_tree_cg): the vector work of solvers.pcg
 // (solvers.py:35-82, no preconditioner) for every band of a cube in one launch per step.  Band = blockIdx.y; each band
 // keeps its own scalars in a CgCtl, and a band whose `stop` is set is skipped by every kernel (frozen).
 //

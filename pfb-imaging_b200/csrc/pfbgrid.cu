@@ -77,7 +77,7 @@ void pfbg_scratch_put(int device, void* p) {
   } while (0)
 
 extern "C" const char* pfbg_last_error(void) { return g_err.c_str(); }
-extern "C" int pfbg_version(void) { return 100; }
+extern "C" int pfbg_version(void) { return 101; }
 extern "C" int64_t pfbg_launch_count(void) { return g_launches.load(); }
 extern "C" int pfbg_device_count(int32_t* count) {
   int n = 0;

@@ -592,7 +592,7 @@ extern "C" int pfbs_clark_run(pfbs_clark* h, const void* dirty, const uint8_t* m
 
 // ---------------------------------------------------------------------------
 // Batched conjugate gradients on sums of PSF-convolution terms (cg.cuh): the one CG driver of the library.
-// pfbs_psf_cg is the case of one group per system and scale 1.
+// HessPSF.idot calls it with one group per system and scale 1.
 // ---------------------------------------------------------------------------
 
 static const int64_t kCgAlign = 256;
@@ -604,11 +604,6 @@ static int cg_grid(int64_t npix) { return (int)std::min<int64_t>((npix + CG_THRE
 static int64_t cg_work_bytes(int64_t nsys, int64_t npix, bool pingpong) {
   return 3 * cg_round(nsys * npix * 8) + cg_round(nsys * CG_GMAX * 2 * 8) + cg_round(nsys * (int64_t)sizeof(CgCtl)) +
          (pingpong ? cg_round(npix * 8) : 0);
-}
-
-extern "C" int64_t pfbs_psf_cg_work_bytes(int32_t nband, int64_t npix) {
-  if (nband < 1 || npix < 1) return -1;
-  return cg_work_bytes(nband, npix, false);
 }
 
 extern "C" int64_t pfbs_tree_cg_work_bytes(int32_t nsys, const int32_t* group_start, int64_t npix) {
@@ -717,16 +712,4 @@ extern "C" int pfbs_tree_cg(int32_t device, int32_t nsys, const int32_t* group_s
     stop[b] = h[b].stop;
   }
   return PFBG_OK;
-}
-
-extern "C" int pfbs_psf_cg(int32_t device, int32_t nband, pfbg_conv* const* conv, const void* const* beam,
-                           const double* eta, const void* rhs, void* x, int64_t npix, double tol, int32_t maxit,
-                           int32_t minit, void* work, int64_t work_bytes, int32_t* iters, double* eps, int32_t* stop,
-                           void* stream) {
-  if (nband < 1 || nband > 65535) return pfbg_fail(PFBG_ERR_ARG, "nband %d not in 1..65535", nband);
-  std::vector<int32_t> group_start(nband + 1);
-  for (int b = 0; b <= nband; ++b) group_start[b] = b;
-  const std::vector<double> scale(nband, 1.0);
-  return pfbs_tree_cg(device, nband, group_start.data(), conv, beam, scale.data(), eta, rhs, x, npix, tol, maxit, minit,
-                      work, work_bytes, iters, eps, stop, stream);
 }

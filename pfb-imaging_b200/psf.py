@@ -20,7 +20,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .wgridder import content_hash, current_device
+from .wgridder import HandleCache, content_hash, current_device
 
 _RDT = {np.dtype(np.float32): (_lib.PFBG_F32, np.complex64), np.dtype(np.float64): (_lib.PFBG_F64, np.complex128)}
 
@@ -149,7 +149,7 @@ class PsfConvolver:
             pass
 
 
-_CONV_CACHE: dict = {}
+_CONV_CACHE = HandleCache(16)
 
 
 def _convolver_for(khat, nx, ny, lastsize, rdt):
@@ -158,21 +158,12 @@ def _convolver_for(khat, nx, ny, lastsize, rdt):
     ny_psf = int(lastsize) if lastsize is not None else 2 * (khat.shape[1] - 1)
     key = (khat.ctypes.data, khat.shape, khat.dtype.str, nx, ny, ny_psf, np.dtype(rdt).str)
     chk = content_hash(khat)  # the whole spectrum: an in-place edit of any element rebuilds the convolver
-    hit = _CONV_CACHE.get(key)
-    if hit is not None and hit[1] == chk:
-        return hit[0]
-    if hit is not None:
-        hit[0].close()
-    while len(_CONV_CACHE) >= 16:
-        _CONV_CACHE.pop(next(iter(_CONV_CACHE)))[0].close()
-    cv = PsfConvolver(nx, ny, nx_psf, ny_psf, dtype=rdt).set_kernel(khat)
-    _CONV_CACHE[key] = (cv, chk, khat)
-    return cv
+    return _CONV_CACHE.get(key, chk, lambda: PsfConvolver(nx, ny, nx_psf, ny_psf, dtype=rdt).set_kernel(khat),
+                           keep=khat)
 
 
 def clear_convolver_cache():
-    while _CONV_CACHE:
-        _CONV_CACHE.popitem()[1][0].close()
+    _CONV_CACHE.clear()
 
 
 def psf_convolve_slice(xpad, xhat, xout, psfhat, lastsize, x, nthreads=1):
@@ -224,7 +215,7 @@ def taperf(shape, taper_width):
     return np.outer(*tapers1d)
 
 
-_DIRECT_CACHE: dict = {}
+_DIRECT_CACHE = HandleCache(8)
 
 
 def hess_direct_slice(x, xpad=None, xhat=None, xout=None, abspsf=None, taperxy=None, lastsize=None, nthreads=1, eta=1,
@@ -234,19 +225,15 @@ def hess_direct_slice(x, xpad=None, xhat=None, xout=None, abspsf=None, taperxy=N
     x = np.asarray(x)
     abspsf = np.asarray(abspsf)
     key = (abspsf.ctypes.data, abspsf.shape, float(eta), mode, x.shape, np.dtype(x.dtype).str, int(lastsize))
-    chk = content_hash(abspsf)
-    hit = _DIRECT_CACHE.get(key)
-    if hit is None or hit[1] != chk:
-        if hit is not None:
-            hit[0].close()
-        while len(_DIRECT_CACHE) >= 8:
-            _DIRECT_CACHE.pop(next(iter(_DIRECT_CACHE)))[0].close()
+
+    def make():
         k = abspsf.astype(np.float64) + float(eta)
         if mode != "forward":
             k = 1.0 / k
-        cv = PsfConvolver(x.shape[0], x.shape[1], abspsf.shape[0], int(lastsize), dtype=x.dtype).set_kernel(k)
-        hit = _DIRECT_CACHE[key] = (cv, chk, abspsf)
-    res = hit[0].apply(x, beam=None if taperxy is None else np.ascontiguousarray(taperxy, dtype=x.dtype))
+        return PsfConvolver(x.shape[0], x.shape[1], abspsf.shape[0], int(lastsize), dtype=x.dtype).set_kernel(k)
+
+    cv = _DIRECT_CACHE.get(key, content_hash(abspsf), make, keep=abspsf)
+    res = cv.apply(x, beam=None if taperxy is None else np.ascontiguousarray(taperxy, dtype=x.dtype))
     if xout is None:
         return res
     np.copyto(xout, res)
@@ -261,6 +248,77 @@ def hess_direct(x, xpad=None, xhat=None, xout=None, abspsf=None, taperxy=None, l
     for b in range(x.shape[0]):
         out[b] = hess_direct_slice(x[b], abspsf=abspsf[b], taperxy=taperxy, lastsize=lastsize, eta=eta, mode=mode)
     return out
+
+
+def _upload(a, device):
+    """A float64 copy of the host array `a` on cuda:`device` (None stays None)."""
+    import torch
+
+    return None if a is None else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).to(
+        torch.device("cuda", device))
+
+
+def _dev_cube(x, shape, device, name="input"):
+    """`x` as a contiguous float64 CUDA tensor of `shape` on cuda:`device` (None: any device); raises before anything
+    is launched, TypeError for a tensor that is not CUDA float64, ValueError for a wrong shape or device."""
+    import torch
+
+    if not getattr(x, "is_cuda", False) or x.dtype != torch.float64:
+        raise TypeError(f"{name} must be a float64 CUDA tensor, got {getattr(x, 'dtype', type(x))} on "
+                        f"{getattr(x, 'device', 'the host')}")
+    if tuple(x.shape) != tuple(shape):
+        raise ValueError(f"{name} shape {tuple(x.shape)} does not match {tuple(shape)}")
+    if device is not None and x.device.index != device:
+        raise ValueError(f"{name} is on {x.device}, the operator on cuda:{device}")
+    return x.contiguous()
+
+
+def _apply_groups(groups, x, out, eta, scale, stream):
+    """``out = scale sum_g beam_g conv_g(beam_g x) + eta x`` on device images, one ``pfbg_conv_apply_scaled`` per
+    ``(convolver, device beam or None)`` group on `stream`: the first group adds the ridge term, each later one the
+    running sum (eta = 1) from a second buffer, and the parity puts the last group's output in `out`.  One group with
+    scale 1 gives the bits of ``pfbg_conv_apply``."""
+    import torch
+
+    pong = torch.empty_like(out) if len(groups) > 1 else None
+    prev = x
+    for i, (cv, bm) in enumerate(groups):
+        dst = out if (len(groups) - 1 - i) % 2 == 0 else pong
+        _lib.check(cv._lib.pfbg_conv_apply_scaled(
+            cv._h, C.c_void_p(x.data_ptr()), None if bm is None else C.c_void_p(bm.data_ptr()),
+            C.c_void_p(prev.data_ptr()), eta if i == 0 else 1.0, scale, C.c_void_p(dst.data_ptr()), _lib.DEVICE_PTRS,
+            stream))
+        prev = dst
+
+
+CG_STOP = {1: "converged", 2: "maxit", 3: "stalled", 4: "initial residual zero", 5: "exact"}  # pfbsara.h PFBS_CG_*
+
+
+def _batched_cg(systems, rhs, sol, tol, maxit, minit, stream):
+    """One ``pfbs_tree_cg`` on `stream` (a ``torch.cuda.Stream``) over `systems`, a list of ``(groups, scale, eta)``
+    with the groups of :func:`_apply_groups`: solves system s for ``rhs[s]`` in place in `sol`, which holds the
+    starting point (both ``(nsys, nx, ny)`` contiguous float64 on the convolvers' device).  Returns a dict of
+    per-system ``iters``, ``eps`` and ``stop`` (``CG_STOP`` strings)."""
+    import torch
+
+    n, npix = len(systems), rhs[0].numel()
+    group_start, convs, beams = [0], [], []
+    for groups, _, _ in systems:
+        convs += [cv._h.value for cv, _ in groups]
+        beams += [None if bm is None else bm.data_ptr() for _, bm in groups]
+        group_start.append(len(convs))
+    lib, ng, device = _lib.load(), len(convs), rhs.device.index
+    gs_arr = (C.c_int32 * (n + 1))(*group_start)
+    nbytes = int(lib.pfbs_tree_cg_work_bytes(n, gs_arr, npix))
+    with torch.cuda.stream(stream):
+        work = torch.empty(nbytes, dtype=torch.uint8, device=torch.device("cuda", device))
+    iters, eps, stop = (C.c_int32 * n)(), (C.c_double * n)(), (C.c_int32 * n)()
+    _lib.check(lib.pfbs_tree_cg(device, n, gs_arr, (C.c_void_p * ng)(*convs), (C.c_void_p * ng)(*beams),
+                                (C.c_double * n)(*[float(sc) for _, sc, _ in systems]),
+                                (C.c_double * n)(*[float(e) for _, _, e in systems]), C.c_void_p(rhs.data_ptr()),
+                                C.c_void_p(sol.data_ptr()), npix, float(tol), int(maxit), int(minit),
+                                C.c_void_p(work.data_ptr()), nbytes, iters, eps, stop, stream.cuda_stream))
+    return dict(iters=np.array(iters[:], dtype=np.int64), eps=np.array(eps[:]), stop=[CG_STOP.get(v, str(v)) for v in stop])
 
 
 class HessianTree:
@@ -311,11 +369,8 @@ class HessianTree:
         self._dev_beams = None  # device copies of the group beams, uploaded on the first device call
 
     def _beams_dev(self):
-        import torch
-
         if self._dev_beams is None:
-            dev = torch.device("cuda", self.device)
-            self._dev_beams = [None if bm is None else torch.from_numpy(bm).to(dev) for _, bm, _ in self._groups]
+            self._dev_beams = [_upload(bm, self.device) for _, bm, _ in self._groups]
         return self._dev_beams
 
     def corr_groups(self, c):
@@ -325,32 +380,15 @@ class HessianTree:
     def _dot_dev(self, x, out=None):
         import torch
 
-        if x.dtype != torch.float64:
-            raise TypeError(f"device input must be float64, got {x.dtype}")
-        if x.device.index != self.device:
-            raise ValueError(f"input is on {x.device}, the operator on cuda:{self.device}")
         xt = x if x.dim() == 3 else x[None]
         ncorr, nx, ny = xt.shape
         assert ncorr == self.ncorr, f"expected {self.ncorr} correlations on axis 0, got {ncorr}"
         assert nx == self.nx and ny == self.ny
-        xt = xt.contiguous()
+        xt = _dev_cube(xt, (ncorr, nx, ny), self.device)
         out = torch.empty_like(xt) if out is None else out
         s = torch.cuda.current_stream(xt.device).cuda_stream
-        pong = None
         for c in range(ncorr):
-            gs = self.corr_groups(c)
-            if len(gs) > 1 and pong is None:
-                pong = torch.empty_like(xt[0])
-            prev = None
-            for i, (cv, bm) in enumerate(gs):
-                # the last group writes out[c]; the ridge term comes in with the first, the running sum with the others
-                dst = out[c] if (len(gs) - 1 - i) % 2 == 0 else pong
-                xin, eta = (xt[c], float(self.eta)) if i == 0 else (prev, 1.0)
-                _lib.check(cv._lib.pfbg_conv_apply_scaled(
-                    cv._h, C.c_void_p(xt[c].data_ptr()), None if bm is None else C.c_void_p(bm.data_ptr()),
-                    C.c_void_p(xin.data_ptr()), eta, 1.0 / float(self.wsum[c]), C.c_void_p(dst.data_ptr()),
-                    _lib.DEVICE_PTRS, s))
-                prev = dst
+            _apply_groups(self.corr_groups(c), xt[c], out[c], float(self.eta), 1.0 / float(self.wsum[c]), s)
         return out
 
     def dot(self, x):
@@ -377,9 +415,6 @@ class HessianTree:
         self._dev_beams = None
 
 
-CG_STOP = {1: "converged", 2: "maxit", 3: "stalled", 4: "initial residual zero", 5: "exact"}  # pfbsara.h PFBS_CG_*
-
-
 def tree_cg(trees, rhs_t, x0_t, tol, maxit, minit, stream=None):
     """Batched CG over the corr-0 systems of `trees` (HessianTrees on one device, sharing (nx, ny)): solves
     ``trees[s].dot(v)[0] = rhs_t[s]`` for every s with one ``pfbs_tree_cg``, the stopping rules of ``solvers.pcg``.
@@ -399,38 +434,12 @@ def tree_cg(trees, rhs_t, x0_t, tol, maxit, minit, stream=None):
         if t.device != t0.device or (t.nx, t.ny) != (t0.nx, t0.ny):
             raise ValueError("the trees of one batched solve must share the device and (nx, ny)")
     shape = (n, t0.nx, t0.ny)
-    for name, v in (("rhs", rhs_t), ("x0", x0_t)):
-        if v is None:
-            continue
-        if v.dtype != torch.float64:
-            raise TypeError(f"{name} must be float64, got {v.dtype}")
-        if tuple(v.shape) != shape:
-            raise ValueError(f"{name} shape {tuple(v.shape)} does not match {shape}")
-        if not v.is_cuda or v.device.index != t0.device:
-            raise ValueError(f"{name} is on {v.device}, the trees on cuda:{t0.device}")
-    dev = torch.device("cuda", t0.device)
-    stream = torch.cuda.current_stream(dev) if stream is None else stream
+    stream = torch.cuda.current_stream(torch.device("cuda", t0.device)) if stream is None else stream
     with torch.cuda.stream(stream):
-        rhs = rhs_t.contiguous()
-        sol = torch.zeros(shape, dtype=torch.float64, device=dev) if x0_t is None else x0_t.clone(
-            memory_format=torch.contiguous_format)
-        group_start, convs, beams = [0], [], []
-        for t in trees:
-            gs = t.corr_groups(0)
-            convs += [cv._h.value for cv, _ in gs]
-            beams += [None if bm is None else bm.data_ptr() for _, bm in gs]
-            group_start.append(len(convs))
-        lib, ng, npix = _lib.load(), len(convs), t0.nx * t0.ny
-        gs_arr = (C.c_int32 * (n + 1))(*group_start)
-        nbytes = int(lib.pfbs_tree_cg_work_bytes(n, gs_arr, npix))
-        work = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        iters, eps, stop = (C.c_int32 * n)(), (C.c_double * n)(), (C.c_int32 * n)()
-        _lib.check(lib.pfbs_tree_cg(t0.device, n, gs_arr, (C.c_void_p * ng)(*convs), (C.c_void_p * ng)(*beams),
-                                    (C.c_double * n)(*[1.0 / float(t.wsum[0]) for t in trees]),
-                                    (C.c_double * n)(*[float(t.eta) for t in trees]), C.c_void_p(rhs.data_ptr()),
-                                    C.c_void_p(sol.data_ptr()), npix, float(tol), int(maxit), int(minit),
-                                    C.c_void_p(work.data_ptr()), nbytes, iters, eps, stop, stream.cuda_stream))
-    info = dict(iters=np.array(iters[:], dtype=np.int64), eps=np.array(eps[:]), stop=[CG_STOP.get(v, str(v)) for v in stop])
+        rhs = _dev_cube(rhs_t, shape, t0.device, "rhs")
+        sol = torch.zeros_like(rhs) if x0_t is None else _dev_cube(x0_t, shape, t0.device, "x0").clone()
+    info = _batched_cg([(t.corr_groups(0), 1.0 / float(t.wsum[0]), t.eta) for t in trees], rhs, sol, tol, maxit, minit,
+                       stream)
     return sol, info
 
 
@@ -488,7 +497,8 @@ class HessPSF:
     numpy in, numpy out as in the reference.  A float64 CUDA tensor on the convolvers' device, ``(nband, nx, ny)`` or
     ``(nx, ny)`` when ``nband == 1``, stays on the device: ``dot`` and ``idot`` then return a new ``(nband, nx, ny)``
     tensor computed on torch's current stream, ``idot(mode="psf")`` solves every band in one batched CG
-    (``pfbs_psf_cg``) and leaves the per-band ``iters`` / ``eps`` / ``stop`` in :attr:`last_idot_info`."""
+    (``pfbs_tree_cg``, one group per band) and leaves the per-band ``iters`` / ``eps`` / ``stop`` in
+    :attr:`last_idot_info`.  The beams are uploaded on the first device call and again after :meth:`set_beam`."""
 
     def __init__(self, nx, ny, abspsf, beam=None, eta=1.0, nthreads=1, cgtol=1e-3, cgmaxit=300, cgverbose=2, cgrf=25,
                  taper_width=32, min_beam=5e-3):
@@ -510,13 +520,15 @@ class HessPSF:
         self.min_beam = min_beam
         self.conv = [PsfConvolver(nx, ny, self.nx_psf, self.ny_psf, dtype=np.float64).set_kernel(abspsf[b])
                      for b in range(self.nband)]
-        self._dev_consts = None  # device copies of the beams and the taper, uploaded on the first device call
+        self.device = self.conv[0].device
+        self._dev_beams = None  # device copies of the beams, uploaded on the first device call
+        self._dev_taper = None  # and of the taper, on the first device call of mode="direct"
         self.last_idot_info = None
 
     def set_beam(self, beam):
         assert beam.shape == (self.nband, self.nx, self.ny)
         self.beam = beam
-        self._dev_consts = None
+        self._dev_beams = None
 
     def _cube(self, x):
         if x.ndim == 3:
@@ -527,44 +539,30 @@ class HessPSF:
 
     def _dev_input(self, x):
         """The (nband, nx, ny) contiguous view of a device input; raises before anything is launched."""
-        import torch
+        return _dev_cube(x[None] if x.dim() == 2 and self.nband == 1 else x, (self.nband, self.nx, self.ny), self.device)
 
-        if x.dtype != torch.float64:
-            raise TypeError(f"device input must be float64, got {x.dtype}")
-        if x.dim() == 2 and self.nband == 1:
-            x = x[None]
-        if tuple(x.shape) != (self.nband, self.nx, self.ny):
-            raise ValueError(f"input shape {tuple(x.shape)} does not match ({self.nband}, {self.nx}, {self.ny})")
-        if x.device.index != self.conv[0].device:
-            raise ValueError(f"input is on {x.device}, the operator on cuda:{self.conv[0].device}")
-        return x.contiguous()
+    def _beams_dev(self):
+        if self._dev_beams is None:
+            self._dev_beams = [_upload(b, self.device) for b in self.beam]
+        return self._dev_beams
 
-    def _consts(self, device):
-        import torch
-
-        if self._dev_consts is None:
-            up = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float64)).to(device)  # noqa: E731
-            self._dev_consts = dict(beam=[None if b is None else up(b) for b in self.beam], taper=up(self.taperxy))
-        return self._dev_consts
-
-    def _direct_dev(self, xt, out, consts, stream):
+    def _direct_dev(self, xt, out, stream):
         """Device :meth:`_direct` of every band: the same shifted spectrum from each band's own convolver."""
+        if self._dev_taper is None:
+            self._dev_taper = _upload(self.taperxy, self.device)
         c0 = np.sqrt(self.nx * self.ny)
         for b in range(self.nband):
-            self.conv[b].apply_shifted_dev(xt[b].data_ptr(), out[b].data_ptr(), consts["taper"].data_ptr(),
+            self.conv[b].apply_shifted_dev(xt[b].data_ptr(), out[b].data_ptr(), self._dev_taper.data_ptr(),
                                            c=float(self.eta[b]) * c0, inverse=True, stream=stream)
 
-    def _dot_dev(self, x, out=None):
+    def _dot_dev(self, x):
         import torch
 
         xt = self._dev_input(x)
-        consts = self._consts(xt.device)
-        s = torch.cuda.current_stream(xt.device).cuda_stream
         out = torch.empty_like(xt)
-        for b in range(self.nband):
-            bm = consts["beam"][b]
-            self.conv[b].apply_dev(xt[b].data_ptr(), out[b].data_ptr(), None if bm is None else bm.data_ptr(),
-                                   float(self.eta[b]), s)
+        s = torch.cuda.current_stream(xt.device).cuda_stream
+        for b, bm in enumerate(self._beams_dev()):
+            _apply_groups([(self.conv[b], bm)], xt[b], out[b], float(self.eta[b]), 1.0, s)
         return out
 
     def _idot_dev(self, x, mode, x0, init_x0):
@@ -573,12 +571,11 @@ class HessPSF:
         xt = self._dev_input(x)
         if mode not in ("direct", "psf"):
             raise ValueError(f"Unknown mode {mode}")
-        consts = self._consts(xt.device)
-        s = torch.cuda.current_stream(xt.device).cuda_stream
+        st = torch.cuda.current_stream(xt.device)
         if mode == "direct":
             out = torch.empty_like(xt)
-            self._direct_dev(xt, out, consts, s)
-            for b, bm in enumerate(consts["beam"]):
+            self._direct_dev(xt, out, st.cuda_stream)
+            for b, bm in enumerate(self._beams_dev()):
                 if bm is not None:
                     mask = (out[b] > 0) & (bm > self.min_beam)
                     out[b] = torch.where(mask, out[b] / (bm * bm), out[b])
@@ -586,20 +583,11 @@ class HessPSF:
         # the starting point of the host path: the direct estimate, or zero (a passed x0 is not used, as there)
         if x0 is None and init_x0:
             sol = torch.empty_like(xt)
-            self._direct_dev(xt, sol, consts, s)
+            self._direct_dev(xt, sol, st.cuda_stream)
         else:
             sol = torch.zeros_like(xt)
-        lib, nb, npix = self.conv[0]._lib, self.nband, self.nx * self.ny
-        nbytes = int(lib.pfbs_psf_cg_work_bytes(nb, npix))
-        work = torch.empty(nbytes, dtype=torch.uint8, device=xt.device)
-        iters, eps, stop = (C.c_int32 * nb)(), (C.c_double * nb)(), (C.c_int32 * nb)()
-        _lib.check(lib.pfbs_psf_cg(self.conv[0].device, nb, (C.c_void_p * nb)(*[c._h.value for c in self.conv]),
-                                   (C.c_void_p * nb)(*[None if bm is None else bm.data_ptr() for bm in consts["beam"]]),
-                                   (C.c_double * nb)(*[float(e) for e in self.eta]), C.c_void_p(xt.data_ptr()),
-                                   C.c_void_p(sol.data_ptr()), npix, float(self.cgtol), int(self.cgmaxit), 3,
-                                   C.c_void_p(work.data_ptr()), nbytes, iters, eps, stop, s))
-        self.last_idot_info = dict(iters=np.array(iters[:], dtype=np.int64), eps=np.array(eps[:]),
-                                   stop=[CG_STOP.get(v, str(v)) for v in stop])
+        systems = [([(cv, bm)], 1.0, e) for cv, bm, e in zip(self.conv, self._beams_dev(), self.eta)]
+        self.last_idot_info = _batched_cg(systems, xt, sol, self.cgtol, self.cgmaxit, 3, st)
         return sol
 
     def dot(self, x):
@@ -660,7 +648,7 @@ class HessPSF:
     def close(self):
         for c in self.conv:
             c.close()
-        self._dev_consts = None
+        self._dev_beams = self._dev_taper = None
 
 
 class PsfGradient:
@@ -675,27 +663,15 @@ class PsfGradient:
         self.dirty = np.ascontiguousarray(dirty, dtype=np.float64)
         if self.dirty.shape != (hess.nband, hess.nx, hess.ny):
             raise ValueError("dirty must have shape (nband, nx, ny)")
-        self._dev = None
+        self._dev_dirty = None  # uploaded on the first device call
 
     def __call__(self, x):
         return self.hess.dot(x) - self.dirty
 
     def device_apply(self, x_t, out_t):
+        """``out_t = hess.dot(x_t) - dirty`` on the device: the Hessian's own device ``dot``."""
         import torch
 
-        tree = not isinstance(self.hess, HessPSF)
-        if self._dev is None:
-            dev = x_t.device
-            self._dev = dict(dirty=torch.from_numpy(self.dirty).to(dev),
-                             beam=[] if tree else [None if b is None else
-                                                   torch.from_numpy(np.ascontiguousarray(b, dtype=np.float64)).to(dev)
-                                                   for b in self.hess.beam])
-        if tree:
-            torch.sub(self.hess.dot(x_t), self._dev["dirty"], out=out_t)
-            return
-        s = torch.cuda.current_stream(x_t.device).cuda_stream
-        for b in range(self.hess.nband):
-            bm = self._dev["beam"][b]
-            self.hess.conv[b].apply_dev(x_t[b].data_ptr(), out_t[b].data_ptr(), None if bm is None else bm.data_ptr(),
-                                        float(self.hess.eta[b]), s)
-        out_t -= self._dev["dirty"]
+        if self._dev_dirty is None:
+            self._dev_dirty = _upload(self.dirty, x_t.device.index)
+        torch.sub(self.hess.dot(x_t), self._dev_dirty, out=out_t)

@@ -36,6 +36,34 @@ def content_hash(a) -> int:
     return int(h.value)
 
 
+class HandleCache:
+    """Device handles (anything with ``close()``) keyed by a key plus a content check, such as the buffer address and
+    shape of a host array and its :func:`content_hash`: a hit needs both to match, so an array rewritten in place
+    rebuilds its handle.  Each entry keeps the arrays its key was taken from alive, so that their addresses cannot be
+    reused by other arrays while it stands.  A stale entry, and the oldest entries beyond `cap`, are closed."""
+
+    def __init__(self, cap):
+        self.cap = cap
+        self._entries: dict = {}
+
+    def get(self, key, check, make, keep=()):
+        """The handle of `key` when its check equals `check`, else ``make()``, cached with `keep`."""
+        hit = self._entries.get(key)
+        if hit is not None:
+            if hit[1] == check:
+                return hit[0]
+            self._entries.pop(key)[0].close()
+        while len(self._entries) >= self.cap:
+            self._entries.pop(next(iter(self._entries)))[0].close()
+        h = make()
+        self._entries[key] = (h, check, keep)
+        return h
+
+    def clear(self):
+        while self._entries:
+            self._entries.popitem()[1][0].close()
+
+
 def current_device() -> int:
     import os
 

@@ -1,5 +1,5 @@
 """GPU: the device inverse of the PSF-convolution Hessian, ``HessPSF.idot`` on CUDA tensors (``pfbg_conv_apply_shifted``
-for the direct estimate, the batched conjugate gradients ``pfbs_psf_cg`` for ``mode="psf"``), against the numpy path of
+for the direct estimate, the batched conjugate gradients ``pfbs_tree_cg`` for ``mode="psf"``), against the numpy path of
 the same operator, which runs ``solvers.pcg`` band by band.
 
 * ``mode="direct"`` is bit-identical to the numpy path: the column pass forms ``Re khat + c`` and its reciprocal in
@@ -260,7 +260,27 @@ def test_set_beam(gpu):
     P._DIRECT_CACHE.clear()
 
 
-def test_errors_before_launch(gpu):
+def test_gradient_follows_set_beam(gpu):
+    """PsfGradient.device_apply uses the Hessian's current beams: after set_beam it still equals the numpy gradient."""
+    import torch
+
+    nband, nx, ny, nxp, nyp = 2, 64, 64, 128, 128
+    rng = np.random.default_rng(13)
+    abspsf = gaussian_abspsf(nband, nxp, nyp, 1.5)
+    H = P.HessPSF(nx, ny, abspsf, beam=rng.uniform(0.5, 1.0, (nband, nx, ny)), eta=0.1, cgverbose=0)
+    grad = P.PsfGradient(H, rng.standard_normal((nband, nx, ny)))
+    x = rng.standard_normal((nband, nx, ny))
+    xt = dev(x)
+    out = torch.empty_like(xt)
+    grad.device_apply(xt, out)
+    assert np.array_equal(host(out), grad(x))
+    H.set_beam(rng.uniform(0.0, 1.0, (nband, nx, ny)))
+    grad.device_apply(xt, out)
+    assert np.array_equal(host(out), grad(x))
+    H.close()
+
+
+def test_errors_before_launch_tree_cg(gpu):
     import torch
 
     lib = _lib.load()
@@ -287,25 +307,27 @@ def test_errors_before_launch(gpu):
     # the C entry points
     other = P.PsfConvolver(nx, ny + 1, nxp, nyp).set_kernel(np.ones((nxp, nyp // 2 + 1)))
     npix = nx * ny
-    need = int(lib.pfbs_psf_cg_work_bytes(nband, npix))
+    gs = (C.c_int32 * (nband + 1))(*range(nband + 1))  # one group per system
+    need = int(lib.pfbs_tree_cg_work_bytes(nband, gs, npix))
     work = torch.empty(need, dtype=torch.uint8, device="cuda")
     sol = torch.zeros_like(x)
     iters, eps, stop = (C.c_int32 * nband)(), (C.c_double * nband)(), (C.c_int32 * nband)()
     beams = (C.c_void_p * nband)(None, None)
+    scales = (C.c_double * nband)(1.0, 1.0)
     etas = (C.c_double * nband)(0.1, 0.1)
     s = torch.cuda.current_stream().cuda_stream
 
     def run(convs, rhs=x.data_ptr(), n=npix, wb=need):
-        return lib.pfbs_psf_cg(H.conv[0].device, nband, (C.c_void_p * nband)(*[c._h.value for c in convs]), beams, etas,
-                               None if rhs is None else C.c_void_p(rhs), C.c_void_p(sol.data_ptr()), n, 1e-3, 10, 3,
-                               C.c_void_p(work.data_ptr()), wb, iters, eps, stop, s)
+        return lib.pfbs_tree_cg(H.conv[0].device, nband, gs, (C.c_void_p * nband)(*[c._h.value for c in convs]), beams,
+                                scales, etas, None if rhs is None else C.c_void_p(rhs), C.c_void_p(sol.data_ptr()), n,
+                                1e-3, 10, 3, C.c_void_p(work.data_ptr()), wb, iters, eps, stop, s)
 
     n0 = lib.pfbg_launch_count()
     assert run([H.conv[0], other]) == _lib.PFBG_ERR_ARG  # mismatched image sizes
     assert run(H.conv, wb=need - 1) == _lib.PFBG_ERR_ARG
     assert run(H.conv, n=npix + 1) == _lib.PFBG_ERR_ARG
     assert run(H.conv, rhs=None) == _lib.PFBG_ERR_ARG
-    assert lib.pfbs_psf_cg_work_bytes(0, npix) == -1
+    assert lib.pfbs_tree_cg_work_bytes(0, gs, npix) == -1
     g = P.PsfConvolver(nx, ny, nxp, nyp).set_gauss((3.0, 2.0, 0.1))
     xh = np.zeros((nx, ny))
     rc = lib.pfbg_conv_apply_shifted(g._h, C.c_void_p(xh.ctypes.data), None, 1.0, 1, C.c_void_p(xh.ctypes.data),

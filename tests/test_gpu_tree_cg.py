@@ -356,7 +356,7 @@ def test_bands_over_devices(gpu, tmp_path):
     pool.close()
 
 
-def test_abi_errors(gpu, tmp_path):
+def test_tree_cg_abi_errors(gpu, tmp_path):
     import torch
 
     lib = _lib.load()
@@ -398,8 +398,8 @@ def test_abi_errors(gpu, tmp_path):
     rhs = torch.randn((nsys, nx, nx), dtype=torch.float64, device="cuda")
     sol = torch.zeros_like(rhs)
     need = int(lib.pfbs_tree_cg_work_bytes(nsys, (C.c_int32 * 3)(*good_gs), npix))
-    assert need == lib.pfbs_psf_cg_work_bytes(nsys, npix) + ((npix * 8 + 255) // 256) * 256  # one more image
-    assert lib.pfbs_tree_cg_work_bytes(nsys, (C.c_int32 * 3)(0, 1, 2), npix) == lib.pfbs_psf_cg_work_bytes(nsys, npix)
+    one_group = int(lib.pfbs_tree_cg_work_bytes(nsys, (C.c_int32 * 3)(0, 1, 2), npix))
+    assert need == one_group + ((npix * 8 + 255) // 256) * 256  # one more image
     work = torch.empty(need, dtype=torch.uint8, device="cuda")
     iters, eps, stop = (C.c_int32 * nsys)(), (C.c_double * nsys)(), (C.c_int32 * nsys)()
 

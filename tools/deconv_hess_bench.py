@@ -13,8 +13,7 @@ Measured per run, in one process on one GPU, with the card's name and power limi
     solves over (K2 - K1) * bands, so that the start-up cancels (host: on --host-bands bands);
   * a device solve at cgtol 1e-3 (cgmaxit 300): wall time, iterations and stop reason per band;
   * hess_dot of the cube, host and device;
-  * one primal-dual iteration (3 bases, 2 levels) with PsfGradient(HessTreeRay): the difference of maxit = 1 and 3 over 2;
-  * shared-beam run only: the same one-group systems solved by HessPSF.idot (pfbs_psf_cg) next to pfbs_tree_cg.
+  * one primal-dual iteration (3 bases, 2 levels) with PsfGradient(HessTreeRay): the difference of maxit = 1 and 3 over 2.
 With two or more visible GPUs, a second process times the distinct-beam solve with the bands spread over every GPU
 against all bands on one.  Times are host clocks around work that ends in a device synchronise, after a warm-up call.
 
@@ -134,19 +133,6 @@ def run_single(a, distinct):
     del pd, reg
     psi.close()
 
-    # the one-group systems through HessPSF.idot (pfbs_psf_cg): same kernels, same loop
-    if not distinct:
-        abspsf = np.stack([sum(p["psfhat"][0] for p in pb) / sum(p["wsum"][0] for p in pb) for pb in parts])
-        beam = np.stack([pb[0]["beam"][0] for pb in parts])
-        H = P.HessPSF(nx, nx, abspsf, beam=beam, eta=float(eta), cgtol=0.0, cgverbose=0)
-        t_psf = {}
-        for k in (a.k1, a.k2):
-            H.cgmaxit = k
-            H.idot(bt, mode="psf", init_x0=False)
-            t_psf[k], _ = timed(lambda: H.idot(bt, mode="psf", init_x0=False), sync)
-        res["psf_cg_ms_per_iter_per_band"] = round((t_psf[a.k2] - t_psf[a.k1]) * 1e3 / (dk * nb), 3)
-        res["tree_over_psf_cg"] = round(res["device_ms_per_iter_per_band"] / res["psf_cg_ms_per_iter_per_band"], 4)
-        H.close()
     pool.close()
     P.clear_convolver_cache()
     return res

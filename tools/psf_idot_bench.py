@@ -1,5 +1,5 @@
 """Cost of inverting the PSF-convolution Hessian, ``HessPSF.idot``, on the host loop (numpy in: ``solvers.pcg`` per band
-around host-pointer convolutions) and on the device (CUDA tensors in: one batched ``pfbs_psf_cg``).
+around host-pointer convolutions) and on the device (CUDA tensors in: one batched ``pfbs_tree_cg``, one group per band).
 
 Workload (defaults): the C3 shape, 8 bands of 4096^2 with a 5760^2 PSF grid, fp64; the PSF is a Gaussian main lobe
 whose width grows with band (its transfer function, as in tools/clean_bench.py), a beam in [0.5, 1], eta = 1e-3.  The
