@@ -70,7 +70,7 @@ typedef struct pfbg_plan_desc {
   int32_t device;        /* CUDA device ordinal */
   int32_t nx, ny;        /* image size (even) */
   int32_t nu, nv;        /* oversampled grid (multiples of 32) */
-  int32_t W;             /* kernel support, 4..16 */
+  int32_t W;             /* kernel support, 4..16; 4..8 in fp32 */
   int32_t nplanes;       /* w-planes (1 when do_wgridding == 0) */
   int32_t do_wgridding;
   int32_t divide_by_n;
@@ -107,6 +107,7 @@ typedef struct pfbg_plan_info {
 } pfbg_plan_info;
 
 const char* pfbg_last_error(void);
+/* 102: pfbg_plan_create and pfbg_split_helper_create reject PFBG_F32 with W > 8 (PFBG_ERR_ARG) */
 int pfbg_version(void);
 int pfbg_device_count(int32_t* count);
 

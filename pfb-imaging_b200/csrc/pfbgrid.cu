@@ -77,7 +77,7 @@ void pfbg_scratch_put(int device, void* p) {
   } while (0)
 
 extern "C" const char* pfbg_last_error(void) { return g_err.c_str(); }
-extern "C" int pfbg_version(void) { return 101; }
+extern "C" int pfbg_version(void) { return 102; }
 extern "C" int64_t pfbg_launch_count(void) { return g_launches.load(); }
 extern "C" int pfbg_device_count(int32_t* count) {
   int n = 0;
@@ -261,6 +261,7 @@ static int plan_create_impl(const pfbg_plan_desc* d, int stack_planes, pfbg_plan
   if (d->precision != PFBG_F32 && d->precision != PFBG_F64) return fail(PFBG_ERR_ARG, "bad precision");
   if (d->nx <= 0 || d->ny <= 0 || (d->nx & 1) || (d->ny & 1)) return fail(PFBG_ERR_ARG, "nx, ny must be positive and even");
   if (d->W < 4 || d->W > PFBG_MAXW) return fail(PFBG_ERR_ARG, "kernel support W=%d outside [4,%d]", d->W, PFBG_MAXW);
+  if (d->precision == PFBG_F32 && d->W > 8) return fail(PFBG_ERR_ARG, "kernel support W=%d: fp32 plans stop at W=8", d->W);
   if (d->nu % (2 * PFBG_TILE) || d->nv % (2 * PFBG_TILE)) return fail(PFBG_ERR_ARG, "nu, nv must be multiples of %d", 2 * PFBG_TILE);
   if (d->nu < d->nx + d->W || d->nv < d->ny + d->W) return fail(PFBG_ERR_ARG, "grid smaller than image + support");
   if (d->nplanes < 1 || (d->do_wgridding && d->nplanes < d->W)) return fail(PFBG_ERR_ARG, "nplanes=%d too small for W=%d", d->nplanes, d->W);
@@ -832,27 +833,26 @@ static int run_blocks(const pfbg_plan* pl, int64_t nact, int warps_per_cta, int 
   return (int)(want < cap ? (want > 0 ? want : 1) : cap);
 }
 
-static int wide_blocks(const pfbg_plan* pl, int64_t nact, int team) {
+static int wide_blocks(const pfbg_plan* pl, int64_t nact) {
   int sm = 148;
   cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, pl->device);
   int64_t nslice = (nact + WIDE_SLICE - 1) / WIDE_SLICE;
-  int64_t want = (nslice * team + WIDE_WARPS - 1) / WIDE_WARPS;
+  int64_t want = (nslice * WIDE_R + WIDE_WARPS - 1) / WIDE_WARPS;
   int64_t cap = (int64_t)sm * 2;
   return (int)(want < cap ? (want > 0 ? want : 1) : cap);
 }
 
-// kernel family of the spreading / gathering passes of a binding: direct (no per-sample records), the one-warp run
-// kernels (W <= 8), the scalar team kernels wide<3, 6, 4> (W <= 12) and wide<2, 8, 8>, or in fp64 at 9 <= W <= 12 the
-// DMMA run kernels (runs_mma.cuh) unless PFBG_WIDE_MMA=0 asks for the scalar team kernels
-enum RunArm { ARM_DIRECT, ARM_RUNS, ARM_WIDE6, ARM_WIDE8, ARM_MMA };
+// kernel family of the spreading / gathering passes of a binding:
+//   ARM_DIRECT  no per-sample records (k_*_direct)
+//   ARM_RUNS    W <= 8, fp32 and fp64: the one-warp run kernels (k_*_runs)
+//   ARM_MMA     fp64, 9 <= W <= 12: the DMMA run kernels (runs_mma.cuh)
+//   ARM_WIDE    fp64, 13 <= W <= 16: the scalar team kernels (k_*_runs_wide)
+// plan_create_impl rejects fp32 with W > 8, so the last two are fp64 only
+enum RunArm { ARM_DIRECT, ARM_RUNS, ARM_MMA, ARM_WIDE };
 static RunArm run_arm(const pfbg_plan* pl) {
   if (!pl->use_runs) return ARM_DIRECT;
   if (pl->gp.W <= 8) return ARM_RUNS;
-  if (pl->precision == PFBG_F64 && pl->gp.W <= 12) {
-    const char* e = getenv("PFBG_WIDE_MMA");
-    if (!(e && e[0] == '0')) return ARM_MMA;
-  }
-  return pl->gp.W <= 12 ? ARM_WIDE6 : ARM_WIDE8;
+  return pl->gp.W <= 12 ? ARM_MMA : ARM_WIDE;
 }
 
 static int mma_blocks(const pfbg_plan* pl, int64_t nact) {
@@ -1093,15 +1093,11 @@ static int run_spread(pfbg_plan* pl, cudaStream_t s, const void* vis, int64_t rs
             pl->gp, recs, pl->nactive, (const double2*)vis, rs, cs, (const double*)wgt, (double2*)pl->grid.p,
             vis_sorted, apply_phase, queue);
       break;
-    case ARM_WIDE6:
-      k_grid_runs_wide<T, 3, 6, 4><<<wide_blocks(pl, pl->nactive, 4), WIDE_WARPS * 32, 0, s>>>(
-          pl->gp, recs, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p, vis_sorted, apply_phase,
-          queue);
-      break;
-    case ARM_WIDE8:
-      k_grid_runs_wide<T, 2, 8, 8><<<wide_blocks(pl, pl->nactive, 8), WIDE_WARPS * 32, 0, s>>>(
-          pl->gp, recs, pl->nactive, (const C*)vis, rs, cs, (const T*)wgt, (C*)pl->grid.p, vis_sorted, apply_phase,
-          queue);
+    case ARM_WIDE:
+      if constexpr (sizeof(T) == 8)
+        k_grid_runs_wide<<<wide_blocks(pl, pl->nactive), WIDE_WARPS * 32, 0, s>>>(
+            pl->gp, recs, pl->nactive, (const double2*)vis, rs, cs, (const double*)wgt, (double2*)pl->grid.p,
+            vis_sorted, apply_phase, queue);
       break;
     case ARM_RUNS: {
       const int ctas = 3;  // resident CTAs per SM
@@ -1129,7 +1125,7 @@ static int run_gather(pfbg_plan* pl, cudaStream_t s, const void* wgt, void* vis_
   if (pl->nactive == 0) return PFBG_OK;
   const RunArm arm = run_arm(pl);
   const VisRec<T>* recs = (const VisRec<T>*)pl->recs.p;
-  const bool team = arm == ARM_WIDE6 || arm == ARM_WIDE8 || arm == ARM_MMA;
+  const bool team = arm == ARM_MMA || arm == ARM_WIDE;
   if (team) {
     // the R warps of a team add their row-partials atomically: start from zero
     if (out_sorted) CK(cudaMemsetAsync(out_sorted, 0, (size_t)pl->nactive * sizeof(C), s));
@@ -1142,9 +1138,6 @@ static int run_gather(pfbg_plan* pl, cudaStream_t s, const void* wgt, void* vis_
   // slice counters of this launch: one per row group (<= 8) for the team kernels
   unsigned long long* queue = (unsigned long long*)((char*)pl->flag.p + (team ? 32 : 24));
   if (arm != ARM_DIRECT) CK(cudaMemsetAsync(queue, 0, team ? 64 : 8, s));
-  // per-sample lane partials of the team kernels (see k_degrid_runs_wide); the attribute is per device and cheap: set
-  // on every launch rather than cached per process
-  const size_t psm = (size_t)WIDE_WARPS * 16 * 32 * sizeof(C);
   switch (arm) {
     case ARM_MMA:
       if constexpr (sizeof(T) == 8)
@@ -1152,17 +1145,16 @@ static int run_gather(pfbg_plan* pl, cudaStream_t s, const void* wgt, void* vis_
             pl->gp, recs, pl->nactive, (const double2*)pl->grid.p, (const double*)wgt, (double2*)vis_out,
             (double2*)out_sorted, apply_phase, queue);
       break;
-    case ARM_WIDE6:
-      CK(cudaFuncSetAttribute(k_degrid_runs_wide<T, 3, 6, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
-      k_degrid_runs_wide<T, 3, 6, 4><<<wide_blocks(pl, pl->nactive, 4), WIDE_WARPS * 32, psm, s>>>(
-          pl->gp, recs, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out, (C*)out_sorted, apply_phase,
-          queue);
-      break;
-    case ARM_WIDE8:
-      CK(cudaFuncSetAttribute(k_degrid_runs_wide<T, 2, 8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
-      k_degrid_runs_wide<T, 2, 8, 8><<<wide_blocks(pl, pl->nactive, 8), WIDE_WARPS * 32, psm, s>>>(
-          pl->gp, recs, pl->nactive, (const C*)pl->grid.p, (const T*)wgt, (C*)vis_out, (C*)out_sorted, apply_phase,
-          queue);
+    case ARM_WIDE:
+      if constexpr (sizeof(T) == 8) {
+        // per-sample lane partials (see k_degrid_runs_wide); the attribute is per device and cheap: set on every
+        // launch rather than cached per process
+        const size_t psm = (size_t)WIDE_WARPS * WIDE_NB * 32 * sizeof(double2);
+        CK(cudaFuncSetAttribute(k_degrid_runs_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
+        k_degrid_runs_wide<<<wide_blocks(pl, pl->nactive), WIDE_WARPS * 32, psm, s>>>(
+            pl->gp, recs, pl->nactive, (const double2*)pl->grid.p, (const double*)wgt, (double2*)vis_out,
+            (double2*)out_sorted, apply_phase, queue);
+      }
       break;
     case ARM_RUNS: {
       const int ctas = 5;  // resident CTAs per SM

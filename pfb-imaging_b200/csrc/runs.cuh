@@ -574,18 +574,22 @@ k_degrid_runs(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
 }
 
 // ===========================================================================
-// Wide-support run kernels (9 <= W <= 16; the fp64 production settings, epsilon <= 1e-7).
+// Wide-support run kernels (fp64, 13 <= W <= 16; fp64 at 9 <= W <= 12 runs on the DMMA kernels of runs_mma.cuh,
+// and fp32 stops at W = 8).
 //
-// The footprint no longer fits one warp's registers, so a TEAM of R warps shares every run: warp r of
-// the team owns the u-rows  i = r*RPW .. r*RPW+RPW-1.  Lane = (j, q2) with j = v-offset (0..15) and
-// q2 = plane slot (0..1); a lane holds RPW rows x NQ planes (q = q2 + 2*qq).
-//   9..12 : RPW = 3, NQ = 6, R = 4        13..16 : RPW = 2, NQ = 8, R = 8
-// The team works on one batch of samples at a time: warp 0 stages weight * phase * vis, ALL R warps
+// The footprint no longer fits one warp's registers, so a TEAM of WIDE_R warps shares every run: warp r of
+// the team owns the u-rows  i = r*WIDE_RPW .. r*WIDE_RPW+WIDE_RPW-1.  Lane = (j, q2) with j = v-offset (0..15) and
+// q2 = plane slot (0..1); a lane holds WIDE_RPW rows x WIDE_NQ planes (q = q2 + 2*qq), so a team covers the
+// 16 x 16 x 16 footprint.
+// The team works on one batch of samples at a time: warp 0 stages weight * phase * vis, ALL WIDE_R warps
 // evaluate the 3 W taps of the batch together (each tap once per team: in fp64 the tap evaluation costs
-// more than the FMAs, and evaluating it per warp made it 4-8 times redundant), then every warp runs the
+// more than the FMAs, and evaluating it per warp made it 8 times redundant), then every warp runs the
 // FMA stage for its rows.  Named barriers (one id per team) separate the stages.
 // ===========================================================================
 #define WIDE_WARPS 8
+#define WIDE_R 8     // warps per team
+#define WIDE_RPW 2   // u-rows per warp
+#define WIDE_NQ 8    // planes per lane
 #define WIDE_SLICE 256  /* samples per (statically strided) slice of a team */
 #define WIDE_NB 16   // samples staged per batch
 #define WIDE_NT 48   // tap slots per sample: 16 u, 16 v, 16 w (the first W of each are live)
@@ -595,15 +599,14 @@ __device__ __forceinline__ void team_sync(int team, int nthreads) {
 }
 
 // all threads of the team: tap t = axis * W + k of sample v
-template <typename T>
-__device__ __forceinline__ void wide_taps(const GParams& p, const T (*x0s)[4], T (*taps)[WIDE_NT], int nb, int ttid,
-                                          int tthreads, T bscale, T xs) {
+__device__ __forceinline__ void wide_taps(const GParams& p, const double (*x0s)[4], double (*taps)[WIDE_NT], int nb,
+                                          int ttid, int tthreads, double bscale, double xs) {
   const int W = p.W, nt = 3 * W;
   for (int idx = ttid; idx < nt * nb; idx += tthreads) {
     const int v = idx / nt, t = idx - v * nt;
     const int axis = t / W, k = t - axis * W;
-    T val = tap_eval(p, x0s[v][axis], k, bscale, xs);
-    if (axis == 2 && !p.do_wgridding) val = (k == 0) ? (T)1 : (T)0;
+    double val = tap_eval(p, x0s[v][axis], k, bscale, xs);
+    if (axis == 2 && !p.do_wgridding) val = (k == 0) ? 1.0 : 0.0;
     taps[v][axis * 16 + k] = val;
   }
   if (W < 16) {  // slots beyond the support are read (times zero grid values / never flushed): keep them zero
@@ -611,34 +614,32 @@ __device__ __forceinline__ void wide_taps(const GParams& p, const T (*x0s)[4], T
     for (int idx = ttid; idx < nz * nb; idx += tthreads) {
       const int v = idx / nz, t = idx - v * nz;
       const int axis = t / (16 - W), k = W + (t - axis * (16 - W));
-      taps[v][axis * 16 + k] = (T)0;
+      taps[v][axis * 16 + k] = 0.0;
     }
   }
 }
 
-template <typename T, int RPW, int NQ>
-__device__ __forceinline__ void wide_flush(const GParams& p, typename cplx_of<T>::type* __restrict__ grid,
-                                           T (&accr)[RPW][NQ], T (&acci)[RPW][NQ], uint64_t origin, int j, int q2,
-                                           int row0) {
+__device__ __forceinline__ void wide_flush(const GParams& p, double2* __restrict__ grid,
+                                           double (&accr)[WIDE_RPW][WIDE_NQ], double (&acci)[WIDE_RPW][WIDE_NQ],
+                                           uint64_t origin, int j, int q2, int row0) {
   const int W = p.W, npl = p.do_wgridding ? W : 1;
   int iv = (int)(origin & 0xffffu) + j;
   int iu0 = (int)((origin >> 16) & 0xffffu);
   int ip = origin_plane(origin);
   if (iv >= p.nv) iv -= p.nv;
-  const int plane_sz = p.nu * p.nv;
   const bool jok = j < W;
 #pragma unroll
-  for (int qq = 0; qq < NQ; ++qq) {
+  for (int qq = 0; qq < WIDE_NQ; ++qq) {
     const int q = q2 + 2 * qq;
     const bool ok = jok && q < npl;
 #pragma unroll
-    for (int ii = 0; ii < RPW; ++ii) {
+    for (int ii = 0; ii < WIDE_RPW; ++ii) {
       const int i = row0 + ii;
       if (ok && i < W) {
         int iu = iu0 + i;
         if (iu >= p.nu) iu -= p.nu;
         bool cj;
-        typename cplx_of<T>::type* g = grid + plane_cell(p, ip + q, iu, iv, cj);
+        double2* g = grid + plane_cell(p, ip + q, iu, iv, cj);
         atomic_add_c(g, accr[ii][qq], cj ? -acci[ii][qq] : acci[ii][qq]);
       }
       accr[ii][qq] = 0;
@@ -647,37 +648,34 @@ __device__ __forceinline__ void wide_flush(const GParams& p, typename cplx_of<T>
   }
 }
 
-template <typename T, int RPW, int NQ, int R>
 __global__ void __launch_bounds__(WIDE_WARPS * 32)
-k_grid_runs_wide(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
-                 const typename cplx_of<T>::type* __restrict__ vis, int64_t vis_rs, int64_t vis_cs,
-                 const T* __restrict__ wgt, typename cplx_of<T>::type* __restrict__ grid, int vis_sorted,
-                 int apply_phase, unsigned long long* __restrict__ queue) {
-  using C = typename cplx_of<T>::type;
-  constexpr int NB = WIDE_NB, NTEAM = WIDE_WARPS / R;
-  __shared__ T taps[NTEAM][NB][WIDE_NT];
-  __shared__ __align__(16) T x0s[NTEAM][NB][4];
-  __shared__ C amp[NTEAM][NB];
+k_grid_runs_wide(GParams p, const VisRec<double>* __restrict__ recs, int64_t nact, const double2* __restrict__ vis,
+                 int64_t vis_rs, int64_t vis_cs, const double* __restrict__ wgt, double2* __restrict__ grid,
+                 int vis_sorted, int apply_phase, unsigned long long* __restrict__ queue) {
+  constexpr int NB = WIDE_NB, NTEAM = WIDE_WARPS / WIDE_R;
+  __shared__ double taps[NTEAM][NB][WIDE_NT];
+  __shared__ __align__(16) double x0s[NTEAM][NB][4];
+  __shared__ double2 amp[NTEAM][NB];
   __shared__ unsigned long long team_slice[NTEAM];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int team = warp / R, r = warp - team * R;
+  const int team = warp / WIDE_R, r = warp - team * WIDE_R;
   const int ttid = r * 32 + lane;
   const int j = lane & 15, q2 = lane >> 4;
-  const int row0 = r * RPW;
-  const T bscale = es_scale((T)p.beta), xs = (T)(2.0 / p.W);
-  T accr[RPW][NQ], acci[RPW][NQ];
+  const int row0 = r * WIDE_RPW;
+  const double bscale = es_scale(p.beta), xs = 2.0 / p.W;
+  double accr[WIDE_RPW][WIDE_NQ], acci[WIDE_RPW][WIDE_NQ];
 #pragma unroll
-  for (int ii = 0; ii < RPW; ++ii)
+  for (int ii = 0; ii < WIDE_RPW; ++ii)
 #pragma unroll
-    for (int qq = 0; qq < NQ; ++qq) { accr[ii][qq] = 0; acci[ii][qq] = 0; }
+    for (int qq = 0; qq < WIDE_NQ; ++qq) { accr[ii][qq] = 0; acci[ii][qq] = 0; }
   uint64_t cur = ~0ull;
   const int64_t nslice = (nact + WIDE_SLICE - 1) / WIDE_SLICE;
   for (;;) {
     // the team's next slice, drawn by its first thread from the launch's counter (see k_grid_runs)
     if (ttid == 0) team_slice[team] = atomicAdd(queue, 1ull);
-    team_sync(team, 32 * R);
+    team_sync(team, 32 * WIDE_R);
     const int64_t sl = (int64_t)team_slice[team];
-    team_sync(team, 32 * R);  // everybody has read it before the next draw overwrites it
+    team_sync(team, 32 * WIDE_R);  // everybody has read it before the next draw overwrites it
     if (sl >= nslice) break;
     const int64_t kend = min(nact, (sl + 1) * WIDE_SLICE);
     for (int64_t k0 = sl * WIDE_SLICE; k0 < kend; k0 += NB) {
@@ -685,20 +683,20 @@ k_grid_runs_wide(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
       uint64_t org = ~0ull;
       if (lane < nb) {  // every warp reads the records (it needs the run origins); warp 0 stages the rest
         const int64_t k = k0 + lane;
-        const VisRec<T> rec = recs[k];
+        const VisRec<double> rec = recs[k];
         org = pack_origin(rec.iu, rec.iv, rec.ip);
         if (r == 0) {
-          C a;
+          double2 a;
           if (vis_sorted) a = vis[k];
           else {
             int64_t row = rec.idx / p.nchan;
             int chan = (int)(rec.idx - row * p.nchan);
             a = vis[row * vis_rs + chan * vis_cs];
           }
-          T w = wgt ? wgt[rec.idx] : (T)1;
-          T pc = apply_phase ? rec.pc : (T)1, ps = apply_phase ? rec.ps : (T)0;
+          double w = wgt ? wgt[rec.idx] : 1.0;
+          double pc = apply_phase ? rec.pc : 1.0, ps = apply_phase ? rec.ps : 0.0;
           if (apply_phase && (rec.ip & REC_CONJ_BIT)) a.y = -a.y;  // folded sample (the Hessian path stays folded)
-          C sa;
+          double2 sa;
           sa.x = (a.x * pc - a.y * ps) * w;
           sa.y = (a.x * ps + a.y * pc) * w;
           amp[team][lane] = sa;
@@ -706,97 +704,86 @@ k_grid_runs_wide(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
         }
       }
       const uint32_t starts = run_starts(org, cur, lane, nb);
-      team_sync(team, 32 * R);
-      wide_taps<T>(p, x0s[team], taps[team], nb, ttid, 32 * R, bscale, xs);
-      team_sync(team, 32 * R);
+      team_sync(team, 32 * WIDE_R);
+      wide_taps(p, x0s[team], taps[team], nb, ttid, 32 * WIDE_R, bscale, xs);
+      team_sync(team, 32 * WIDE_R);
       for (int v = 0; v < nb; ++v) {
         if ((starts >> v) & 1u) {
-          if (cur != ~0ull) wide_flush<T, RPW, NQ>(p, grid, accr, acci, cur, j, q2, row0);
+          if (cur != ~0ull) wide_flush(p, grid, accr, acci, cur, j, q2, row0);
           cur = shfl_u64(org, v);
         }
-        const T* tp = taps[team][v];
-        const T tv = tp[16 + j];
-        const C a = amp[team][v];
-        const T ar = a.x * tv, ai = a.y * tv;
-        T ur[RPW], ui[RPW];
+        const double* tp = taps[team][v];
+        const double tv = tp[16 + j];
+        const double2 a = amp[team][v];
+        const double ar = a.x * tv, ai = a.y * tv;
+        double ur[WIDE_RPW], ui[WIDE_RPW];
 #pragma unroll
-        for (int ii = 0; ii < RPW; ++ii) { ur[ii] = ar * tp[row0 + ii]; ui[ii] = ai * tp[row0 + ii]; }
+        for (int ii = 0; ii < WIDE_RPW; ++ii) { ur[ii] = ar * tp[row0 + ii]; ui[ii] = ai * tp[row0 + ii]; }
 #pragma unroll
-        for (int qq = 0; qq < NQ; ++qq) {
-          const T wq = tp[32 + q2 + 2 * qq];
+        for (int qq = 0; qq < WIDE_NQ; ++qq) {
+          const double wq = tp[32 + q2 + 2 * qq];
 #pragma unroll
-          for (int ii = 0; ii < RPW; ++ii) {
+          for (int ii = 0; ii < WIDE_RPW; ++ii) {
             accr[ii][qq] += ur[ii] * wq;
             acci[ii][qq] += ui[ii] * wq;
           }
         }
       }
-      team_sync(team, 32 * R);  // the next batch overwrites the staging buffers
+      team_sync(team, 32 * WIDE_R);  // the next batch overwrites the staging buffers
     }
   }
-  if (cur != ~0ull) wide_flush<T, RPW, NQ>(p, grid, accr, acci, cur, j, q2, row0);
+  if (cur != ~0ull) wide_flush(p, grid, accr, acci, cur, j, q2, row0);
 }
 
 // Degridding keeps INDEPENDENT warps (measured on B200, C2 band in fp64 at epsilon 1e-7: the cooperative
 // variant with team barriers was 17 % slower here, because every new run starts with a footprint fetch whose
 // latency the barriers then serialise across the team; for gridding, whose flushes are fire-and-forget, the
 // cooperative form above is 19 % faster).  Each warp stages the records and evaluates the taps it needs itself.
-template <typename T, int RPW, int NQ>
-struct WideCfg {
-  static constexpr int NB = 16;              // samples staged per batch
-  static constexpr int NT = RPW + 32;        // taps per sample and warp: RPW u-taps, 16 v-taps, 16 w-taps
-};
-
-template <typename T, int RPW, int NQ>
-__device__ __forceinline__ void wide_taps_warp(const GParams& p, const T (*x0s)[4], T (*taps)[RPW + 32], int nb, int lane,
-                                          int row0, T bscale, T xs) {
-  constexpr int NT = RPW + 32;
+__device__ __forceinline__ void wide_taps_warp(const GParams& p, const double (*x0s)[4], double (*taps)[WIDE_RPW + 32],
+                                               int nb, int lane, int row0, double bscale, double xs) {
+  constexpr int NT = WIDE_RPW + 32;
   for (int idx = lane; idx < NT * nb; idx += 32) {
     const int v = idx / NT, t = idx - v * NT;
     int axis, k;
-    if (t < RPW) { axis = 0; k = row0 + t; }
-    else if (t < RPW + 16) { axis = 1; k = t - RPW; }
-    else { axis = 2; k = t - RPW - 16; }
-    T val = es_fast((x0s[v][axis] + (T)k) * xs, bscale);
-    if (axis == 2 && !p.do_wgridding) val = (k == 0) ? (T)1 : (T)0;
+    if (t < WIDE_RPW) { axis = 0; k = row0 + t; }
+    else if (t < WIDE_RPW + 16) { axis = 1; k = t - WIDE_RPW; }
+    else { axis = 2; k = t - WIDE_RPW - 16; }
+    double val = es_fast((x0s[v][axis] + (double)k) * xs, bscale);
+    if (axis == 2 && !p.do_wgridding) val = (k == 0) ? 1.0 : 0.0;
     taps[v][t] = val;
   }
 }
 
-// degridding: each warp of the team produces the partial sum over its rows; partials of the R
+// degridding: each warp of the team produces the partial sum over its rows; partials of the WIDE_R
 // warps are combined with one atomicAdd per sample and warp into a zero-initialised output.
-template <typename T, int RPW, int NQ, int R>
 __global__ void __launch_bounds__(WIDE_WARPS * 32)
-k_degrid_runs_wide(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
-                   const typename cplx_of<T>::type* __restrict__ grid, const T* __restrict__ wgt,
-                   typename cplx_of<T>::type* __restrict__ vis_out,
-                   typename cplx_of<T>::type* __restrict__ out_sorted, int apply_phase,
-                   unsigned long long* __restrict__ queue) {
-  using C = typename cplx_of<T>::type;
-  constexpr int NB = WideCfg<T, RPW, NQ>::NB, NT = WideCfg<T, RPW, NQ>::NT;
-  __shared__ T taps[WIDE_WARPS][NB][NT];
-  __shared__ __align__(16) T x0s[WIDE_WARPS][NB][4];
+k_degrid_runs_wide(GParams p, const VisRec<double>* __restrict__ recs, int64_t nact, const double2* __restrict__ grid,
+                   const double* __restrict__ wgt, double2* __restrict__ vis_out, double2* __restrict__ out_sorted,
+                   int apply_phase, unsigned long long* __restrict__ queue) {
+  constexpr int NB = WIDE_NB, NT = WIDE_RPW + 32;  // taps per sample and warp: WIDE_RPW u, 16 v, 16 w
+  __shared__ double taps[WIDE_WARPS][NB][NT];
+  __shared__ __align__(16) double x0s[WIDE_WARPS][NB][4];
   __shared__ uint64_t orgs[WIDE_WARPS][NB];
   // per-sample partial sums of the 32 lanes: summed lane <-> sample after the batch (skewed, conflict-free) instead
   // of a 5-level shuffle reduction per sample, whose dependent latency dominated this kernel (ncu: "wait" stalls)
   extern __shared__ __align__(16) unsigned char wide_part_raw[];  // WIDE_WARPS * NB * 32 complex (dynamic: > 48 KB in fp64)
-  C (*part)[NB][32] = reinterpret_cast<C (*)[NB][32]>(wide_part_raw);
+  double2 (*part)[NB][32] = reinterpret_cast<double2 (*)[NB][32]>(wide_part_raw);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int j = lane & 15, q2 = lane >> 4;
   const int64_t gwarp = (int64_t)blockIdx.x * WIDE_WARPS + warp;
-  const int row0 = (int)(gwarp % R) * RPW;
+  const int row0 = (int)(gwarp % WIDE_R) * WIDE_RPW;
   const int W = p.W, npl = p.do_wgridding ? W : 1;
-  const T bscale = es_scale((T)p.beta), xs = (T)(2.0 / p.W);
+  const double bscale = es_scale(p.beta), xs = 2.0 / p.W;
   const int plane_sz = p.nu * p.nv;
-  T gr[RPW][NQ], gi[RPW][NQ];
+  double gr[WIDE_RPW][WIDE_NQ], gi[WIDE_RPW][WIDE_NQ];
 #pragma unroll
-  for (int ii = 0; ii < RPW; ++ii)
+  for (int ii = 0; ii < WIDE_RPW; ++ii)
 #pragma unroll
-    for (int qq = 0; qq < NQ; ++qq) { gr[ii][qq] = 0; gi[ii][qq] = 0; }
+    for (int qq = 0; qq < WIDE_NQ; ++qq) { gr[ii][qq] = 0; gi[ii][qq] = 0; }
   uint64_t cur = ~0ull;
   const int64_t nslice = (nact + WIDE_SLICE - 1) / WIDE_SLICE;
   // the warps are independent: every (slice, row group) pair is drawn exactly once from the row group's own counter
-  unsigned long long* myq = queue + (gwarp % R);
+  unsigned long long* myq = queue + (gwarp % WIDE_R);
   for (;;) {
     unsigned long long t = 0;
     if (lane == 0) t = atomicAdd(myq, 1ull);
@@ -805,14 +792,14 @@ k_degrid_runs_wide(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
     const int64_t kend = min(nact, (sl + 1) * WIDE_SLICE);
     for (int64_t k0 = sl * WIDE_SLICE; k0 < kend; k0 += NB) {
       const int nb = (int)min((int64_t)NB, kend - k0);
-      VisRec<T> r;
+      VisRec<double> r;
       if (lane < nb) {
         r = recs[k0 + lane];
         x0s[warp][lane][0] = r.x0[0]; x0s[warp][lane][1] = r.x0[1]; x0s[warp][lane][2] = r.x0[2];
         orgs[warp][lane] = pack_origin(r.iu, r.iv, r.ip);
       }
       __syncwarp();
-      wide_taps_warp<T, RPW, NQ>(p, x0s[warp], taps[warp], nb, lane, row0, bscale, xs);
+      wide_taps_warp(p, x0s[warp], taps[warp], nb, lane, row0, bscale, xs);
       __syncwarp();
       for (int v = 0; v < nb; ++v) {
         const uint64_t org = orgs[warp][v];
@@ -826,15 +813,15 @@ k_degrid_runs_wide(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
           if (iu0 >= 1 && iu0 + W <= p.nu) {  // rows do not wrap: constant stride (see wide_flush)
             const int mv = iv ? p.nv - iv : 0;
 #pragma unroll
-            for (int qq = 0; qq < NQ; ++qq) {
+            for (int qq = 0; qq < WIDE_NQ; ++qq) {
               const int q = q2 + 2 * qq, pl = ip + q;
               const bool ok = jok && q < npl, mir = pl < 0;
-              const C* g = grid + (mir ? (int64_t)(-pl - 1) * plane_sz + (int64_t)(p.nu - iu0 - row0) * p.nv + mv
-                                       : (int64_t)pl * plane_sz + (int64_t)(iu0 + row0) * p.nv + iv);
+              const double2* g = grid + (mir ? (int64_t)(-pl - 1) * plane_sz + (int64_t)(p.nu - iu0 - row0) * p.nv + mv
+                                             : (int64_t)pl * plane_sz + (int64_t)(iu0 + row0) * p.nv + iv);
               const int step = mir ? -p.nv : p.nv;
 #pragma unroll
-              for (int ii = 0; ii < RPW; ++ii) {
-                C val; val.x = 0; val.y = 0;
+              for (int ii = 0; ii < WIDE_RPW; ++ii) {
+                double2 val; val.x = 0; val.y = 0;
                 if (ok && row0 + ii < W) {
                   val = g[ii * step];
                   if (mir) val.y = -val.y;
@@ -844,13 +831,13 @@ k_degrid_runs_wide(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
             }
           } else {
 #pragma unroll
-          for (int qq = 0; qq < NQ; ++qq) {
+          for (int qq = 0; qq < WIDE_NQ; ++qq) {
             const int q = q2 + 2 * qq;
             const bool ok = jok && q < npl;
 #pragma unroll
-            for (int ii = 0; ii < RPW; ++ii) {
+            for (int ii = 0; ii < WIDE_RPW; ++ii) {
               const int i = row0 + ii;
-              C val; val.x = 0; val.y = 0;
+              double2 val; val.x = 0; val.y = 0;
               if (ok && i < W) {
                 int iu = iu0 + i;
                 if (iu >= p.nu) iu -= p.nu;
@@ -863,36 +850,36 @@ k_degrid_runs_wide(GParams p, const VisRec<T>* __restrict__ recs, int64_t nact,
           }
           }
         }
-        const T* tp = taps[warp][v];
-        T sr = 0, si = 0;
+        const double* tp = taps[warp][v];
+        double sr = 0, si = 0;
 #pragma unroll
-        for (int qq = 0; qq < NQ; ++qq) {
-          T pr = 0, pi = 0;
+        for (int qq = 0; qq < WIDE_NQ; ++qq) {
+          double pr = 0, pi = 0;
 #pragma unroll
-          for (int ii = 0; ii < RPW; ++ii) { pr += gr[ii][qq] * tp[ii]; pi += gi[ii][qq] * tp[ii]; }
-          const T wq = tp[RPW + 16 + q2 + 2 * qq];
+          for (int ii = 0; ii < WIDE_RPW; ++ii) { pr += gr[ii][qq] * tp[ii]; pi += gi[ii][qq] * tp[ii]; }
+          const double wq = tp[WIDE_RPW + 16 + q2 + 2 * qq];
           sr += pr * wq; si += pi * wq;
         }
-        const T tv = tp[RPW + j];
-        C pv; pv.x = sr * tv; pv.y = si * tv;
+        const double tv = tp[WIDE_RPW + j];
+        double2 pv; pv.x = sr * tv; pv.y = si * tv;
         part[warp][v][lane] = pv;
       }
       __syncwarp();
       if (lane < nb) {
-        T myr = 0, myi = 0;
+        double myr = 0, myi = 0;
 #pragma unroll 8
         for (int l = 0; l < 32; ++l) {
-          const C pv = part[warp][lane][(lane + l) & 31];
+          const double2 pv = part[warp][lane][(lane + l) & 31];
           myr += pv.x; myi += pv.y;
         }
-        T re = myr, im = myi;
+        double re = myr, im = myi;
         if (apply_phase) {
           re = myr * r.pc + myi * r.ps;
           im = myi * r.pc - myr * r.ps;
         }
         if (apply_phase && (r.ip & REC_CONJ_BIT)) im = -im;
-        if (wgt) { T w = wgt[r.idx]; re *= w; im *= w; }
-        C* dst = out_sorted ? (out_sorted + k0 + lane) : (vis_out + r.idx);
+        if (wgt) { double w = wgt[r.idx]; re *= w; im *= w; }
+        double2* dst = out_sorted ? (out_sorted + k0 + lane) : (vis_out + r.idx);
         atomicAdd(&dst->x, re);
         atomicAdd(&dst->y, im);
       }

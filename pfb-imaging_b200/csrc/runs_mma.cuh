@@ -9,10 +9,10 @@
 //               vis_s            = sum_q kw_s[q] (D[s,(q,0)] + i D[s,(q,1)])
 //
 // with c = real / imaginary part.  On B200 DMMA runs at the DFMA flop rate (measured: 37 against 34 TFLOP/s), but one
-// DMMA replaces 8 DFMA warp instructions, and the scalar kernels (k_*_runs_wide) are ISSUE bound: ncu on the C2 band at
-// epsilon 1e-7 shows 680 / 980 warp instructions per sample (gridding / degridding) against ~200 that are DFMAs, the
-// fp64 pipe ~25 % busy.  Here a sample costs 13.5 DMMAs per direction for the whole team and every tap is evaluated
-// once per team.
+// DMMA replaces 8 DFMA warp instructions, and scalar team kernels (k_*_runs_wide, which serve 13 <= W <= 16) are ISSUE
+// bound: ncu on the C2 band at epsilon 1e-7 shows 680 / 980 warp instructions per sample (gridding / degridding)
+// against ~200 that are DFMAs, the fp64 pipe ~25 % busy.  Here a sample costs 13.5 DMMAs per direction for the whole
+// team and every tap is evaluated once per team.
 //
 // Team = 3 warps; warp r owns the u-rows 4r .. 4r+3 (48 of the 144 (i,j) cells).
 //   gridding:   6 M-tiles (2 rows x 4 columns each) x 3 N-tiles per warp = 36 accumulator doubles per lane; the C

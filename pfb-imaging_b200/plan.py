@@ -214,13 +214,13 @@ def vis_cost(precision, W, ndim, nvis=0):
     """Run kernels: one warp per run for W <= 8; fp64 9 <= W <= 12: a team of 3 warps on the DMMA path
     (csrc/runs_mma.cuh; measured 5.1e-10 s per sample and direction on the C2 band of 25 M samples, whatever W is in
     that range, and 1.15e-9 on the 1 M samples of C1, which do not fill the GPU);
-    scalar teams of 8 warps for W <= 16 (and of 4 for a single-precision W <= 12, which W_LIMIT rules out)."""
+    fp64 13 <= W <= 16: scalar teams of 8 warps.  Single precision stops at W_LIMIT = 8."""
     if W <= RUNS_MAX_W:
         # W < 8 with w-gridding leaves the constant-stride / cyclic-column flush and fetch of the one-warp kernels for
         # their general path (C1 in fp64, W = 7 against W = 8: degrid 1.18 against 0.40 ms, grid 0.74 against 0.47 ms)
         return COST_VIS_RUNS[precision] * (2.0 if (W < RUNS_MAX_W and ndim == 3) else 1.0)
     if W <= 12:
-        return COST_VIS_RUNS[precision] * ((1.3 if nvis >= 4_000_000 else 3.0) if precision == "double" else 5.0)
+        return COST_VIS_RUNS[precision] * (1.3 if nvis >= 4_000_000 else 3.0)
     return COST_VIS_RUNS[precision] * 9.0
 
 

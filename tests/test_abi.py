@@ -47,6 +47,29 @@ def test_struct_layout_matches_header():
     assert ctypes.sizeof(_lib.PlanInfo) == 5 * 8 + 6 * 4
 
 
+@pytest.mark.parametrize("w", [9, 16])
+def test_fp32_plans_stop_at_w8(w):
+    """An fp32 descriptor with W > 8 (the planner's W_LIMIT) is an argument error of pfbg_plan_create and of
+    pfbg_split_helper_create, named as such, before any CUDA call: so it also holds without a GPU."""
+    lib = _lib.load()
+    keep = [np.ones(64), np.ones(64), np.linspace(0.1, 0.9, 4), np.full(4, 0.25)]
+    d = _lib.PlanDesc(precision=_lib.PFBG_F32, device=0, nx=64, ny=64, nu=96, nv=96, W=w, nplanes=16, do_wgridding=1,
+                      divide_by_n=1, beta=2.3 * w, pixsize_x=1e-5, pixsize_y=1e-5, usign=1.0, vsign=1.0, wsign=1.0,
+                      w0=0.0, dw=1.0, corr_u=keep[0].ctypes.data, corr_v=keep[1].ctypes.data,
+                      gl_x=keep[2].ctypes.data, gl_w=keep[3].ctypes.data, n_gl=4)
+    out = ctypes.c_void_p()
+    assert lib.pfbg_plan_create(ctypes.byref(d), ctypes.byref(out)) == _lib.PFBG_ERR_ARG
+    assert b"fp32 plans stop at W=8" in lib.pfbg_last_error()
+    assert not out.value
+    window = np.array([0, 96, 0, 96], dtype=np.int32)
+    blobs = ctypes.create_string_buffer(4 * _lib.IPC_BLOB_BYTES)
+    mailbox = ctypes.create_string_buffer(_lib.IPC_BLOB_BYTES)
+    rc = lib.pfbg_split_helper_create(ctypes.byref(d), 1, window.ctypes.data, blobs, ctypes.byref(out), mailbox)
+    assert rc == _lib.PFBG_ERR_ARG
+    assert b"fp32 plans stop at W=8" in lib.pfbg_last_error()
+    assert not out.value
+
+
 def _no_gpu():
     try:
         return _lib.device_count() == 0

@@ -1,8 +1,7 @@
 """fp64 run kernels on the DMMA path (csrc/runs_mma.cuh, 9 <= W <= 12) against the explicit DFT and against the
-scalar team kernels they replace (PFBG_WIDE_MMA=0).  Tolerance: rel-L2 <= epsilon vs the DFT (north_star), and
-fp64 round-off between the two kernel families (same taps, different summation order)."""
-import os
-
+direct kernels (k_grid_direct / k_degrid_direct, PFBG_FORCE_DIRECT=1), which evaluate every tap with the library's
+exp / sqrt straight from uvw.  Tolerance: rel-L2 <= epsilon vs the DFT (north_star), and fp64 round-off between the
+two kernel families (the same kernel, different tap arithmetic and summation order)."""
 import numpy as np
 import pytest
 
@@ -13,20 +12,14 @@ from pfbg_testutil import rel_l2, small_problem
 pytestmark = pytest.mark.gpu
 
 
-def _both(fn):
-    """fn() with the DMMA kernels and with the scalar team kernels"""
-    old = os.environ.get("PFBG_WIDE_MMA")
-    try:
-        os.environ["PFBG_WIDE_MMA"] = "1"
-        a = fn()
-        os.environ["PFBG_WIDE_MMA"] = "0"
-        b = fn()
-    finally:
-        if old is None:
-            os.environ.pop("PFBG_WIDE_MMA", None)
-        else:
-            os.environ["PFBG_WIDE_MMA"] = old
-    return a, b
+def _both(monkeypatch, make):
+    """make() bound as usual (the DMMA kernels) and bound with PFBG_FORCE_DIRECT=1 (the direct kernels: the variable
+    is read when uvw is bound)"""
+    gp = make()
+    with monkeypatch.context() as m:
+        m.setenv("PFBG_FORCE_DIRECT", "1")
+        gd = make()
+    return gp, gd
 
 
 # (epsilon, sigma range) chosen so that the plan lands on W = 9 .. 12
@@ -38,32 +31,35 @@ def _both(fn):
     (3e-7, 1.35, 1.35, dict(flip_u=True, flip_w=True)),
     (3e-7, 1.85, 1.85, dict(flip_v=True)),
 ])
-def test_mma_kernels_vs_dft_and_scalar_kernels(gpu, eps, smin, smax, geom):
+def test_mma_kernels_vs_dft_and_direct_kernels(gpu, monkeypatch, eps, smin, smax, geom):
     p = small_problem(nrow=900, nchan=4, nx=96, ny=64, wscale=3.0)
     kw = dict(center_x=0.0, center_y=0.0, flip_u=False, flip_v=False, flip_w=False, do_wgridding=True, divide_by_n=True)
     kw.update(geom)
-    gp = W.plan_for(p["uvw"], p["freq"], npix_x=p["nx"], npix_y=p["ny"], pixsize_x=p["cell"], pixsize_y=p["cell"],
-                    epsilon=eps, precision="double", mask=p["mask"], sigma_min=smin, sigma_max=smax, **kw)
+    gp, gd = _both(monkeypatch, lambda: W.plan_for(
+        p["uvw"], p["freq"], npix_x=p["nx"], npix_y=p["ny"], pixsize_x=p["cell"], pixsize_y=p["cell"], epsilon=eps,
+        precision="double", mask=p["mask"], sigma_min=smin, sigma_max=smax, **kw))
     assert 9 <= gp.info()["W"] <= 12, gp.info()
     act = p["mask"] != 0
-    v_mma, v_old = _both(lambda: gp.degrid(p["img"]))
+    v_mma, v_dir = gp.degrid(p["img"]), gd.degrid(p["img"])
     ref = dft.dft_dirty2vis(p["uvw"], p["freq"], p["img"], p["cell"], p["cell"], **kw)
     assert rel_l2(v_mma[act], ref[act]) <= eps
     assert np.all(v_mma[~act] == 0)
-    assert rel_l2(v_mma, v_old) <= 1e-13
-    d_mma, d_old = _both(lambda: gp.grid(p["vis"], p["wgt"]))
+    d_mma, d_dir = gp.grid(p["vis"], p["wgt"]), gd.grid(p["vis"], p["wgt"])
+    print(f"W={gp.info()['W']}: DMMA vs direct: degrid {rel_l2(v_mma, v_dir):.2e}, grid {rel_l2(d_mma, d_dir):.2e}")
+    assert rel_l2(v_mma, v_dir) <= 1e-13
     dref = dft.dft_vis2dirty(p["uvw"], p["freq"], p["vis"], p["wgt"], p["mask"], p["nx"], p["ny"], p["cell"],
                              p["cell"], **kw)
     assert rel_l2(d_mma, dref) <= eps
-    assert rel_l2(d_mma, d_old) <= 1e-13
+    assert rel_l2(d_mma, d_dir) <= 1e-13
     # adjointness of the DMMA pair
     lhs = np.vdot(v_mma, p["vis"] * p["wgt"] * act).real
     rhs = float((d_mma * p["img"]).sum())
     assert abs(lhs - rhs) <= 1e-12 * abs(rhs)
     gp.close()
+    gd.close()
 
 
-def test_mma_hessian_long_runs_and_tail_batches(gpu):
+def test_mma_hessian_long_runs_and_tail_batches(gpu, monkeypatch):
     """Many samples per footprint origin (runs longer than a batch), a sample count that is not a multiple of the
     batch, and the fused Hessian (bucket-order model visibilities, phases skipped)."""
     rng = np.random.default_rng(5)
@@ -74,15 +70,18 @@ def test_mma_hessian_long_runs_and_tail_batches(gpu):
     x = p["img"]
     kw = dict(npix_x=64, npix_y=64, pixsize_x=p["cell"], pixsize_y=p["cell"], epsilon=1e-7, precision="double",
               mask=mask, sigma_min=1.4, sigma_max=1.4, flip_v=True, divide_by_n=False)
-    gp = W.plan_for(uvw, p["freq"], **kw)
+    gp, gd = _both(monkeypatch, lambda: W.plan_for(uvw, p["freq"], **kw))
     assert 9 <= gp.info()["W"] <= 12
     gp.bind_weights(wgt)
-    h_mma, h_old = _both(lambda: gp.hessian(x, wsum=1.0, eta=0.0))
+    gd.bind_weights(wgt)
+    h_mma, h_dir = gp.hessian(x, wsum=1.0, eta=0.0), gd.hessian(x, wsum=1.0, eta=0.0)
     v = gp.degrid(x)
     ref = gp.grid(v, wgt)
-    assert rel_l2(h_mma, h_old) <= 1e-13
+    print(f"W={gp.info()['W']}: DMMA vs direct: hessian {rel_l2(h_mma, h_dir):.2e}")
+    assert rel_l2(h_mma, h_dir) <= 1e-13
     assert rel_l2(h_mma, ref) <= 1e-12
     gp.close()
+    gd.close()
 
 
 @pytest.mark.parametrize("beta", [13.7, 16.4, 23.34, 31.0, 37.0])

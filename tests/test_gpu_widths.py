@@ -7,9 +7,8 @@ w-gridding).  That reaches, by construction rather than by whatever W an epsilon
 
     W < 8, or W = 8 without w-gridding     k_grid_runs / k_degrid_runs, general flush / fetch
     W = 8 with w-gridding                  the same kernels' W = 8 fast path (fp32: fast and accurate w-screen)
-    fp64 9 <= W <= 12                      the DMMA run kernels (runs_mma.cuh), and the scalar teams <T, 3, 6, 4>
-                                           with PFBG_WIDE_MMA=0
-    fp64 13 <= W <= 16                     the scalar team kernels <T, 2, 8, 8>
+    fp64 9 <= W <= 12                      the DMMA run kernels (runs_mma.cuh)
+    fp64 13 <= W <= 16                     the scalar team kernels k_grid_runs_wide / k_degrid_runs_wide
     any W with PFBG_FORCE_DIRECT=1         k_grid_direct / k_degrid_direct (read when uvw is bound)
 
 `FLOOR` is the round-off floor of each precision: fp64 the 5e-13 of the restatement (the kernels measure <= 4e-14 at
@@ -144,19 +143,6 @@ def test_run_kernels_at_the_kernel_error_bound(gpu, problems, geom, prec, w, sig
         lhs = np.vdot(v.astype(np.complex128), (r["vis"] * r["wgt"] * act).astype(np.complex128)).real
         rhs = float((d.astype(np.float64) * r["img"]).sum())
         assert abs(lhs - rhs) <= ADJ[prec] * abs(rhs)
-
-
-@pytest.mark.parametrize("geom", list(GEOMS))
-@pytest.mark.parametrize("w", range(9, 13))
-@pytest.mark.parametrize("sigma", [1.5, 2.0])
-def test_scalar_team_kernels_at_the_kernel_error_bound(gpu, problems, monkeypatch, geom, w, sigma):
-    """fp64 9 <= W <= 12 on the scalar team kernels <T, 3, 6, 4> (PFBG_WIDE_MMA=0, read per call) against the DFT,
-    not only against the DMMA kernels."""
-    prob = problems[geom]
-    with _plan(prob, "double", w, sigma) as gp:
-        _check_geometry(gp, geom, w, sigma)
-        monkeypatch.setenv("PFBG_WIDE_MMA", "0")
-        _check_bound(gp, _dft_errors(prob, "double", _apply(gp, prob["ref"]["double"])), f"teams/{geom}")
 
 
 @pytest.mark.parametrize("geom", list(GEOMS))
